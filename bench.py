@@ -3,6 +3,7 @@
 roofline of the step kernel and the CPU baseline timed beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2]): BoatEnv experiment 6 (changing velocity, random
 direction), fp32 production mode, uniform(-1,1) policy "A1" (SURVEY.md 8d) so episodes end by
@@ -24,6 +25,12 @@ state (118 MB) fits the L2, which the config line says.
 by oracle/make_ref.py into oracle/_ref so that it travels to the GPU box) on all host cores, one
 process per core in the reference's own fan-out style (main.py:215-235), on bounded samples of the
 same workload; if the staged copy is missing it falls back to the C port (oracle/boat_oracle.c).
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed step gave its caller (the policy's
+actions and BoatEnv.step's obs / reward / done / term / final_obs) as DIR/<name>.npy, float32, for a fixed
+seeded sample of DUMP_ENVS envs of rank 0 (all of them when it has fewer), and the sampled env ids as
+DIR/env_index.npy, float64.  The inputs depend only on the arguments, so two builds run with the same
+arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -47,6 +54,8 @@ SEED = 1
 ALGO_BYTES_PER_STEP = 165  # SURVEY.md 8(d): fp32, K=1, exp 6: action 4 + state 56 read + 56 write + obs 44 + reward 4 + done 1
 STATS_EVERY = 250          # NCCL all-reduce of the 64-byte statistics vector every M steps (and once per timed region)
 PREROLL = 1000             # untimed steps before warm-up: brings the reset rate to its steady state (episodes last ~360 steps)
+DUMP_ENVS = 1 << 18        # --dump-outputs: envs sampled (26 floats each: ~27 MB in all, under the 64 MB cap)
+DUMP_SEED = 12345
 
 
 def workload_config(n_gpus: int, envs_per_gpu: int, scaling: str = "weak", total_envs: int | None = None) -> dict:
@@ -337,11 +346,12 @@ def run_ours(args) -> None:
         env.uniform_actions(t, args.action_scale, out=actions)       # the policy (1 launch)
         if ev is not None:
             ev[0].record()
-        env.step(actions)                               # BoatEnv.step for every env (1 launch)
+        out = env.step(actions)                         # BoatEnv.step for every env (1 launch)
         if ev is not None:
             ev[1].record()
         if (t + 1) % STATS_EVERY == 0 or force_stats:   # occasional statistics all-reduce
             reduce_stats()
+        return out
 
     def barrier():
         if world > 1:
@@ -371,13 +381,17 @@ def run_ours(args) -> None:
     start.record()
     for k in range(args.steps):
         # the statistics all-reduce fires inside every timed region, however short (here: at its middle step)
-        one_step(t, kernel_events[k], force_stats=(k == args.steps // 2))
+        last = one_step(t, kernel_events[k], force_stats=(k == args.steps // 2))
         t += 1
     end.record()
     barrier()
     launches = lib.boatenv_kernel_launches() - launches0
     clocks = sampler.stop()
     allreduces_timed = n_allreduce[0]
+    if args.dump_outputs and rank == 0:
+        obs, reward, done, info = last
+        dump_outputs(args.dump_outputs, {"action": actions, "obs": obs, "reward": reward, "done": done,
+                                         "term": info["term"], "final_obs": info["final_obs"]})
     reduce_stats()
     # episodes that ended in warm-up + timed steps, scaled to the timed steps (the rate is steady after the pre-roll;
     # counting exactly would need a host read-back between warm-up and timed region, i.e. the idle gap avoided above)
@@ -484,6 +498,21 @@ def run_ours(args) -> None:
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """--dump-outputs: the rows of a fixed seeded env sample of every output tensor, as float32 .npy files."""
+    import numpy as np
+    import torch
+    n = outputs["obs"].shape[0]
+    idx = np.arange(n)
+    if n > DUMP_ENVS:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=DUMP_ENVS, replace=False))
+    rows = torch.from_numpy(idx).to(outputs["obs"].device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for name, x in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x.index_select(0, rows).float().cpu().numpy())
+
+
 def toy_timings(S, torch, device: int) -> dict:
     """BASELINE.json configs[3]: toy_car and toy_parachute, 1,048,576 envs each, fp32, on one B200.  Device-timed
     (CUDA events), whole scripts: 5001 iterations of toy_car.py:19-32, 2654 of toy_parachute.py:16-40."""
@@ -526,7 +555,13 @@ def main():
     ap.add_argument("--total-envs", type=int, default=ENVS_PER_GPU, help="--scaling strong: envs over all GPUs")
     ap.add_argument("--e2e-k", type=int, default=8, help="sub-steps per host round trip of the second e2e line (0: skip)")
     ap.add_argument("--no-toys", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (a fixed sample of the envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

@@ -23,6 +23,22 @@ def load_golden(name):
     return out
 
 
+AGENT_KEYS = ("learning_rate_alpha", "learning_rate_beta", "gamma", "tvn_parameter_modulation_tau", "reward_scale")
+
+
+def reference_config_record():
+    """The values of the reference's configs/original_config.yaml that tests/golden recorded (oracle/make_golden.py,
+    make_agent_golden.py): the hot-path keys stored beside the reference roll-outs, which set
+    base_settings.experiment per file (left out here), and the agent keys of the recorded SAC update."""
+    cfgs = [load_golden(f"ref_rollout_exp{e}")["config"] for e in range(1, 7)]
+    for e, cfg in enumerate(cfgs, 1):
+        assert cfg["base_settings"].pop("experiment") == e
+    assert all(cfg == cfgs[0] for cfg in cfgs)
+    rec = np.load(os.path.join(GOLDEN, "agent_update.npz"))
+    cfgs[0]["agent"] = {k: rec["meta/" + k].item() for k in AGENT_KEYS}
+    return cfgs[0]
+
+
 def scaled_err(a, b, scale=1.0):
     """|a-b| / max(|b|, scale): the parity metric of SURVEY.md H6."""
     a = np.asarray(a, dtype=np.float64)

@@ -103,6 +103,45 @@ def test_gpu_arm_line():
 
 
 @pytest.mark.gpu
+def test_gpu_arm_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs: the last timed step's outputs for a fixed env sample, identical from run to run, with
+    --steps timed steps (one policy launch + one step launch each)."""
+    import numpy as np
+    import torch
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    n, steps = 1 << 19, 7
+    flags = ["--steps", str(steps), "--warmup", "3", "--envs-per-gpu", str(n), "--e2e-steps", "3", "--e2e-k", "0",
+             "--no-cpu-baseline", "--no-toys"]
+    runs = []
+    for i in range(2):
+        d = run_bench(*flags, "--dump-outputs", str(tmp_path / str(i)))
+        assert d["steps"] == steps and 2 * steps <= d["gpu_launches"] <= 2 * steps + 4
+        runs.append({f[:-4]: np.load(tmp_path / str(i) / f) for f in sorted(os.listdir(tmp_path / str(i)))})
+    a, b = runs
+    m = 1 << 18
+    assert sorted(a) == ["action", "done", "env_index", "final_obs", "obs", "reward", "term"]
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert all(x.dtype in (np.float32, np.float64) for x in a.values())
+    assert a["obs"].shape == a["final_obs"].shape == (m, 11) and a["reward"].shape == a["done"].shape == (m,)
+    idx = a["env_index"]
+    assert len(np.unique(idx)) == m and idx.min() >= 0 and idx.max() < n and np.all(idx == np.floor(idx))
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    assert np.isfinite(a["obs"]).all() and np.array_equal(a["done"], (a["term"] != 0).astype(np.float32))
+    # the dumped actions are the policy's draw for the last timed step (after pre-roll and warm-up) at the sampled ids
+    import bench
+    import sac_agent_b200 as S
+    env = S.BatchedBoatEnv(S.load_config(base_settings__experiment=bench.EXPERIMENT), n, seed=bench.SEED,
+                           precision="fp32", device=0)
+    rows = idx.astype(np.int64)
+    last = bench.PREROLL + 3 + steps - 1
+    assert np.array_equal(a["action"], env.uniform_actions(last).cpu().numpy()[rows])
+    assert not np.array_equal(a["action"], env.uniform_actions(last - 1).cpu().numpy()[rows])
+    env.close()
+
+
+@pytest.mark.gpu
 def test_gpu_arm_strong_scaling_line():
     import torch
     if not torch.cuda.is_available():
