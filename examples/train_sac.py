@@ -60,7 +60,12 @@ def main(argv=None):
                          "bottom quarter adopts the best member's weights + hyper-parameters and perturbs them")
     ap.add_argument("--overlap", action="store_true",
                     help="acting and learning on two streams (OverlappedActorLearner: the policy lags one update)")
+    ap.add_argument("--record-envs", type=int, default=0, metavar="K",
+                    help="record every step of the first K envs of each rank's shard into its experiment's episodes/ "
+                         "(the reference's Recorder CSVs, DeviceRecorder); flushed at every log interval")
     args = ap.parse_args(argv)
+    if args.record_envs and not args.experiments_root:
+        ap.error("--record-envs requires --experiments-root")
 
     rank, local_rank, world = S.sharding.dist_info()
     torch.cuda.set_device(local_rank)
@@ -88,7 +93,13 @@ def main(argv=None):
                               use_cuda_graph=not args.no_graph, memory=mem, policy_precision=args.policy_precision)
     act = agent.choose_action if args.no_graph else agent.choose_action_graphed
     obs = env.reset()
-    pipe = S.OverlappedActorLearner(agent, env, done_flag_mode=1) if args.overlap else None
+    rec = None
+    if args.record_envs:   # main.py:79: a recorder row every step; the ring holds a log interval (+ the first row)
+        k = min(args.record_envs, env.n_envs)
+        rec = S.DeviceRecorder(env, range(env.env_id_offset, env.env_id_offset + k), exp.experiment_dir,
+                               capacity=max(1024, args.log_every + 1))
+        rec.start()
+    pipe = S.OverlappedActorLearner(agent, env, done_flag_mode=1, recorder=rec) if args.overlap else None
     losses = None
     rows, best, prev = [], float("-inf"), {"episodes": 0.0, "return_sum": 0.0}
     import random as _random
@@ -104,6 +115,8 @@ def main(argv=None):
         else:
             actions = act(obs).squeeze(-1)
             agent.step_and_remember(env, actions, done_flag_mode=1)   # env.step + agent.remember, one kernel
+            if rec:
+                rec.capture(actions)
             for _ in range(args.updates_per_iter):
                 out = agent.learn()
                 losses = out if out is not None else losses
@@ -122,6 +135,8 @@ def main(argv=None):
                             "ranking": info["ranking"]})
         if pipe and args.log_every and it % args.log_every == 0:
             pipe.sync()   # counters, losses and checkpoints below run on the default stream: order it after the pipeline
+        if rec and args.log_every and it % args.log_every == 0:
+            rec.flush()
         if exp and args.log_every and it % args.log_every == 0:
             # one console.csv row per logging interval: the mean return of the episodes that ended in it
             c = env.counters()
@@ -147,6 +162,11 @@ def main(argv=None):
     if world > 1:
         torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
     stats = S.all_reduce_counters(env.counters_tensor())
+    if rec:
+        rec.close()
+        recorded = torch.tensor([len(rec.ids), rec.episodes_finished], dtype=torch.float64, device="cuda")
+        if world > 1:
+            torch.distributed.all_reduce(recorded)
     sec = float(ms.item()) * 1e-3
     summary = {"example": "train_sac", "overrides": overrides, "n_gpus": world, "envs_total": args.envs, "iters": args.iters,
                "updates_per_iter": args.updates_per_iter, "cuda_graph": not args.no_graph, "overlap": bool(args.overlap),
@@ -156,6 +176,8 @@ def main(argv=None):
                "ms_per_iter": 1e3 * sec / args.iters, "episodes": stats["episodes"],
                "mean_return": stats["return_mean"], "reached_goal": stats["reached_goal"],
                "losses_v_pi_q": [float(x) for x in losses] if losses is not None else None}
+    if rec:   # over all ranks: envs recorded, and their episodes that ended (one info.csv row each)
+        summary["recorded_envs"], summary["recorded_episodes"] = int(recorded[0]), int(recorded[1])
     if args.pbt_every:
         summary["pbt_rounds"] = len(pbt_log)
         summary["pbt_adoptions_rank0"] = [e for e in pbt_log if e["adopted_from"] is not None]

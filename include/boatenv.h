@@ -176,6 +176,29 @@ BOATENV_API int boatenv_wind_table(boatenv_t h, int64_t env_index, double *wind_
                        double *wind_angle_out, void *stream);
 BOATENV_API int boatenv_wind_length(boatenv_t h); /* int(t_max/dt)  wind.py:14-15 */
 
+/* ---- episode recording (postprocessing/recorder.py:18-56, main.py:79) -------------- */
+
+/* Caller-owned device columns of a recording ring, each [capacity][n_ids] row-major: row t holds
+ * the recorded envs in `ids` order.  The eight state / step columns are T; term is
+ * BOATENV_TERM_*; episode is BOATENV_F_EPISODE of the env when the row was taken. */
+typedef struct boatenv_record_ring {
+    void *s_x, *s_y, *v_x, *v_y, *s_r, *rudder_angle, *action, *reward;
+    uint8_t *term;
+    uint32_t *episode;
+    int64_t capacity;
+} boatenv_record_ring;
+
+/* One recorder row of recorder.py:24-36 (return_all_data, boat_env.py:128-140) for n_ids envs in one
+ * launch: writes row (row % capacity) of `ring` from local env ids int64[n_ids] (device; each in
+ * [0, n_envs) -- an id outside is skipped, its entries left as they were).  s_x .. rudder_angle are
+ * the values boatenv_get_field returns, bit for bit; action / reward / term are entry ids[j] of the
+ * step's actions T[n_envs], reward T[n_envs] and term uint8[n_envs], each of which may be NULL
+ * (zeros: the row of a state no step led to, e.g. right after reset).  Queued on `stream` after
+ * the step it records; no synchronisation. */
+BOATENV_API int boatenv_record_rows(boatenv_t h, const int64_t *ids, int64_t n_ids, const void *actions,
+                        const void *reward, const uint8_t *term, const boatenv_record_ring *ring, int64_t row,
+                        void *stream);
+
 /* Validation hook: replace the Philox draws by caller-supplied ones for every episode
  * started after this call (fixture replay, differential tests against the reference).
  *   s_y_start int32[n_envs] or NULL; knots double[n_envs][2][fixed_points] or NULL

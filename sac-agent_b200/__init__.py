@@ -12,14 +12,14 @@ from ._lib import BoatEnvError, lib, library_path  # noqa: F401
 from .boat_env import BatchedBoatEnv, BoatEnv, Box, TERM_NAMES  # noqa: F401
 from .buffer import ReplayBuffer  # noqa: F401
 from .toy_envs import ToyCar, ToyParachute  # noqa: F401
-from .csv_export import BatchedRecorder  # noqa: F401
+from .csv_export import BatchedRecorder, DeviceRecorder  # noqa: F401
 from .sharding import all_reduce_counters, make_sharded_env, shard_range  # noqa: F401
 from .experiment import Experiment, HPTuner, get_experiment_config, info_from_counters  # noqa: F401
 from . import population  # noqa: F401
 
 __all__ = ["AttrDict", "load_config", "params_from_config", "BoatEnvError", "lib", "library_path",
            "BatchedBoatEnv", "BoatEnv", "Box", "TERM_NAMES", "ReplayBuffer", "ToyCar", "ToyParachute",
-           "BatchedRecorder", "all_reduce_counters", "make_sharded_env", "shard_range",
+           "BatchedRecorder", "DeviceRecorder", "all_reduce_counters", "make_sharded_env", "shard_range",
            "Experiment", "HPTuner", "get_experiment_config", "info_from_counters",
            "ContinuousAgent", "SACLearner", "OverlappedActorLearner"]
 

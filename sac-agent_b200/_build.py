@@ -31,6 +31,7 @@ UNITS = {
     "toys.cu": ["-fmad=false"],
     "agent_ops.cu": [],
     "policy_mlp.cu": [],
+    "record.cu": [],
 }
 
 

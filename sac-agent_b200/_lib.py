@@ -32,6 +32,12 @@ _lib = None
 vp, i64, u64, i32, u32, dbl = C.c_void_p, C.c_int64, C.c_uint64, C.c_int32, C.c_uint32, C.c_double
 PP = C.POINTER(BoatEnvParams)
 
+
+class RecordRing(C.Structure):
+    """boatenv_record_ring: device column pointers [capacity][n_ids] of a recording ring."""
+    _fields_ = [(name, vp) for name in ("s_x", "s_y", "v_x", "v_y", "s_r", "rudder_angle", "action", "reward",
+                                        "term", "episode")] + [("capacity", i64)]
+
 # name -> (restype, argtypes): one row per declaration in include/boatenv.h
 SIGNATURES = {
     "boatenv_create": (C.c_int, [PP, i64, u64, i64, C.c_int, C.c_int, C.POINTER(vp)]),
@@ -47,6 +53,7 @@ SIGNATURES = {
     "boatenv_set_field": (C.c_int, [vp, C.c_int, vp, vp]),
     "boatenv_env_state_host": (C.c_int, [vp, i64, C.POINTER(dbl)]),
     "boatenv_wind_table": (C.c_int, [vp, i64, vp, vp, vp]),
+    "boatenv_record_rows": (C.c_int, [vp, vp, i64, vp, vp, vp, C.POINTER(RecordRing), i64, vp]),
     "boatenv_wind_length": (C.c_int, [vp]),
     "boatenv_set_episode_draws": (C.c_int, [vp, vp, vp, vp]),
     "boatenv_episode_draws_host": (C.c_int, [PP, u64, i64, u32, C.POINTER(i32), C.POINTER(dbl)]),

@@ -200,6 +200,16 @@ class BatchedBoatEnv:
         assert v.numel() == self.n_envs
         _lib.check(self._L.boatenv_set_field(self._h, f, v.data_ptr(), self._stream()), "boatenv_set_field")
 
+    def record_rows(self, ids, ring, row, actions=None, reward=None, term=None):
+        """One recorder row (boatenv_record_rows): state, action, reward and termination code of the LOCAL env ids
+        ``ids`` (int64 device tensor) into row ``row % ring.capacity`` of ``ring`` (a ``_lib.RecordRing``).
+        ``actions`` / ``reward`` / ``term`` are the step's [n_envs] device tensors, or None for zeros.  One launch on
+        the current stream, no synchronisation."""
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        _lib.check(self._L.boatenv_record_rows(self._h, ids.data_ptr(), ids.numel(), ptr(actions), ptr(reward),
+                                               ptr(term), C.byref(ring), int(row), self._stream()),
+                   "boatenv_record_rows")
+
     @property
     def wind_length(self):
         return int(self._L.boatenv_wind_length(self._h))

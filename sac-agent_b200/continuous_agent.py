@@ -465,8 +465,9 @@ class OverlappedActorLearner:
     next ``step()`` then waits for the caller's stream in turn.  ``finish()`` is ``sync()`` at the end of a run.
     """
 
-    def __init__(self, agent: ContinuousAgent, env, done_flag_mode=1):
+    def __init__(self, agent: ContinuousAgent, env, done_flag_mode=1, recorder=None):
         self.agent, self.env, self.done_flag_mode = agent, env, int(done_flag_mode)
+        self.recorder = recorder   # a DeviceRecorder: captures every step on the env stream
         dev = agent.device
         # the learner's small kernels go first whenever an SM frees up: without a priority they queue behind
         # the thousand CTAs of each policy GEMM and the two streams do not overlap at all
@@ -527,6 +528,8 @@ class OverlappedActorLearner:
             self.s_env.wait_event(self.ev_sample)           # sample(t - 1) is done with the ring
             a.step_and_remember(self.env, actions.squeeze(-1), done_flag_mode=self.done_flag_mode)
             self.ev_store.record(self.s_env)
+            if self.recorder is not None:
+                self.recorder.capture(actions.squeeze(-1))
         with torch.cuda.stream(self.s_learn):
             self.s_learn.wait_event(self.ev_store)          # the rows of step t are complete
             if a.memory.mem_cntr >= a.batch_size:
