@@ -330,6 +330,32 @@ BOATENV_API int boatagent_policy_act(const void *weight_blob, const float *obs, 
                          const float *max_action, uint64_t seed, uint64_t step, int64_t n, int32_t obs_dim,
                          int32_t n_actions, float *action_out, void *stream);
 
+/* Closed-loop rollout of the tcgen05 policy on a BoatEnv handle (render_model, main.py:137-172, over every env of
+ * the handle): the forward pass of boatagent_policy_act and one K = 1 boatenv_step sub-step without
+ * BOATENV_AUTO_RESET, fused in one persistent kernel.  fp32 handles, n_actions = 1, weight_blob and max_action as
+ * for boatagent_policy_act.  Sub-step t of env i acts with the action boatagent_policy_act gives row i with
+ * step = step0 + t (Philox(seed; i, step) + Box-Muller), or with eps = 0 under BOATAGENT_ROLLOUT_DETERMINISTIC
+ * (action = tanh(mean) * max_action).
+ * Every env takes min(max_steps, steps until its episode ends) steps.  An env whose episode ends is then frozen:
+ * no auto-reset and no further steps; its counters are updated once, as the step kernel does, and its state stays
+ * the terminal state.  An env whose episode had already ended before the call is stepped on from its terminal
+ * state, as boatenv_step would: reset it first.
+ * obs_in float32 [N][11] is each env's last observation (what reset / step wrote); the first action needs it,
+ * because the observation holds the last sub-step's accelerations, which the state does not.  Outputs, per env:
+ *   obs_out    float32 [N][11]  the last observation (the terminal one if the episode ended); may alias obs_in
+ *   return_out float32 [N]      the episode_reward slot (BOATENV_F_EPISODE_REWARD) after the last step
+ *   steps_out  int32 [N]        steps taken in this call
+ *   term_out   uint8 [N]        BOATENV_TERM_* of the ending step, 0 = still running after max_steps
+ * At the end every env's state is written back (dyn slots, step index, wind coefficients; the episode number is
+ * untouched), so get_field, export_state, step and another rollout continue exactly where the rollout stopped.
+ * Errors: BOATENV_EUNSUPPORTED for an fp64 handle, BOATENV_ESTATE before reset, BOATENV_EINVAL for NULL
+ * pointers, max_steps < 1 or unknown flags, BOATENV_EALIGN for a weight_blob that is not 16-byte aligned. */
+#define BOATAGENT_ROLLOUT_DETERMINISTIC 1u   /* action = tanh(mean) * max_action */
+BOATENV_API int boatagent_rollout(boatenv_t h, const void *weight_blob, const float *max_action, uint64_t seed,
+                                  uint64_t step0, int32_t max_steps, uint32_t flags, const float *obs_in,
+                                  float *obs_out, float *return_out, int32_t *steps_out, uint8_t *term_out,
+                                  void *stream);
+
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 
 typedef struct boattoy_handle *boattoy_t;

@@ -32,6 +32,7 @@ UNITS = {
     "agent_ops.cu": [],
     "policy_mlp.cu": [],
     "record.cu": [],
+    "rollout.cu": [],
 }
 
 

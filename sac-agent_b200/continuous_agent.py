@@ -25,6 +25,7 @@ from __future__ import annotations
 
 import copy
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -257,6 +258,36 @@ class ContinuousAgent:
             from .networks import TensorCorePolicy
             self._tc_policy = TensorCorePolicy(self.actor, seed=0x5ac)
         return self._tc_policy
+
+    @torch.no_grad()
+    def evaluate(self, env, max_steps=None, deterministic=True):
+        """render_model (main.py:137-172) over every env of the fp32 BatchedBoatEnv `env`: one episode per env
+        under the current actor, run from the env's current state (call ``env.reset()`` first for fresh episodes)
+        in one fused kernel (TensorCorePolicy.rollout).  Always acts through the tcgen05 copy of the actor, whatever
+        `policy_precision` is, so evaluation acts with bf16 inputs (fp32 accumulation).  `max_steps` defaults to
+        enough steps for every episode to end, at the latest by timeout (t_max / dt).  `deterministic`: the mean
+        action tanh(mean) * max_action, else a draw as in training.  After ``OverlappedActorLearner`` use, call its
+        ``sync()`` first.  Returns (returns, steps, term, summary): the per-env device tensors of the rollout and a
+        host dict -- envs, episodes ended, still running, counts per termination kind, goal fraction (of all envs),
+        mean / std / min / max return and mean length of the ended episodes."""
+        from .boat_env import TERM_NAMES
+        if max_steps is None:
+            max_steps = int(math.ceil(env.params.t_max / env.params.dt)) + 1
+        pol = self.tensor_core_policy()
+        pol.refresh()
+        returns, steps, term = pol.rollout(env, max_steps, deterministic=deterministic)
+        t, r, s = term.cpu().numpy(), returns.double().cpu().numpy(), steps.cpu().numpy()
+        ended = t != 0
+        rr = r[ended]
+        summary = {"envs": int(t.size), "episodes": int(ended.sum()), "running": int((~ended).sum()),
+                   "terminations": {TERM_NAMES[k]: int((t == k).sum()) for k in range(1, len(TERM_NAMES))},
+                   "goal_fraction": float((t == 1).mean()) if t.size else float("nan"),
+                   "return_mean": float(rr.mean()) if rr.size else float("nan"),
+                   "return_std": float(rr.std()) if rr.size else float("nan"),
+                   "return_min": float(rr.min()) if rr.size else float("nan"),
+                   "return_max": float(rr.max()) if rr.size else float("nan"),
+                   "length_mean": float(s[ended].mean()) if rr.size else float("nan")}
+        return returns, steps, term, summary
 
     def choose_action_graphed(self, observation):
         """`choose_action` for a PERSISTENT observation tensor (BatchedBoatEnv.obs): the policy's forward

@@ -225,6 +225,40 @@ __device__ __forceinline__ void substep(const DevCfg &c, float (&d)[D_COUNT], Fx
     d[D_SY] = s_y; d[D_SR] = s_r; d[D_RET] += r;
 }
 
+// The wind sample wind[index] of an env (wind.py:26-63, boat_env.py:230-236) from its carried piece coefficients
+// wa / wb; j, r: the spline piece of the sample and its remainder (piece_of), for next_sample_in_next_piece.
+template <typename T, int WK>
+__device__ __forceinline__ void wind_sample(const DevCfg &c, int index, const T (&wa)[4], const T (&wb)[4], T inv_Lm1,
+                                            T &w, T &th, int &j, int &r) {
+    constexpr bool kCurves = (WK == WIND_VEL_CURVE || WK == WIND_ANGLE_RECT || WK == WIND_BOTH);
+    w = (T)0; th = (T)0;
+    j = 0; r = 0;
+    if (kCurves) {
+        piece_of(c, min(index, c.L - 1), j, r);
+        const T s = (T)r * inv_Lm1;
+        const T va = ((wa[3] * s + wa[2]) * s + wa[1]) * s + wa[0];
+        if (WK == WIND_ANGLE_RECT) {
+            if (sizeof(T) == 8) {  // wind.py:57-58,95: (value<=0.25 ? 0 : 1)*pi + pi/2
+                w = (T)c.p.max_velocity;
+                th = (T)(((double)va <= 0.25 ? 0.0 : 1.0) * 3.14159265358979323846 + 3.14159265358979323846 / 2.0);
+            } else {
+                th = va;  // the fp32 path thresholds inside substep()
+            }
+        } else {
+            w = va;
+            th = (T)c.direction_rad;
+        }
+        if (WK == WIND_BOTH) th = ((wb[3] * s + wb[2]) * s + wb[1]) * s + wb[0];
+    }
+    if (WK == WIND_CONST) { w = (T)c.p.max_velocity; th = (T)c.direction_rad; }
+}
+
+// Does wind[index + 1] (the next sub-step's sample) live in the next spline piece, given piece j and remainder r of
+// wind[index]?  Then the env needs the next piece's coefficients (wind_setup_*) before its next sub-step.
+__device__ __forceinline__ bool next_sample_in_next_piece(const DevCfg &c, int j, int r) {
+    return r + c.npieces >= c.Lm1 && j + 1 <= c.npieces - 1;
+}
+
 // A NaN bit pattern that no arithmetic instruction produces (their NaNs are canonical): see the stage-refill vote.
 __device__ __forceinline__ bool is_poison(float v) { return __float_as_uint(v) == 0x7fc00001u; }
 __device__ __forceinline__ bool is_poison(double v) { return __double_as_longlong(v) == 0x7ff8000000000001ll; }
@@ -674,26 +708,9 @@ boat_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ StepA
             bool need_setup = false;
             if (alive) {
                 // ---- wind sample wind[index] from the carried piece coefficients ----
-                T w = (T)0, th = (T)0;
-                int j = 0, r = 0;
-                if (kCurves) {
-                    piece_of(c, min(index, c.L - 1), j, r);
-                    const T s = (T)r * inv_Lm1;
-                    const T va = ((wa[3] * s + wa[2]) * s + wa[1]) * s + wa[0];
-                    if (WK == WIND_ANGLE_RECT) {
-                        if (sizeof(T) == 8) {  // wind.py:57-58,95: (value<=0.25 ? 0 : 1)*pi + pi/2
-                            w = (T)c.p.max_velocity;
-                            th = (T)(((double)va <= 0.25 ? 0.0 : 1.0) * 3.14159265358979323846 + 3.14159265358979323846 / 2.0);
-                        } else {
-                            th = va;  // the fp32 path thresholds inside substep()
-                        }
-                    } else {
-                        w = va;
-                        th = (T)c.direction_rad;
-                    }
-                    if (WK == WIND_BOTH) th = ((wb[3] * s + wb[2]) * s + wb[1]) * s + wb[0];
-                }
-                if (WK == WIND_CONST) { w = (T)c.p.max_velocity; th = (T)c.direction_rad; }
+                T w, th;
+                int j, r;
+                wind_sample<T, WK>(c, index, wa, wb, inv_Lm1, w, th, j, r);
 
                 T rew, acc[3];
 #ifdef BOAT_DEBUG_NOCOMPUTE  // memory-pattern experiment only: stream the state through untouched
@@ -710,7 +727,7 @@ boat_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ StepA
                     need_setup = true;  // statistics, and the reset if AUTO_RESET
                 } else if (kCurves) {
                     // does wind[index] (the next sub-step) live in the next spline piece?
-                    if (r + c.npieces >= c.Lm1 && j + 1 <= c.npieces - 1) need_setup = true;
+                    if (next_sample_in_next_piece(c, j, r)) need_setup = true;
                 }
             }
             if (!KMULTI) store_results();

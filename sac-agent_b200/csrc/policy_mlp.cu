@@ -18,140 +18,17 @@
 //     under the other's MMAs; observations are fetched one tile ahead;
 //   * HBM traffic is the input and the output: 4 * obs_dim + 4 * A bytes per env.
 // Inputs are rounded to bf16 (fp32 accumulation): acting only, the learner never sees this kernel.
-#include <cstdint>
-#include <cuda_bf16.h>
-#include <cuda_runtime.h>
+// The rollout kernel (rollout.cu) runs the same pass through the copies of these steps in actor_tc.cuh
+// (actor_prologue .. actor_normal_draw), which must stay statement for statement equal to the code below: a change
+// here is made there too (tests/test_gpu_rollout.py checks the two kernels' actions bit for bit).
 #include <mutex>
 
-#include "../../include/boatenv.h"
-#include "common.cuh"
+#include "actor_tc.cuh"
 #include "launch.h"
 
 namespace {
 
-constexpr int kHidden = 256, kTileM = 128, kK1 = 16, kN3 = 16;
-// 8 epilogue warps in two groups of four (warp w: TMEM lanes 32 (w % 4) .. + 31, the hardware's lane window of a
-// warp; group w / 4); warp 8 issues the MMAs.
-constexpr int kEpiThreads = 256, kThreads = kEpiThreads + 32, kMmaWarp = kEpiThreads / 32;
-// shared-memory map (bytes).  Operand layout: element (row, k) of an R-row operand sits at
-// (k / 8) * (R * 16) + row * 16 + (k % 8) * 2  -- 8x8 core matrices, K-adjacent cores R*16 bytes apart (LBO),
-// row groups 128 bytes apart (SBO).
-constexpr int kOffW1 = 0;                                   // [256 rows][16]
-constexpr int kOffW2 = kOffW1 + kHidden * kK1 * 2;          // [256 rows][256]
-constexpr int kOffW3 = kOffW2 + kHidden * kHidden * 2;      // fp32 [16 rows][256], row-major: the heads stay in fp32
-constexpr int kOffB1 = kOffW3 + kN3 * kHidden * 4;          // fp32[256]
-constexpr int kOffB2 = kOffB1 + kHidden * 4;
-constexpr int kOffB3 = kOffB2 + kHidden * 4;                // fp32[16]
-constexpr int kBlobBytes = kOffB3 + kN3 * 4;                // what the host packs (BOATAGENT_POLICY_BLOB_BYTES)
-static_assert(kBlobBytes == BOATAGENT_POLICY_BLOB_BYTES, "header and kernel disagree on the weight blob");
-
-__device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// UMMA shared-memory descriptor, K-major, no swizzle (cute::UMMA::SmemDescriptor: start >> 4 at [0,14), LBO >> 4 at
-// [16,30), SBO >> 4 at [32,46), version 1 at [46,48), layout type 0 at [61,64)).
-__device__ __forceinline__ uint64_t umma_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)((lbo_bytes >> 4) & 0x3fffu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3fffu) << 32) | (1ull << 46);
-}
-// Instruction descriptor of tcgen05.mma.kind::f16 (cute::UMMA::InstrDescriptor): D = f32, A = B = bf16, both K-major.
-__host__ __device__ constexpr uint32_t umma_idesc(int m, int n) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t *bar) {   // arrives on `bar` when every MMA issued so far is done
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_addr(bar)) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void bar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "W_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra D_%=;\n\t"
-        "bra W_%=;\n\t"
-        "D_%=:\n\t"
-        "}" ::"r"(smem_addr(bar)), "r"(parity) : "memory");
-}
-// 32 consecutive fp32 accumulator columns of this thread's TMEM lane: asynchronous load (the registers are valid after
-// tmem_ld_wait()), so the next chunk can be in flight while the current one is processed
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-}
-// The registers are tied to the wait as in/out operands: nothing that reads them can be scheduled above it.
-__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
-                   "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]), "+r"(r[16]),
-                   "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]),
-                   "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
-                 :
-                 : "memory");
-}
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-    const __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<const uint32_t *>(&p);
-}
-
-// Two tiles in flight per CTA.  Epilogue group g (warps 4g .. 4g + 3, one env row = one TMEM lane per thread) owns
-// the TMEM columns 256 g .. 256 g + 255 and every other tile of the CTA.  The layer-1 activations never go to
-// shared memory: the epilogue packs them to bf16 pairs and stores them back into TMEM (tcgen05.st, in place over
-// the accumulator columns it has already read), and layer 2 takes its A operand from TMEM.  Layer 2 runs as two
-// N = 128 halves into the upper 128 columns of the region, so while one group is in an epilogue the tensor pipe
-// works for the other.  Hand-offs are mbarriers (no CTA-wide barrier in the loop); the MMA warp polls them.
-constexpr int kOffA0 = (kBlobBytes + 127) / 128 * 128;      // two [128 rows][16] tiles
-constexpr int kOffBar = kOffA0 + 2 * kTileM * kK1 * 2;      // 2 groups x {a0_ready, d1_ready, h1_ready, d2_ready, d2_free}
-constexpr int kSmemBytes = kOffBar + 2 * 5 * 8;
-static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
-enum { B_A0 = 0, B_D1 = 1, B_H1 = 2, B_D2 = 3, B_FREE = 4 };
-
-__device__ __forceinline__ void bar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_addr(bar)) : "memory");
-}
-__device__ __forceinline__ bool bar_test(uint64_t *bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}" : "=r"(ok) : "r"(smem_addr(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
-// D[tmem] (+)= A[tmem, bf16 pairs per column] . B[smem]^T
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t"
-        "}" ::"r"(tmem_d), "r"(tmem_a), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr), "r"(r[0]), "r"(r[1]),
-        "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]),
-        "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-        : "memory");
-}
+using namespace boatenv;
 
 template <int NA>
 __global__ void __launch_bounds__(kThreads, 1)

@@ -237,3 +237,31 @@ class TensorCorePolicy:
                             "boatagent_policy_act")
         self.steps += 1
         return out
+
+    @torch.no_grad()
+    def rollout(self, env, max_steps, deterministic=False):
+        """Runs every env of the fp32 BatchedBoatEnv `env` under this policy for up to `max_steps` steps in ONE
+        kernel (boatagent_rollout, csrc/rollout.cu): each step is the action `act` would draw for that env's row at
+        that call, then one env step without auto-reset.  An env whose episode ends is frozen in its terminal state
+        (reset() starts the next round).  `deterministic`: action = tanh(mean) * max_action.  Reads and updates
+        `env.obs` (the last, or terminal, observation of every env) and advances `steps` by `max_steps`, so later
+        `act` calls draw fresh noise.  Returns device tensors (returns float32: the episode_reward slot, steps int32:
+        steps taken in this call, term uint8: the termination code, 0 = still running); launches on the current
+        stream and does not synchronise."""
+        if self.n_actions != 1 or self.obs_dim != 11:
+            raise ValueError("rollout: the BoatEnv actor (11 observations, one action)")
+        if env.device != self.blob.device:
+            raise ValueError("rollout: the env and the policy must be on the same device")
+        n = env.n_envs
+        returns = torch.empty(n, dtype=torch.float32, device=env.device)
+        steps = torch.empty(n, dtype=torch.int32, device=env.device)
+        term = torch.empty(n, dtype=torch.uint8, device=env.device)
+        flags = 1 if deterministic else 0   # BOATAGENT_ROLLOUT_DETERMINISTIC
+        with torch.cuda.device(env.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            self._lib.check(self._L.boatagent_rollout(env._h, self.blob.data_ptr(), self.actor.max_action.data_ptr(),
+                                                      self.seed, self.steps, int(max_steps), flags, env.obs.data_ptr(),
+                                                      env.obs.data_ptr(), returns.data_ptr(), steps.data_ptr(),
+                                                      term.data_ptr(), stream), "boatagent_rollout")
+        self.steps += int(max_steps)
+        return returns, steps, term
