@@ -13,12 +13,6 @@
 
 using namespace boatenv;
 
-#define CUDA_TRY(expr)                                  \
-    do {                                                \
-        cudaError_t _e = (expr);                        \
-        if (_e != cudaSuccess) return (int)_e;          \
-    } while (0)
-
 namespace boatenv {
 static std::atomic<long long> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
@@ -417,6 +411,18 @@ int boatenv_step(boatenv_t h, const void *actions, void *obs_out, void *reward_o
     return step_common(h, a, (cudaStream_t)stream);
 }
 
+// The episode-end queue of the K > 1 kernels with wind curves under auto-reset (StepArgs::kq_*), allocated on first
+// use.  Sized for every env plus the rounding of up to 1024 per-CTA regions to whole warp tiles; a launch whose
+// regions do not fit sets the wind up inline instead (step_impl.inl).
+static int ensure_episode_queue(boatenv_t h) {
+    if (h->kq_entries) return BOATENV_OK;
+    GUARD_DEVICE(h);
+    h->kq_total = num_blocks(h->cfg.n_envs) * 32 + 1024LL * kWarpsPerCta * 32;
+    CUDA_TRY(cudaMalloc((void **)&h->kq_entries, (size_t)h->kq_total * sizeof(uint2)));
+    CUDA_TRY(cudaMalloc((void **)&h->kq_counts, 4096 * sizeof(unsigned)));
+    return BOATENV_OK;
+}
+
 int boatenv_step_k(boatenv_t h, const void *actions, int64_t action_stride, int32_t k, void *obs_out,
                    void *reward_out, uint8_t *done_out, uint8_t *term_out, int32_t *steps_out, uint32_t flags,
                    void *stream) {
@@ -435,12 +441,8 @@ int boatenv_step_k(boatenv_t h, const void *actions, int64_t action_stride, int3
     a.steps_out = steps_out;
     a.flags = flags;
     if (k > 1 && h->cfg.ncurves > 0 && (flags & BOATENV_AUTO_RESET)) {  // episode-end queue of the fused kernels
-        if (!h->kq_entries) {
-            GUARD_DEVICE(h);
-            h->kq_total = num_blocks(h->cfg.n_envs) * 32 + 1024LL * kWarpsPerCta * 32;
-            CUDA_TRY(cudaMalloc((void **)&h->kq_entries, (size_t)h->kq_total * sizeof(uint2)));
-            CUDA_TRY(cudaMalloc((void **)&h->kq_counts, 4096 * sizeof(unsigned)));
-        }
+        const int rc = ensure_episode_queue(h);
+        if (rc) return rc;
         a.kq_entries = h->kq_entries;
         a.kq_counts = h->kq_counts;
         a.kq_total = h->kq_total;
@@ -575,10 +577,9 @@ static int step_host_impl(boatenv_t h, const void *actions_host, int k, void *ob
         }
         act_dev = h->h_act_k;
         if (steps_host && !h->h_steps) CUDA_TRY(cudaMalloc((void **)&h->h_steps, (size_t)n * sizeof(int32_t)));
-        if (h->cfg.ncurves > 0 && (flags & BOATENV_AUTO_RESET) && !h->kq_entries) {  // episode-end queue of the fused kernels
-            h->kq_total = num_blocks(n) * 32 + 1024LL * kWarpsPerCta * 32;
-            CUDA_TRY(cudaMalloc((void **)&h->kq_entries, (size_t)h->kq_total * sizeof(uint2)));
-            CUDA_TRY(cudaMalloc((void **)&h->kq_counts, 4096 * sizeof(unsigned)));
+        if (h->cfg.ncurves > 0 && (flags & BOATENV_AUTO_RESET)) {  // episode-end queue of the fused kernels
+            rc = ensure_episode_queue(h);
+            if (rc) return rc;
         }
     }
     // chunks are multiples of the CTA tile so that every tile keeps its 16-byte alignment
@@ -791,7 +792,7 @@ int boatenv_fill_uniform_actions(boatenv_t h, uint64_t step_counter, double scal
 
 }  // extern "C"
 
-// accessors for the other translation units (replay.cu's fused step+store)
+// the handle accessors of launch.h
 namespace boatenv {
 DevCfg *handle_cfg(boatenv_t h) { return &h->cfg; }
 int handle_precision(boatenv_t h) { return h->precision; }

@@ -2,13 +2,13 @@
 // as building blocks shared by the acting kernel (policy_mlp.cu) and the closed-loop rollout kernel (rollout.cu).
 // Both kernels run the same warp roles on the same shared-memory map: 8 epilogue warps in two groups of four
 // (warp w: TMEM lanes 32 (w % 4) .. + 31, the hardware's lane window of a warp; group w / 4), and warp 8 issues
-// the MMAs.  The pass functions below (actor_prologue .. actor_normal_draw) are the steps of policy_mlp_kernel,
-// statement for statement, so the rollout's actions are bit-identical to boatagent_policy_act's.  The acting
-// kernel keeps them written out inline: calling them there changes its register allocation.
+// the MMAs.  Both kernels run the pass through the functions below (actor_prologue .. actor_normal_draw), so the
+// rollout's actions are bit-identical to boatagent_policy_act's.
 #pragma once
 #include <cstdint>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
+#include <mutex>
 
 #include "../../include/boatenv.h"
 #include "common.cuh"
@@ -29,8 +29,6 @@ constexpr int kOffB3 = kOffB2 + kHidden * 4;                // fp32[16]
 constexpr int kBlobBytes = kOffB3 + kN3 * 4;                // what the host packs (BOATAGENT_POLICY_BLOB_BYTES)
 static_assert(kBlobBytes == BOATAGENT_POLICY_BLOB_BYTES, "header and kernel disagree on the weight blob");
 
-__device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
 // UMMA shared-memory descriptor, K-major, no swizzle (cute::UMMA::SmemDescriptor: start >> 4 at [0,14), LBO >> 4 at
 // [16,30), SBO >> 4 at [32,46), version 1 at [46,48), layout type 0 at [61,64)).
 __device__ __forceinline__ uint64_t umma_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
@@ -50,22 +48,10 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t a_desc, uint
         "}" ::"r"(tmem_d), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint64_t *bar) {   // arrives on `bar` when every MMA issued so far is done
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_addr(bar)) : "memory");
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void bar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "W_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra D_%=;\n\t"
-        "bra W_%=;\n\t"
-        "D_%=:\n\t"
-        "}" ::"r"(smem_addr(bar)), "r"(parity) : "memory");
-}
 // 32 consecutive fp32 accumulator columns of this thread's TMEM lane: asynchronous load (the registers are valid after
 // tmem_ld_wait()), so the next chunk can be in flight while the current one is processed
 __device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
@@ -106,17 +92,17 @@ constexpr int kSmemBytes = kOffBar + 2 * 5 * 8;
 static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
 enum { B_A0 = 0, B_D1 = 1, B_H1 = 2, B_D2 = 3, B_FREE = 4 };
 
-__device__ __forceinline__ void bar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_addr(bar)) : "memory");
+__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ bool bar_test(uint64_t *bar, uint32_t parity) {
+__device__ __forceinline__ bool mbar_test(uint64_t *bar, uint32_t parity) {
     uint32_t ok;
     asm volatile(
         "{\n\t"
         ".reg .pred p;\n\t"
         "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
         "selp.u32 %0, 1, 0, p;\n\t"
-        "}" : "=r"(ok) : "r"(smem_addr(bar)), "r"(parity) : "memory");
+        "}" : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
     return ok != 0;
 }
 // D[tmem] (+)= A[tmem, bf16 pairs per column] . B[smem]^T
@@ -147,19 +133,19 @@ __device__ __forceinline__ uint32_t actor_prologue(const unsigned char *__restri
         reinterpret_cast<uint4 *>(smem)[i] = __ldg(reinterpret_cast<const uint4 *>(blob) + i);
     if (tid == 0) {
         for (int g = 0; g < 2; ++g) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 128;" ::"r"(smem_addr(bars + 5 * g + B_A0)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bars + 5 * g + B_D1)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 128;" ::"r"(smem_addr(bars + 5 * g + B_H1)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bars + 5 * g + B_D2)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 128;" ::"r"(smem_addr(bars + 5 * g + B_FREE)) : "memory");
+            mbar_init(bars + 5 * g + B_A0, 128);
+            mbar_init(bars + 5 * g + B_D1, 1);
+            mbar_init(bars + 5 * g + B_H1, 128);
+            mbar_init(bars + 5 * g + B_D2, 1);
+            mbar_init(bars + 5 * g + B_FREE, 128);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
     if (warp == kMmaWarp) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_addr(tmem_base_slot)) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_base_slot)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    proxy_fence();
+    fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -171,7 +157,7 @@ __device__ __forceinline__ uint32_t actor_prologue(const unsigned char *__restri
 // Returns true when the group's pass through the network is fully issued (the caller advances its parity).
 __device__ __forceinline__ bool actor_mma_poll(uint64_t *b, int &state, uint32_t par, uint32_t region, uint32_t sbase, int g) {
     if (state == 0) {          // observations staged -> layer 1: D1[128][256] = A0 . W1^T
-        if (!bar_test(b + B_A0, par)) return false;
+        if (!mbar_test(b + B_A0, par)) return false;
         tc_fence_after();
         umma_bf16(region, umma_desc(sbase + kOffA0 + g * (kTileM * kK1 * 2), kTileM * 16, 128),
                   umma_desc(sbase + kOffW1, kHidden * 16, 128), umma_idesc(kTileM, kHidden), 0u);
@@ -180,7 +166,7 @@ __device__ __forceinline__ bool actor_mma_poll(uint64_t *b, int &state, uint32_t
         return false;
     }
     // h1 is in TMEM (state 1) / the first half has been read (state 2)
-    if (!bar_test(b + (state == 1 ? B_H1 : B_FREE), par)) return false;
+    if (!mbar_test(b + (state == 1 ? B_H1 : B_FREE), par)) return false;
     tc_fence_after();
     const int half = state - 1;   // output columns 128 half .. + 127 of layer 2
 #pragma unroll 1
@@ -206,14 +192,14 @@ __device__ __forceinline__ void actor_stage_a0(uint64_t *b, unsigned char *a0, i
         out.w = pack_bf16(o[j * 8 + 6], o[j * 8 + 7]);
         *reinterpret_cast<uint4 *>(a0 + j * (kTileM * 16) + row * 16) = out;
     }
-    proxy_fence();
+    fence_proxy_async_smem();
     tc_fence_before();
-    bar_arrive(b + B_A0);
+    mbar_arrive(b + B_A0);
 }
 
 // Layer-1 epilogue: accumulator -> + bias -> ReLU -> bf16 pairs, back into TMEM in place; then signals h1_ready.
 __device__ __forceinline__ void actor_layer1_epilogue(uint64_t *b, uint32_t par, uint32_t region, const float *b1) {
-    bar_wait(b + B_D1, par);
+    mbar_wait(b + B_D1, par);
     tc_fence_after();
     {
         uint32_t ra[32], rb[32];
@@ -240,7 +226,7 @@ __device__ __forceinline__ void actor_layer1_epilogue(uint64_t *b, uint32_t par,
     }
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
     tc_fence_before();
-    bar_arrive(b + B_H1);
+    mbar_arrive(b + B_H1);
 }
 
 // Layer-2 epilogue (two halves of 128 columns) fused with the fp32 heads: acc[j] = relu(h2) . w3[j] (bias not added).
@@ -251,7 +237,7 @@ __device__ __forceinline__ void actor_layer2_heads(uint64_t *b, uint32_t region,
     for (int j = 0; j < NH; ++j) acc[j] = 0.f;
 #pragma unroll 1
     for (int half = 0; half < 2; ++half) {
-        bar_wait(b + B_D2, (uint32_t)half);   // two completions per pass: parities 0, 1
+        mbar_wait(b + B_D2, (uint32_t)half);   // two completions per pass: parities 0, 1
         tc_fence_after();
         uint32_t ra[32], rb[32];
         auto chunk = [&](const uint32_t (&r)[32], int c) {   // c: 32-column chunk of the 256 layer-2 outputs
@@ -285,7 +271,7 @@ __device__ __forceinline__ void actor_layer2_heads(uint64_t *b, uint32_t region,
         tmem_ld_wait(rb); chunk(rb, half * 4 + 3);
         if (half == 0) {   // the columns may be overwritten by the second half now
             tc_fence_before();
-            bar_arrive(b + B_FREE);
+            mbar_arrive(b + B_FREE);
         }
     }
 }
@@ -300,6 +286,32 @@ __device__ __forceinline__ float actor_normal_draw(long long env, unsigned long 
     const float u1 = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
     const float u2 = ((float)(r.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
     return sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
+}
+
+// Launch set-up of a family of kernels built on this pass, on the current device: raises their dynamic shared-memory
+// limit to kSmemBytes and returns the SM count in n_sm.  Done once per device and family (the statics belong to the
+// instantiation) under a mutex, so that alternating devices or host threads neither thrash nor race.
+template <auto... Kernels>
+cudaError_t actor_kernels_setup(int &n_sm) {
+    static std::mutex mu;
+    static int n_sm_of[64] = {0};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    if (dev < 0 || dev >= 64) return cudaErrorInvalidDevice;
+    std::lock_guard<std::mutex> lock(mu);
+    if (n_sm_of[dev] == 0) {
+        for (const void *k : {(const void *)Kernels...}) {
+            e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+            if (e != cudaSuccess) return e;
+        }
+        int v = 0;
+        e = cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
+        if (e != cudaSuccess) return e;
+        n_sm_of[dev] = v;
+    }
+    n_sm = n_sm_of[dev];
+    return cudaSuccess;
 }
 
 }  // namespace boatenv

@@ -259,6 +259,18 @@ __device__ __forceinline__ bool next_sample_in_next_piece(const DevCfg &c, int j
     return r + c.npieces >= c.Lm1 && j + 1 <= c.npieces - 1;
 }
 
+// Statistics of an episode that ended with termination `code` and return `ret` (info dict, boat_env.py:24-32,87-113),
+// counted in fp64 into the counter row of state block `blk`: sparse events -> per-env REDs.
+template <typename T>
+__device__ __forceinline__ void count_episode_end(const DevCfg &c, int blk, int code, T ret) {
+    double *cnt = c.counters + (blk & (kCounterSlots - 1)) * 32;
+    const double r = (double)ret;
+    atomicAdd(cnt + (code - 1), 1.0);
+    atomicAdd(cnt + 5, 1.0);
+    atomicAdd(cnt + 6, r);
+    atomicAdd(cnt + 7, r * r);
+}
+
 // A NaN bit pattern that no arithmetic instruction produces (their NaNs are canonical): see the stage-refill vote.
 __device__ __forceinline__ bool is_poison(float v) { return __float_as_uint(v) == 0x7fc00001u; }
 __device__ __forceinline__ bool is_poison(double v) { return __double_as_longlong(v) == 0x7ff8000000000001ll; }
@@ -309,30 +321,11 @@ __device__ __forceinline__ void stage_reset_obs(const DevCfg &c, T *row, T s_y0)
 }
 
 // ---------------------------------------------------------------------------------
-// TMA bulk-copy + mbarrier primitives (sm_90+/sm_100a PTX).  The copies are 1-D
+// TMA bulk-copy primitives (sm_90+/sm_100a PTX; the mbarrier ones are in common.cuh).  The copies are 1-D
 // (cp.async.bulk, no tensor map): a warp's state block is contiguous in HBM.
 // ---------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_fence_init() {
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t"
-        "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
 // global -> shared bulk copy, completion counted in bytes on `bar`.  Default L2 policy: an evict_first
 // cache hint measured 3 % slower (the alternating sweep lets the tail of a launch hit L2 in the next one).
@@ -349,8 +342,6 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 // wait until the bulk stores of all committed groups have finished READING shared memory
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// generic-proxy writes (st.shared) -> visible to the async proxy (the bulk store that follows)
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 // Build-time switches.  BOAT_MINBLOCKS_F32 / BOAT_STAGES / BOAT_SETUP_WARPS / BOAT_CTA_THREADS are tuning
 // knobs (defaults = measured optimum); the BOAT_DEBUG_* macros remove parts of the kernel for the
 // ablation measurements quoted in DESIGN.md section 4 and are never defined in a product build.
@@ -788,14 +779,7 @@ boat_step_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ StepA
                 // when an episode ends
                 uint32_t *epi_g = reinterpret_cast<uint32_t *>(gb + c.off_epi) + lane;
                 uint32_t episode = KMULTI ? episode_k : ((need_setup && active) ? *epi_g : 0u);
-                if (is_done) {  // statistics (info dict, boat_env.py:24-32,87-113): sparse events -> per-env REDs
-                    double *cnt = c.counters + (blk & (kCounterSlots - 1)) * 32;
-                    const double ret = (double)d[D_RET];
-                    atomicAdd(cnt + (code - 1), 1.0);
-                    atomicAdd(cnt + 5, 1.0);
-                    atomicAdd(cnt + 6, ret);
-                    atomicAdd(cnt + 7, ret * ret);
-                }
+                if (is_done) count_episode_end(c, blk, code, d[D_RET]);
                 if (is_done) {  // the terminal observation leaves before a reset overwrites the row
                     if (a.final_obs_out) {
                         T *fo = reinterpret_cast<T *>(a.final_obs_out) + (size_t)i * kObsDim;

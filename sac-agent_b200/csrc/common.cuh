@@ -273,6 +273,32 @@ template <> struct Fx<float> {
     }
 };
 
+// ---------------------------------------------------------------------------------
+// mbarrier and proxy-fence primitives (sm_90+/sm_100a PTX), shared by the step kernels' TMA pipeline
+// (boat_step.cuh) and the tcgen05 actor pass (actor_tc.cuh)
+// ---------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_fence_init() {
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "WAIT_%=:\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
+        "@p bra DONE_%=;\n\t"
+        "bra WAIT_%=;\n\t"
+        "DONE_%=:\n\t"
+        "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+// generic-proxy writes (st.shared) -> visible to the async proxy (a bulk store or an MMA that reads them next)
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
 // round-to-nearest integer of x * k for |x * k| < 2^22 without the conversion pipe (one FFMA + one IADD)
 __device__ __forceinline__ int fixed_increment(float x, float k) {
     return __float_as_int(fmaf(x, k, 12582912.0f)) - 0x4B400000;

@@ -1,5 +1,5 @@
-// launch.h -- launcher prototypes shared between the per-precision translation units
-// (step_f32.cu, step_f64.cu) and the C-ABI front end (abi.cu).
+// launch.h -- declarations shared by the translation units of libboatenv: the launcher prototypes of the
+// per-precision units (step_f32.cu, step_f64.cu), the env-handle accessors (abi.cu) and CUDA_TRY.
 #pragma once
 #include "common.cuh"
 
@@ -26,10 +26,23 @@ private:
     boatenv::DeviceGuard _guard((h)->device);                      \
     if (!_guard.ok()) return (int)_guard.error()
 
+// In an int-returning entry point: return a CUDA call's error code unless it succeeded.
+#define CUDA_TRY(expr)                                  \
+    do {                                                \
+        cudaError_t _e = (expr);                        \
+        if (_e != cudaSuccess) return (int)_e;          \
+    } while (0)
 
 namespace boatenv {
 
 void count_launch();
+
+// Access to an env handle from the other translation units (the handle is defined in abi.cu).
+DevCfg *handle_cfg(boatenv_t h);
+int handle_precision(boatenv_t h);
+int handle_device(boatenv_t h);
+bool handle_was_reset(boatenv_t h);
+int handle_next_parity(boatenv_t h);   // the sweep direction of the next step launch (alternates)
 
 cudaError_t launch_step_f32(const DevCfg &, const StepArgs &, cudaStream_t);
 cudaError_t launch_step_f64(const DevCfg &, const StepArgs &, cudaStream_t);

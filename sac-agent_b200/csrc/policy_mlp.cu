@@ -18,11 +18,8 @@
 //     under the other's MMAs; observations are fetched one tile ahead;
 //   * HBM traffic is the input and the output: 4 * obs_dim + 4 * A bytes per env.
 // Inputs are rounded to bf16 (fp32 accumulation): acting only, the learner never sees this kernel.
-// The rollout kernel (rollout.cu) runs the same pass through the copies of these steps in actor_tc.cuh
-// (actor_prologue .. actor_normal_draw), which must stay statement for statement equal to the code below: a change
-// here is made there too (tests/test_gpu_rollout.py checks the two kernels' actions bit for bit).
-#include <mutex>
-
+// The pass is the building blocks of actor_tc.cuh (actor_prologue .. actor_normal_draw), which the rollout kernel
+// (rollout.cu) runs too: the two kernels' actions agree bit for bit (tests/test_gpu_rollout.py).
 #include "actor_tc.cuh"
 #include "launch.h"
 
@@ -40,29 +37,8 @@ policy_mlp_kernel(const unsigned char *__restrict__ blob, const float *__restric
     constexpr int NH = 2 * NA;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + kOffBar);
-
-    for (int i = tid; i < kBlobBytes / 16; i += kThreads)
-        reinterpret_cast<uint4 *>(smem)[i] = __ldg(reinterpret_cast<const uint4 *>(blob) + i);
-    if (tid == 0) {
-        for (int g = 0; g < 2; ++g) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 128;" ::"r"(smem_addr(bars + 5 * g + B_A0)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bars + 5 * g + B_D1)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 128;" ::"r"(smem_addr(bars + 5 * g + B_H1)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bars + 5 * g + B_D2)) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 128;" ::"r"(smem_addr(bars + 5 * g + B_FREE)) : "memory");
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == kMmaWarp) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_addr(&tmem_base_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    proxy_fence();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_base_slot;
-    const uint32_t sbase = smem_addr(smem);
+    const uint32_t tmem = actor_prologue(blob, smem, &tmem_base_slot);
+    const uint32_t sbase = smem_u32(smem);
     const long long n_tiles = (n + kTileM - 1) / kTileM;
     const long long G = gridDim.x;
     // local tile j of this CTA is global tile blockIdx.x + j * G; group g takes the local tiles j = 2 i + g
@@ -76,32 +52,9 @@ policy_mlp_kernel(const unsigned char *__restrict__ blob, const float *__restric
             const long long cnt[2] = {(my_tiles + 1) / 2, my_tiles / 2};
             while (it[0] < cnt[0] || it[1] < cnt[1]) {
 #pragma unroll
-                for (int g = 0; g < 2; ++g) {
-                    if (it[g] >= cnt[g]) continue;
-                    uint64_t *b = bars + 5 * g;
-                    const uint32_t par = (uint32_t)(it[g] & 1);
-                    const uint32_t region = tmem + 256u * g;
-                    if (state[g] == 0) {          // observations staged -> layer 1: D1[128][256] = A0 . W1^T
-                        if (!bar_test(b + B_A0, par)) continue;
-                        tc_fence_after();
-                        umma_bf16(region, umma_desc(sbase + kOffA0 + g * (kTileM * kK1 * 2), kTileM * 16, 128),
-                                  umma_desc(sbase + kOffW1, kHidden * 16, 128), umma_idesc(kTileM, kHidden), 0u);
-                        umma_commit(b + B_D1);
-                        state[g] = 1;
-                    } else {                      // h1 is in TMEM (state 1) / the first half has been read (state 2)
-                        if (!bar_test(b + (state[g] == 1 ? B_H1 : B_FREE), par)) continue;
-                        tc_fence_after();
-                        const int half = state[g] - 1;   // output columns 128 half .. + 127 of layer 2
-#pragma unroll 1
-                        for (int k = 0; k < kHidden / 16; ++k)
-                            umma_bf16_ts(region + 128u, region + 8u * k,
-                                         umma_desc(sbase + kOffW2 + half * (128 * 16) + k * 2 * (kHidden * 16), kHidden * 16, 128),
-                                         umma_idesc(kTileM, 128), k > 0 ? 1u : 0u);
-                        umma_commit(b + B_D2);
-                        if (state[g] == 1) state[g] = 2;
-                        else { state[g] = 0; ++it[g]; }
-                    }
-                }
+                for (int g = 0; g < 2; ++g)
+                    if (it[g] < cnt[g] && actor_mma_poll(bars + 5 * g, state[g], (uint32_t)(it[g] & 1), tmem + 256u * g, sbase, g))
+                        ++it[g];
             }
         }
     } else {
@@ -122,110 +75,17 @@ policy_mlp_kernel(const unsigned char *__restrict__ blob, const float *__restric
         fetch_obs(0);
         for (long long i = 0; i < cnt; ++i) {
             const long long env = ((long long)blockIdx.x + (2 * i + g) * G) * kTileM + row;
-            const uint32_t par = (uint32_t)(i & 1);
-            // ---- observations -> bf16 A0 (the previous tile's epilogue, i.e. every read of this region, is behind us) ----
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                uint4 out;
-                out.x = pack_bf16(o[j * 8 + 0], o[j * 8 + 1]);
-                out.y = pack_bf16(o[j * 8 + 2], o[j * 8 + 3]);
-                out.z = pack_bf16(o[j * 8 + 4], o[j * 8 + 5]);
-                out.w = pack_bf16(o[j * 8 + 6], o[j * 8 + 7]);
-                *reinterpret_cast<uint4 *>(a0 + j * (kTileM * 16) + row * 16) = out;
-            }
-            proxy_fence();
-            tc_fence_before();
-            bar_arrive(b + B_A0);
-            fetch_obs(i + 1);
-            // ---- layer-1 epilogue: accumulator -> + bias -> ReLU -> bf16 pairs, back into TMEM in place ----
-            bar_wait(b + B_D1, par);
-            tc_fence_after();
-            {
-                uint32_t ra[32], rb[32];
-                auto chunk = [&](const uint32_t (&r)[32], int c) {
-                    uint32_t packed[16];
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const float4 bb = *reinterpret_cast<const float4 *>(b1 + c * 32 + 4 * q);
-                        packed[2 * q] = pack_bf16(fmaxf(__uint_as_float(r[4 * q + 0]) + bb.x, 0.f),
-                                                  fmaxf(__uint_as_float(r[4 * q + 1]) + bb.y, 0.f));
-                        packed[2 * q + 1] = pack_bf16(fmaxf(__uint_as_float(r[4 * q + 2]) + bb.z, 0.f),
-                                                      fmaxf(__uint_as_float(r[4 * q + 3]) + bb.w, 0.f));
-                    }
-                    tmem_st16(region + 16u * c, packed);   // columns 16 c .. 16 c + 15 <= what has been read so far
-                };
-                tmem_ld32_issue(region, ra);
-#pragma unroll
-                for (int c = 0; c < 8; c += 2) {
-                    tmem_ld_wait(ra); tmem_ld32_issue(region + 32u * (c + 1), rb); chunk(ra, c);
-                    tmem_ld_wait(rb);
-                    if (c + 2 < 8) tmem_ld32_issue(region + 32u * (c + 2), ra);
-                    chunk(rb, c + 1);
-                }
-            }
-            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-            tc_fence_before();
-            bar_arrive(b + B_H1);
-            // ---- layer-2 epilogue (two halves of 128 columns) fused with the fp32 heads ----
+            actor_stage_a0(b, a0, row, o);
+            fetch_obs(i + 1);   // the next tile's observations load under this tile's MMAs
+            actor_layer1_epilogue(b, (uint32_t)(i & 1), region, b1);
             float acc[NH];
-#pragma unroll
-            for (int j = 0; j < NH; ++j) acc[j] = 0.f;
-#pragma unroll 1
-            for (int half = 0; half < 2; ++half) {
-                bar_wait(b + B_D2, (uint32_t)half);   // two completions per tile: parities 0, 1
-                tc_fence_after();
-                uint32_t ra[32], rb[32];
-                auto chunk = [&](const uint32_t (&r)[32], int c) {   // c: 32-column chunk of the 256 layer-2 outputs
-                    float v[32];
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const float4 bb = *reinterpret_cast<const float4 *>(b2 + c * 32 + 4 * q);
-                        v[4 * q + 0] = fmaxf(__uint_as_float(r[4 * q + 0]) + bb.x, 0.f);
-                        v[4 * q + 1] = fmaxf(__uint_as_float(r[4 * q + 1]) + bb.y, 0.f);
-                        v[4 * q + 2] = fmaxf(__uint_as_float(r[4 * q + 2]) + bb.z, 0.f);
-                        v[4 * q + 3] = fmaxf(__uint_as_float(r[4 * q + 3]) + bb.w, 0.f);
-                    }
-#pragma unroll
-                    for (int j = 0; j < NH; ++j) {
-                        const float4 *w = reinterpret_cast<const float4 *>(w3 + j * kHidden + c * 32);
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) {
-                            const float4 ww = w[q];
-                            acc[j] = fmaf(v[4 * q + 0], ww.x, acc[j]);
-                            acc[j] = fmaf(v[4 * q + 1], ww.y, acc[j]);
-                            acc[j] = fmaf(v[4 * q + 2], ww.z, acc[j]);
-                            acc[j] = fmaf(v[4 * q + 3], ww.w, acc[j]);
-                        }
-                    }
-                };
-                const uint32_t d2 = region + 128u;
-                tmem_ld32_issue(d2, ra);
-                tmem_ld_wait(ra); tmem_ld32_issue(d2 + 32u, rb); chunk(ra, half * 4 + 0);
-                tmem_ld_wait(rb); tmem_ld32_issue(d2 + 64u, ra); chunk(rb, half * 4 + 1);
-                tmem_ld_wait(ra); tmem_ld32_issue(d2 + 96u, rb); chunk(ra, half * 4 + 2);
-                tmem_ld_wait(rb); chunk(rb, half * 4 + 3);
-                if (half == 0) {   // the columns may be overwritten by the second half now
-                    tc_fence_before();
-                    bar_arrive(b + B_FREE);
-                }
-            }
+            actor_layer2_heads<NH>(b, region, b2, w3, acc);
             if (env < n) {
 #pragma unroll
                 for (int a = 0; a < NA; ++a) {   // sample_normal, networks.py:47-65
                     const float mean = acc[a] + b3[a];
                     const float log_std = -5.0f + 3.5f * (tanhf(acc[NA + a] + b3[NA + a]) + 1.0f);
-                    float e;
-                    if (eps) {
-                        e = __ldg(eps + env * NA + a);
-                    } else {   // Box-Muller on Philox(seed; env, step, action)
-                        const boatenv::Philox4 r = boatenv::philox4x32_10(
-                            (uint32_t)env, (uint32_t)((unsigned long long)env >> 32), (uint32_t)step,
-                            0xD0000000u | ((uint32_t)a << 16) | (uint32_t)((step >> 32) & 0xffffu), (uint32_t)seed,
-                            (uint32_t)(seed >> 32));
-                        const float u1 = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
-                        const float u2 = ((float)(r.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
-                        e = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
-                    }
+                    const float e = eps ? __ldg(eps + env * NA + a) : actor_normal_draw(env, step, a, seed);
                     action_out[env * NA + a] = tanhf(mean + e * expf(log_std)) * __ldg(max_action + a);
                 }
             }
@@ -254,30 +114,10 @@ extern "C" int boatagent_policy_act(const void *weight_blob, const float *obs, c
     case 8: kern = policy_mlp_kernel<8>; break;
     default: return BOATENV_EUNSUPPORTED;
     }
-    // per-device configuration (max dynamic shared memory of the four instantiations, SM count): done once per
-    // device under a mutex, so that alternating devices or host threads neither thrash nor race
-    static std::mutex mu;
-    static int n_sm_of[64] = {0};
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return (int)e;
-    if (dev < 0 || dev >= 64) return (int)cudaErrorInvalidDevice;
     int n_sm = 0;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        if (n_sm_of[dev] == 0) {
-            for (kern_t k : {(kern_t)policy_mlp_kernel<1>, (kern_t)policy_mlp_kernel<2>, (kern_t)policy_mlp_kernel<4>,
-                             (kern_t)policy_mlp_kernel<8>}) {
-                e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-                if (e != cudaSuccess) return (int)e;
-            }
-            int v = 0;
-            e = cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
-            if (e != cudaSuccess) return (int)e;
-            n_sm_of[dev] = v;
-        }
-        n_sm = n_sm_of[dev];
-    }
+    const cudaError_t e = actor_kernels_setup<policy_mlp_kernel<1>, policy_mlp_kernel<2>, policy_mlp_kernel<4>,
+                                              policy_mlp_kernel<8>>(n_sm);
+    if (e != cudaSuccess) return (int)e;
     const long long tiles = (n + kTileM - 1) / kTileM;
     const unsigned grid = (unsigned)(tiles < n_sm ? tiles : n_sm);
     kern<<<grid, kThreads, kSmemBytes, (cudaStream_t)stream>>>((const unsigned char *)weight_blob, obs, eps, max_action, seed,

@@ -7,11 +7,6 @@
 using namespace boatenv;
 
 namespace boatenv {
-DevCfg *handle_cfg(boatenv_t h);
-int handle_precision(boatenv_t h);
-int handle_device(boatenv_t h);
-bool handle_was_reset(boatenv_t h);
-
 constexpr int kRecordBlock = 128;
 
 // One thread per recorded env.  The state is decoded by read_field, the same decode boat_get_field_kernel

@@ -13,20 +13,6 @@
 
 using namespace boatenv;
 
-#define CUDA_TRY(expr)                                  \
-    do {                                                \
-        cudaError_t _e = (expr);                        \
-        if (_e != cudaSuccess) return (int)_e;          \
-    } while (0)
-
-namespace boatenv {
-DevCfg *handle_cfg(boatenv_t h);
-int handle_precision(boatenv_t h);
-int handle_device(boatenv_t h);
-bool handle_was_reset(boatenv_t h);
-int handle_next_parity(boatenv_t h);
-}  // namespace boatenv
-
 struct boatreplay_handle {
     void *state, *new_state, *action, *reward;
     uint8_t *terminal;

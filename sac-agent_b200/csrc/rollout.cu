@@ -16,20 +16,11 @@
 //     wind_setup_lane_any: the envs of a freshly reset tile cross piece boundaries at the same step, so it runs
 //     converged.
 // fp32 handles and one action only.  Design notes and measurements: DESIGN.md sections 4 and 8.
-#include <mutex>
-
 #include "actor_tc.cuh"
 #include "boat_step.cuh"
 #include "launch.h"
 
 using namespace boatenv;
-
-namespace boatenv {
-DevCfg *handle_cfg(boatenv_t h);
-int handle_precision(boatenv_t h);
-int handle_device(boatenv_t h);
-bool handle_was_reset(boatenv_t h);
-}  // namespace boatenv
 
 namespace {
 
@@ -68,7 +59,7 @@ boat_rollout_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Ro
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + kOffBar);
     if (tid < 2) group_done[tid] = 0;
     const uint32_t tmem = actor_prologue(a.blob, smem, &tmem_base_slot);   // its __syncthreads orders group_done
-    const uint32_t sbase = smem_addr(smem);
+    const uint32_t sbase = smem_u32(smem);
     const long long n = c.n_envs;
     const long long n_tiles = (n + kTileM - 1) / kTileM;
     const long long G = gridDim.x;
@@ -86,7 +77,7 @@ boat_rollout_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Ro
                     if (!live[g]) continue;
                     // a group raises its flag only after waiting for its last pass's layer 2, i.e. once every pass
                     // it asked for has been issued: state 0 and no A0 pending
-                    if (state[g] == 0 && group_done[g] && !bar_test(bars + 5 * g + B_A0, (uint32_t)(it[g] & 1))) {
+                    if (state[g] == 0 && group_done[g] && !mbar_test(bars + 5 * g + B_A0, (uint32_t)(it[g] & 1))) {
                         live[g] = false;
                         continue;
                     }
@@ -161,13 +152,8 @@ boat_rollout_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Ro
                     index += 1;
                     stage_obs(c, o, d, fx, accel, index);
                     if (code != BOATENV_TERM_NONE) {
-                        alive = false;   // statistics (info dict, boat_env.py:24-32,87-113), as the step kernel counts them
-                        double *cnt_row = c.counters + (blk & (kCounterSlots - 1)) * 32;
-                        const double ret = (double)d[D_RET];
-                        atomicAdd(cnt_row + (code - 1), 1.0);
-                        atomicAdd(cnt_row + 5, 1.0);
-                        atomicAdd(cnt_row + 6, ret);
-                        atomicAdd(cnt_row + 7, ret * ret);
+                        alive = false;   // statistics as the step kernel counts them
+                        count_episode_end(c, blk, code, d[D_RET]);
                     } else if (kCurves && next_sample_in_next_piece(c, j, r)) {
                         double cf[8];
                         wind_setup_lane_any(c, env, episode, index, cf);
@@ -238,28 +224,11 @@ extern "C" int boatagent_rollout(boatenv_t h, const void *weight_blob, const flo
     const DevCfg &c = *handle_cfg(h);
     const kern_t kern = kernel_for(c.wind_kind);
     if (!kern) return BOATENV_EINVAL;
-    // per-device configuration (max dynamic shared memory of the five instantiations, SM count), once per device
-    static std::mutex mu;
-    static int n_sm_of[64] = {0};
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return (int)e;
-    if (dev < 0 || dev >= 64) return (int)cudaErrorInvalidDevice;
     int n_sm = 0;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        if (n_sm_of[dev] == 0) {
-            for (int wk = WIND_NONE; wk <= WIND_BOTH; ++wk) {
-                e = cudaFuncSetAttribute(kernel_for(wk), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-                if (e != cudaSuccess) return (int)e;
-            }
-            int v = 0;
-            e = cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
-            if (e != cudaSuccess) return (int)e;
-            n_sm_of[dev] = v;
-        }
-        n_sm = n_sm_of[dev];
-    }
+    const cudaError_t e = actor_kernels_setup<boat_rollout_kernel<WIND_NONE>, boat_rollout_kernel<WIND_CONST>,
+                                              boat_rollout_kernel<WIND_VEL_CURVE>, boat_rollout_kernel<WIND_ANGLE_RECT>,
+                                              boat_rollout_kernel<WIND_BOTH>>(n_sm);
+    if (e != cudaSuccess) return (int)e;
     RolloutArgs a;
     a.blob = static_cast<const unsigned char *>(weight_blob);
     a.max_action = max_action;

@@ -17,12 +17,6 @@
 
 using namespace boatenv;
 
-#define CUDA_TRY(expr)                                  \
-    do {                                                \
-        cudaError_t _e = (expr);                        \
-        if (_e != cudaSuccess) return (int)_e;          \
-    } while (0)
-
 constexpr int kToyMaxParams = 9;
 constexpr int kCarParams = 4;        // accel, v_limit, dtheta, dt
 constexpr int kParachuteParams = 9;  // h0, h1, area_free, area_chute, mass, c_w, rho, g, dt_integrator
