@@ -14,6 +14,8 @@ networks/networks.py, the `agent:` block of original_config.yaml); the update is
 recorded run of the reference's own learn() in tests/test_agent_golden.py.
 
     python examples/train_sac.py --envs 65536 --iters 200
+    python examples/train_sac.py --envs 8192 --policy-precision tcgen05 --collect-steps 8 --updates-per-iter 8
+                                          # 8 steps of act + step + remember per launch (ContinuousAgent.collect)
     torchrun --nproc-per-node 8 examples/train_sac.py --envs 65536        # replicas: one agent per GPU shard
     torchrun --nproc-per-node 8 examples/train_sac.py --experiments-root experiments --tune
                                           # the reference's `main.py -p 8`: a tuned_configs.yaml draw per member
@@ -38,7 +40,8 @@ import sac_agent_b200 as S  # noqa: E402
 def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--envs", type=int, default=65536, help="total envs over all ranks")
-    ap.add_argument("--iters", type=int, default=200, help="env steps (each over every env)")
+    ap.add_argument("--iters", type=int, default=200, help="iterations: env steps (each over every env), or "
+                    "--collect-steps of them each")
     ap.add_argument("--warmup-iters", type=int, default=20, help="untimed iterations (graph capture happens here)")
     ap.add_argument("--updates-per-iter", type=int, default=1)
     ap.add_argument("--experiment", type=int, default=5)
@@ -63,9 +66,23 @@ def main(argv=None):
     ap.add_argument("--record-envs", type=int, default=0, metavar="K",
                     help="record every step of the first K envs of each rank's shard into its experiment's episodes/ "
                          "(the reference's Recorder CSVs, DeviceRecorder); flushed at every log interval")
+    ap.add_argument("--collect-steps", type=int, default=0, metavar="T",
+                    help="one iteration = T env steps of every env collected by ONE fused kernel (policy, env step with "
+                         "auto-reset and replay store; ContinuousAgent.collect), then --updates-per-iter updates; "
+                         "needs --policy-precision tcgen05.  0: one env step per iteration, policy and step launched "
+                         "separately")
     args = ap.parse_args(argv)
     if args.record_envs and not args.experiments_root:
         ap.error("--record-envs requires --experiments-root")
+    if args.collect_steps < 0:
+        ap.error("--collect-steps must be >= 0")
+    if args.collect_steps:   # checked before any CUDA work
+        if args.policy_precision != "tcgen05":
+            ap.error("--collect-steps acts through the fused tcgen05 kernel: it needs --policy-precision tcgen05")
+        if args.overlap:
+            ap.error("--collect-steps and --overlap cannot be combined")
+        if args.record_envs:
+            ap.error("--collect-steps and --record-envs cannot be combined (the fused kernel records no steps)")
 
     rank, local_rank, world = S.sharding.dist_info()
     torch.cuda.set_device(local_rank)
@@ -86,7 +103,7 @@ def main(argv=None):
         if args.tune:
             cfg = tuned
     env = S.make_sharded_env(cfg, args.envs, seed=args.seed, precision="fp32", auto_reset=True)
-    mem = S.ReplayBuffer(max(args.buffer, env.n_envs), (11,), 1, precision="fp32", device=local_rank,
+    mem = S.ReplayBuffer(max(args.buffer, env.n_envs * max(args.collect_steps, 1)), (11,), 1, precision="fp32", device=local_rank,
                          seed=args.seed + rank, as_torch=True)
     agent = S.ContinuousAgent(cfg, exp.experiment_dir if exp else None, env.observation_space.shape, env,
                               device=local_rank, seed=args.seed + rank,
@@ -112,6 +129,11 @@ def main(argv=None):
             t0.record()
         if pipe:
             losses = pipe.step()
+        elif args.collect_steps:
+            agent.collect(env, args.collect_steps, done_flag_mode=1)   # T x (act, env.step, remember), one kernel
+            for _ in range(args.updates_per_iter):
+                out = agent.learn()
+                losses = out if out is not None else losses
         else:
             actions = act(obs).squeeze(-1)
             agent.step_and_remember(env, actions, done_flag_mode=1)   # env.step + agent.remember, one kernel
@@ -168,10 +190,11 @@ def main(argv=None):
         if world > 1:
             torch.distributed.all_reduce(recorded)
     sec = float(ms.item()) * 1e-3
+    steps_per_iter = max(args.collect_steps, 1)
     summary = {"example": "train_sac", "overrides": overrides, "n_gpus": world, "envs_total": args.envs, "iters": args.iters,
                "updates_per_iter": args.updates_per_iter, "cuda_graph": not args.no_graph, "overlap": bool(args.overlap),
-               "policy_precision": args.policy_precision,
-               "env_steps_per_s": args.iters * args.envs / sec,
+               "policy_precision": args.policy_precision, "collect_steps": args.collect_steps,
+               "env_steps_per_s": args.iters * steps_per_iter * args.envs / sec,
                "updates_per_s_per_replica": args.iters * args.updates_per_iter / sec,
                "ms_per_iter": 1e3 * sec / args.iters, "episodes": stats["episodes"],
                "mean_return": stats["return_mean"], "reached_goal": stats["reached_goal"],

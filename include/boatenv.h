@@ -356,6 +356,29 @@ BOATENV_API int boatagent_rollout(boatenv_t h, const void *weight_blob, const fl
                                   float *obs_out, float *return_out, int32_t *steps_out, uint8_t *term_out,
                                   void *stream);
 
+/* Experience collection with the tcgen05 policy (the main.py:78-90 loop body -- choose_action, env.step,
+ * agent.remember -- over `steps` steps and every env of the handle) in one persistent kernel.  Each step is exactly
+ * boatagent_policy_act (step = step0 + t, Philox draws, never deterministic) followed by
+ * boatenv_step_store(..., BOATENV_AUTO_RESET): fp32 handles, n_actions = 1, weight_blob and max_action as for
+ * boatagent_policy_act.  Row i of step t goes to ring slot (mem_cntr + t * n_envs + i) % mem_size:
+ *   state = the observation the env acted on, action, reward, new_state = the observation after the step (the
+ *   terminal one if the episode ended, written before the reset), terminal = (term == reached_goal) for
+ *   done_flag_mode 1, (term != 0) for done_flag_mode 0.
+ * An env whose episode ends is reset in the kernel as BOATENV_AUTO_RESET does (counters updated once, episode
+ * number + 1, the new episode's draws) and keeps stepping.  On return the handle, the ring and the outputs are what
+ * `steps` rounds of boatagent_policy_act and boatenv_step_store leave behind:
+ *   obs_inout  float32 [N][11]  the current observations on entry, the last (post-reset) ones on return
+ *   reward_out float32 [N], done_out / term_out uint8 [N] (either may be NULL, not both)  of the last step
+ * and mem_cntr has grown by steps * n_envs.
+ * Errors (a rejected call changes nothing): BOATENV_EUNSUPPORTED for an fp64 handle or a ring that is not fp32 with
+ * obs_dim 11 and one action, BOATENV_ESTATE before reset, BOATENV_EINVAL for NULL pointers, steps < 1, a
+ * done_flag_mode other than 0 / 1, ring and handle on different devices, or steps * n_envs > mem_size (rows of one
+ * call may not share a slot), BOATENV_EALIGN for a weight_blob that is not 16-byte aligned. */
+BOATENV_API int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action,
+                                  uint64_t seed, uint64_t step0, int32_t steps, int done_flag_mode,
+                                  float *obs_inout, float *reward_out, uint8_t *done_out, uint8_t *term_out,
+                                  void *stream);
+
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 
 typedef struct boattoy_handle *boattoy_t;

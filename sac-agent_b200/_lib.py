@@ -69,6 +69,7 @@ SIGNATURES = {
     "boatagent_adam_polyak_step": (C.c_int, [vp, i32, C.c_float, C.c_float, C.c_float, C.c_float, vp, vp]),
     "boatagent_policy_act": (C.c_int, [vp, vp, vp, vp, u64, u64, i64, i32, i32, vp, vp]),
     "boatagent_rollout": (C.c_int, [vp, vp, vp, u64, u64, i32, u32, vp, vp, vp, vp, vp, vp]),
+    "boatagent_collect": (C.c_int, [vp, vp, vp, vp, u64, u64, i32, C.c_int, vp, vp, vp, vp, vp]),
     "boatreplay_create": (C.c_int, [i64, i32, i32, C.c_int, C.c_int, C.POINTER(vp)]),
     "boatreplay_destroy": (C.c_int, [vp]),
     "boatreplay_store": (C.c_int, [vp, i64, vp, vp, vp, vp, vp, vp]),

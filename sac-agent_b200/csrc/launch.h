@@ -61,4 +61,17 @@ cudaError_t launch_env_state_f64(const DevCfg &, long long env, double *out, cud
 cudaError_t launch_wind_table(const DevCfg &, long long env, double *wv, double *wa, cudaStream_t);
 cudaError_t launch_reduce_counters(const double *counters, double *out, cudaStream_t);
 
+// boatagent_collect (replay.cu checks the arguments, rollout.cu holds the kernel): T steps of policy, env step with
+// auto-reset and replay store, fused
+struct CollectArgs {
+    const unsigned char *blob;
+    const float *max_action;
+    unsigned long long seed, step0;
+    int steps;
+    float *obs_inout, *reward_out;
+    uint8_t *done_out, *term_out;   // either may be NULL
+    ReplayView rp;
+};
+cudaError_t launch_collect(const DevCfg &, const CollectArgs &, cudaStream_t);
+
 }  // namespace boatenv

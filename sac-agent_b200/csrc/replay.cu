@@ -1,6 +1,7 @@
 // replay.cu -- device-resident ReplayBuffer (agent/buffer.py:3-35): ring store,
-// uniform-with-replacement sample-gather, and the fused env.step + agent.remember
-// launch (main.py:81-88).  Rows are kept exactly as the reference keeps them --
+// uniform-with-replacement sample-gather, the fused env.step + agent.remember
+// launch (main.py:81-88) and the entry point of the fused act + step + remember
+// collection kernel (rollout.cu).  Rows are kept exactly as the reference keeps them --
 // five parallel arrays state[size][obs], new_state[size][obs], action[size][na],
 // reward[size], terminal[size] -- so a sampled batch is five dense tensors the
 // learner can consume without a transpose.
@@ -305,6 +306,44 @@ int boatenv_step_store(boatenv_t h, boatreplay_t r, const void *actions, void *o
     CUDA_TRY(r->precision == 32 ? launch_step_f32(c, a, (cudaStream_t)stream)
                                 : launch_step_f64(c, a, (cudaStream_t)stream));
     r->mem_cntr += c.n_envs;
+    return BOATENV_OK;
+}
+
+int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action, uint64_t seed,
+                      uint64_t step0, int32_t steps, int done_flag_mode, float *obs_inout, float *reward_out,
+                      uint8_t *done_out, uint8_t *term_out, void *stream) {
+    if (!h || !r || !weight_blob || !max_action || !obs_inout || !reward_out || (!done_out && !term_out) || steps < 1 ||
+        (done_flag_mode != 0 && done_flag_mode != 1))
+        return BOATENV_EINVAL;
+    if (handle_precision(h) != 32 || r->precision != 32 || r->obs_dim != kObsDim || r->n_actions != 1)
+        return BOATENV_EUNSUPPORTED;
+    if (!handle_was_reset(h)) return BOATENV_ESTATE;
+    const DevCfg &c = *handle_cfg(h);
+    // tiles advance at different rates: two rows of one call in the same slot would race
+    if (handle_device(h) != r->device || (long long)steps * c.n_envs > r->mem_size) return BOATENV_EINVAL;
+    if ((reinterpret_cast<uintptr_t>(weight_blob) & 15u) != 0) return BOATENV_EALIGN;
+    GUARD_DEVICE(r);
+    CollectArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.blob = static_cast<const unsigned char *>(weight_blob);
+    a.max_action = max_action;
+    a.seed = seed;
+    a.step0 = step0;
+    a.steps = steps;
+    a.obs_inout = obs_inout;
+    a.reward_out = reward_out;
+    a.done_out = done_out;
+    a.term_out = term_out;
+    a.rp.state = r->state;
+    a.rp.new_state = r->new_state;
+    a.rp.action = r->action;
+    a.rp.reward = r->reward;
+    a.rp.terminal = r->terminal;
+    a.rp.mem_size = r->mem_size;
+    a.rp.base_slot = r->mem_cntr % r->mem_size;
+    a.rp.done_flag_mode = done_flag_mode;
+    CUDA_TRY(launch_collect(c, a, (cudaStream_t)stream));
+    r->mem_cntr += (long long)steps * c.n_envs;
     return BOATENV_OK;
 }
 

@@ -265,3 +265,33 @@ class TensorCorePolicy:
                                                       term.data_ptr(), stream), "boatagent_rollout")
         self.steps += int(max_steps)
         return returns, steps, term
+
+    @torch.no_grad()
+    def collect(self, env, memory, steps, done_flag_mode=1):
+        """`steps` rounds of the training loop body -- `act(env.obs)`, then `memory.step_store(env, actions,
+        done_flag_mode)` -- over every env of the fp32 auto-resetting BatchedBoatEnv `env`, in ONE kernel
+        (boatagent_collect, csrc/rollout.cu): the same actions, env steps, resets and ring rows (fp32 ReplayBuffer
+        `memory`) as that loop.  Advances `steps` by `steps`.  Returns (env.obs, env.reward, env.done, {"term":
+        env.term}) of the last step, as ReplayBuffer.step_store does; launches on the current stream and does not
+        synchronise."""
+        steps = int(steps)
+        if self.n_actions != 1 or self.obs_dim != 11:
+            raise ValueError("collect: the BoatEnv actor (11 observations, one action)")
+        if not env.auto_reset:
+            raise ValueError("collect: the env must auto-reset (created with auto_reset=True)")
+        if env.precision != 32 or memory.precision != 32:
+            raise ValueError("collect: fp32 env and replay buffer only")
+        if env.device != self.blob.device or memory.device != self.blob.device:
+            raise ValueError("collect: the env, the replay buffer and the policy must be on the same device")
+        if steps * env.n_envs > memory.mem_size:
+            raise ValueError(f"collect: {steps} steps x {env.n_envs} envs exceed the ring's {memory.mem_size} slots "
+                             "(rows of one call may not share a slot)")
+        with torch.cuda.device(env.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            self._lib.check(self._L.boatagent_collect(env._h, memory._h, self.blob.data_ptr(),
+                                                      self.actor.max_action.data_ptr(), self.seed, self.steps, steps,
+                                                      int(done_flag_mode), env.obs.data_ptr(), env.reward.data_ptr(),
+                                                      env.done.data_ptr(), env.term.data_ptr(), stream),
+                            "boatagent_collect")
+        self.steps += steps
+        return env.obs, env.reward, env.done, {"term": env.term}
