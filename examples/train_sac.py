@@ -56,6 +56,10 @@ def main(argv=None):
                     help="population mode (main.py -p): every rank trains with its own tuned_configs.yaml draw")
     ap.add_argument("--policy-precision", default="fp32", choices=["fp32", "tf32", "bf16", "tcgen05"],
                     help="dense layers of choose_action on tensor-core inputs (acting only; the learner stays fp32)")
+    ap.add_argument("--learner-precision", default="fp32", choices=["fp32", "tcgen05"],
+                    help="tcgen05: each update runs as libboatenv's two fused kernels (bf16 operands for the 256-wide "
+                         "products, fp32 accumulation) instead of the captured fp32 graph; the batch size must be a "
+                         "multiple of 128")
     ap.add_argument("--set", action="append", default=[], metavar="SECTION__KEY=VALUE",
                     help="override a config key, e.g. --set agent__learning_rate_alpha=0.001 (original_config.yaml names)")
     ap.add_argument("--pbt-every", type=int, default=0,
@@ -107,7 +111,8 @@ def main(argv=None):
                          seed=args.seed + rank, as_torch=True)
     agent = S.ContinuousAgent(cfg, exp.experiment_dir if exp else None, env.observation_space.shape, env,
                               device=local_rank, seed=args.seed + rank,
-                              use_cuda_graph=not args.no_graph, memory=mem, policy_precision=args.policy_precision)
+                              use_cuda_graph=not args.no_graph, memory=mem, policy_precision=args.policy_precision,
+                              learner_precision=args.learner_precision)
     act = agent.choose_action if args.no_graph else agent.choose_action_graphed
     obs = env.reset()
     rec = None
@@ -193,7 +198,8 @@ def main(argv=None):
     steps_per_iter = max(args.collect_steps, 1)
     summary = {"example": "train_sac", "overrides": overrides, "n_gpus": world, "envs_total": args.envs, "iters": args.iters,
                "updates_per_iter": args.updates_per_iter, "cuda_graph": not args.no_graph, "overlap": bool(args.overlap),
-               "policy_precision": args.policy_precision, "collect_steps": args.collect_steps,
+               "policy_precision": args.policy_precision, "learner_precision": args.learner_precision,
+               "collect_steps": args.collect_steps,
                "env_steps_per_s": args.iters * steps_per_iter * args.envs / sec,
                "updates_per_s_per_replica": args.iters * args.updates_per_iter / sec,
                "ms_per_iter": 1e3 * sec / args.iters, "episodes": stats["episodes"],

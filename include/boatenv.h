@@ -379,6 +379,33 @@ BOATENV_API int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weigh
                                   float *obs_inout, float *reward_out, uint8_t *done_out, uint8_t *term_out,
                                   void *stream);
 
+/* One SAC-v1 update (SACLearner.update) of the BoatEnv agent -- obs_dim 11, one action, 256-wide layers -- in two
+ * tcgen05 kernels: the five networks' forward and backward passes per 128-row tile of the batch, then the gradient
+ * reductions, Adam and the Polyak average of the target value network.  The 256 x 256 products (fc2 forward, its
+ * input gradient and its weight gradient) and fc1's forward run with bf16 operands and fp32 accumulation; the heads,
+ * the Gaussian head, fc1's gradients, the losses and the optimiser run in fp32.  Reductions run in a fixed order
+ * without float atomics: an update is bit-reproducible.
+ *   state, new_state float32 [batch][11]; action, reward float32 [batch]; done uint8 [batch]; eps float32 [2][batch]
+ *   (the standard-normal draws of the two sample_normal calls); max_action float32 [1] (device);
+ *   batch a positive multiple of 128;
+ *   slots_host: the 26 slots of boatagent_adam_polyak_step in DeviceAdam's order -- actor fc1 w, b, fc2 w, b, mean w,
+ *   b, std w, b; critic 1 and critic 2 fc1 w, b, fc2 w, b, q w, b; value fc1 w, b, fc2 w, b, v w, b with `target`
+ *   the target value network's tensors (NULL for every other slot).  `param` is read, `grad` receives the batch
+ *   gradient (as the fp32 learner leaves p.grad), then Adam (beta1, beta2, adam_eps, the slot's lr) and the Polyak
+ *   average (tau) run as in boatagent_adam_polyak_step, with adam_state int64[2] as there;
+ *   losses_out float32 [3] (device): value, actor, critic loss;
+ *   workspace: boatagent_sac_update_workspace_bytes(batch) device bytes, 16-byte aligned.
+ * Errors: BOATENV_EINVAL for NULL pointers, a batch that is not a positive multiple of 128, n_slots != 26, a slot
+ * whose numel is not the agent's shape, a missing or extra target, a workspace that is too small; BOATENV_EALIGN for
+ * a workspace or parameter that is not 16-byte aligned. */
+BOATENV_API int64_t boatagent_sac_update_workspace_bytes(int64_t batch);   /* BOATENV_EINVAL for a bad batch */
+BOATENV_API int boatagent_sac_update(const float *state, const float *action, const float *reward,
+                                     const float *new_state, const uint8_t *done, const float *eps,
+                                     const float *max_action, int64_t batch, float gamma, float reward_scale,
+                                     const boatagent_adam_slot *slots_host, int32_t n_slots, float beta1,
+                                     float beta2, float adam_eps, float tau, int64_t *adam_state, float *losses_out,
+                                     void *workspace, int64_t workspace_bytes, void *stream);
+
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 
 typedef struct boattoy_handle *boattoy_t;

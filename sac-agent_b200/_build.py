@@ -33,6 +33,7 @@ UNITS = {
     "policy_mlp.cu": [],
     "record.cu": [],
     "rollout.cu": [],
+    "learner.cu": [],
 }
 
 

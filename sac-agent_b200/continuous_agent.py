@@ -186,7 +186,7 @@ class ContinuousAgent:
     """agent/continuous_agent.py:9-154 on the GPU-resident env and replay ring."""
 
     def __init__(self, config, experiment_dir, input_dims, env, device=None, seed=0, use_cuda_graph=True,
-                 memory=None, policy_precision="fp32"):
+                 memory=None, policy_precision="fp32", learner_precision="fp32"):
         if not torch.cuda.is_available():
             raise RuntimeError("sac_agent_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.env = env
@@ -212,6 +212,12 @@ class ContinuousAgent:
         # "tcgen05" is libboatenv's fused kernel (csrc/policy_mlp.cu: bf16 inputs, fp32 accumulation, the
         # whole forward pass and the draw in one launch, weights re-packed after every update)
         self.policy_precision = policy_precision
+        if learner_precision not in ("fp32", "tcgen05"):
+            raise ValueError("learner_precision: fp32 or tcgen05")
+        # "tcgen05": one update is libboatenv's two fused kernels (csrc/learner.cu: bf16 operands for the 256-wide
+        # products, fp32 accumulation, everything else fp32) instead of the captured fp32 graph; same tensors, state
+        # and checkpoints
+        self.learner_precision = learner_precision
         self._tc_policy = None
         self._weight_listeners = []   # callables run after load_models / load_state_dict (acting copies republish)
         B, O, A = self.batch_size, int(np.prod(self.input_dims)), self.get_n_actions()
@@ -225,6 +231,8 @@ class ContinuousAgent:
         self._losses = None
         self._act_graphs = {}
         self.updates = 0
+        if learner_precision == "tcgen05":
+            self._init_fused_learner()
 
     # -- base_agent.py:7-19 -------------------------------------------------------------
     def get_n_actions(self):
@@ -335,8 +343,41 @@ class ContinuousAgent:
         s, a, r, s2, d = self._batch
         return self.learner.update(s, a, r, s2, d.bool(), eps_sample=self._eps[0], eps_rsample=self._eps[1])
 
+    def _init_fused_learner(self):
+        B, L = self.batch_size, self.learner
+        if self.input_dims != (11,) or self.get_n_actions() != 1 or B <= 0 or B % 128:
+            raise ValueError("learner_precision='tcgen05': the BoatEnv agent (11 observations, one action) and a "
+                             f"batch size that is a positive multiple of 128 (got {self.input_dims}, "
+                             f"{self.get_n_actions()} actions, batch {B})")
+        if any(tuple(p.shape) != (256, 256) for p in (L.actor.fc2.weight, L.critic_1.fc2.weight,
+                                                      L.critic_2.fc2.weight, L.value.fc2.weight)):
+            raise ValueError("learner_precision='tcgen05': 256-wide hidden layers only")
+        nbytes = int(L.optimizer._L.boatagent_sac_update_workspace_bytes(B))
+        self._ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        self._loss_buf = torch.zeros(3, dtype=torch.float32, device=self.device)
+        self._losses = tuple(self._loss_buf[k] for k in range(3))
+
+    def _fused_update(self):
+        """One update in the two kernels of boatagent_sac_update on the current stream (no sync)."""
+        L, o = self.learner, self.learner.optimizer
+        for k, p in enumerate(o.params):   # the kernels write the batch gradient where the fp32 learner leaves it
+            if p.grad is None:
+                p.grad = torch.zeros_like(p)
+            o._slots[k].grad = p.grad.data_ptr()
+        s, a, r, s2, d = self._batch
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            o._lib.check(o._L.boatagent_sac_update(
+                s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), self._eps.data_ptr(),
+                L.actor.max_action.data_ptr(), self.batch_size, float(L.gamma), float(L.scale), o._slots, len(o.params),
+                o.betas[0], o.betas[1], o.eps, o.tau, o.state.data_ptr(), self._loss_buf.data_ptr(),
+                self._ws.data_ptr(), self._ws.numel(), stream), "boatagent_sac_update")
+        return self._losses
+
     def _run_update(self):
-        if not self.use_cuda_graph:
+        if self.learner_precision == "tcgen05":
+            self._fused_update()
+        elif not self.use_cuda_graph:
             self._losses = self._update_static()
         else:
             if self._graph is None:
@@ -350,7 +391,8 @@ class ContinuousAgent:
     def learn(self):
         """continuous_agent.py:96-154.  Returns None before the memory holds one batch (like the
         reference); afterwards the three losses (value, actor, critic) as device tensors (no sync).
-        Three launches: the sample-gather kernel, the Gaussian draws, the captured update."""
+        Three launches: the sample-gather kernel, the Gaussian draws, the captured update (learner_precision
+        "tcgen05": the two kernels of the fused update)."""
         if self.memory.mem_cntr < self.batch_size:
             return None
         self.memory.sample_buffer(self.batch_size, as_torch=True, out=self._batch)

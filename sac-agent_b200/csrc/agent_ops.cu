@@ -1,26 +1,19 @@
 // agent_ops.cu -- the tanh-squashed Gaussian head of the reference's actor
 // (networks/networks.py:47-70, ActorNetwork.sample_normal) as ONE kernel forward and ONE kernel
 // backward.  In PyTorch the head is ~23 element-wise launches forward and ~35 backward on [B, n_actions]
-// tensors -- 80 of the ~190 kernels of a captured SAC update, all launch-latency.
-//
-//   t = tanh(raw_std);  log_std = -5 + 3.5 (t + 1);  std = exp(log_std)          (:53-56)
-//   u = mean + eps * std                     (Normal.rsample / .sample, :60-63; eps ~ N(0, 1) supplied)
-//   action = tanh(u) * max_action                                               (:65)
-//   log_prob = sum_a [ -(u - mean)^2 / (2 std^2) - log_std - log sqrt(2 pi) - log(1 - action^2 + 1e-6) ]   (:66-68)
-//
-// Backward is for the reparameterised draw (u a function of mean and std).  The Gaussian term is then
-// -eps^2 / 2 exactly: autograd's two paths into it cancel, so its gradient is 0 here.
+// tensors -- 80 of the ~190 kernels of a captured SAC update, all launch-latency.  The formulas are in
+// agent_math.cuh, shared with the fused learner (learner.cu).
 #include <cstdint>
 #include <cuda_runtime.h>
 
 #include "../../include/boatenv.h"
+#include "agent_math.cuh"
 #include "launch.h"
 
 namespace {
 
-constexpr float kLogStdMin = -5.0f, kLogStdHalfSpan = 3.5f;  // 0.5 * (LOG_STD_MAX - LOG_STD_MIN)
-constexpr float kHalfLog2Pi = 0.91893853320467274178f;
-constexpr float kReparamNoise = 1e-6f;
+using boatenv::gaussian_head_bwd;
+using boatenv::gaussian_head_fwd;
 
 __global__ void __launch_bounds__(256) gaussian_head_fwd_kernel(const float *__restrict__ mean,
                                                                 const float *__restrict__ raw_std,
@@ -33,13 +26,8 @@ __global__ void __launch_bounds__(256) gaussian_head_fwd_kernel(const float *__r
     float lp = 0.0f;
     for (int a = 0; a < n_actions; ++a) {
         const long long i = b * n_actions + a;
-        const float m = mean[i];
-        const float log_std = kLogStdMin + kLogStdHalfSpan * (tanhf(raw_std[i]) + 1.0f);
-        const float sd = expf(log_std);
-        const float u = m + eps[i] * sd;
-        const float act = tanhf(u) * max_action[a];
-        const float d = u - m;
-        lp += -(d * d) / (2.0f * sd * sd) - log_std - kHalfLog2Pi - logf(1.0f - act * act + kReparamNoise);
+        float act;
+        lp += gaussian_head_fwd(mean[i], raw_std[i], eps[i], max_action[a], act);
         action_out[i] = act;
     }
     log_prob_out[b] = lp;
@@ -55,19 +43,8 @@ __global__ void __launch_bounds__(256) gaussian_head_bwd_kernel(
     const float glp = grad_log_prob ? grad_log_prob[b] : 0.0f;
     for (int a = 0; a < n_actions; ++a) {
         const long long i = b * n_actions + a;
-        const float t = tanhf(raw_std[i]);
-        const float dls = kLogStdHalfSpan * (1.0f - t * t);          // d log_std / d raw_std
-        const float sd = expf(kLogStdMin + kLogStdHalfSpan * (t + 1.0f));
-        const float e = eps[i];
-        const float th = tanhf(mean[i] + e * sd);
-        const float ma = max_action[a];
-        const float act = th * ma;
-        const float dact = ma * (1.0f - th * th);                      // d action / d u
-        const float ga = grad_action ? grad_action[i] : 0.0f;
-        // d/du of -log(1 - action^2 + 1e-6) is 2 action dact / (1 - action^2 + 1e-6)
-        const float gu = ga * dact + glp * (2.0f * act * dact) / (1.0f - act * act + kReparamNoise);
-        grad_mean[i] = gu;
-        grad_raw_std[i] = gu * e * sd * dls - glp * dls;              // through std (u) and through -log_std
+        gaussian_head_bwd(mean[i], raw_std[i], eps[i], max_action[a], grad_action ? grad_action[i] : 0.0f, glp,
+                          grad_mean[i], grad_raw_std[i]);
     }
 }
 
@@ -131,9 +108,9 @@ __global__ void __launch_bounds__(kAdamThreads) adam_polyak_kernel(const __grid_
         }
         s_slot = k;
         s_first = chunk * kAdamChunk;
-        const double t = (double)(*reinterpret_cast<volatile long long *>(state) + 1);  // this step's number
-        s_bc1 = (float)(1.0 - pow((double)tab.beta1, t));
-        s_bc2_sqrt = (float)sqrt(1.0 - pow((double)tab.beta2, t));
+        // this step's number
+        boatenv::adam_bias_corrections(*reinterpret_cast<volatile long long *>(state) + 1, tab.beta1, tab.beta2, s_bc1,
+                                       s_bc2_sqrt);
     }
     __syncthreads();
     if (s_slot < tab.n_slots) {
@@ -141,15 +118,7 @@ __global__ void __launch_bounds__(kAdamThreads) adam_polyak_kernel(const __grid_
         const float step_size = sl.lr / s_bc1;
         const long long end = min(s_first + (long long)kAdamChunk, (long long)sl.numel);
         for (long long i = s_first + threadIdx.x; i < end; i += kAdamThreads) {
-            const float g = sl.grad[i];
-            const float m = sl.exp_avg[i] + (g - sl.exp_avg[i]) * (1.0f - tab.beta1);   // lerp_(grad, 1 - beta1)
-            const float v = sl.exp_avg_sq[i] * tab.beta2 + (1.0f - tab.beta2) * g * g;  // mul_(beta2).addcmul_(g, g, 1 - beta2)
-            const float denom = sqrtf(v) / s_bc2_sqrt + tab.eps;
-            const float p = sl.param[i] - step_size * (m / denom);                       // addcdiv_(m, denom, -step_size)
-            sl.exp_avg[i] = m;
-            sl.exp_avg_sq[i] = v;
-            sl.param[i] = p;
-            if (sl.target) sl.target[i] = tab.tau * p + (1.0f - tab.tau) * sl.target[i];
+            boatenv::adam_polyak_element(sl, i, sl.grad[i], tab.beta1, tab.beta2, tab.eps, tab.tau, step_size, s_bc2_sqrt);
         }
     }
     __syncthreads();
