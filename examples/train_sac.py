@@ -19,9 +19,13 @@ recorded run of the reference's own learn() in tests/test_agent_golden.py.
     torchrun --nproc-per-node 8 examples/train_sac.py --envs 65536        # replicas: one agent per GPU shard
     torchrun --nproc-per-node 8 examples/train_sac.py --experiments-root experiments --tune
                                           # the reference's `main.py -p 8`: a tuned_configs.yaml draw per member
+    torchrun --nproc-per-node 8 examples/train_sac.py --envs 65536 --data-parallel
+                                          # ONE agent over all ranks: every update averages 8 batches' gradients
 
-Multi-GPU is "replicas only" (SURVEY.md 8e): every rank trains its own agent on its own env shard,
+By default multi-GPU is "replicas only" (SURVEY.md 8e): every rank trains its own agent on its own env shard,
 like the reference's `-p` mode runs independent models; only the episode statistics are all-reduced.
+`--data-parallel` trains one agent instead: each rank samples its own ring, one all-reduce per update averages the
+gradients, and rank 0 writes the one experiment directory from the all-reduced episode statistics.
 The last line printed by rank 0 is a JSON summary (device-timed after `--warmup-iters`).
 """
 from __future__ import annotations
@@ -75,6 +79,10 @@ def main(argv=None):
                          "auto-reset and replay store; ContinuousAgent.collect), then --updates-per-iter updates; "
                          "needs --policy-precision tcgen05.  0: one env step per iteration, policy and step launched "
                          "separately")
+    ap.add_argument("--data-parallel", action="store_true",
+                    help="train ONE agent over all ranks (ContinuousAgent(data_parallel=True)): every update all-reduces "
+                         "the gradients of the ranks' batches, an effective batch of world x batch_size; --envs must "
+                         "divide evenly over the ranks")
     args = ap.parse_args(argv)
     if args.record_envs and not args.experiments_root:
         ap.error("--record-envs requires --experiments-root")
@@ -89,9 +97,18 @@ def main(argv=None):
             ap.error("--collect-steps and --record-envs cannot be combined (the fused kernel records no steps)")
 
     rank, local_rank, world = S.sharding.dist_info()
+    if args.data_parallel:   # checked before any CUDA work
+        for flag, on in (("--tune", args.tune), ("--pbt-every", args.pbt_every), ("--overlap", args.overlap)):
+            if on:
+                ap.error(f"--data-parallel and {flag} cannot be combined")
+        if args.envs % world:
+            ap.error(f"--data-parallel needs --envs divisible by the world size ({args.envs} envs, {world} ranks)")
     torch.cuda.set_device(local_rank)
     if world > 1:
         torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    elif args.data_parallel:   # a one-rank group: the agent all-reduces as it would over several
+        torch.distributed.init_process_group("nccl", store=torch.distributed.HashStore(), rank=0, world_size=1,
+                                             device_id=torch.device("cuda", local_rank))
     torch.manual_seed(args.seed + rank)
     overrides = {}
     for item in args.set:
@@ -99,7 +116,7 @@ def main(argv=None):
         overrides[k] = float(v) if any(ch in v for ch in ".e") else int(v)
     cfg = S.load_config(base_settings__experiment=args.experiment, **overrides)
     exp = None
-    if args.experiments_root:   # utils/build_experiment.py: one experiment directory per population member
+    if args.experiments_root and not (args.data_parallel and rank > 0):   # data-parallel: rank 0's directory only   # utils/build_experiment.py: one experiment directory per population member
         import random
         exp = S.Experiment(experiment_name=f"experiment_r{rank}", subdir=f"setting_{args.experiment}",
                            root=args.experiments_root, rng=random.Random(args.seed + rank))
@@ -112,11 +129,11 @@ def main(argv=None):
     agent = S.ContinuousAgent(cfg, exp.experiment_dir if exp else None, env.observation_space.shape, env,
                               device=local_rank, seed=args.seed + rank,
                               use_cuda_graph=not args.no_graph, memory=mem, policy_precision=args.policy_precision,
-                              learner_precision=args.learner_precision)
+                              learner_precision=args.learner_precision, data_parallel=args.data_parallel or None)
     act = agent.choose_action if args.no_graph else agent.choose_action_graphed
     obs = env.reset()
     rec = None
-    if args.record_envs:   # main.py:79: a recorder row every step; the ring holds a log interval (+ the first row)
+    if args.record_envs and exp:   # main.py:79: a recorder row every step; the ring holds a log interval (+ the first row)
         k = min(args.record_envs, env.n_envs)
         rec = S.DeviceRecorder(env, range(env.env_id_offset, env.env_id_offset + k), exp.experiment_dir,
                                capacity=max(1024, args.log_every + 1))
@@ -164,9 +181,12 @@ def main(argv=None):
             pipe.sync()   # counters, losses and checkpoints below run on the default stream: order it after the pipeline
         if rec and args.log_every and it % args.log_every == 0:
             rec.flush()
+        if args.data_parallel and args.experiments_root and args.log_every and it % args.log_every == 0:
+            c = S.all_reduce_counters(env.counters_tensor())   # collective: the one agent's episodes on every rank
         if exp and args.log_every and it % args.log_every == 0:
             # one console.csv row per logging interval: the mean return of the episodes that ended in it
-            c = env.counters()
+            if not args.data_parallel:
+                c = env.counters()
             n = c["episodes"] - prev["episodes"]
             score = (c["return_sum"] - prev["return_sum"]) / n if n else float("nan")
             prev = c
@@ -189,9 +209,11 @@ def main(argv=None):
     if world > 1:
         torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
     stats = S.all_reduce_counters(env.counters_tensor())
-    if rec:
-        rec.close()
-        recorded = torch.tensor([len(rec.ids), rec.episodes_finished], dtype=torch.float64, device="cuda")
+    if args.record_envs:
+        recorded = torch.zeros(2, dtype=torch.float64, device="cuda")
+        if rec:
+            rec.close()
+            recorded += torch.tensor([len(rec.ids), rec.episodes_finished], dtype=torch.float64, device="cuda")
         if world > 1:
             torch.distributed.all_reduce(recorded)
     sec = float(ms.item()) * 1e-3
@@ -205,28 +227,30 @@ def main(argv=None):
                "ms_per_iter": 1e3 * sec / args.iters, "episodes": stats["episodes"],
                "mean_return": stats["return_mean"], "reached_goal": stats["reached_goal"],
                "losses_v_pi_q": [float(x) for x in losses] if losses is not None else None}
-    if rec:   # over all ranks: envs recorded, and their episodes that ended (one info.csv row each)
+    if args.data_parallel:
+        summary["data_parallel"], summary["effective_batch"] = True, world * agent.batch_size
+    if args.record_envs:   # over all ranks: envs recorded, and their episodes that ended (one info.csv row each)
         summary["recorded_envs"], summary["recorded_episodes"] = int(recorded[0]), int(recorded[1])
     if args.pbt_every:
         summary["pbt_rounds"] = len(pbt_log)
         summary["pbt_adoptions_rank0"] = [e for e in pbt_log if e["adopted_from"] is not None]
         summary["hyperparameters_rank0"] = agent.hyperparameters()
     if exp:
-        c = env.counters()
+        c = stats if args.data_parallel else env.counters()
         exp.write_console(rows)
         exp.append_overview(best)
         exp.write_terminations(S.info_from_counters(c, max(S.TERM_NAMES[1:], key=lambda k: c[k])))
         summary["experiment_dir"], summary["best_interval_return"] = exp.experiment_dir, best
         if args.tune:
             summary["hpset"] = exp.tuner.hpset
-        if world > 1:   # the population's best member, like reading overview.csv after a `-p` run
+        if world > 1 and not args.data_parallel:   # the population's best member, like reading overview.csv after a `-p` run
             scores = [None] * world
             torch.distributed.all_gather_object(scores, (best, rank, exp.experiment_name))
             summary["population_best"] = max(scores)
     if rank == 0:
         print(json.dumps(summary), flush=True)
     env.close(); mem.close()
-    if world > 1:
+    if world > 1 or args.data_parallel:
         torch.distributed.destroy_process_group()
     return summary
 

@@ -405,6 +405,20 @@ BOATENV_API int boatagent_sac_update(const float *state, const float *action, co
                                      const boatagent_adam_slot *slots_host, int32_t n_slots, float beta1,
                                      float beta2, float adam_eps, float tau, int64_t *adam_state, float *losses_out,
                                      void *workspace, int64_t workspace_bytes, void *stream);
+/* The gradients of boatagent_sac_update without its optimiser step, for data-parallel training: every replica
+ * computes the gradients of its own batch, the replicas all-reduce them, and each applies the same Adam step.
+ * Arguments and errors as boatagent_sac_update's, without the Adam hyper-parameters and state.  Each slot's `grad`
+ * receives grad_scale times the batch gradient and losses_out grad_scale times the three losses; parameters, targets,
+ * Adam moments and step counter are only read (the moments not at all).  grad_scale = 1 / world makes a SUM
+ * all-reduce the mean, exactly when world is a power of two.
+ * With grad_scale = 1, this call followed by boatagent_adam_polyak_step on the same slots (and the same adam_state)
+ * equals one boatagent_sac_update bit for bit: gradients, weights, targets, Adam moments, step counter and losses.
+ * The split costs one extra launch (the Adam kernel). */
+BOATENV_API int boatagent_sac_gradients(const float *state, const float *action, const float *reward,
+                                        const float *new_state, const uint8_t *done, const float *eps,
+                                        const float *max_action, int64_t batch, float gamma, float reward_scale,
+                                        const boatagent_adam_slot *slots_host, int32_t n_slots, float grad_scale,
+                                        float *losses_out, void *workspace, int64_t workspace_bytes, void *stream);
 
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 

@@ -73,6 +73,8 @@ SIGNATURES = {
     "boatagent_sac_update_workspace_bytes": (i64, [i64]),
     "boatagent_sac_update": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, i64, C.c_float, C.c_float, vp, i32, C.c_float,
                                        C.c_float, C.c_float, C.c_float, vp, vp, vp, i64, vp]),
+    "boatagent_sac_gradients": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, i64, C.c_float, C.c_float, vp, i32, C.c_float,
+                                          vp, vp, i64, vp]),
     "boatreplay_create": (C.c_int, [i64, i32, i32, C.c_int, C.c_int, C.POINTER(vp)]),
     "boatreplay_destroy": (C.c_int, [vp]),
     "boatreplay_store": (C.c_int, [vp, i64, vp, vp, vp, vp, vp, vp]),

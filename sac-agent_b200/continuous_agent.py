@@ -13,6 +13,8 @@ the data lives and how the update is driven:
   fused Adam + Polyak kernel for all networks (`DeviceAdam`) are captured once and replayed (about a
   hundred small kernels whose launch latency otherwise dominates a 1024 x 256 update); batch and
   Gaussian draws are static inputs of the graph;
+* with `data_parallel`, the ranks of a process group train ONE agent: each samples its own ring and computes the
+  gradients of its own batch, one all-reduce averages them, and every rank applies the same Adam step;
 * `choose_action` takes the [N, 11] observation tensor of a BatchedBoatEnv and returns [N, 1]
   actions without leaving the GPU (the reference syncs one action per env step through
   `.cpu().numpy()`, continuous_agent.py:61); a numpy observation of one env still works and
@@ -147,6 +149,29 @@ class SACLearner:
         """One update on a batch (state [B, obs], action [B, n_actions], reward [B], new_state [B, obs],
         done [B] bool).  eps_*: optional standard-normal draws for the two `sample_normal` calls.
         Returns (value_loss, actor_loss, critic_loss) as 0-d tensors."""
+        losses, grads_v, grads_a, grads_c = self._losses_and_grads(state, action, reward, new_state, done, eps_sample,
+                                                                   eps_rsample)
+        for p, g in zip(self._value_params + self._actor_params + self._critic_params, grads_v + grads_a + grads_c):
+            p.grad = g
+        if isinstance(self.optimizer, DeviceAdam):   # Adam for all four networks + update_network_parameters (:154)
+            self.optimizer.step(grads_a + grads_c + grads_v)
+        else:
+            self.optimizer.step()
+            self.update_network_parameters()                                    # :154
+        return losses
+
+    def gradients(self, state, action, reward, new_state, done, eps_sample, eps_rsample, out, scale=1.0):
+        """`update` without the optimiser step: writes `scale` times the batch gradients into `out[:-3]` (one tensor
+        per parameter in DeviceAdam's order: actor, critic 1, critic 2, value) and `scale` times the three losses
+        into `out[-3:]` (0-d tensors).  Leaves weights, optimiser state and `.grad` bindings alone."""
+        losses, grads_v, grads_a, grads_c = self._losses_and_grads(state, action, reward, new_state, done, eps_sample,
+                                                                   eps_rsample)
+        torch._foreach_copy_(out, list(grads_a + grads_c + grads_v) + list(losses))
+        if scale != 1.0:
+            torch._foreach_mul_(out, scale)
+
+    def _losses_and_grads(self, state, action, reward, new_state, done, eps_sample, eps_rsample):
+        """The three losses (detached) and the gradients of the value, actor and critic parameters."""
         with torch.no_grad():
             value_ = self.target_value(new_state).view(-1)
             value_ = torch.where(done, torch.zeros_like(value_), value_)        # value_[done] = 0.0   (:111)
@@ -171,22 +196,25 @@ class SACLearner:
         q2_old = self.critic_2(state, action).view(-1)
         critic_loss = 0.5 * F.mse_loss(q1_old, q_hat) + 0.5 * F.mse_loss(q2_old, q_hat)
         grads_c = torch.autograd.grad(critic_loss, self._critic_params)
+        return (value_loss.detach(), actor_loss.detach(), critic_loss.detach()), grads_v, grads_a, grads_c
 
-        for p, g in zip(self._value_params + self._actor_params + self._critic_params, grads_v + grads_a + grads_c):
-            p.grad = g
-        if isinstance(self.optimizer, DeviceAdam):   # Adam for all four networks + update_network_parameters (:154)
-            self.optimizer.step(grads_a + grads_c + grads_v)
-        else:
-            self.optimizer.step()
-            self.update_network_parameters()                                    # :154
-        return value_loss.detach(), actor_loss.detach(), critic_loss.detach()
+
+class DataParallelState(list):
+    """`training_tensors()` of a data-parallel agent: ONE agent's state, held equal by every rank of its group, so
+    population rounds (population.exploit_explore) must not hand it between ranks."""
 
 
 class ContinuousAgent:
-    """agent/continuous_agent.py:9-154 on the GPU-resident env and replay ring."""
+    """agent/continuous_agent.py:9-154 on the GPU-resident env and replay ring.
+
+    data_parallel: a torch.distributed process group (True: the default group) whose ranks train this one agent.  Each
+    rank keeps its own env shard, ring, sampler seed and Gaussian draws; every update averages the ranks' gradients and
+    losses with one all-reduce and applies the same Adam step everywhere, so the weights stay bit-identical without
+    being re-broadcast.  Rank 0's weights and optimiser state are broadcast at construction.  Every rank must hold the
+    same number of envs (`learn()` updates on all ranks or on none without a vote)."""
 
     def __init__(self, config, experiment_dir, input_dims, env, device=None, seed=0, use_cuda_graph=True,
-                 memory=None, policy_precision="fp32", learner_precision="fp32"):
+                 memory=None, policy_precision="fp32", learner_precision="fp32", data_parallel=None):
         if not torch.cuda.is_available():
             raise RuntimeError("sac_agent_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.env = env
@@ -233,6 +261,9 @@ class ContinuousAgent:
         self.updates = 0
         if learner_precision == "tcgen05":
             self._init_fused_learner()
+        self._dp = None   # (group, flat gradient + loss buffer, its gradient views, grad_scale) in data-parallel mode
+        if data_parallel is not None and data_parallel is not False:
+            self._init_data_parallel(None if data_parallel is True else data_parallel)
 
     # -- base_agent.py:7-19 -------------------------------------------------------------
     def get_n_actions(self):
@@ -374,8 +405,92 @@ class ContinuousAgent:
                 self._ws.data_ptr(), self._ws.numel(), stream), "boatagent_sac_update")
         return self._losses
 
-    def _run_update(self):
+    def _init_data_parallel(self, group):
+        import torch.distributed as dist
+        if not (dist.is_available() and dist.is_initialized()):
+            raise ValueError("data_parallel needs an initialised torch.distributed process group")
+        world = dist.get_world_size(group)
+        n = torch.tensor([getattr(self.env, "n_envs", 1)] * 2, dtype=torch.int64, device=self.device)
+        n[1].neg_()
+        dist.all_reduce(n, op=dist.ReduceOp.MAX, group=group)
+        if int(n[0]) != -int(n[1]):
+            raise ValueError(f"data_parallel: every rank needs the same number of envs (they hold {-int(n[1])} to "
+                             f"{int(n[0])}); make the total divisible by the world size {world}")
+        o = self.learner.optimizer
+        # every trained parameter's .grad is a view into one flat buffer, followed by the three losses: ONE all-reduce
+        flat = torch.zeros(sum(p.numel() for p in o.params) + 3, dtype=torch.float32, device=self.device)
+        grads, off = [], 0
+        for p in o.params:
+            p.grad = flat[off:off + p.numel()].view_as(p)
+            grads.append(p.grad)
+            off += p.numel()
+        self._losses = tuple(flat[off + k] for k in range(3))
+        # grad_scale 1 / world: the SUM all-reduce is the mean (exact for power-of-two world sizes)
+        self._dp = (group, flat, grads, 1.0 / world)
+        src = 0 if group is None else dist.get_global_rank(group, 0)
+        for t in self.training_tensors():   # the ranks start from rank 0's agent
+            dist.broadcast(t, src=src, group=group)
+        self._weights_changed()
+
+    @property
+    def data_parallel(self):
+        """True when this agent is trained by a process group (constructor argument `data_parallel`)."""
+        return self._dp is not None
+
+    def _dp_gradients_static(self):
+        s, a, r, s2, d = self._batch
+        _, flat, grads, scale = self._dp
+        self.learner.gradients(s, a, r, s2, d.bool(), self._eps[0], self._eps[1], grads + list(self._losses), scale)
+
+    def _dp_update(self):
+        """gradients (scaled by 1 / world) -> all-reduce of gradients and losses -> Adam + Polyak on every rank."""
+        import torch.distributed as dist
+        group, flat, grads, scale = self._dp
+        L, o = self.learner, self.learner.optimizer
         if self.learner_precision == "tcgen05":
+            for k, g in enumerate(grads):
+                o._slots[k].grad = g.data_ptr()
+            s, a, r, s2, d = self._batch
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            with torch.cuda.device(self.device):
+                o._lib.check(o._L.boatagent_sac_gradients(
+                    s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), self._eps.data_ptr(),
+                    L.actor.max_action.data_ptr(), self.batch_size, float(L.gamma), float(L.scale), o._slots,
+                    len(o.params), scale, self._losses[0].data_ptr(), self._ws.data_ptr(), self._ws.numel(), stream),
+                    "boatagent_sac_gradients")
+        elif not self.use_cuda_graph:
+            self._dp_gradients_static()
+        else:
+            if self._graph is None:
+                self._capture_dp()
+            self._graph[0].replay()
+        dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)   # eager, between the graphs (NCCL and gloo)
+        if self.learner_precision == "fp32" and self.use_cuda_graph:
+            self._graph[1].replay()
+        else:
+            o.step(grads)
+
+    def _capture_dp(self):
+        """Capture the data-parallel update as two graphs around the all-reduce: A = forward and backward passes into
+        the flat buffer, B = DeviceAdam's step.  A writes nothing but the buffer, so its warm-up runs need no undo."""
+        cur = torch.cuda.current_stream(self.device)
+        side = torch.cuda.Stream(self.device)
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            for _ in range(3):
+                self._dp_gradients_static()
+        cur.wait_stream(side)
+        ga, gb = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
+        with torch.cuda.graph(ga, stream=self.capture_stream):
+            self._dp_gradients_static()
+        with torch.cuda.graph(gb, stream=self.capture_stream):
+            self.learner.optimizer.step(self._dp[2])
+        self._graph = (ga, gb)
+
+    def _run_update(self):
+        if self._dp is not None:
+            self._dp_update()
+        elif self.learner_precision == "tcgen05":
             self._fused_update()
         elif not self.use_cuda_graph:
             self._losses = self._update_static()
@@ -475,7 +590,8 @@ class ContinuousAgent:
     def training_tensors(self):
         """Weights of the five networks + Adam moments and step counter: what a population member hands over."""
         L = self.learner
-        return [p.data for net in L.networks() for p in net.parameters()] + L.optimizer.state_tensors()
+        tensors = [p.data for net in L.networks() for p in net.parameters()] + L.optimizer.state_tensors()
+        return DataParallelState(tensors) if self._dp is not None else tensors
 
     def _weights_changed(self):
         if self._tc_policy is not None:
@@ -548,6 +664,8 @@ class OverlappedActorLearner:
     """
 
     def __init__(self, agent: ContinuousAgent, env, done_flag_mode=1, recorder=None):
+        if agent.data_parallel:
+            raise ValueError("OverlappedActorLearner: a data-parallel agent is not supported")
         self.agent, self.env, self.done_flag_mode = agent, env, int(done_flag_mode)
         self.recorder = recorder   # a DeviceRecorder: captures every step on the env stream
         dev = agent.device

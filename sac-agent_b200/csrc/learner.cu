@@ -8,7 +8,10 @@
 //                     inputs and output gradients) and the tile's loss sums to the workspace.
 //   sac_params_kernel reduces the gradients over the batch in a fixed order (tcgen05 for the four fc2 weights, one
 //                     warp per hidden unit for the rest), writes them to the parameters' .grad tensors, applies Adam
-//                     and the Polyak average (agent_math.cuh, as adam_polyak_kernel) and sums the loss partials.
+//                     and the Polyak average (agent_math.cuh, as adam_polyak_kernel) and sums the loss partials.  Its
+//                     gradients-only instantiation (boatagent_sac_gradients) writes the gradients and the losses times
+//                     grad_scale and leaves the parameters and the optimiser state alone, so that the gradients of
+//                     several replicas can be all-reduced before one Adam step.
 //
 // Operands in shared memory and in the workspace use the 8x8 core-matrix layout of actor_tc.cuh: element (r, c) of
 // an R-row matrix at (c / 8) * (R * 16) + r * 16 + (c % 8) * 2.  The same bytes are a K-major operand with rows = M/N
@@ -87,6 +90,7 @@ struct ParamArgs {
     const unsigned char *ws;
     long long *state;   // [steps taken, ticket]
     float *losses;
+    float grad_scale;   // gradients-only instantiation: factor on the written gradients and losses
 };
 
 __device__ __forceinline__ uint32_t core_off(int r, int c, int rows) { return (uint32_t)((c >> 3) * (rows * 16) + r * 16 + (c & 7) * 2); }
@@ -418,20 +422,28 @@ __global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_con
 // slot of tensor `t` (0 w1, 1 b1, 2 w2, 3 b2, 4 / 6 head weights, 5 / 7 head biases) of trained network `n`
 __device__ __forceinline__ int slot_of(int n, int t) { return n == 0 ? t : 8 + 6 * (n - 1) + t; }
 
+// kAdam: write the gradients, apply Adam + Polyak and count the step; else write grad_scale times the gradients only
+template <bool kAdam>
 __global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_constant__ ParamArgs args) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
     __shared__ float s_bc1, s_bc2_sqrt;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const long long B = args.batch, tiles = B / kRows;
-    if (tid == 0) adam_bias_corrections(*reinterpret_cast<volatile long long *>(args.state) + 1, args.beta1, args.beta2,
-                                        s_bc1, s_bc2_sqrt);
-    __syncthreads();
+    if constexpr (kAdam) {
+        if (tid == 0) adam_bias_corrections(*reinterpret_cast<volatile long long *>(args.state) + 1, args.beta1,
+                                            args.beta2, s_bc1, s_bc2_sqrt);
+        __syncthreads();
+    }
     const float bc2_sqrt = s_bc2_sqrt;
     auto adam = [&](int k, long long i, float g) {
         const boatagent_adam_slot &sl = args.slot[k];
-        const_cast<float *>(sl.grad)[i] = g;
-        adam_polyak_element(sl, i, g, args.beta1, args.beta2, args.eps, args.tau, sl.lr / s_bc1, bc2_sqrt);
+        if constexpr (kAdam) {
+            const_cast<float *>(sl.grad)[i] = g;
+            adam_polyak_element(sl, i, g, args.beta1, args.beta2, args.eps, args.tau, sl.lr / s_bc1, bc2_sqrt);
+        } else {
+            const_cast<float *>(sl.grad)[i] = g * args.grad_scale;
+        }
     };
     const int blk = blockIdx.x;
     if (blk < 2 * kNets) {
@@ -538,17 +550,25 @@ __global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_cons
         for (long long t = 0; t < tiles; ++t)
             for (int q = 0; q < 4; ++q) s[q] += p[t * kWsLoss + q];
         const float invB = 1.0f / (float)B;
-        args.losses[0] = 0.5f * (s[0] * invB);
-        args.losses[1] = s[1] * invB;
-        args.losses[2] = 0.5f * (s[2] * invB) + 0.5f * (s[3] * invB);
+        if constexpr (kAdam) {
+            args.losses[0] = 0.5f * (s[0] * invB);
+            args.losses[1] = s[1] * invB;
+            args.losses[2] = 0.5f * (s[2] * invB) + 0.5f * (s[3] * invB);
+        } else {
+            args.losses[0] = (0.5f * (s[0] * invB)) * args.grad_scale;
+            args.losses[1] = (s[1] * invB) * args.grad_scale;
+            args.losses[2] = (0.5f * (s[2] * invB) + 0.5f * (s[3] * invB)) * args.grad_scale;
+        }
     }
-    __syncthreads();
-    if (tid == 0) {   // the last CTA to finish publishes the new step count
-        __threadfence();
-        const unsigned long long done = atomicAdd(reinterpret_cast<unsigned long long *>(args.state + 1), 1ULL) + 1ULL;
-        if (done == gridDim.x) {
-            args.state[1] = 0;
-            args.state[0] += 1;
+    if constexpr (kAdam) {
+        __syncthreads();
+        if (tid == 0) {   // the last CTA to finish publishes the new step count
+            __threadfence();
+            const unsigned long long done = atomicAdd(reinterpret_cast<unsigned long long *>(args.state + 1), 1ULL) + 1ULL;
+            if (done == gridDim.x) {
+                args.state[1] = 0;
+                args.state[0] += 1;
+            }
         }
     }
 }
@@ -572,19 +592,19 @@ extern "C" int64_t boatagent_sac_update_workspace_bytes(int64_t batch) {
     return (int64_t)ws_bytes(batch / kRows);
 }
 
-extern "C" int boatagent_sac_update(const float *state, const float *action, const float *reward, const float *new_state,
-                                    const uint8_t *done, const float *eps, const float *max_action, int64_t batch,
-                                    float gamma, float reward_scale, const boatagent_adam_slot *slots_host,
-                                    int32_t n_slots, float beta1, float beta2, float adam_eps, float tau,
-                                    int64_t *adam_state, float *losses_out, void *workspace, int64_t workspace_bytes,
-                                    void *stream) {
-    if (!state || !action || !reward || !new_state || !done || !eps || !max_action || !slots_host || !adam_state ||
-        !losses_out || !workspace)
+namespace {
+
+// The arguments of both kernels from the ABI's (checks as documented in boatenv.h); pa's optimiser fields stay unset.
+int sac_args(const float *state, const float *action, const float *reward, const float *new_state, const uint8_t *done,
+             const float *eps, const float *max_action, int64_t batch, float gamma, float reward_scale,
+             const boatagent_adam_slot *slots_host, int32_t n_slots, float *losses_out, void *workspace,
+             int64_t workspace_bytes, RowArgs &ra, ParamArgs &pa) {
+    if (!state || !action || !reward || !new_state || !done || !eps || !max_action || !slots_host || !losses_out ||
+        !workspace)
         return BOATENV_EINVAL;
     if (batch <= 0 || batch % kRows != 0 || n_slots != kSlots) return BOATENV_EINVAL;
     if (workspace_bytes < (int64_t)ws_bytes(batch / kRows)) return BOATENV_EINVAL;
     if ((reinterpret_cast<uintptr_t>(workspace) & 15u) != 0) return BOATENV_EALIGN;
-    ParamArgs pa;
     for (int k = 0; k < kSlots; ++k) {
         const boatagent_adam_slot &s = slots_host[k];
         if (!s.param || !s.grad || !s.exp_avg || !s.exp_avg_sq || s.numel != expected_numel(k)) return BOATENV_EINVAL;
@@ -592,16 +612,10 @@ extern "C" int boatagent_sac_update(const float *state, const float *action, con
         if ((reinterpret_cast<uintptr_t>(s.param) & 15u) != 0) return BOATENV_EALIGN;
         pa.slot[k] = s;
     }
-    pa.beta1 = beta1;
-    pa.beta2 = beta2;
-    pa.eps = adam_eps;
-    pa.tau = tau;
     pa.batch = batch;
     pa.ws = (const unsigned char *)workspace;
-    pa.state = (long long *)adam_state;
     pa.losses = losses_out;
 
-    RowArgs ra;
     ra.state = state;
     ra.action = action;
     ra.reward = reward;
@@ -629,7 +643,11 @@ extern "C" int boatagent_sac_update(const float *state, const float *action, con
     ra.net[2] = net(14, kObs + 1, false, false);
     ra.net[3] = net(20, kObs, false, false);
     ra.net[4] = net(20, kObs, false, true);
+    return 0;
+}
 
+template <bool kAdam>
+int sac_launch(const RowArgs &ra, const ParamArgs &pa, void *stream) {
     static std::mutex mu;
     static bool set_of[64] = {false};
     int dev = 0;
@@ -639,14 +657,54 @@ extern "C" int boatagent_sac_update(const float *state, const float *action, con
         std::lock_guard<std::mutex> lock(mu);
         if (!set_of[dev]) {
             CUDA_TRY(cudaFuncSetAttribute(sac_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
-            CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+            CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+            CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
             set_of[dev] = true;
         }
     }
-    sac_rows_kernel<<<(unsigned)(batch / kRows), kLThreads, kLSmem, (cudaStream_t)stream>>>(ra);
+    sac_rows_kernel<<<(unsigned)(ra.batch / kRows), kLThreads, kLSmem, (cudaStream_t)stream>>>(ra);
     boatenv::count_launch();
     CUDA_TRY(cudaGetLastError());
-    sac_params_kernel<<<kParamBlocks, kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+    sac_params_kernel<kAdam><<<kParamBlocks, kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
     boatenv::count_launch();
     return (int)cudaGetLastError();
+}
+
+}  // namespace
+
+extern "C" int boatagent_sac_update(const float *state, const float *action, const float *reward, const float *new_state,
+                                    const uint8_t *done, const float *eps, const float *max_action, int64_t batch,
+                                    float gamma, float reward_scale, const boatagent_adam_slot *slots_host,
+                                    int32_t n_slots, float beta1, float beta2, float adam_eps, float tau,
+                                    int64_t *adam_state, float *losses_out, void *workspace, int64_t workspace_bytes,
+                                    void *stream) {
+    if (!adam_state) return BOATENV_EINVAL;
+    RowArgs ra;
+    ParamArgs pa;
+    const int rc = sac_args(state, action, reward, new_state, done, eps, max_action, batch, gamma, reward_scale,
+                            slots_host, n_slots, losses_out, workspace, workspace_bytes, ra, pa);
+    if (rc != 0) return rc;
+    pa.beta1 = beta1;
+    pa.beta2 = beta2;
+    pa.eps = adam_eps;
+    pa.tau = tau;
+    pa.state = (long long *)adam_state;
+    pa.grad_scale = 1.0f;
+    return sac_launch<true>(ra, pa, stream);
+}
+
+extern "C" int boatagent_sac_gradients(const float *state, const float *action, const float *reward,
+                                       const float *new_state, const uint8_t *done, const float *eps,
+                                       const float *max_action, int64_t batch, float gamma, float reward_scale,
+                                       const boatagent_adam_slot *slots_host, int32_t n_slots, float grad_scale,
+                                       float *losses_out, void *workspace, int64_t workspace_bytes, void *stream) {
+    RowArgs ra;
+    ParamArgs pa;
+    const int rc = sac_args(state, action, reward, new_state, done, eps, max_action, batch, gamma, reward_scale,
+                            slots_host, n_slots, losses_out, workspace, workspace_bytes, ra, pa);
+    if (rc != 0) return rc;
+    pa.beta1 = pa.beta2 = pa.eps = pa.tau = 0.f;
+    pa.state = nullptr;
+    pa.grad_scale = grad_scale;
+    return sac_launch<false>(ra, pa, stream);
 }

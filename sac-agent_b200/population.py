@@ -43,6 +43,10 @@ def exploit_explore(tensors, hp: dict, score: float, rng: random.Random, bottom_
     member adopts.  Collective: every member of ``group`` must call it."""
     import torch
     import torch.distributed as dist
+    from .continuous_agent import DataParallelState
+    if isinstance(tensors, DataParallelState):
+        raise ValueError("exploit_explore: these are the tensors of a data-parallel agent, one agent shared by its "
+                         "ranks; population rounds need one agent per member")
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) < 2:
         return dict(hp), {"adopted_from": None, "ranking": [0], "scores": [score]}
     world, rank = dist.get_world_size(group), dist.get_rank(group)
