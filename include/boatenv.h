@@ -379,6 +379,23 @@ BOATENV_API int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weigh
                                   float *obs_inout, float *reward_out, uint8_t *done_out, uint8_t *term_out,
                                   void *stream);
 
+/* boatagent_collect that also records selected envs (the Recorder of main.py:79, postprocessing/recorder.py:18-56)
+ * inside the kernel: after step t (and after its auto-reset), the recorder row of every env in `ids` goes to row
+ * (row + t) % ring->capacity of `ring` -- exactly what boatenv_record_rows(h, ids, n_ids, actions, reward, term,
+ * ring, row + t, ...) writes after the t-th round of boatagent_policy_act + boatenv_step_store: the state as
+ * boatenv_get_field returns it (an ended episode's row holds the next episode's first state), the step's action,
+ * reward and term code, and the episode number after the reset.  ids int64[n_ids] (device) are local env ids in any
+ * order and must be unique; an id outside [0, n_envs) is skipped, its entries left as they were.  The ring is fp32
+ * (the handle's precision).  Everything else -- ring rows, write-back, outputs, counters -- is boatagent_collect's.
+ * Errors: those of boatagent_collect, and BOATENV_EINVAL for NULL ids, ring or ring column, n_ids <= 0 or
+ * > 2^31 - 1, capacity <= 0, row < 0, or steps > capacity (one call would overwrite its own rows).  A rejected call
+ * changes nothing. */
+BOATENV_API int boatagent_collect_record(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action,
+                                         uint64_t seed, uint64_t step0, int32_t steps, int done_flag_mode,
+                                         float *obs_inout, float *reward_out, uint8_t *done_out, uint8_t *term_out,
+                                         const int64_t *ids, int64_t n_ids, const boatenv_record_ring *ring,
+                                         int64_t row, void *stream);
+
 /* One SAC-v1 update (SACLearner.update) of the BoatEnv agent -- obs_dim 11, one action, 256-wide layers -- in two
  * tcgen05 kernels: the five networks' forward and backward passes per 128-row tile of the batch, then the gradient
  * reductions, Adam and the Polyak average of the target value network.  The 256 x 256 products (fc2 forward, its

@@ -70,6 +70,8 @@ SIGNATURES = {
     "boatagent_policy_act": (C.c_int, [vp, vp, vp, vp, u64, u64, i64, i32, i32, vp, vp]),
     "boatagent_rollout": (C.c_int, [vp, vp, vp, u64, u64, i32, u32, vp, vp, vp, vp, vp, vp]),
     "boatagent_collect": (C.c_int, [vp, vp, vp, vp, u64, u64, i32, C.c_int, vp, vp, vp, vp, vp]),
+    "boatagent_collect_record": (C.c_int, [vp, vp, vp, vp, u64, u64, i32, C.c_int, vp, vp, vp, vp, vp, i64,
+                                           C.POINTER(RecordRing), i64, vp]),
     "boatagent_sac_update_workspace_bytes": (i64, [i64]),
     "boatagent_sac_update": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, i64, C.c_float, C.c_float, vp, i32, C.c_float,
                                        C.c_float, C.c_float, C.c_float, vp, vp, vp, i64, vp]),

@@ -360,14 +360,16 @@ class ContinuousAgent:
         """main.py:81-88 for every env in one kernel: env.step + remember (ReplayBuffer.step_store)."""
         return self.memory.step_store(env, actions, done_flag_mode=done_flag_mode)
 
-    def collect(self, env, steps, done_flag_mode=1):
+    def collect(self, env, steps, done_flag_mode=1, recorder=None):
         """`steps` rounds of choose_action + step_and_remember over every env in ONE kernel
         (TensorCorePolicy.collect): the same actions, steps, resets and ring rows as that loop with
-        policy_precision "tcgen05", the only precision it serves."""
+        policy_precision "tcgen05", the only precision it serves.  `recorder`: a DeviceRecorder of `env`, which
+        gets the rows a capture() after every round would give, written by the same kernel."""
         if self.policy_precision != "tcgen05":
             raise ValueError(f"collect acts through the tcgen05 policy; this agent acts in {self.policy_precision!r} "
                              "(create it with policy_precision='tcgen05')")
-        return self.tensor_core_policy().collect(env, self.memory, steps, done_flag_mode=done_flag_mode)
+        return self.tensor_core_policy().collect(env, self.memory, steps, done_flag_mode=done_flag_mode,
+                                                 recorder=recorder)
 
     # -- learning -------------------------------------------------------------------------
     def _update_static(self):

@@ -153,13 +153,7 @@ __device__ __forceinline__ double read_field(const DevCfg &c, long long i, int f
 }
 __device__ __forceinline__ double read_field(const DevCfg &c, long long i, int field, float) {
     const float raw = *dyn_scalar<float>(c, i, field);
-    if (field == D_RUDDER) {
-        const long long rud = ((long long)__float_as_int(raw) << kRudLoBits) | (long long)(*index_ptr(c, i) >> kIndexBits);
-        return (double)rud * (1.0 / 4398046511104.0);
-    }
-    if (field == D_SX) return (double)__float_as_int(raw) * (double)c.f.sx_inv;
-    if (field == D_SY) return (double)__float_as_int(raw) * (double)c.f.sy_inv;
-    return (double)raw;
+    return decode_field(c, field, raw, field == D_RUDDER ? *index_ptr(c, i) : 0u);
 }
 __device__ __forceinline__ void write_field(const DevCfg &c, long long i, int field, double v, double) {
     *dyn_scalar<double>(c, i, field) = v;

@@ -273,6 +273,20 @@ template <> struct Fx<float> {
     }
 };
 
+// The plain value of dyn slot `field` of an fp32 env from the bits Fx<float>::pack stores: `raw` the slot, `ixw` the
+// step-index word (read for the rudder only).  The fixed-point carriers (rudder_angle, s_x, s_y) are decoded; the
+// other slots are plain floats.  boatenv_get_field, boatenv_record_rows and the recording collect kernel all read
+// the state through this one decode.
+__device__ __forceinline__ double decode_field(const DevCfg &c, int field, float raw, uint32_t ixw) {
+    if (field == D_RUDDER) {
+        const long long rud = ((long long)__float_as_int(raw) << kRudLoBits) | (long long)(ixw >> kIndexBits);
+        return (double)rud * (1.0 / 4398046511104.0);
+    }
+    if (field == D_SX) return (double)__float_as_int(raw) * (double)c.f.sx_inv;
+    if (field == D_SY) return (double)__float_as_int(raw) * (double)c.f.sy_inv;
+    return (double)raw;
+}
+
 // ---------------------------------------------------------------------------------
 // mbarrier and proxy-fence primitives (sm_90+/sm_100a PTX), shared by the step kernels' TMA pipeline
 // (boat_step.cuh) and the tcgen05 actor pass (actor_tc.cuh)

@@ -61,8 +61,8 @@ cudaError_t launch_env_state_f64(const DevCfg &, long long env, double *out, cud
 cudaError_t launch_wind_table(const DevCfg &, long long env, double *wv, double *wa, cudaStream_t);
 cudaError_t launch_reduce_counters(const double *counters, double *out, cudaStream_t);
 
-// boatagent_collect (replay.cu checks the arguments, rollout.cu holds the kernel): T steps of policy, env step with
-// auto-reset and replay store, fused
+// boatagent_collect / boatagent_collect_record (replay.cu checks the arguments, rollout.cu holds the kernel): T steps
+// of policy, env step with auto-reset and replay store, fused
 struct CollectArgs {
     const unsigned char *blob;
     const float *max_action;
@@ -71,6 +71,13 @@ struct CollectArgs {
     float *obs_inout, *reward_out;
     uint8_t *done_out, *term_out;   // either may be NULL
     ReplayView rp;
+    // recording (boatagent_collect_record only; rec_ids == NULL: plain collection).  Appended, so that the fields
+    // above keep their parameter offsets.  Step t's row goes to row (rec_row0 + t) % rec_ring.capacity, with
+    // 0 <= rec_row0 < capacity and T <= capacity.
+    const long long *rec_ids;
+    int rec_n_ids;
+    boatenv_record_ring rec_ring;
+    long long rec_row0;
 };
 cudaError_t launch_collect(const DevCfg &, const CollectArgs &, cudaStream_t);
 

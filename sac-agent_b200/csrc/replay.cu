@@ -309,9 +309,12 @@ int boatenv_step_store(boatenv_t h, boatreplay_t r, const void *actions, void *o
     return BOATENV_OK;
 }
 
-int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action, uint64_t seed,
-                      uint64_t step0, int32_t steps, int done_flag_mode, float *obs_inout, float *reward_out,
-                      uint8_t *done_out, uint8_t *term_out, void *stream) {
+
+// boatagent_collect, and boatagent_collect_record with rec_ids != NULL (its own arguments checked by the caller)
+static int collect(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action, uint64_t seed,
+                   uint64_t step0, int32_t steps, int done_flag_mode, float *obs_inout, float *reward_out,
+                   uint8_t *done_out, uint8_t *term_out, const int64_t *rec_ids, int64_t rec_n_ids,
+                   const boatenv_record_ring *rec_ring, int64_t rec_row, void *stream) {
     if (!h || !r || !weight_blob || !max_action || !obs_inout || !reward_out || (!done_out && !term_out) || steps < 1 ||
         (done_flag_mode != 0 && done_flag_mode != 1))
         return BOATENV_EINVAL;
@@ -342,9 +345,35 @@ int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weight_blob, cons
     a.rp.mem_size = r->mem_size;
     a.rp.base_slot = r->mem_cntr % r->mem_size;
     a.rp.done_flag_mode = done_flag_mode;
+    if (rec_ids) {
+        a.rec_ids = (const long long *)rec_ids;
+        a.rec_n_ids = (int)rec_n_ids;
+        a.rec_ring = *rec_ring;
+        a.rec_row0 = rec_row % rec_ring->capacity;
+    }
     CUDA_TRY(launch_collect(c, a, (cudaStream_t)stream));
     r->mem_cntr += (long long)steps * c.n_envs;
     return BOATENV_OK;
+}
+
+int boatagent_collect(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action, uint64_t seed,
+                      uint64_t step0, int32_t steps, int done_flag_mode, float *obs_inout, float *reward_out,
+                      uint8_t *done_out, uint8_t *term_out, void *stream) {
+    return collect(h, r, weight_blob, max_action, seed, step0, steps, done_flag_mode, obs_inout, reward_out, done_out,
+                   term_out, nullptr, 0, nullptr, 0, stream);
+}
+
+int boatagent_collect_record(boatenv_t h, boatreplay_t r, const void *weight_blob, const float *max_action,
+                             uint64_t seed, uint64_t step0, int32_t steps, int done_flag_mode, float *obs_inout,
+                             float *reward_out, uint8_t *done_out, uint8_t *term_out, const int64_t *ids,
+                             int64_t n_ids, const boatenv_record_ring *ring, int64_t row, void *stream) {
+    if (!ids || n_ids <= 0 || n_ids > 2147483647LL || !ring || row < 0) return BOATENV_EINVAL;
+    if (!ring->s_x || !ring->s_y || !ring->v_x || !ring->v_y || !ring->s_r || !ring->rudder_angle || !ring->action ||
+        !ring->reward || !ring->term || !ring->episode || ring->capacity <= 0)
+        return BOATENV_EINVAL;
+    if (steps > ring->capacity) return BOATENV_EINVAL;   // one call would overwrite its own rows
+    return collect(h, r, weight_blob, max_action, seed, step0, steps, done_flag_mode, obs_inout, reward_out, done_out,
+                   term_out, ids, n_ids, ring, row, stream);
 }
 
 }  // extern "C"

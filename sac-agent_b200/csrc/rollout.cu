@@ -7,7 +7,9 @@
 //     or max_steps is reached.
 //   * boat_collect_kernel: experience collection (the main.py:78-90 loop body: act, step, remember) over T steps.
 //     Every step writes its transition into the replay ring, and an env whose episode ends is reset in its own lane
-//     as BOATENV_AUTO_RESET does in the step kernel; every tile runs exactly T steps.
+//     as BOATENV_AUTO_RESET does in the step kernel; every tile runs exactly T steps.  Its <WK, true>
+//     instantiations (boatagent_collect_record) also write each step's recorder row of selected envs into a
+//     boatenv_record_ring, as boatenv_record_rows would after every step.
 // Common to both:
 //   * an epilogue group owns a 128-env tile (four 32-env state blocks); warp w % 4 of the group loads block
 //     4 tile + w % 4 into registers once and keeps it there for the whole call;
@@ -166,6 +168,47 @@ __device__ __forceinline__ void tile_env_store(const DevCfg &c, char *gb, int la
     if (episode_dirty) reinterpret_cast<uint32_t *>(gb + c.off_epi)[lane] = s.episode;
 }
 
+// Barrier of the 128 threads of epilogue group g (named barrier 1 + g; the MMA warp never joins it).
+__device__ __forceinline__ void group_sync(int g) { asm volatile("bar.sync %0, 128;" ::"r"(1 + g) : "memory"); }
+
+// The recording ring's column j (ids[j] == env) of each env of the tile whose first env is `first`, -1 for an env
+// that is not recorded.  The group's 128 threads scan the ids together, ceil(n_ids / 128) loads each, into the
+// group's table; ids outside [0, n) match no env.  The first barrier keeps every thread's clearing of its own entry
+// ahead of the others' writes, the second keeps their writes ahead of its read.
+__device__ __forceinline__ int tile_record_column(const CollectArgs &a, int g, int row, long long first, long long n,
+                                                  int *table) {
+    table[row] = -1;
+    group_sync(g);
+    for (int j = row; j < a.rec_n_ids; j += kTileM) {
+        const long long id = __ldg(a.rec_ids + j);
+        if (id >= first && id < first + kTileM && id < n) table[id - first] = j;
+    }
+    group_sync(g);
+    return table[row];
+}
+
+// The recorder row of an env after its step (and its reset, if the episode ended), entry o of the ring: what
+// boatenv_record_rows writes after the per-step step_store.  The state is decoded from the bits Fx<float>::pack
+// would store, as get_field decodes it once the tile is written back; action, reward and termination code are the
+// step's, the episode number is the one after the reset.
+__device__ __forceinline__ void tile_env_record(const DevCfg &c, const boatenv_record_ring &ring, long long o,
+                                                const TileEnv &s, float action, float rew, int code) {
+    float dd[D_COUNT];
+#pragma unroll
+    for (int q = 0; q < D_COUNT; ++q) dd[q] = s.d[q];
+    const uint32_t ixw = s.fx.pack(dd, s.index);
+    static_cast<float *>(ring.s_x)[o] = (float)decode_field(c, D_SX, dd[D_SX], ixw);
+    static_cast<float *>(ring.s_y)[o] = (float)decode_field(c, D_SY, dd[D_SY], ixw);
+    static_cast<float *>(ring.v_x)[o] = (float)decode_field(c, D_VX, dd[D_VX], ixw);
+    static_cast<float *>(ring.v_y)[o] = (float)decode_field(c, D_VY, dd[D_VY], ixw);
+    static_cast<float *>(ring.s_r)[o] = (float)decode_field(c, D_SR, dd[D_SR], ixw);
+    static_cast<float *>(ring.rudder_angle)[o] = (float)decode_field(c, D_RUDDER, dd[D_RUDDER], ixw);
+    static_cast<float *>(ring.action)[o] = action;
+    static_cast<float *>(ring.reward)[o] = rew;
+    ring.term[o] = (uint8_t)code;
+    ring.episode[o] = s.episode;
+}
+
 // New wind coefficients for the lanes of this warp that ask for them (`need`: an episode was reset, or the next
 // sample lies in the next spline piece), for sample s.index of episode s.episode.  Collection resets envs at scattered
 // steps, so requests are sparse: the whole warp serves one env at a time (wind_setup_warp, the step kernel's slow
@@ -276,8 +319,9 @@ boat_rollout_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Ro
 
 // Collection: T steps of every env with auto-reset, each step's transition stored in the replay ring.  Row i of step
 // t goes to slot (base_slot + t N + i) mod mem_size; the host guarantees T N <= mem_size, so no two rows of a call
-// share a slot (tiles advance at different rates).
-template <int WK>
+// share a slot (tiles advance at different rates).  kRecord: every step also writes the recorder row of each
+// recorded env (a.rec_ids) to row (rec_row0 + t) % capacity of a.rec_ring; the host guarantees T <= capacity.
+template <int WK, bool kRecord>
 __global__ void __launch_bounds__(kThreads, 1)
 boat_collect_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ CollectArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -285,6 +329,7 @@ boat_collect_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Co
     __shared__ volatile int group_done[2];
     constexpr bool kCurves = (WK == WIND_VEL_CURVE || WK == WIND_ANGLE_RECT || WK == WIND_BOTH);
     __shared__ double setup_scratch[kCurves ? kEpiThreads / 32 : 1][kScratchDoubles];   // per epilogue warp
+    __shared__ int record_column[kRecord ? 2 : 1][kRecord ? kTileM : 1];                 // per epilogue group
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + kOffBar);
     if (tid < 2) group_done[tid] = 0;
@@ -325,6 +370,12 @@ boat_collect_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Co
             float rew = 0.f;
             long long slot = a.rp.base_slot + env;   // < 2 mem_size: base_slot < mem_size and env < N <= mem_size
             if (slot >= mem_size) slot -= mem_size;
+            int rec_col = -1;                        // the env's column in the recording ring, -1: not recorded
+            long long rec_row = 0;
+            if (kRecord) {
+                rec_col = tile_record_column(a, g, row, tile * kTileM, n, record_column[kRecord ? g : 0]);
+                rec_row = a.rec_row0;
+            }
             for (int t = 0; t < a.steps; ++t) {
                 actor_stage_a0(b, a0, row, s.o);
                 actor_layer1_epilogue(b, (uint32_t)(pass & 1), region, b1);
@@ -358,6 +409,8 @@ boat_collect_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Co
                     } else if (kCurves && next_sample_in_next_piece(c, j, r)) {
                         need_wind = true;
                     }
+                    if (kRecord && rec_col >= 0)
+                        tile_env_record(c, a.rec_ring, rec_row * a.rec_n_ids + rec_col, s, action, rew, code);
                 }
                 if (kCurves) {
                     warp_wind_setups(c, need_wind, env, s, scratch);
@@ -365,6 +418,7 @@ boat_collect_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ Co
                 }
                 slot += n;
                 if (slot >= mem_size) slot -= mem_size;
+                if (kRecord && ++rec_row == a.rec_ring.capacity) rec_row = 0;
             }
             if (active) {
                 tile_env_store<WK>(c, gb, lane, s, wind_dirty, episode_dirty);
@@ -397,15 +451,23 @@ kern_t kernel_for(int wind_kind) {
 
 using collect_kern_t = void (*)(const DevCfg, const CollectArgs);
 
+template <bool kRecord>
 collect_kern_t collect_kernel_for(int wind_kind) {
     switch (wind_kind) {
-    case WIND_NONE: return boat_collect_kernel<WIND_NONE>;
-    case WIND_CONST: return boat_collect_kernel<WIND_CONST>;
-    case WIND_VEL_CURVE: return boat_collect_kernel<WIND_VEL_CURVE>;
-    case WIND_ANGLE_RECT: return boat_collect_kernel<WIND_ANGLE_RECT>;
-    case WIND_BOTH: return boat_collect_kernel<WIND_BOTH>;
+    case WIND_NONE: return boat_collect_kernel<WIND_NONE, kRecord>;
+    case WIND_CONST: return boat_collect_kernel<WIND_CONST, kRecord>;
+    case WIND_VEL_CURVE: return boat_collect_kernel<WIND_VEL_CURVE, kRecord>;
+    case WIND_ANGLE_RECT: return boat_collect_kernel<WIND_ANGLE_RECT, kRecord>;
+    case WIND_BOTH: return boat_collect_kernel<WIND_BOTH, kRecord>;
     default: return nullptr;
     }
+}
+
+template <bool kRecord>
+cudaError_t collect_kernels_setup(int &n_sm) {
+    return actor_kernels_setup<boat_collect_kernel<WIND_NONE, kRecord>, boat_collect_kernel<WIND_CONST, kRecord>,
+                               boat_collect_kernel<WIND_VEL_CURVE, kRecord>, boat_collect_kernel<WIND_ANGLE_RECT, kRecord>,
+                               boat_collect_kernel<WIND_BOTH, kRecord>>(n_sm);
 }
 
 // one CTA per SM at most: with fewer tiles than SMs every tile gets a CTA (and an SM) of its own rather than
@@ -426,12 +488,11 @@ unsigned grid_for(long long n_envs, int n_sm) {
 namespace boatenv {
 
 cudaError_t launch_collect(const DevCfg &c, const CollectArgs &a, cudaStream_t stream) {
-    const collect_kern_t kern = collect_kernel_for(c.wind_kind);
+    const bool record = a.rec_ids != nullptr;
+    const collect_kern_t kern = record ? collect_kernel_for<true>(c.wind_kind) : collect_kernel_for<false>(c.wind_kind);
     if (!kern) return cudaErrorInvalidValue;
     int n_sm = 0;
-    const cudaError_t e = actor_kernels_setup<boat_collect_kernel<WIND_NONE>, boat_collect_kernel<WIND_CONST>,
-                                              boat_collect_kernel<WIND_VEL_CURVE>, boat_collect_kernel<WIND_ANGLE_RECT>,
-                                              boat_collect_kernel<WIND_BOTH>>(n_sm);
+    const cudaError_t e = record ? collect_kernels_setup<true>(n_sm) : collect_kernels_setup<false>(n_sm);
     if (e != cudaSuccess) return e;
     kern<<<grid_for(c.n_envs, n_sm), kThreads, kSmemBytes, stream>>>(c, a);
     count_launch();

@@ -141,6 +141,12 @@ class DeviceRecorder:
         for t in ...: env.step(a)  (or memory.step_store(env, a));  rec.capture(a)
         rec.close()
 
+    The fused collection kernel records inside itself: ``agent.collect(env, T, recorder=rec)`` (or
+    ``TensorCorePolicy.collect(env, memory, T, recorder=rec)``) writes the T rows that T rounds of act +
+    ``step_store`` + ``capture()`` would, in the same launch, so collection keeps one launch per T steps.  T may
+    not exceed ``capacity``; rows that would not fit beside the pending ones are preceded by a flush.  Collect calls
+    and ``capture()`` steps may be mixed on one recorder.
+
     ``env_ids`` are GLOBAL env ids (``env.env_id_offset`` + local index) inside the env's shard; files are named
     by them.  Rows: ``start()`` takes the state after reset, each ``capture()`` the state after the step (under
     auto-reset the next episode's first state) with that step's action / reward.  The result equals
@@ -189,18 +195,25 @@ class DeviceRecorder:
         """Episodes of the recorded envs that ended in the flushed rows (one info.csv row each)."""
         return sum(self.book.episode.values())
 
-    def _take(self, stepped, actions=None):
+    def _record(self, n, stepped, launch):
+        """Reserves the next ``n`` rows (flushing first if they do not fit beside the pending ones), calls
+        ``launch(row)``, which queues the writes of rows ``row .. row + n - 1`` on the current stream, and books
+        them: the event marks their end, each is taken after a step (``stepped``) or after reset."""
         import torch
-        if self.pending == self.capacity:
+        if self.pending + n > self.capacity:
             self.flush()
+        launch(self._rows)
+        self._ev.record(torch.cuda.current_stream(self.env.device))
+        self._rows += n
+        self._stepped.extend([stepped] * n)
+
+    def _take(self, stepped, actions=None):
         env = self.env
         if stepped:
-            env.record_rows(self._local, self._ring, self._rows, env._actions(actions), env.reward, env.term)
+            self._record(1, True, lambda row: env.record_rows(self._local, self._ring, row, env._actions(actions),
+                                                              env.reward, env.term))
         else:
-            env.record_rows(self._local, self._ring, self._rows)
-        self._ev.record(torch.cuda.current_stream(env.device))
-        self._rows += 1
-        self._stepped.append(stepped)
+            self._record(1, False, lambda row: env.record_rows(self._local, self._ring, row))
 
     def start(self):
         """Captures the current state (call it after ``env.reset()``) and writes each env's wind.csv."""

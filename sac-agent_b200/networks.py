@@ -9,6 +9,7 @@ graph per update, batch gathered on the device by libboatenv's replay kernels).
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 import os
 
@@ -267,13 +268,16 @@ class TensorCorePolicy:
         return returns, steps, term
 
     @torch.no_grad()
-    def collect(self, env, memory, steps, done_flag_mode=1):
+    def collect(self, env, memory, steps, done_flag_mode=1, recorder=None):
         """`steps` rounds of the training loop body -- `act(env.obs)`, then `memory.step_store(env, actions,
         done_flag_mode)` -- over every env of the fp32 auto-resetting BatchedBoatEnv `env`, in ONE kernel
         (boatagent_collect, csrc/rollout.cu): the same actions, env steps, resets and ring rows (fp32 ReplayBuffer
         `memory`) as that loop.  Advances `steps` by `steps`.  Returns (env.obs, env.reward, env.done, {"term":
         env.term}) of the last step, as ReplayBuffer.step_store does; launches on the current stream and does not
-        synchronise."""
+        synchronise.
+        `recorder`: a DeviceRecorder of `env`; the same kernel (boatagent_collect_record) then writes the `steps`
+        rows that a `recorder.capture(actions)` after each round would, flushing the recorder first if they do not
+        fit beside its pending rows.  `steps` may not exceed its capacity."""
         steps = int(steps)
         if self.n_actions != 1 or self.obs_dim != 11:
             raise ValueError("collect: the BoatEnv actor (11 observations, one action)")
@@ -286,12 +290,23 @@ class TensorCorePolicy:
         if steps * env.n_envs > memory.mem_size:
             raise ValueError(f"collect: {steps} steps x {env.n_envs} envs exceed the ring's {memory.mem_size} slots "
                              "(rows of one call may not share a slot)")
+        if recorder is not None:
+            if recorder.env is not env:
+                raise ValueError("collect: the recorder records another env")
+            if steps > recorder.capacity:
+                raise ValueError(f"collect: {steps} steps exceed the recorder's {recorder.capacity} rows "
+                                 "(one call would overwrite its own rows)")
+        args = (env._h, memory._h, self.blob.data_ptr(), self.actor.max_action.data_ptr(), self.seed, self.steps, steps,
+                int(done_flag_mode), env.obs.data_ptr(), env.reward.data_ptr(), env.done.data_ptr(),
+                env.term.data_ptr())
         with torch.cuda.device(env.device):
             stream = torch.cuda.current_stream().cuda_stream
-            self._lib.check(self._L.boatagent_collect(env._h, memory._h, self.blob.data_ptr(),
-                                                      self.actor.max_action.data_ptr(), self.seed, self.steps, steps,
-                                                      int(done_flag_mode), env.obs.data_ptr(), env.reward.data_ptr(),
-                                                      env.done.data_ptr(), env.term.data_ptr(), stream),
-                            "boatagent_collect")
+            if recorder is None:
+                self._lib.check(self._L.boatagent_collect(*args, stream), "boatagent_collect")
+            else:
+                recorder._record(steps, True, lambda row: self._lib.check(
+                    self._L.boatagent_collect_record(*args, recorder._local.data_ptr(), recorder._local.numel(),
+                                                     C.byref(recorder._ring), int(row), stream),
+                    "boatagent_collect_record"))
         self.steps += steps
         return env.obs, env.reward, env.done, {"term": env.term}
