@@ -21,6 +21,8 @@ recorded run of the reference's own learn() in tests/test_agent_golden.py.
                                           # the reference's `main.py -p 8`: a tuned_configs.yaml draw per member
     torchrun --nproc-per-node 8 examples/train_sac.py --envs 65536 --data-parallel
                                           # ONE agent over all ranks: every update averages 8 batches' gradients
+    python examples/train_sac.py --envs 8192 --population 8 --policy-precision tcgen05 --learner-precision tcgen05 \
+        --collect-steps 8 --updates-per-iter 8 --tune    # 8 members on one GPU (AgentPopulation): one update launch pair
 
 By default multi-GPU is "replicas only" (SURVEY.md 8e): every rank trains its own agent on its own env shard,
 like the reference's `-p` mode runs independent models; only the episode statistics are all-reduced.
@@ -83,6 +85,11 @@ def main(argv=None):
                     help="train ONE agent over all ranks (ContinuousAgent(data_parallel=True)): every update all-reduces "
                          "the gradients of the ranks' batches, an effective batch of world x batch_size; --envs must "
                          "divide evenly over the ranks")
+    ap.add_argument("--population", type=int, default=0, metavar="P",
+                    help="train P independent members per process on its GPU (AgentPopulation, 1 to 16): each on the "
+                         "env shard a replica gets, with its own ring, experiment directory and --tune draw; every "
+                         "update round is one batched launch pair for all members.  Needs both precisions tcgen05 and "
+                         "--collect-steps")
     args = ap.parse_args(argv)
     if args.record_envs and not args.experiments_root:
         ap.error("--record-envs requires --experiments-root")
@@ -97,6 +104,21 @@ def main(argv=None):
             ap.error("--collect-steps and --record-envs cannot be combined (the fused kernel records no steps)")
 
     rank, local_rank, world = S.sharding.dist_info()
+    if args.population:   # checked before any CUDA work
+        if not 1 <= args.population <= 16:
+            ap.error("--population takes 1 to 16 members per process")
+        if args.policy_precision != "tcgen05" or args.learner_precision != "tcgen05":
+            ap.error("--population needs --policy-precision tcgen05 and --learner-precision tcgen05")
+        if args.collect_steps < 1:
+            ap.error("--population needs --collect-steps T >= 1")
+        for flag, on in (("--data-parallel", args.data_parallel), ("--overlap", args.overlap),
+                         ("--record-envs", args.record_envs)):
+            if on:
+                ap.error(f"--population and {flag} cannot be combined")
+        if args.pbt_every and world > 1:
+            ap.error("--population with --pbt-every runs on one process: population rounds across ranks hold one "
+                     "member per rank")
+        return train_population(args, rank, local_rank, world)
     if args.data_parallel:   # checked before any CUDA work
         for flag, on in (("--tune", args.tune), ("--pbt-every", args.pbt_every), ("--overlap", args.overlap)):
             if on:
@@ -251,6 +273,131 @@ def main(argv=None):
         print(json.dumps(summary), flush=True)
     env.close(); mem.close()
     if world > 1 or args.data_parallel:
+        torch.distributed.destroy_process_group()
+    return summary
+
+
+def _overrides(args):
+    out = {}
+    for item in args.set:
+        k, v = item.split("=", 1)
+        out[k] = float(v) if any(ch in v for ch in ".e") else int(v)
+    return out
+
+
+def train_population(args, rank, local_rank, world):
+    """--population P: P members per process (AgentPopulation), each trained as a replica would be."""
+    import random
+    torch.cuda.set_device(local_rank)
+    if world > 1:
+        torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    torch.manual_seed(args.seed + rank)   # the Gaussian draws of the updates; each member's weights use seed + g
+    P, overrides = args.population, _overrides(args)
+    cfg = S.load_config(base_settings__experiment=args.experiment, **overrides)
+    _, n_local = S.shard_range(args.envs, rank, world)
+    configs, exps = [cfg] * P, [None] * P
+    if args.experiments_root:
+        for m in range(P):
+            g = rank * P + m
+            exps[m] = S.Experiment(experiment_name=f"experiment_r{rank}_m{m}", subdir=f"setting_{args.experiment}",
+                                   root=args.experiments_root, rng=random.Random(args.seed + g))
+            tuned = exps[m].save_configs(cfg)
+            if args.tune:
+                configs[m] = tuned
+    pop = S.AgentPopulation(cfg, P, n_local, seed=args.seed, rank=rank, device=local_rank, configs=configs,
+                            experiment_dirs=[e.experiment_dir if e else None for e in exps],
+                            buffer_size=max(args.buffer, n_local * args.collect_steps))
+    pop.reset()
+    losses = None
+    rows, best = [[] for _ in range(P)], [float("-inf")] * P
+    prev = [{"episodes": 0.0, "return_sum": 0.0} for _ in range(P)]
+    pbt_prev = [{"episodes": 0.0, "return_sum": 0.0} for _ in range(P)]
+    pbt_log, pbt_rng = [], random.Random(1000 + args.seed + rank)
+
+    def interval_score(c, p):
+        n = c["episodes"] - p["episodes"]
+        return (c["return_sum"] - p["return_sum"]) / n if n else float("nan")
+
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for it in range(1, args.warmup_iters + args.iters + 1):
+        if it == args.warmup_iters + 1:
+            t0.record()
+        pop.collect(args.collect_steps)
+        for _ in range(args.updates_per_iter):
+            out = pop.learn()
+            losses = out if out is not None else losses
+        if args.pbt_every and it % args.pbt_every == 0:
+            counters = [env.counters() for env in pop.envs]
+            scores = [interval_score(c, p) for c, p in zip(counters, pbt_prev)]
+            pbt_prev = counters
+            info = pop.exploit_explore(scores, pbt_rng)
+            pbt_log.append({"iter": it, "scores": info["scores"], "ranking": info["ranking"],
+                            "adopted": {m: {"from": info["best"], "hp": hp} for m, hp in info["adopted"].items()}})
+        if args.log_every and it % args.log_every == 0:
+            for m, (a, env, exp) in enumerate(zip(pop.members, pop.envs, exps)):
+                if exp is None:
+                    continue
+                c = env.counters()
+                score = interval_score(c, prev[m])
+                n = c["episodes"] - prev[m]["episodes"]
+                prev[m] = c
+                if n and score > best[m]:
+                    best[m] = score
+                    a.save_models()
+                kind = max(S.TERM_NAMES[1:], key=lambda k: c[k])
+                avg = c["return_sum"] / c["episodes"] if c["episodes"] else float("nan")
+                rows[m].append([(rank, it), f"{kind}-{int(c[kind])}", score, best[m], avg, "", ""])
+            if rank == 0:
+                c = [env.counters() for env in pop.envs]
+                lv = [float(x) for x in losses[0]] if losses is not None else [float("nan")] * 3
+                print(f"iter {it:6d}  episodes {sum(x['episodes'] for x in c):.0f}  goals "
+                      f"{sum(x['reached_goal'] for x in c):.0f}  member 0 losses v/pi/q {lv[0]:.3g} {lv[1]:.3g} "
+                      f"{lv[2]:.3g}", flush=True)
+    t1.record()
+    torch.cuda.synchronize()
+    ms = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device="cuda")
+    if world > 1:
+        torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
+    total = torch.stack([env.counters_tensor() for env in pop.envs]).sum(0)
+    stats = S.all_reduce_counters(total)
+    sec = float(ms.item()) * 1e-3
+    members_total = P * world
+    summary = {"example": "train_sac", "overrides": overrides, "n_gpus": world, "envs_total": args.envs,
+               "iters": args.iters, "updates_per_iter": args.updates_per_iter, "cuda_graph": not args.no_graph,
+               "overlap": False, "policy_precision": args.policy_precision,
+               "learner_precision": args.learner_precision, "collect_steps": args.collect_steps,
+               "members": members_total, "members_per_gpu": P, "envs_per_member": n_local,
+               "env_steps_per_s": args.iters * args.collect_steps * n_local * members_total / sec,
+               "updates_per_s_per_replica": args.iters * args.updates_per_iter / sec,
+               "updates_per_s_aggregate": args.iters * args.updates_per_iter * members_total / sec,
+               "ms_per_iter": 1e3 * sec / args.iters, "episodes": stats["episodes"],
+               "mean_return": stats["return_mean"], "reached_goal": stats["reached_goal"],
+               "losses_v_pi_q": [[float(x) for x in l] for l in losses] if losses is not None else None}
+    summary["env_steps_per_s_aggregate"] = summary["env_steps_per_s"]
+    if args.pbt_every:
+        summary["pbt_rounds"] = len(pbt_log)
+        summary["pbt_adoptions"] = [e for e in pbt_log if e["adopted"]]
+        summary["hyperparameters"] = [a.hyperparameters() for a in pop.members]
+    if args.experiments_root:
+        for m, (a, env, exp) in enumerate(zip(pop.members, pop.envs, exps)):
+            c = env.counters()
+            exp.write_console(rows[m])
+            exp.append_overview(best[m])
+            exp.write_terminations(S.info_from_counters(c, max(S.TERM_NAMES[1:], key=lambda k: c[k])))
+        summary["experiment_dirs"] = [e.experiment_dir for e in exps]
+        summary["best_interval_return"] = best
+        if args.tune:
+            summary["hpsets"] = [e.tuner.hpset for e in exps]
+        mine = max((b, rank, e.experiment_name) for b, e in zip(best, exps))
+        if world > 1:
+            scores = [None] * world
+            torch.distributed.all_gather_object(scores, mine)
+            mine = max(scores)
+        summary["population_best"] = mine
+    if rank == 0:
+        print(json.dumps(summary), flush=True)
+    pop.close()
+    if world > 1:
         torch.distributed.destroy_process_group()
     return summary
 

@@ -269,6 +269,19 @@ BOATENV_API int boatreplay_gather(boatreplay_t r, int64_t batch, const int64_t *
                       void *r_out, void *s2_out, uint8_t *done_out, void *stream);
 /* Checkpoint restore: sets the store counter (buffer.py:6 mem_cntr).  The next store goes to slot mem_cntr % mem_size,
  * samples draw from [0, min(mem_cntr, mem_size)). */
+/* boatreplay_sample for the rings of a population in ONE launch (member m on blockIdx.y = m): member m's rows equal
+ * boatreplay_sample(m.ring, batch, m.seed, m.counter, m.s_out, m.a_out, m.r_out, m.s2_out, m.done_out, NULL) bit for
+ * bit.  members_host: HOST array of n_members (1..BOATAGENT_SAC_MAX_MEMBERS) entries; the rings share precision
+ * and device.  Errors (checked before anything is launched): BOATENV_EINVAL for a bad count, a NULL table, ring or
+ * output, mixed precisions or devices; BOATENV_ESTATE for an empty ring. */
+typedef struct boatreplay_sample_member {
+    boatreplay_t ring;
+    uint64_t seed, counter;
+    void *s_out, *a_out, *r_out, *s2_out;
+    uint8_t *done_out;
+} boatreplay_sample_member;
+BOATENV_API int boatreplay_sample_members(const boatreplay_sample_member *members_host, int32_t n_members,
+                                          int64_t batch, void *stream);
 BOATENV_API int boatreplay_set_mem_cntr(boatreplay_t r, int64_t mem_cntr);
 BOATENV_API int64_t boatreplay_mem_cntr(boatreplay_t r); /* buffer.py:6  */
 BOATENV_API int64_t boatreplay_mem_size(boatreplay_t r); /* buffer.py:5  */
@@ -436,6 +449,35 @@ BOATENV_API int boatagent_sac_gradients(const float *state, const float *action,
                                         const float *max_action, int64_t batch, float gamma, float reward_scale,
                                         const boatagent_adam_slot *slots_host, int32_t n_slots, float grad_scale,
                                         float *losses_out, void *workspace, int64_t workspace_bytes, void *stream);
+
+/* Population training on one GPU: one SAC update of each of n_members INDEPENDENT agents (the reference's `main.py -p N`
+ * members, main.py:215-235, each with its own utils/hyperparameter_tuner.py draw) in the two kernels of
+ * boatagent_sac_update, launched once for all of them (member m on blockIdx.y = m).  Member m computes exactly what
+ * boatagent_sac_update computes with its entry's arguments, bit for bit.  Each entry of members_host (a HOST array,
+ * copied into the kernel arguments) names one agent:
+ *   state .. max_action, slots / n_slots, gamma, reward_scale, adam_state, losses: as for boatagent_sac_update (the
+ *   slots carry the member's learning rates); tau: the member's Polyak factor.
+ * Shared by all members: batch (a positive multiple of 128), beta1, beta2, adam_eps.  Members must not share
+ * parameters, gradients, moments, adam_state or losses.
+ *   workspace: n_members * boatagent_sac_update_workspace_bytes(batch) device bytes, 16-byte aligned; member m uses
+ *   the slice at m times that size.
+ * Errors (checked for every member before anything is launched): BOATENV_EINVAL for n_members outside
+ * 1..BOATAGENT_SAC_MAX_MEMBERS, a NULL table, workspace or adam_state, a workspace that is too small, and every
+ * argument error of boatagent_sac_update; BOATENV_EALIGN as there. */
+#define BOATAGENT_SAC_MAX_MEMBERS 16   /* the member tables fill most of the 32,764 bytes of kernel parameters */
+typedef struct boatagent_sac_member {
+    const float *state, *action, *reward, *new_state;
+    const uint8_t *done;
+    const float *eps, *max_action;
+    const boatagent_adam_slot *slots;   /* HOST array of n_slots (26) slots */
+    int32_t n_slots;
+    float gamma, reward_scale, tau;
+    int64_t *adam_state;
+    float *losses;
+} boatagent_sac_member;
+BOATENV_API int boatagent_sac_update_members(const boatagent_sac_member *members_host, int32_t n_members,
+                                             int64_t batch, float beta1, float beta2, float adam_eps, void *workspace,
+                                             int64_t workspace_bytes, void *stream);
 
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 

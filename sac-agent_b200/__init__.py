@@ -16,11 +16,12 @@ from .csv_export import BatchedRecorder, DeviceRecorder  # noqa: F401
 from .sharding import all_reduce_counters, make_sharded_env, shard_range  # noqa: F401
 from .experiment import Experiment, HPTuner, get_experiment_config, info_from_counters  # noqa: F401
 from . import population  # noqa: F401
+from .population import AgentPopulation  # noqa: F401
 
 __all__ = ["AttrDict", "load_config", "params_from_config", "BoatEnvError", "lib", "library_path",
            "BatchedBoatEnv", "BoatEnv", "Box", "TERM_NAMES", "ReplayBuffer", "ToyCar", "ToyParachute",
            "BatchedRecorder", "DeviceRecorder", "all_reduce_counters", "make_sharded_env", "shard_range",
-           "Experiment", "HPTuner", "get_experiment_config", "info_from_counters",
+           "Experiment", "HPTuner", "get_experiment_config", "info_from_counters", "AgentPopulation",
            "ContinuousAgent", "SACLearner", "OverlappedActorLearner"]
 
 

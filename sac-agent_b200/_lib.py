@@ -38,6 +38,19 @@ class RecordRing(C.Structure):
     _fields_ = [(name, vp) for name in ("s_x", "s_y", "v_x", "v_y", "s_r", "rudder_angle", "action", "reward",
                                         "term", "episode")] + [("capacity", i64)]
 
+class SacMember(C.Structure):
+    """boatagent_sac_member: one population member's arguments of boatagent_sac_update_members."""
+    _fields_ = [(name, vp) for name in ("state", "action", "reward", "new_state", "done", "eps", "max_action",
+                                        "slots")] + [("n_slots", i32), ("gamma", C.c_float), ("reward_scale", C.c_float),
+                                                     ("tau", C.c_float), ("adam_state", vp), ("losses", vp)]
+
+
+class SampleMember(C.Structure):
+    """boatreplay_sample_member: one ring's arguments of boatreplay_sample_members."""
+    _fields_ = [("ring", vp), ("seed", u64), ("counter", u64)] + [(name, vp) for name in ("s_out", "a_out", "r_out",
+                                                                                            "s2_out", "done_out")]
+
+
 # name -> (restype, argtypes): one row per declaration in include/boatenv.h
 SIGNATURES = {
     "boatenv_create": (C.c_int, [PP, i64, u64, i64, C.c_int, C.c_int, C.POINTER(vp)]),
@@ -77,6 +90,9 @@ SIGNATURES = {
                                        C.c_float, C.c_float, C.c_float, vp, vp, vp, i64, vp]),
     "boatagent_sac_gradients": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, i64, C.c_float, C.c_float, vp, i32, C.c_float,
                                           vp, vp, i64, vp]),
+    "boatagent_sac_update_members": (C.c_int, [C.POINTER(SacMember), i32, i64, C.c_float, C.c_float, C.c_float, vp,
+                                               i64, vp]),
+    "boatreplay_sample_members": (C.c_int, [C.POINTER(SampleMember), i32, i64, vp]),
     "boatreplay_create": (C.c_int, [i64, i32, i32, C.c_int, C.c_int, C.POINTER(vp)]),
     "boatreplay_destroy": (C.c_int, [vp]),
     "boatreplay_store": (C.c_int, [vp, i64, vp, vp, vp, vp, vp, vp]),

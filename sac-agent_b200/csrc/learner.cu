@@ -13,12 +13,16 @@
 //                     grad_scale and leaves the parameters and the optimiser state alone, so that the gradients of
 //                     several replicas can be all-reduced before one Adam step.
 //
+// boatagent_sac_update_members runs the same two bodies for up to 16 independent agents in one launch each:
+// member m on blockIdx.y = m, with its own arguments, workspace slice and step counter.
+//
 // Operands in shared memory and in the workspace use the 8x8 core-matrix layout of actor_tc.cuh: element (r, c) of
 // an R-row matrix at (c / 8) * (R * 16) + r * 16 + (c % 8) * 2.  The same bytes are a K-major operand with rows = M/N
 // (LBO = R * 16, SBO = 128) and an MN-major operand with rows = K (LBO = 128, SBO = R * 16): so W2 [out][in] is the B
 // operand of both H1 . W2^T (forward) and dZ2 . W2 (input gradient), and the workspace tiles of dZ2 and H1 [rows][256]
 // are the A and B operands of dW2 = dZ2^T . H1 without a transpose.
 #include <cstdint>
+#include <cstring>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
@@ -92,6 +96,17 @@ struct ParamArgs {
     float *losses;
     float grad_scale;   // gradients-only instantiation: factor on the written gradients and losses
 };
+
+// The population launch (boatagent_sac_update_members): every member's arguments, member m on blockIdx.y = m.  Both
+// tables travel as kernel parameters, within the 32,764-byte limit of CUDA 12.1+.
+struct MemberRowArgs {
+    RowArgs m[BOATAGENT_SAC_MAX_MEMBERS];
+};
+struct MemberParamArgs {
+    ParamArgs m[BOATAGENT_SAC_MAX_MEMBERS];
+};
+static_assert(sizeof(MemberRowArgs) <= 32764, "kernel parameter limit");
+static_assert(sizeof(MemberParamArgs) <= 32764, "kernel parameter limit");
 
 __device__ __forceinline__ uint32_t core_off(int r, int c, int rows) { return (uint32_t)((c >> 3) * (rows * 16) + r * 16 + (c & 7) * 2); }
 
@@ -309,10 +324,12 @@ __device__ __forceinline__ void put_small(unsigned char *ws, int tid, const floa
 // min(a, b)'s gradient share of a, as torch's backward of torch.min(a, b): ties split the gradient in halves
 __device__ __forceinline__ float min_share(float a, float b) { return a < b ? 1.f : (a == b ? 0.5f : 0.f); }
 
-__global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_constant__ RowArgs args) {
+// The row pass of one 128-row tile.  blockIdx.x is the tile and gridDim.x the tile count of ONE update: the
+// population launch puts its members on blockIdx.y, so both stay per member.
+__device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
-    const int tid = threadIdx.x, warp = tid >> 5;
+    const int warp = tid >> 5;
     Rows R;
     R.smem = smem;
     R.sbase = smem_u32(smem);
@@ -419,16 +436,27 @@ __global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_con
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(R.tmem) : "memory");
 }
 
+__global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_constant__ RowArgs args) {
+    sac_rows_tile(args, threadIdx.x);
+}
+
+// population launch: member blockIdx.y, its tiles on blockIdx.x
+__global__ void __launch_bounds__(kLThreads, 1) sac_rows_members_kernel(const __grid_constant__ MemberRowArgs args) {
+    sac_rows_tile(args.m[blockIdx.y], threadIdx.x);
+}
+
 // slot of tensor `t` (0 w1, 1 b1, 2 w2, 3 b2, 4 / 6 head weights, 5 / 7 head biases) of trained network `n`
 __device__ __forceinline__ int slot_of(int n, int t) { return n == 0 ? t : 8 + 6 * (n - 1) + t; }
 
-// kAdam: write the gradients, apply Adam + Polyak and count the step; else write grad_scale times the gradients only
+// kAdam: write the gradients, apply Adam + Polyak and count the step; else write grad_scale times the gradients only.
+// blockIdx.x is the CTA and gridDim.x the CTA count of ONE update (the population launch: member = blockIdx.y), so
+// the step-counter ticket counts one member's CTAs.
 template <bool kAdam>
-__global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_constant__ ParamArgs args) {
+__device__ __forceinline__ void sac_params_block(const ParamArgs &args, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
     __shared__ float s_bc1, s_bc2_sqrt;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int warp = tid >> 5, lane = tid & 31;
     const long long B = args.batch, tiles = B / kRows;
     if constexpr (kAdam) {
         if (tid == 0) adam_bias_corrections(*reinterpret_cast<volatile long long *>(args.state) + 1, args.beta1,
@@ -573,6 +601,15 @@ __global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_cons
     }
 }
 
+template <bool kAdam>
+__global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_constant__ ParamArgs args) {
+    sac_params_block<kAdam>(args, threadIdx.x);   // read here, where the launch bounds bound it
+}
+
+__global__ void __launch_bounds__(kPThreads) sac_params_members_kernel(const __grid_constant__ MemberParamArgs args) {
+    sac_params_block<true>(args.m[blockIdx.y], threadIdx.x);
+}
+
 constexpr int kParamBlocks = 2 * kNets + kNets * (kHidden / 8) + 1;
 
 // numel of slot k, in DeviceAdam's order (actor: fc1 w, b, fc2 w, b, mean w, b, std w, b; critics and value: fc1 w, b,
@@ -646,22 +683,29 @@ int sac_args(const float *state, const float *action, const float *reward, const
     return 0;
 }
 
-template <bool kAdam>
-int sac_launch(const RowArgs &ra, const ParamArgs &pa, void *stream) {
+// the dynamic shared memory opt-in of every learner kernel, once per device
+int set_smem_attributes() {
     static std::mutex mu;
     static bool set_of[64] = {false};
     int dev = 0;
     CUDA_TRY(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64) return (int)cudaErrorInvalidDevice;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        if (!set_of[dev]) {
-            CUDA_TRY(cudaFuncSetAttribute(sac_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
-            CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
-            CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
-            set_of[dev] = true;
-        }
+    std::lock_guard<std::mutex> lock(mu);
+    if (!set_of[dev]) {
+        CUDA_TRY(cudaFuncSetAttribute(sac_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac_rows_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac_params_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+        set_of[dev] = true;
     }
+    return 0;
+}
+
+template <bool kAdam>
+int sac_launch(const RowArgs &ra, const ParamArgs &pa, void *stream) {
+    const int rc = set_smem_attributes();
+    if (rc != 0) return rc;
     sac_rows_kernel<<<(unsigned)(ra.batch / kRows), kLThreads, kLSmem, (cudaStream_t)stream>>>(ra);
     boatenv::count_launch();
     CUDA_TRY(cudaGetLastError());
@@ -707,4 +751,40 @@ extern "C" int boatagent_sac_gradients(const float *state, const float *action, 
     pa.state = nullptr;
     pa.grad_scale = grad_scale;
     return sac_launch<false>(ra, pa, stream);
+}
+
+extern "C" int boatagent_sac_update_members(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch,
+                                            float beta1, float beta2, float adam_eps, void *workspace,
+                                            int64_t workspace_bytes, void *stream) {
+    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
+    if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
+    const size_t slice = ws_bytes(batch / kRows);   // a multiple of 16: every slice stays 16-byte aligned
+    if (workspace_bytes < 0 || (uint64_t)workspace_bytes < slice * (uint64_t)n_members) return BOATENV_EINVAL;
+    static thread_local MemberRowArgs ra;   // ~32 KB together: kept off the stack
+    static thread_local MemberParamArgs pa;
+    std::memset(&ra, 0, sizeof(ra));
+    std::memset(&pa, 0, sizeof(pa));
+    for (int m = 0; m < n_members; ++m) {
+        const boatagent_sac_member &b = members_host[m];
+        if (!b.adam_state) return BOATENV_EINVAL;
+        unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
+        const int rc = sac_args(b.state, b.action, b.reward, b.new_state, b.done, b.eps, b.max_action, batch, b.gamma,
+                                b.reward_scale, b.slots, b.n_slots, b.losses, ws, (int64_t)slice, ra.m[m], pa.m[m]);
+        if (rc != 0) return rc;
+        pa.m[m].beta1 = beta1;
+        pa.m[m].beta2 = beta2;
+        pa.m[m].eps = adam_eps;
+        pa.m[m].tau = b.tau;
+        pa.m[m].state = (long long *)b.adam_state;
+        pa.m[m].grad_scale = 1.0f;
+    }
+    const int rc = set_smem_attributes();
+    if (rc != 0) return rc;
+    sac_rows_members_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem,
+                              (cudaStream_t)stream>>>(ra);
+    boatenv::count_launch();
+    CUDA_TRY(cudaGetLastError());
+    sac_params_members_kernel<<<dim3(kParamBlocks, (unsigned)n_members), kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+    boatenv::count_launch();
+    return (int)cudaGetLastError();
 }

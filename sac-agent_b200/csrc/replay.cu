@@ -92,9 +92,10 @@ __device__ __forceinline__ long long replay_index(unsigned long long seed, unsig
 // (consecutive threads = consecutive output elements: coalesced stores, row-contiguous loads) and the
 // first threads move action / reward / done.
 // USE_IDX: indices supplied by the caller; otherwise drawn in-kernel (and optionally exported).
+// blockIdx.x / gridDim.x stride over ONE ring's batch (the population launch puts its members on blockIdx.y).
 constexpr int kGatherRows = 128;
 template <typename T, bool USE_IDX>
-__global__ void __launch_bounds__(256) replay_gather_kernel(
+__device__ __forceinline__ void gather_rows(
     const T *__restrict__ state, const T *__restrict__ new_state, const T *__restrict__ action,
     const T *__restrict__ reward, const uint8_t *__restrict__ terminal, const long long *__restrict__ idx_in,
     long long *__restrict__ idx_out, T *__restrict__ s_out, T *__restrict__ a_out, T *__restrict__ r_out,
@@ -130,6 +131,40 @@ __global__ void __launch_bounds__(256) replay_gather_kernel(
         }
         __syncthreads();  // jrow is reused by the next group of rows
     }
+}
+
+template <typename T, bool USE_IDX>
+__global__ void __launch_bounds__(256) replay_gather_kernel(
+    const T *__restrict__ state, const T *__restrict__ new_state, const T *__restrict__ action,
+    const T *__restrict__ reward, const uint8_t *__restrict__ terminal, const long long *__restrict__ idx_in,
+    long long *__restrict__ idx_out, T *__restrict__ s_out, T *__restrict__ a_out, T *__restrict__ r_out,
+    T *__restrict__ s2_out, uint8_t *__restrict__ d_out, long long batch, long long max_mem, long long size,
+    unsigned long long seed, unsigned long long counter, int obs_dim, int n_actions) {
+    gather_rows<T, USE_IDX>(state, new_state, action, reward, terminal, idx_in, idx_out, s_out, a_out, r_out, s2_out,
+                            d_out, batch, max_mem, size, seed, counter, obs_dim, n_actions);
+}
+
+// boatreplay_sample_members: one ring's in-kernel draw and gather per blockIdx.y
+struct GatherMember {
+    const void *state, *new_state, *action, *reward;
+    const uint8_t *terminal;
+    void *s_out, *a_out, *r_out, *s2_out;
+    uint8_t *d_out;
+    long long max_mem, size;
+    unsigned long long seed, counter;
+    int obs_dim, n_actions;
+};
+struct GatherMembers {
+    GatherMember m[BOATAGENT_SAC_MAX_MEMBERS];
+};
+
+template <typename T>
+__global__ void __launch_bounds__(256) replay_gather_members_kernel(const __grid_constant__ GatherMembers args,
+                                                                    long long batch) {
+    const GatherMember &g = args.m[blockIdx.y];
+    gather_rows<T, false>((const T *)g.state, (const T *)g.new_state, (const T *)g.action, (const T *)g.reward,
+                          g.terminal, nullptr, nullptr, (T *)g.s_out, (T *)g.a_out, (T *)g.r_out, (T *)g.s2_out, g.d_out,
+                          batch, g.max_mem, g.size, g.seed, g.counter, g.obs_dim, g.n_actions);
 }
 
 template <typename T>
@@ -249,6 +284,50 @@ int boatreplay_sample(boatreplay_t r, int64_t batch, uint64_t seed, uint64_t cou
                                         s2_out, done_out, (cudaStream_t)stream)
                  : launch_gather<double>(r, batch, nullptr, (long long *)idx_out, seed, counter, s_out, a_out, r_out,
                                          s2_out, done_out, (cudaStream_t)stream));
+    return BOATENV_OK;
+}
+
+int boatreplay_sample_members(const boatreplay_sample_member *members_host, int32_t n_members, int64_t batch,
+                              void *stream) {
+    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || batch <= 0) return BOATENV_EINVAL;
+    const boatreplay_t r0 = members_host[0].ring;
+    if (!r0) return BOATENV_EINVAL;
+    GatherMembers a;
+    std::memset(&a, 0, sizeof(a));
+    for (int m = 0; m < n_members; ++m) {
+        const boatreplay_sample_member &e = members_host[m];
+        const boatreplay_t r = e.ring;
+        if (!r || !e.s_out || !e.a_out || !e.r_out || !e.s2_out || !e.done_out) return BOATENV_EINVAL;
+        if (r->precision != r0->precision || r->device != r0->device) return BOATENV_EINVAL;
+        if (r->mem_cntr <= 0) return BOATENV_ESTATE;
+        GatherMember &g = a.m[m];
+        g.state = r->state;
+        g.new_state = r->new_state;
+        g.action = r->action;
+        g.reward = r->reward;
+        g.terminal = r->terminal;
+        g.s_out = e.s_out;
+        g.a_out = e.a_out;
+        g.r_out = e.r_out;
+        g.s2_out = e.s2_out;
+        g.d_out = e.done_out;
+        g.max_mem = r->mem_cntr < r->mem_size ? r->mem_cntr : r->mem_size;
+        g.size = r->mem_size;
+        g.seed = e.seed;
+        g.counter = e.counter;
+        g.obs_dim = r->obs_dim;
+        g.n_actions = r->n_actions;
+    }
+    GUARD_DEVICE(r0);
+    long long blocks = (batch + kGatherRows - 1) / kGatherRows;
+    blocks = std::max(1LL, std::min(blocks, 148LL * 32));
+    const dim3 grid((unsigned)blocks, (unsigned)n_members);
+    if (r0->precision == 32)
+        replay_gather_members_kernel<float><<<grid, 256, 0, (cudaStream_t)stream>>>(a, batch);
+    else
+        replay_gather_members_kernel<double><<<grid, 256, 0, (cudaStream_t)stream>>>(a, batch);
+    count_launch();
+    CUDA_TRY(cudaGetLastError());
     return BOATENV_OK;
 }
 

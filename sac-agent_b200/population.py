@@ -11,9 +11,15 @@ the members never talk.  With one member per GPU under ``torchrun`` the members 
   explore   perturb the adopted hyper-parameters by x0.8 or x1.25, clipped to the tuner's ranges.
 
 ``exploit_explore`` works on any list of tensors and any process group (NCCL on GPUs, gloo in the CPU test).
+
+On ONE GPU, ``AgentPopulation`` trains P members in one process: each member is an ordinary ``ContinuousAgent`` with its
+own env, ring, experiment directory and hyper-parameters, and one ``learn()`` updates all of them in four launches (one
+sample-gather for every ring, one Gaussian draw, the two kernels of ``boatagent_sac_update_members``).
+``exploit_explore_local`` is ``exploit_explore`` over such members, with device copies instead of collectives.
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 import random
 
@@ -33,6 +39,18 @@ def perturb(hp: dict, rng: random.Random, factors=(0.8, 1.25)) -> dict:
         v = 1.0 - (1.0 - hp[k]) * f if k == "gamma" else hp[k] * f
         out[k] = round(min(max(v, lo), hi), 4)
     return out
+
+
+def select(scores, bottom_fraction: float = 0.25):
+    """The ranking of one population round.  ``scores``: one per member, higher is better, NaN / -inf = no finished
+    episode.  Returns (ranking best first with ties broken by index, the best member, the losers that adopt it: the
+    bottom ``bottom_fraction`` (at least one) of the ranking, without the best and without members scoring as well
+    as it; nobody adopts when no member has a score)."""
+    n = len(scores)
+    ranking = sorted(range(n), key=lambda r: (-scores[r], r))
+    best = ranking[0]
+    n_bottom = max(1, int(n * bottom_fraction)) if scores[best] > -float("inf") else 0
+    return ranking, best, [r for r in ranking[n - n_bottom:] if r != best and scores[r] < scores[best]]
 
 
 def exploit_explore(tensors, hp: dict, score: float, rng: random.Random, bottom_fraction: float = 0.25, group=None):
@@ -57,10 +75,7 @@ def exploit_explore(tensors, hp: dict, score: float, rng: random.Random, bottom_
     dist.all_gather(table, mine, group=group)
     table = torch.stack(table).cpu()
     scores = table[:, 0].tolist()
-    ranking = sorted(range(world), key=lambda r: (-scores[r], r))       # best first; ties by rank: the same everywhere
-    best = ranking[0]
-    n_bottom = max(1, int(world * bottom_fraction)) if scores[best] > -float("inf") else 0
-    losers = [r for r in ranking[world - n_bottom:] if r != best and scores[r] < scores[best]]
+    ranking, best, losers = select(scores, bottom_fraction)              # ties by rank: the same everywhere
     info = {"adopted_from": None, "ranking": ranking, "scores": scores}
     if not losers:
         return dict(hp), info
@@ -81,3 +96,174 @@ def exploit_explore(tensors, hp: dict, score: float, rng: random.Random, bottom_
     info["adopted_from"] = best
     best_hp = dict(zip(HP_KEYS, table[best, 1:].tolist()))
     return perturb(best_hp, rng), info
+
+
+def exploit_explore_local(members, scores, rng: random.Random, bottom_fraction: float = 0.25):
+    """``exploit_explore`` for members held by one process (``ContinuousAgent`` objects on one device): the same
+    ranking (``select``) and perturbation, with each loser's ``training_tensors()`` overwritten by device copies of the
+    best member's.  ``scores``: one per member (NaN = no finished episode).  Returns
+    {"ranking", "scores", "best", "adopted": {loser index: perturbed hyper-parameters}}."""
+    import torch
+    scores = [-float("inf") if math.isnan(float(x)) else float(x) for x in scores]
+    if len(scores) != len(members):
+        raise ValueError(f"exploit_explore_local: {len(scores)} scores for {len(members)} members")
+    ranking, best, losers = select(scores, bottom_fraction)
+    info = {"ranking": ranking, "scores": scores, "best": best, "adopted": {}}
+    if not losers:
+        return info
+    src, best_hp = members[best].training_tensors(), members[best].hyperparameters()
+    for r in losers:
+        with torch.no_grad():
+            torch._foreach_copy_(members[r].training_tensors(), src)
+        hp = perturb(best_hp, rng)
+        members[r].set_hyperparameters(**hp)
+        members[r]._weights_changed()
+        info["adopted"][r] = hp
+    return info
+
+
+class AgentPopulation:
+    """P independent SAC members on one GPU, updated together (the reference's ``main.py -p P`` on one device).
+
+    Member m of process ``rank`` has the global index g = rank * P + m.  It is a ``ContinuousAgent`` with
+    policy and learner precision "tcgen05", its own ``BatchedBoatEnv`` (``envs_per_member`` envs, global env ids from
+    g * envs_per_member, so no two members share wind draws), its own ``ReplayBuffer`` (ring seed ``seed + g``), its
+    initial weights drawn under torch seed ``seed + g`` and its tcgen05 acting seed 0x5ac + g.  With P = 1 and rank 0
+    that is the agent ``examples/train_sac.py`` builds with the same seed, bit for bit.
+
+    ``configs``: one config per member (e.g. its tuned_configs.yaml draw), else ``config`` for all; the batch size must
+    be the same.  Change a member's hyper-parameters through ``set_hyperparameters`` or ``exploit_explore`` so that
+    the next ``learn()`` sees them."""
+
+    def __init__(self, config, members, envs_per_member, seed=0, rank=0, device=None, configs=None,
+                 experiment_dirs=None, buffer_size=None, done_flag_mode=1):
+        import torch
+        from . import _lib
+        from .boat_env import BatchedBoatEnv
+        from .buffer import ReplayBuffer
+        from .continuous_agent import ContinuousAgent
+        from .networks import TensorCorePolicy
+        P = int(members)
+        if not 1 <= P <= 16:
+            raise ValueError(f"AgentPopulation: 1 to 16 members per process (BOATAGENT_SAC_MAX_MEMBERS), got {P}")
+        configs = list(configs) if configs is not None else [config] * P
+        dirs = list(experiment_dirs) if experiment_dirs is not None else [None] * P
+        if len(configs) != P or len(dirs) != P:
+            raise ValueError("AgentPopulation: one config and one experiment directory per member")
+        self.batch_size = int(configs[0].agent.batch_size)
+        if any(int(c.agent.batch_size) != self.batch_size for c in configs):
+            raise ValueError("AgentPopulation: the members share one batch size")
+        self._L, self._lib = _lib.lib(), _lib
+        self.device = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        self.rank, self.seed, self.done_flag_mode = int(rank), int(seed), int(done_flag_mode)
+        self.envs, self.members = [], []
+        for m in range(P):
+            g = self.rank * P + m
+            cfg = configs[m]
+            env = BatchedBoatEnv(cfg, envs_per_member, seed=seed, precision="fp32", device=self.device.index,
+                                 env_id_offset=g * int(envs_per_member), auto_reset=True)
+            size = int(cfg.agent.max_size) if buffer_size is None else int(buffer_size)
+            mem = ReplayBuffer(size, (11,), 1, precision="fp32", device=self.device.index, seed=seed + g, as_torch=True)
+            with torch.random.fork_rng(devices=[self.device]):
+                torch.manual_seed(seed + g)
+                agent = ContinuousAgent(cfg, dirs[m], env.observation_space.shape, env, device=self.device.index,
+                                        seed=seed + g, memory=mem, policy_precision="tcgen05",
+                                        learner_precision="tcgen05")
+            agent._tc_policy = TensorCorePolicy(agent.actor, seed=0x5ac + g)
+            self.envs.append(env)
+            self.members.append(agent)
+        B = self.batch_size
+        # the members' Gaussian draws are slices of one tensor: one normal_() per learn()
+        self.eps = torch.zeros((P, 2, B, 1), dtype=torch.float32, device=self.device)
+        for m, a in enumerate(self.members):
+            a._eps = self.eps[m]
+        self._ws = torch.empty(P * int(self._L.boatagent_sac_update_workspace_bytes(B)), dtype=torch.uint8,
+                               device=self.device)
+        self._sample = (_lib.SampleMember * P)()
+        self._table = None
+
+    def __len__(self):
+        return len(self.members)
+
+    def reset(self):
+        """Resets every member's env; returns their observations."""
+        return [env.reset() for env in self.envs]
+
+    def collect(self, steps):
+        """``steps`` env steps of every member's envs (``ContinuousAgent.collect``, one launch per member).  Each
+        member's packed acting weights are refreshed once, here, instead of after every update."""
+        for a, env in zip(self.members, self.envs):
+            a._tc_policy.refresh()
+            a.collect(env, steps, done_flag_mode=self.done_flag_mode)
+
+    def _build_table(self):
+        """The member table of boatagent_sac_update_members.  Every pointer in it is stable: parameters, moments,
+        gradients, the batch and the draws are updated in place."""
+        import torch
+        t = (self._lib.SacMember * len(self.members))()
+        for m, a in enumerate(self.members):
+            o, L = a.learner.optimizer, a.learner
+            for k, p in enumerate(o.params):
+                if p.grad is None:
+                    p.grad = torch.zeros_like(p)
+                o._slots[k].grad = p.grad.data_ptr()
+            s, act, r, s2, d = a._batch
+            t[m] = self._lib.SacMember(s.data_ptr(), act.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(),
+                                       a._eps.data_ptr(), L.actor.max_action.data_ptr(),
+                                       C.cast(o._slots, C.c_void_p), len(o.params), float(L.gamma), float(L.scale),
+                                       float(o.tau), o.state.data_ptr(), a._loss_buf.data_ptr())
+            self._sample[m] = self._lib.SampleMember(a.memory._h, a.memory.seed, 0, s.data_ptr(), act.data_ptr(),
+                                                     r.data_ptr(), s2.data_ptr(), d.data_ptr())
+        self._table = t   # its slot pointers are the members' own DeviceAdam arrays, which live as long as they do
+
+    def learn(self):
+        """One update of every member: the batched sample-gather, one Gaussian draw for all, and the two kernels of
+        boatagent_sac_update_members (no sync).  Returns each member's (value, actor, critic) losses as device
+        tensors, or None (nothing launched) while some member's ring holds less than a batch."""
+        if any(a.memory.mem_cntr < self.batch_size for a in self.members):
+            return None
+        import torch
+        if self._table is None:
+            self._build_table()
+        P, B = len(self.members), self.batch_size
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        for m, a in enumerate(self.members):
+            self._sample[m].counter = a.memory._samples
+        self._lib.check(self._L.boatreplay_sample_members(self._sample, P, B, stream), "boatreplay_sample_members")
+        for a in self.members:
+            a.memory._samples += 1
+        self.eps.normal_()
+        o = self.members[0].learner.optimizer
+        self._lib.check(self._L.boatagent_sac_update_members(self._table, P, B, o.betas[0], o.betas[1], o.eps,
+                                                             self._ws.data_ptr(), self._ws.numel(), stream),
+                        "boatagent_sac_update_members")
+        for a in self.members:
+            a.updates += 1
+        return [a._losses for a in self.members]
+
+    def set_hyperparameters(self, m, **hp):
+        """``ContinuousAgent.set_hyperparameters`` of member m, seen by the next ``learn()``."""
+        self.members[m].set_hyperparameters(**hp)
+        self._table = None
+
+    def exploit_explore(self, scores, rng: random.Random, bottom_fraction: float = 0.25):
+        """One population round over the members (``exploit_explore_local``)."""
+        info = exploit_explore_local(self.members, scores, rng, bottom_fraction)
+        self._table = None
+        return info
+
+    def state_dict(self):
+        """The members' ``ContinuousAgent.state_dict()``, in member order."""
+        return [a.state_dict() for a in self.members]
+
+    def load_state_dict(self, sd):
+        if len(sd) != len(self.members):
+            raise ValueError(f"checkpoint of {len(sd)} members for a population of {len(self.members)}")
+        for a, s in zip(self.members, sd):
+            a.load_state_dict(s)
+        self._table = None
+
+    def close(self):
+        for a, env in zip(self.members, self.envs):
+            env.close()
+            a.memory.close()
