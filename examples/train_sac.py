@@ -23,6 +23,9 @@ recorded run of the reference's own learn() in tests/test_agent_golden.py.
                                           # ONE agent over all ranks: every update averages 8 batches' gradients
     python examples/train_sac.py --envs 8192 --population 8 --policy-precision tcgen05 --learner-precision tcgen05 \
         --collect-steps 8 --updates-per-iter 8 --tune    # 8 members on one GPU (AgentPopulation): one update launch pair
+    torchrun --nproc-per-node 8 examples/train_sac.py --envs 65536 --population 8 --data-parallel --tune --pbt-every 50 \
+        --policy-precision tcgen05 --learner-precision tcgen05 --collect-steps 8
+                                          # 8 members, each ONE agent over all ranks, with population rounds
 
 By default multi-GPU is "replicas only" (SURVEY.md 8e): every rank trains its own agent on its own env shard,
 like the reference's `-p` mode runs independent models; only the episode statistics are all-reduced.
@@ -89,7 +92,9 @@ def main(argv=None):
                     help="train P independent members per process on its GPU (AgentPopulation, 1 to 16): each on the "
                          "env shard a replica gets, with its own ring, experiment directory and --tune draw; every "
                          "update round is one batched launch pair for all members.  Needs both precisions tcgen05 and "
-                         "--collect-steps")
+                         "--collect-steps.  With --data-parallel under torchrun (2+ ranks) every member is ONE agent "
+                         "trained by all ranks, --envs counts each member's envs over all ranks, and --tune and "
+                         "--pbt-every draw and rank the members the same way on every rank")
     args = ap.parse_args(argv)
     if args.record_envs and not args.experiments_root:
         ap.error("--record-envs requires --experiments-root")
@@ -111,14 +116,26 @@ def main(argv=None):
             ap.error("--population needs --policy-precision tcgen05 and --learner-precision tcgen05")
         if args.collect_steps < 1:
             ap.error("--population needs --collect-steps T >= 1")
-        for flag, on in (("--data-parallel", args.data_parallel), ("--overlap", args.overlap),
+        for flag, on in (("--data-parallel", args.data_parallel and world < 2), ("--overlap", args.overlap),
                          ("--record-envs", args.record_envs)):
             if on:
-                ap.error(f"--population and {flag} cannot be combined")
-        if args.pbt_every and world > 1:
+                ap.error(f"--population and {flag} cannot be combined" +
+                         (" on one process (a one-rank group is plain --population)" if flag == "--data-parallel" else ""))
+        if args.pbt_every and world > 1 and not args.data_parallel:
             ap.error("--population with --pbt-every runs on one process: population rounds across ranks hold one "
-                     "member per rank")
-        return train_population(args, rank, local_rank, world)
+                     "member per rank (or add --data-parallel: every member trained by all ranks)")
+        if args.data_parallel and args.envs % world:
+            ap.error(f"--population --data-parallel needs --envs (each member's envs over all ranks) divisible by the "
+                     f"world size ({args.envs} envs, {world} ranks)")
+        torch.cuda.set_device(local_rank)
+        if world > 1:
+            torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+        try:
+            return train_population(args, rank, local_rank, world,
+                                    group=torch.distributed.group.WORLD if args.data_parallel else None)
+        finally:
+            if world > 1:
+                torch.distributed.destroy_process_group()
     if args.data_parallel:   # checked before any CUDA work
         for flag, on in (("--tune", args.tune), ("--pbt-every", args.pbt_every), ("--overlap", args.overlap)):
             if on:
@@ -285,34 +302,41 @@ def _overrides(args):
     return out
 
 
-def train_population(args, rank, local_rank, world):
-    """--population P: P members per process (AgentPopulation), each trained as a replica would be."""
+def train_population(args, rank, local_rank, world, group=None):
+    """--population P: P members per process (AgentPopulation), each trained as a replica would be.  With a process
+    group (--data-parallel) every member is one agent trained by all ranks of `group` (rank and world are then this
+    process's rank in it and its size): the ranks tune and rank the members alike, and rank 0 writes the experiments."""
     import random
-    torch.cuda.set_device(local_rank)
-    if world > 1:
-        torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    dp = group is not None
     torch.manual_seed(args.seed + rank)   # the Gaussian draws of the updates; each member's weights use seed + g
     P, overrides = args.population, _overrides(args)
     cfg = S.load_config(base_settings__experiment=args.experiment, **overrides)
-    _, n_local = S.shard_range(args.envs, rank, world)
+    n_local = args.envs // world if dp else S.shard_range(args.envs, rank, world)[1]
     configs, exps = [cfg] * P, [None] * P
     if args.experiments_root:
         for m in range(P):
             g = rank * P + m
-            exps[m] = S.Experiment(experiment_name=f"experiment_r{rank}_m{m}", subdir=f"setting_{args.experiment}",
-                                   root=args.experiments_root, rng=random.Random(args.seed + g))
+            if dp and rank > 0:   # rank 0's draw for member m, without writing its directory
+                if args.tune:
+                    configs[m] = S.AttrDict(S.HPTuner(rng=random.Random(args.seed + m)).tuned(cfg))
+                continue
+            exps[m] = S.Experiment(experiment_name=f"experiment_m{m}" if dp else f"experiment_r{rank}_m{m}",
+                                   subdir=f"setting_{args.experiment}", root=args.experiments_root,
+                                   rng=random.Random(args.seed + g))
             tuned = exps[m].save_configs(cfg)
             if args.tune:
                 configs[m] = tuned
     pop = S.AgentPopulation(cfg, P, n_local, seed=args.seed, rank=rank, device=local_rank, configs=configs,
                             experiment_dirs=[e.experiment_dir if e else None for e in exps],
-                            buffer_size=max(args.buffer, n_local * args.collect_steps))
+                            buffer_size=max(args.buffer, n_local * args.collect_steps),
+                            data_parallel=group if dp else None)
     pop.reset()
     losses = None
     rows, best = [[] for _ in range(P)], [float("-inf")] * P
     prev = [{"episodes": 0.0, "return_sum": 0.0} for _ in range(P)]
     pbt_prev = [{"episodes": 0.0, "return_sum": 0.0} for _ in range(P)]
-    pbt_log, pbt_rng = [], random.Random(1000 + args.seed + rank)
+    # data-parallel: one rng for every rank, so that all ranks make the same population rounds
+    pbt_log, pbt_rng = [], random.Random(1000 + args.seed + (0 if dp else rank))
 
     def interval_score(c, p):
         n = c["episodes"] - p["episodes"]
@@ -327,17 +351,18 @@ def train_population(args, rank, local_rank, world):
             out = pop.learn()
             losses = out if out is not None else losses
         if args.pbt_every and it % args.pbt_every == 0:
-            counters = [env.counters() for env in pop.envs]
+            counters = pop.counters()   # data-parallel: summed over the ranks
             scores = [interval_score(c, p) for c, p in zip(counters, pbt_prev)]
             pbt_prev = counters
             info = pop.exploit_explore(scores, pbt_rng)
             pbt_log.append({"iter": it, "scores": info["scores"], "ranking": info["ranking"],
                             "adopted": {m: {"from": info["best"], "hp": hp} for m, hp in info["adopted"].items()}})
         if args.log_every and it % args.log_every == 0:
-            for m, (a, env, exp) in enumerate(zip(pop.members, pop.envs, exps)):
+            counters = pop.counters() if dp or args.experiments_root or rank == 0 else None
+            for m, (a, exp) in enumerate(zip(pop.members, exps)):
                 if exp is None:
                     continue
-                c = env.counters()
+                c = counters[m]
                 score = interval_score(c, prev[m])
                 n = c["episodes"] - prev[m]["episodes"]
                 prev[m] = c
@@ -348,7 +373,7 @@ def train_population(args, rank, local_rank, world):
                 avg = c["return_sum"] / c["episodes"] if c["episodes"] else float("nan")
                 rows[m].append([(rank, it), f"{kind}-{int(c[kind])}", score, best[m], avg, "", ""])
             if rank == 0:
-                c = [env.counters() for env in pop.envs]
+                c = counters
                 lv = [float(x) for x in losses[0]] if losses is not None else [float("nan")] * 3
                 print(f"iter {it:6d}  episodes {sum(x['episodes'] for x in c):.0f}  goals "
                       f"{sum(x['reached_goal'] for x in c):.0f}  member 0 losses v/pi/q {lv[0]:.3g} {lv[1]:.3g} "
@@ -357,30 +382,33 @@ def train_population(args, rank, local_rank, world):
     torch.cuda.synchronize()
     ms = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device="cuda")
     if world > 1:
-        torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
+        torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX, group=group)
     total = torch.stack([env.counters_tensor() for env in pop.envs]).sum(0)
-    stats = S.all_reduce_counters(total)
+    stats = S.all_reduce_counters(total, group=group)
+    final = pop.counters()   # data-parallel: summed over the ranks
     sec = float(ms.item()) * 1e-3
-    members_total = P * world
+    members_total = P if dp else P * world
     summary = {"example": "train_sac", "overrides": overrides, "n_gpus": world, "envs_total": args.envs,
                "iters": args.iters, "updates_per_iter": args.updates_per_iter, "cuda_graph": not args.no_graph,
                "overlap": False, "policy_precision": args.policy_precision,
                "learner_precision": args.learner_precision, "collect_steps": args.collect_steps,
                "members": members_total, "members_per_gpu": P, "envs_per_member": n_local,
-               "env_steps_per_s": args.iters * args.collect_steps * n_local * members_total / sec,
+               "env_steps_per_s": args.iters * args.collect_steps * n_local * P * world / sec,
                "updates_per_s_per_replica": args.iters * args.updates_per_iter / sec,
                "updates_per_s_aggregate": args.iters * args.updates_per_iter * members_total / sec,
                "ms_per_iter": 1e3 * sec / args.iters, "episodes": stats["episodes"],
                "mean_return": stats["return_mean"], "reached_goal": stats["reached_goal"],
                "losses_v_pi_q": [[float(x) for x in l] for l in losses] if losses is not None else None}
     summary["env_steps_per_s_aggregate"] = summary["env_steps_per_s"]
+    if dp:
+        summary["data_parallel"], summary["effective_batch"] = True, world * pop.batch_size
     if args.pbt_every:
         summary["pbt_rounds"] = len(pbt_log)
         summary["pbt_adoptions"] = [e for e in pbt_log if e["adopted"]]
         summary["hyperparameters"] = [a.hyperparameters() for a in pop.members]
-    if args.experiments_root:
-        for m, (a, env, exp) in enumerate(zip(pop.members, pop.envs, exps)):
-            c = env.counters()
+    if args.experiments_root and exps[0] is not None:
+        for m, (a, exp) in enumerate(zip(pop.members, exps)):
+            c = final[m]
             exp.write_console(rows[m])
             exp.append_overview(best[m])
             exp.write_terminations(S.info_from_counters(c, max(S.TERM_NAMES[1:], key=lambda k: c[k])))
@@ -389,7 +417,7 @@ def train_population(args, rank, local_rank, world):
         if args.tune:
             summary["hpsets"] = [e.tuner.hpset for e in exps]
         mine = max((b, rank, e.experiment_name) for b, e in zip(best, exps))
-        if world > 1:
+        if world > 1 and not dp:
             scores = [None] * world
             torch.distributed.all_gather_object(scores, mine)
             mine = max(scores)
@@ -397,8 +425,6 @@ def train_population(args, rank, local_rank, world):
     if rank == 0:
         print(json.dumps(summary), flush=True)
     pop.close()
-    if world > 1:
-        torch.distributed.destroy_process_group()
     return summary
 
 

@@ -478,6 +478,30 @@ typedef struct boatagent_sac_member {
 BOATENV_API int boatagent_sac_update_members(const boatagent_sac_member *members_host, int32_t n_members,
                                              int64_t batch, float beta1, float beta2, float adam_eps, void *workspace,
                                              int64_t workspace_bytes, void *stream);
+/* Data-parallel population training: boatagent_sac_update_members split as boatagent_sac_gradients splits
+ * boatagent_sac_update, so that each member's gradients can be all-reduced over the ranks that train it.
+ *
+ * boatagent_sac_gradients_members: boatagent_sac_gradients of every member in one launch pair.  Each slot's `grad`
+ * receives grad_scale times the member's batch gradient and `losses` grad_scale times its three losses; parameters,
+ * targets, Adam moments and step counters are not written, `tau` and `adam_state` are not read (adam_state may be
+ * NULL).  Member m's results equal a boatagent_sac_gradients call with its entry's arguments, bit for bit.  Table,
+ * workspace and errors as boatagent_sac_update_members, without the adam_state check.
+ *
+ * boatagent_adam_polyak_members: boatagent_adam_polyak_step(slots, 26, beta1, beta2, adam_eps, tau, adam_state) of
+ * every member in one launch (member m on blockIdx.y = m, the same 2048-element chunks on blockIdx.x): each member
+ * reads its slots' `grad`, steps with its slots' learning rates, its `tau` and its adam_state, bit for bit as that
+ * call.  The batch, draw and loss pointers are not read.  Members must not share parameters, moments, targets or
+ * adam_state.  Errors (checked for every member before anything is launched): BOATENV_EINVAL for a NULL table,
+ * n_members outside 1..BOATAGENT_SAC_MAX_MEMBERS, n_slots != 26, a NULL slot pointer, a slot whose numel is not the
+ * agent's shape, a missing or extra target, a NULL adam_state.
+ *
+ * With grad_scale = 1, boatagent_sac_gradients_members followed by boatagent_adam_polyak_members equals
+ * boatagent_sac_update_members bit for bit: gradients, weights, targets, Adam moments, step counters and losses. */
+BOATENV_API int boatagent_sac_gradients_members(const boatagent_sac_member *members_host, int32_t n_members,
+                                                int64_t batch, float grad_scale, void *workspace,
+                                                int64_t workspace_bytes, void *stream);
+BOATENV_API int boatagent_adam_polyak_members(const boatagent_sac_member *members_host, int32_t n_members, float beta1,
+                                              float beta2, float adam_eps, void *stream);
 
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 

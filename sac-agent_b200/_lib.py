@@ -92,6 +92,8 @@ SIGNATURES = {
                                           vp, vp, i64, vp]),
     "boatagent_sac_update_members": (C.c_int, [C.POINTER(SacMember), i32, i64, C.c_float, C.c_float, C.c_float, vp,
                                                i64, vp]),
+    "boatagent_sac_gradients_members": (C.c_int, [C.POINTER(SacMember), i32, i64, C.c_float, vp, i64, vp]),
+    "boatagent_adam_polyak_members": (C.c_int, [C.POINTER(SacMember), i32, C.c_float, C.c_float, C.c_float, vp]),
     "boatreplay_sample_members": (C.c_int, [C.POINTER(SampleMember), i32, i64, vp]),
     "boatreplay_create": (C.c_int, [i64, i32, i32, C.c_int, C.c_int, C.POINTER(vp)]),
     "boatreplay_destroy": (C.c_int, [vp]),

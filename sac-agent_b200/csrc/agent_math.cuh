@@ -69,4 +69,47 @@ __device__ __forceinline__ void adam_bias_corrections(long long t_steps, float b
     bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, t));
 }
 
+// The coalesced Adam + Polyak step of one agent's n_slots slots (agent_ops.cu's adam_polyak_kernel, and each member
+// of learner.cu's adam_polyak_members_kernel): CTA `chunk` of the `n_ctas` CTAs that step the agent takes kAdamChunk
+// consecutive elements of one slot (the slots' chunks in slot order), and the last of them to finish advances the step
+// counter state[0] (state[1] is its ticket).
+constexpr int kAdamChunk = 2048, kAdamThreads = 256;
+__device__ __forceinline__ void adam_polyak_chunk(const boatagent_adam_slot *slot, int n_slots, float beta1,
+                                                  float beta2, float eps, float tau, long long *__restrict__ state,
+                                                  long long chunk, unsigned n_ctas, int tid) {
+    __shared__ int s_slot;
+    __shared__ long long s_first;
+    __shared__ float s_bc1, s_bc2_sqrt;
+    if (tid == 0) {
+        int k = 0;
+        for (; k < n_slots; ++k) {
+            const long long nchunks = (slot[k].numel + kAdamChunk - 1) / kAdamChunk;
+            if (chunk < nchunks) break;
+            chunk -= nchunks;
+        }
+        s_slot = k;
+        s_first = chunk * kAdamChunk;
+        // this step's number
+        adam_bias_corrections(*reinterpret_cast<volatile long long *>(state) + 1, beta1, beta2, s_bc1, s_bc2_sqrt);
+    }
+    __syncthreads();
+    if (s_slot < n_slots) {
+        const boatagent_adam_slot &sl = slot[s_slot];
+        const float step_size = sl.lr / s_bc1;
+        const long long end = min(s_first + (long long)kAdamChunk, (long long)sl.numel);
+        for (long long i = s_first + tid; i < end; i += kAdamThreads) {
+            adam_polyak_element(sl, i, sl.grad[i], beta1, beta2, eps, tau, step_size, s_bc2_sqrt);
+        }
+    }
+    __syncthreads();
+    if (tid == 0) {  // the last CTA to finish publishes the new step count
+        __threadfence();
+        const unsigned long long done = atomicAdd(reinterpret_cast<unsigned long long *>(state + 1), 1ULL) + 1ULL;
+        if (done == n_ctas) {
+            state[1] = 0;
+            state[0] += 1;
+        }
+    }
+}
+
 }  // namespace boatenv

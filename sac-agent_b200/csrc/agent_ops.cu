@@ -86,7 +86,8 @@ int boatagent_gaussian_head_backward(const float *mean, const float *raw_std, co
 // ---------------------------------------------------------------------------------
 namespace {
 
-constexpr int kAdamChunk = 2048, kAdamThreads = 256;
+using boatenv::kAdamChunk;
+using boatenv::kAdamThreads;
 struct AdamTable {
     boatagent_adam_slot slot[BOATAGENT_ADAM_MAX_SLOTS];
     int n_slots;
@@ -95,41 +96,8 @@ struct AdamTable {
 
 __global__ void __launch_bounds__(kAdamThreads) adam_polyak_kernel(const __grid_constant__ AdamTable tab,
                                                                    long long *__restrict__ state /* [step, ticket] */) {
-    __shared__ int s_slot;
-    __shared__ long long s_first;
-    __shared__ float s_bc1, s_bc2_sqrt;
-    if (threadIdx.x == 0) {
-        long long chunk = blockIdx.x;
-        int k = 0;
-        for (; k < tab.n_slots; ++k) {
-            const long long nchunks = (tab.slot[k].numel + kAdamChunk - 1) / kAdamChunk;
-            if (chunk < nchunks) break;
-            chunk -= nchunks;
-        }
-        s_slot = k;
-        s_first = chunk * kAdamChunk;
-        // this step's number
-        boatenv::adam_bias_corrections(*reinterpret_cast<volatile long long *>(state) + 1, tab.beta1, tab.beta2, s_bc1,
-                                       s_bc2_sqrt);
-    }
-    __syncthreads();
-    if (s_slot < tab.n_slots) {
-        const boatagent_adam_slot &sl = tab.slot[s_slot];
-        const float step_size = sl.lr / s_bc1;
-        const long long end = min(s_first + (long long)kAdamChunk, (long long)sl.numel);
-        for (long long i = s_first + threadIdx.x; i < end; i += kAdamThreads) {
-            boatenv::adam_polyak_element(sl, i, sl.grad[i], tab.beta1, tab.beta2, tab.eps, tab.tau, step_size, s_bc2_sqrt);
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {  // the last CTA to finish publishes the new step count
-        __threadfence();
-        const unsigned long long done = atomicAdd(reinterpret_cast<unsigned long long *>(state + 1), 1ULL) + 1ULL;
-        if (done == gridDim.x) {
-            state[1] = 0;
-            state[0] += 1;
-        }
-    }
+    boatenv::adam_polyak_chunk(tab.slot, tab.n_slots, tab.beta1, tab.beta2, tab.eps, tab.tau, state, blockIdx.x,
+                               gridDim.x, threadIdx.x);
 }
 
 }  // namespace

@@ -14,7 +14,10 @@
 //                     several replicas can be all-reduced before one Adam step.
 //
 // boatagent_sac_update_members runs the same two bodies for up to 16 independent agents in one launch each:
-// member m on blockIdx.y = m, with its own arguments, workspace slice and step counter.
+// member m on blockIdx.y = m, with its own arguments, workspace slice and step counter.  The data-parallel population
+// splits it as boatagent_sac_gradients splits the solo update: boatagent_sac_gradients_members (the row body and the
+// gradients-only parameter body), then, after the all-reduce, boatagent_adam_polyak_members (adam_polyak_kernel's
+// chunk body, agent_math.cuh, for every member in one launch).
 //
 // Operands in shared memory and in the workspace use the 8x8 core-matrix layout of actor_tc.cuh: element (r, c) of
 // an R-row matrix at (c / 8) * (R * 16) + r * 16 + (c % 8) * 2.  The same bytes are a K-major operand with rows = M/N
@@ -610,6 +613,17 @@ __global__ void __launch_bounds__(kPThreads) sac_params_members_kernel(const __g
     sac_params_block<true>(args.m[blockIdx.y], threadIdx.x);
 }
 
+// population gradients (boatagent_sac_gradients_members): member blockIdx.y
+__global__ void __launch_bounds__(kPThreads) sac_grads_members_kernel(const __grid_constant__ MemberParamArgs args) {
+    sac_params_block<false>(args.m[blockIdx.y], threadIdx.x);
+}
+
+// population Adam + Polyak step (boatagent_adam_polyak_members): member blockIdx.y, its chunks on blockIdx.x
+__global__ void __launch_bounds__(kAdamThreads) adam_polyak_members_kernel(const __grid_constant__ MemberParamArgs args) {
+    const ParamArgs &a = args.m[blockIdx.y];
+    adam_polyak_chunk(a.slot, kSlots, a.beta1, a.beta2, a.eps, a.tau, a.state, blockIdx.x, gridDim.x, threadIdx.x);
+}
+
 constexpr int kParamBlocks = 2 * kNets + kNets * (kHidden / 8) + 1;
 
 // numel of slot k, in DeviceAdam's order (actor: fc1 w, b, fc2 w, b, mean w, b, std w, b; critics and value: fc1 w, b,
@@ -617,6 +631,13 @@ constexpr int kParamBlocks = 2 * kNets + kNets * (kHidden / 8) + 1;
 constexpr long long expected_numel(int k) {
     const int t = k < 8 ? k : (k - 8) % 6, in = (k >= 8 && k < 20) ? kObs + 1 : kObs;
     return t == 0 ? (long long)kHidden * in : t == 2 ? (long long)kHidden * kHidden : (t == 5 || t == 7) ? 1 : kHidden;
+}
+
+// the CTAs of one agent's Adam step: the chunks of its 26 slots, as boatagent_adam_polyak_step counts them
+constexpr int adam_chunks() {
+    long long n = 0;
+    for (int k = 0; k < kSlots; ++k) n += (expected_numel(k) + kAdamChunk - 1) / kAdamChunk;
+    return (int)n;
 }
 
 }  // namespace
@@ -697,6 +718,7 @@ int set_smem_attributes() {
         CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac_rows_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac_params_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac_grads_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         set_of[dev] = true;
     }
     return 0;
@@ -710,6 +732,56 @@ int sac_launch(const RowArgs &ra, const ParamArgs &pa, void *stream) {
     boatenv::count_launch();
     CUDA_TRY(cudaGetLastError());
     sac_params_kernel<kAdam><<<kParamBlocks, kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+    boatenv::count_launch();
+    return (int)cudaGetLastError();
+}
+
+MemberRowArgs &member_rows() {   // ~32 KB together: kept off the stack
+    static thread_local MemberRowArgs ra;
+    return ra;
+}
+MemberParamArgs &member_params() {
+    static thread_local MemberParamArgs pa;
+    return pa;
+}
+
+// The member tables of boatagent_sac_update_members and boatagent_sac_gradients_members: every member checked as
+// boatagent_sac_update checks its arguments (its adam_state only with `adam`), before anything is launched.  The
+// shared Adam hyper-parameters stay unset.
+int member_tables(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch, void *workspace,
+                  int64_t workspace_bytes, bool adam, float grad_scale, MemberRowArgs &ra, MemberParamArgs &pa) {
+    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
+    if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
+    const size_t slice = ws_bytes(batch / kRows);   // a multiple of 16: every slice stays 16-byte aligned
+    if (workspace_bytes < 0 || (uint64_t)workspace_bytes < slice * (uint64_t)n_members) return BOATENV_EINVAL;
+    std::memset(&ra, 0, sizeof(ra));
+    std::memset(&pa, 0, sizeof(pa));
+    for (int m = 0; m < n_members; ++m) {
+        const boatagent_sac_member &b = members_host[m];
+        if (adam && !b.adam_state) return BOATENV_EINVAL;
+        unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
+        const int rc = sac_args(b.state, b.action, b.reward, b.new_state, b.done, b.eps, b.max_action, batch, b.gamma,
+                                b.reward_scale, b.slots, b.n_slots, b.losses, ws, (int64_t)slice, ra.m[m], pa.m[m]);
+        if (rc != 0) return rc;
+        pa.m[m].tau = b.tau;
+        pa.m[m].state = (long long *)b.adam_state;
+        pa.m[m].grad_scale = grad_scale;
+    }
+    return 0;
+}
+
+int members_launch(bool adam, int32_t n_members, int64_t batch, const MemberRowArgs &ra, const MemberParamArgs &pa,
+                   void *stream) {
+    const int rc = set_smem_attributes();
+    if (rc != 0) return rc;
+    sac_rows_members_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem,
+                              (cudaStream_t)stream>>>(ra);
+    boatenv::count_launch();
+    CUDA_TRY(cudaGetLastError());
+    if (adam)
+        sac_params_members_kernel<<<dim3(kParamBlocks, (unsigned)n_members), kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+    else
+        sac_grads_members_kernel<<<dim3(kParamBlocks, (unsigned)n_members), kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
     boatenv::count_launch();
     return (int)cudaGetLastError();
 }
@@ -756,35 +828,49 @@ extern "C" int boatagent_sac_gradients(const float *state, const float *action, 
 extern "C" int boatagent_sac_update_members(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch,
                                             float beta1, float beta2, float adam_eps, void *workspace,
                                             int64_t workspace_bytes, void *stream) {
-    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
-    if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
-    const size_t slice = ws_bytes(batch / kRows);   // a multiple of 16: every slice stays 16-byte aligned
-    if (workspace_bytes < 0 || (uint64_t)workspace_bytes < slice * (uint64_t)n_members) return BOATENV_EINVAL;
-    static thread_local MemberRowArgs ra;   // ~32 KB together: kept off the stack
-    static thread_local MemberParamArgs pa;
-    std::memset(&ra, 0, sizeof(ra));
+    MemberRowArgs &ra = member_rows();
+    MemberParamArgs &pa = member_params();
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, 1.0f, ra, pa);
+    if (rc != 0) return rc;
+    for (int m = 0; m < n_members; ++m) {
+        pa.m[m].beta1 = beta1;
+        pa.m[m].beta2 = beta2;
+        pa.m[m].eps = adam_eps;
+    }
+    return members_launch(true, n_members, batch, ra, pa, stream);
+}
+
+extern "C" int boatagent_sac_gradients_members(const boatagent_sac_member *members_host, int32_t n_members,
+                                               int64_t batch, float grad_scale, void *workspace,
+                                               int64_t workspace_bytes, void *stream) {
+    MemberRowArgs &ra = member_rows();
+    MemberParamArgs &pa = member_params();
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, false, grad_scale, ra, pa);
+    if (rc != 0) return rc;
+    return members_launch(false, n_members, batch, ra, pa, stream);
+}
+
+extern "C" int boatagent_adam_polyak_members(const boatagent_sac_member *members_host, int32_t n_members, float beta1,
+                                             float beta2, float adam_eps, void *stream) {
+    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS) return BOATENV_EINVAL;
+    MemberParamArgs &pa = member_params();
     std::memset(&pa, 0, sizeof(pa));
     for (int m = 0; m < n_members; ++m) {
         const boatagent_sac_member &b = members_host[m];
-        if (!b.adam_state) return BOATENV_EINVAL;
-        unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
-        const int rc = sac_args(b.state, b.action, b.reward, b.new_state, b.done, b.eps, b.max_action, batch, b.gamma,
-                                b.reward_scale, b.slots, b.n_slots, b.losses, ws, (int64_t)slice, ra.m[m], pa.m[m]);
-        if (rc != 0) return rc;
+        if (!b.adam_state || !b.slots || b.n_slots != kSlots) return BOATENV_EINVAL;
+        for (int k = 0; k < kSlots; ++k) {
+            const boatagent_adam_slot &s = b.slots[k];
+            if (!s.param || !s.grad || !s.exp_avg || !s.exp_avg_sq || s.numel != expected_numel(k)) return BOATENV_EINVAL;
+            if ((k >= 20) != (s.target != nullptr)) return BOATENV_EINVAL;   // the value network's tensors, and only they
+            pa.m[m].slot[k] = s;
+        }
         pa.m[m].beta1 = beta1;
         pa.m[m].beta2 = beta2;
         pa.m[m].eps = adam_eps;
         pa.m[m].tau = b.tau;
         pa.m[m].state = (long long *)b.adam_state;
-        pa.m[m].grad_scale = 1.0f;
     }
-    const int rc = set_smem_attributes();
-    if (rc != 0) return rc;
-    sac_rows_members_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem,
-                              (cudaStream_t)stream>>>(ra);
-    boatenv::count_launch();
-    CUDA_TRY(cudaGetLastError());
-    sac_params_members_kernel<<<dim3(kParamBlocks, (unsigned)n_members), kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+    adam_polyak_members_kernel<<<dim3(adam_chunks(), (unsigned)n_members), kAdamThreads, 0, (cudaStream_t)stream>>>(pa);
     boatenv::count_launch();
     return (int)cudaGetLastError();
 }

@@ -16,6 +16,9 @@ On ONE GPU, ``AgentPopulation`` trains P members in one process: each member is 
 own env, ring, experiment directory and hyper-parameters, and one ``learn()`` updates all of them in four launches (one
 sample-gather for every ring, one Gaussian draw, the two kernels of ``boatagent_sac_update_members``).
 ``exploit_explore_local`` is ``exploit_explore`` over such members, with device copies instead of collectives.
+With ``data_parallel``, every member is ONE agent trained by all ranks of a process group: each rank holds its own
+env shard and ring of every member, and one update round of all members is one gradient launch pair, one all-reduce
+and one Adam launch.
 """
 from __future__ import annotations
 
@@ -131,12 +134,23 @@ class AgentPopulation:
     initial weights drawn under torch seed ``seed + g`` and its tcgen05 acting seed 0x5ac + g.  With P = 1 and rank 0
     that is the agent ``examples/train_sac.py`` builds with the same seed, bit for bit.
 
+    ``data_parallel``: a torch.distributed process group (True: the default group) of W ranks that train every member
+    together; ``rank`` is then the rank r in that group.  Each rank holds ``envs_per_member`` envs of each member
+    (global env ids from (m W + r) envs_per_member, so a member's W shards are contiguous), its own ring of each member
+    (ring seed ``seed + r P + m``) and its own acting seed 0x5ac + r P + m.  The initial weights are drawn under torch
+    seed ``seed + m`` and rank 0's training tensors are broadcast once; every rank must pass the same P, batch size and
+    ``envs_per_member`` (checked here).  ``learn()`` computes every member's gradients of this rank's batch times 1 / W,
+    sums them over the ranks with one all-reduce and applies the same Adam step on every rank, so the members stay
+    bit-identical across ranks (1 / W is exact for power-of-two W).  At W = 1 this is the plain population, bit for
+    bit.  Population rounds (``exploit_explore``) keep the ranks identical when every rank passes the same scores
+    (``counters()`` sums them over the ranks) and an identically seeded rng.
+
     ``configs``: one config per member (e.g. its tuned_configs.yaml draw), else ``config`` for all; the batch size must
     be the same.  Change a member's hyper-parameters through ``set_hyperparameters`` or ``exploit_explore`` so that
     the next ``learn()`` sees them."""
 
     def __init__(self, config, members, envs_per_member, seed=0, rank=0, device=None, configs=None,
-                 experiment_dirs=None, buffer_size=None, done_flag_mode=1):
+                 experiment_dirs=None, buffer_size=None, done_flag_mode=1, data_parallel=None):
         import torch
         from . import _lib
         from .boat_env import BatchedBoatEnv
@@ -155,17 +169,28 @@ class AgentPopulation:
             raise ValueError("AgentPopulation: the members share one batch size")
         self._L, self._lib = _lib.lib(), _lib
         self.device = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        self._dp = None   # (group, world) in data-parallel mode
+        if data_parallel is not None and data_parallel is not False:
+            import torch.distributed as dist
+            if not (dist.is_available() and dist.is_initialized()):
+                raise ValueError("AgentPopulation: data_parallel needs an initialised torch.distributed process group")
+            group = None if data_parallel is True else data_parallel
+            self._dp = (group, dist.get_world_size(group))
+            rank = dist.get_rank(group)
         self.rank, self.seed, self.done_flag_mode = int(rank), int(seed), int(done_flag_mode)
+        W, E = (self._dp[1] if self._dp else 1), int(envs_per_member)
         self.envs, self.members = [], []
         for m in range(P):
             g = self.rank * P + m
             cfg = configs[m]
-            env = BatchedBoatEnv(cfg, envs_per_member, seed=seed, precision="fp32", device=self.device.index,
-                                 env_id_offset=g * int(envs_per_member), auto_reset=True)
+            # data-parallel: member m's W shards are contiguous, and its weights do not depend on the rank
+            first_env, weight_seed = ((m * W + self.rank) * E, seed + m) if self._dp else (g * E, seed + g)
+            env = BatchedBoatEnv(cfg, E, seed=seed, precision="fp32", device=self.device.index,
+                                 env_id_offset=first_env, auto_reset=True)
             size = int(cfg.agent.max_size) if buffer_size is None else int(buffer_size)
             mem = ReplayBuffer(size, (11,), 1, precision="fp32", device=self.device.index, seed=seed + g, as_torch=True)
             with torch.random.fork_rng(devices=[self.device]):
-                torch.manual_seed(seed + g)
+                torch.manual_seed(weight_seed)
                 agent = ContinuousAgent(cfg, dirs[m], env.observation_space.shape, env, device=self.device.index,
                                         seed=seed + g, memory=mem, policy_precision="tcgen05",
                                         learner_precision="tcgen05")
@@ -181,6 +206,44 @@ class AgentPopulation:
                                device=self.device)
         self._sample = (_lib.SampleMember * P)()
         self._table = None
+        self._flat = None
+        if self._dp is not None:
+            self._init_data_parallel(E)
+
+    def _init_data_parallel(self, envs_per_member):
+        """Checks that every rank holds the same population, points every member's gradients and losses into one flat
+        [P, n_params + 3] buffer (one all-reduce per round) and starts every rank from rank 0's members."""
+        import torch
+        import torch.distributed as dist
+        group, world = self._dp
+        P = len(self.members)
+        shape = torch.tensor([P, self.batch_size, envs_per_member], dtype=torch.int64, device=self.device)
+        both = torch.cat([shape, -shape])
+        dist.all_reduce(both, op=dist.ReduceOp.MAX, group=group)
+        if not torch.equal(both[:3], -both[3:]):
+            raise ValueError(f"AgentPopulation: every rank of the data-parallel group needs the same members, batch "
+                             f"size and envs per member (this rank: {P}, {self.batch_size}, {envs_per_member}; "
+                             f"largest over the ranks: {both[:3].tolist()})")
+        params = self.members[0].learner.optimizer.params
+        n = sum(p.numel() for p in params)
+        self._flat = torch.zeros((P, n + 3), dtype=torch.float32, device=self.device)
+        for m, a in enumerate(self.members):
+            off = 0
+            for p in a.learner.optimizer.params:
+                p.grad = self._flat[m, off:off + p.numel()].view_as(p)
+                off += p.numel()
+            a._loss_buf = self._flat[m, n:]
+            a._losses = tuple(a._loss_buf[k] for k in range(3))
+        src = 0 if group is None else dist.get_global_rank(group, 0)
+        for a in self.members:
+            for t in a.training_tensors():
+                dist.broadcast(t, src=src, group=group)
+            a._weights_changed()
+
+    @property
+    def data_parallel(self):
+        """True when every member is trained by a process group (constructor argument ``data_parallel``)."""
+        return self._dp is not None
 
     def __len__(self):
         return len(self.members)
@@ -219,7 +282,11 @@ class AgentPopulation:
     def learn(self):
         """One update of every member: the batched sample-gather, one Gaussian draw for all, and the two kernels of
         boatagent_sac_update_members (no sync).  Returns each member's (value, actor, critic) losses as device
-        tensors, or None (nothing launched) while some member's ring holds less than a batch."""
+        tensors, or None (nothing launched) while some member's ring holds less than a batch.
+
+        Data-parallel: the update is boatagent_sac_gradients_members (times 1 / W), one all-reduce (SUM) of every
+        member's gradients and losses, and boatagent_adam_polyak_members; the losses are the means over the ranks.
+        The rank shards are equal, so all ranks start updating at the same call without a vote."""
         if any(a.memory.mem_cntr < self.batch_size for a in self.members):
             return None
         import torch
@@ -234,12 +301,34 @@ class AgentPopulation:
             a.memory._samples += 1
         self.eps.normal_()
         o = self.members[0].learner.optimizer
-        self._lib.check(self._L.boatagent_sac_update_members(self._table, P, B, o.betas[0], o.betas[1], o.eps,
-                                                             self._ws.data_ptr(), self._ws.numel(), stream),
-                        "boatagent_sac_update_members")
+        if self._dp is None:
+            self._lib.check(self._L.boatagent_sac_update_members(self._table, P, B, o.betas[0], o.betas[1], o.eps,
+                                                                 self._ws.data_ptr(), self._ws.numel(), stream),
+                            "boatagent_sac_update_members")
+        else:
+            import torch.distributed as dist
+            group, world = self._dp
+            self._lib.check(self._L.boatagent_sac_gradients_members(self._table, P, B, 1.0 / world,
+                                                                    self._ws.data_ptr(), self._ws.numel(), stream),
+                            "boatagent_sac_gradients_members")
+            dist.all_reduce(self._flat, op=dist.ReduceOp.SUM, group=group)
+            self._lib.check(self._L.boatagent_adam_polyak_members(self._table, P, o.betas[0], o.betas[1], o.eps, stream),
+                            "boatagent_adam_polyak_members")
         for a in self.members:
             a.updates += 1
         return [a._losses for a in self.members]
+
+    def counters(self):
+        """Each member's episode counters (``BatchedBoatEnv.counters()`` dicts), in member order.  Data-parallel: summed
+        over the ranks with one all-reduce of a [P, 8] float64 tensor (collective), so every rank gets the same."""
+        if self._dp is None:
+            return [env.counters() for env in self.envs]
+        import torch
+        import torch.distributed as dist
+        from .boat_env import COUNTER_NAMES
+        c = torch.stack([env.counters_tensor() for env in self.envs])
+        dist.all_reduce(c, op=dist.ReduceOp.SUM, group=self._dp[0])
+        return [dict(zip(COUNTER_NAMES, row)) for row in c.cpu().tolist()]
 
     def set_hyperparameters(self, m, **hp):
         """``ContinuousAgent.set_hyperparameters`` of member m, seen by the next ``learn()``."""
@@ -247,7 +336,9 @@ class AgentPopulation:
         self._table = None
 
     def exploit_explore(self, scores, rng: random.Random, bottom_fraction: float = 0.25):
-        """One population round over the members (``exploit_explore_local``)."""
+        """One population round over the members (``exploit_explore_local``).  Data-parallel: every rank must call it
+        with the same scores (e.g. from ``counters()``) and an identically seeded rng, so that all ranks make the same
+        round and their members stay bit-identical."""
         info = exploit_explore_local(self.members, scores, rng, bottom_fraction)
         self._table = None
         return info
