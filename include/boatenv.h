@@ -427,7 +427,8 @@ BOATENV_API int boatagent_collect_record(boatenv_t h, boatreplay_t r, const void
  *   workspace: boatagent_sac_update_workspace_bytes(batch) device bytes, 16-byte aligned.
  * Errors: BOATENV_EINVAL for NULL pointers, a batch that is not a positive multiple of 128, n_slots != 26, a slot
  * whose numel is not the agent's shape, a missing or extra target, a workspace that is too small; BOATENV_EALIGN for
- * a workspace or parameter that is not 16-byte aligned. */
+ * a workspace or parameter that is not 16-byte aligned.
+ * This is the one-member case of boatagent_sac_update_members below. */
 BOATENV_API int64_t boatagent_sac_update_workspace_bytes(int64_t batch);   /* BOATENV_EINVAL for a bad batch */
 BOATENV_API int boatagent_sac_update(const float *state, const float *action, const float *reward,
                                      const float *new_state, const uint8_t *done, const float *eps,
@@ -443,7 +444,8 @@ BOATENV_API int boatagent_sac_update(const float *state, const float *action, co
  * all-reduce the mean, exactly when world is a power of two.
  * With grad_scale = 1, this call followed by boatagent_adam_polyak_step on the same slots (and the same adam_state)
  * equals one boatagent_sac_update bit for bit: gradients, weights, targets, Adam moments, step counter and losses.
- * The split costs one extra launch (the Adam kernel). */
+ * The split costs one extra launch (the Adam kernel).  This is the one-member case of boatagent_sac_gradients_members
+ * below. */
 BOATENV_API int boatagent_sac_gradients(const float *state, const float *action, const float *reward,
                                         const float *new_state, const uint8_t *done, const float *eps,
                                         const float *max_action, int64_t batch, float gamma, float reward_scale,
@@ -493,7 +495,8 @@ BOATENV_API int boatagent_sac_update_members(const boatagent_sac_member *members
  * call.  The batch, draw and loss pointers are not read.  Members must not share parameters, moments, targets or
  * adam_state.  Errors (checked for every member before anything is launched): BOATENV_EINVAL for a NULL table,
  * n_members outside 1..BOATAGENT_SAC_MAX_MEMBERS, n_slots != 26, a NULL slot pointer, a slot whose numel is not the
- * agent's shape, a missing or extra target, a NULL adam_state.
+ * agent's shape, a missing or extra target, a NULL adam_state; BOATENV_EALIGN for a parameter that is not 16-byte
+ * aligned (the slots are checked as boatagent_sac_update checks them).
  *
  * With grad_scale = 1, boatagent_sac_gradients_members followed by boatagent_adam_polyak_members equals
  * boatagent_sac_update_members bit for bit: gradients, weights, targets, Adam moments, step counters and losses. */

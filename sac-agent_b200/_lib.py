@@ -39,7 +39,7 @@ class RecordRing(C.Structure):
                                         "term", "episode")] + [("capacity", i64)]
 
 class SacMember(C.Structure):
-    """boatagent_sac_member: one population member's arguments of boatagent_sac_update_members."""
+    """boatagent_sac_member: one agent's arguments of boatagent_sac_update_members and its split calls."""
     _fields_ = [(name, vp) for name in ("state", "action", "reward", "new_state", "done", "eps", "max_action",
                                         "slots")] + [("n_slots", i32), ("gamma", C.c_float), ("reward_scale", C.c_float),
                                                      ("tau", C.c_float), ("adam_state", vp), ("losses", vp)]

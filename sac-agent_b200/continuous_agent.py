@@ -92,6 +92,94 @@ class DeviceAdam:
         return {"state": self.state, "exp_avg": self.exp_avg, "exp_avg_sq": self.exp_avg_sq}
 
 
+class FusedLearner:
+    """The fused tcgen05 update (csrc/learner.cu) of 1 to 16 `ContinuousAgent`s with learner_precision "tcgen05", one
+    batch size and one device: each agent's batch (`_batch`, `_eps`), networks, `DeviceAdam` and hyper-parameters, one
+    member of every launch.  A launch writes each agent's batch gradients into its parameters' `.grad` tensors and its
+    three losses into its `_loss_buf`, on the current stream (no sync):
+
+      update()          one SAC update of every agent (boatagent_sac_update_members, two launches);
+      gradients(scale)  scale times the gradients and losses only (boatagent_sac_gradients_members, two launches),
+                        for an all-reduce before
+      adam()            Adam + Polyak of every agent from its `.grad` tensors (boatagent_adam_polyak_members, one
+                        launch).
+
+    The learning rates are read from the agents' DeviceAdam slots and gamma, reward scale and tau from their learners at
+    every launch, so `ContinuousAgent.set_hyperparameters` reaches the next one.  The other pointers (batch, draws,
+    `.grad` tensors, losses) are taken at the first launch and must stay the same tensors after it."""
+
+    @staticmethod
+    def check(agent):
+        """The agent the kernels are written for: 11 observations, one action, 256-wide hidden layers and a batch size
+        that is a positive multiple of 128."""
+        B, L = agent.batch_size, agent.learner
+        if agent.input_dims != (11,) or agent.get_n_actions() != 1 or B <= 0 or B % 128:
+            raise ValueError("learner_precision='tcgen05': the BoatEnv agent (11 observations, one action) and a "
+                             f"batch size that is a positive multiple of 128 (got {agent.input_dims}, "
+                             f"{agent.get_n_actions()} actions, batch {B})")
+        if any(tuple(p.shape) != (256, 256) for p in (L.actor.fc2.weight, L.critic_1.fc2.weight,
+                                                      L.critic_2.fc2.weight, L.value.fc2.weight)):
+            raise ValueError("learner_precision='tcgen05': 256-wide hidden layers only")
+
+    def __init__(self, agents):
+        self.agents = list(agents)
+        a0 = self.agents[0]
+        if not 1 <= len(self.agents) <= 16 or any(a.batch_size != a0.batch_size or a.device != a0.device
+                                                  for a in self.agents):
+            raise ValueError("FusedLearner: 1 to 16 agents (BOATAGENT_SAC_MAX_MEMBERS) of one batch size and device")
+        for a in self.agents:
+            self.check(a)
+        o0 = a0.learner.optimizer
+        self._lib, self._L, self.device, self.batch_size = o0._lib, o0._L, a0.device, a0.batch_size
+        self.ws = torch.empty(len(self.agents) * int(self._L.boatagent_sac_update_workspace_bytes(self.batch_size)),
+                              dtype=torch.uint8, device=self.device)
+        self._table = None
+
+    def _launch(self, name, *args):
+        if self._table is None:   # on the first launch: like the fp32 learner, no .grad before the first update
+            self._table = (self._lib.SacMember * len(self.agents))()
+            for m, a in enumerate(self.agents):
+                o = a.learner.optimizer
+                for k, p in enumerate(o.params):   # the batch gradient goes where the fp32 learner leaves it
+                    if p.grad is None:
+                        p.grad = torch.zeros_like(p)
+                    o._slots[k].grad = p.grad.data_ptr()
+                s, act, r, s2, d = a._batch
+                self._table[m] = self._lib.SacMember(
+                    s.data_ptr(), act.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), a._eps.data_ptr(),
+                    a.learner.actor.max_action.data_ptr(), C.cast(o._slots, C.c_void_p), len(o.params), 0.0, 0.0, 0.0,
+                    o.state.data_ptr(), a._loss_buf.data_ptr())
+        for e, a in zip(self._table, self.agents):
+            L = a.learner
+            e.gamma, e.reward_scale, e.tau = float(L.gamma), float(L.scale), float(L.optimizer.tau)
+        with torch.cuda.device(self.device):   # the ABI launches on the current device
+            stream = torch.cuda.current_stream().cuda_stream
+            self._lib.check(getattr(self._L, name)(self._table, len(self.agents), *args, stream), name)
+
+    def update(self):
+        o = self.agents[0].learner.optimizer
+        self._launch("boatagent_sac_update_members", self.batch_size, o.betas[0], o.betas[1], o.eps,
+                     self.ws.data_ptr(), self.ws.numel())
+
+    def gradients(self, scale):
+        self._launch("boatagent_sac_gradients_members", self.batch_size, scale, self.ws.data_ptr(), self.ws.numel())
+
+    def adam(self):
+        o = self.agents[0].learner.optimizer
+        self._launch("boatagent_adam_polyak_members", o.betas[0], o.betas[1], o.eps)
+
+
+def point_grads_into(agent, row):
+    """Makes the agent's `.grad` tensors (DeviceAdam's order) and its three losses (`_loss_buf`, `_losses`) views of
+    `row`, a contiguous float32 tensor of n_params + 3 elements, so that one all-reduce of `row` averages them all."""
+    off = 0
+    for p in agent.learner.optimizer.params:
+        p.grad = row[off:off + p.numel()].view_as(p)
+        off += p.numel()
+    agent._loss_buf = row[off:off + 3]
+    agent._losses = tuple(agent._loss_buf[k] for k in range(3))
+
+
 class SACLearner:
     """The five networks, their Adam optimisers and one SAC-v1 update (continuous_agent.py:96-154)."""
 
@@ -259,8 +347,11 @@ class ContinuousAgent:
         self._losses = None
         self._act_graphs = {}
         self.updates = 0
+        self._fused = None   # this agent's one-member FusedLearner, created by its first update
         if learner_precision == "tcgen05":
-            self._init_fused_learner()
+            FusedLearner.check(self)
+            self._loss_buf = torch.zeros(3, **kw)
+            self._losses = tuple(self._loss_buf[k] for k in range(3))
         self._dp = None   # (group, flat gradient + loss buffer, its gradient views, grad_scale) in data-parallel mode
         if data_parallel is not None and data_parallel is not False:
             self._init_data_parallel(None if data_parallel is True else data_parallel)
@@ -376,35 +467,21 @@ class ContinuousAgent:
         s, a, r, s2, d = self._batch
         return self.learner.update(s, a, r, s2, d.bool(), eps_sample=self._eps[0], eps_rsample=self._eps[1])
 
-    def _init_fused_learner(self):
-        B, L = self.batch_size, self.learner
-        if self.input_dims != (11,) or self.get_n_actions() != 1 or B <= 0 or B % 128:
-            raise ValueError("learner_precision='tcgen05': the BoatEnv agent (11 observations, one action) and a "
-                             f"batch size that is a positive multiple of 128 (got {self.input_dims}, "
-                             f"{self.get_n_actions()} actions, batch {B})")
-        if any(tuple(p.shape) != (256, 256) for p in (L.actor.fc2.weight, L.critic_1.fc2.weight,
-                                                      L.critic_2.fc2.weight, L.value.fc2.weight)):
-            raise ValueError("learner_precision='tcgen05': 256-wide hidden layers only")
-        nbytes = int(L.optimizer._L.boatagent_sac_update_workspace_bytes(B))
-        self._ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-        self._loss_buf = torch.zeros(3, dtype=torch.float32, device=self.device)
-        self._losses = tuple(self._loss_buf[k] for k in range(3))
+    def _fused_learner(self):
+        """This agent's one-member FusedLearner.  Created on first use, so that the members of an AgentPopulation,
+        which the population's own FusedLearner updates, hold no workspace of their own."""
+        if self._fused is None:
+            self._fused = FusedLearner([self])
+        return self._fused
+
+    @property
+    def _ws(self):
+        """The workspace of this agent's one-member FusedLearner (boatagent_sac_update_workspace_bytes(batch) bytes)."""
+        return self._fused_learner().ws
 
     def _fused_update(self):
-        """One update in the two kernels of boatagent_sac_update on the current stream (no sync)."""
-        L, o = self.learner, self.learner.optimizer
-        for k, p in enumerate(o.params):   # the kernels write the batch gradient where the fp32 learner leaves it
-            if p.grad is None:
-                p.grad = torch.zeros_like(p)
-            o._slots[k].grad = p.grad.data_ptr()
-        s, a, r, s2, d = self._batch
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        with torch.cuda.device(self.device):
-            o._lib.check(o._L.boatagent_sac_update(
-                s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), self._eps.data_ptr(),
-                L.actor.max_action.data_ptr(), self.batch_size, float(L.gamma), float(L.scale), o._slots, len(o.params),
-                o.betas[0], o.betas[1], o.eps, o.tau, o.state.data_ptr(), self._loss_buf.data_ptr(),
-                self._ws.data_ptr(), self._ws.numel(), stream), "boatagent_sac_update")
+        """One update in the two fused learner kernels on the current stream (no sync)."""
+        self._fused_learner().update()
         return self._losses
 
     def _init_data_parallel(self, group):
@@ -419,16 +496,10 @@ class ContinuousAgent:
             raise ValueError(f"data_parallel: every rank needs the same number of envs (they hold {-int(n[1])} to "
                              f"{int(n[0])}); make the total divisible by the world size {world}")
         o = self.learner.optimizer
-        # every trained parameter's .grad is a view into one flat buffer, followed by the three losses: ONE all-reduce
         flat = torch.zeros(sum(p.numel() for p in o.params) + 3, dtype=torch.float32, device=self.device)
-        grads, off = [], 0
-        for p in o.params:
-            p.grad = flat[off:off + p.numel()].view_as(p)
-            grads.append(p.grad)
-            off += p.numel()
-        self._losses = tuple(flat[off + k] for k in range(3))
+        point_grads_into(self, flat)
         # grad_scale 1 / world: the SUM all-reduce is the mean (exact for power-of-two world sizes)
-        self._dp = (group, flat, grads, 1.0 / world)
+        self._dp = (group, flat, [p.grad for p in o.params], 1.0 / world)
         src = 0 if group is None else dist.get_global_rank(group, 0)
         for t in self.training_tensors():   # the ranks start from rank 0's agent
             dist.broadcast(t, src=src, group=group)
@@ -448,18 +519,8 @@ class ContinuousAgent:
         """gradients (scaled by 1 / world) -> all-reduce of gradients and losses -> Adam + Polyak on every rank."""
         import torch.distributed as dist
         group, flat, grads, scale = self._dp
-        L, o = self.learner, self.learner.optimizer
         if self.learner_precision == "tcgen05":
-            for k, g in enumerate(grads):
-                o._slots[k].grad = g.data_ptr()
-            s, a, r, s2, d = self._batch
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            with torch.cuda.device(self.device):
-                o._lib.check(o._L.boatagent_sac_gradients(
-                    s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), self._eps.data_ptr(),
-                    L.actor.max_action.data_ptr(), self.batch_size, float(L.gamma), float(L.scale), o._slots,
-                    len(o.params), scale, self._losses[0].data_ptr(), self._ws.data_ptr(), self._ws.numel(), stream),
-                    "boatagent_sac_gradients")
+            self._fused_learner().gradients(scale)
         elif not self.use_cuda_graph:
             self._dp_gradients_static()
         else:
@@ -467,10 +528,12 @@ class ContinuousAgent:
                 self._capture_dp()
             self._graph[0].replay()
         dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)   # eager, between the graphs (NCCL and gloo)
-        if self.learner_precision == "fp32" and self.use_cuda_graph:
+        if self.learner_precision == "tcgen05":
+            self._fused.adam()
+        elif self.use_cuda_graph:
             self._graph[1].replay()
         else:
-            o.step(grads)
+            self.learner.optimizer.step(grads)
 
     def _capture_dp(self):
         """Capture the data-parallel update as two graphs around the all-reduce: A = forward and backward passes into

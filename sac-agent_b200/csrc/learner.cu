@@ -1,6 +1,7 @@
-// learner.cu -- one SAC-v1 update (SACLearner.update, continuous_agent.py) of the BoatEnv agent (11 observations, one
-// action, 256-wide layers) in two kernels, with the 256 x 256 products on the tensor cores (tcgen05, bf16 operands,
-// fp32 accumulation in TMEM) and everything else in fp32:
+// learner.cu -- one SAC-v1 update (SACLearner.update, continuous_agent.py) of each of 1 to 16 independent BoatEnv
+// agents (11 observations, one action, 256-wide layers) in two kernels, with the 256 x 256 products on the tensor cores
+// (tcgen05, bf16 operands, fp32 accumulation in TMEM) and everything else in fp32.  Member m of a launch runs on
+// blockIdx.y = m with its own arguments, workspace slice and step counter:
 //
 //   sac_rows_kernel   one CTA per 128-row tile of the batch, one row per thread (= TMEM lane).  Runs the forward and
 //                     backward passes of the five networks for its rows in the dependency order of the update and
@@ -9,15 +10,13 @@
 //   sac_params_kernel reduces the gradients over the batch in a fixed order (tcgen05 for the four fc2 weights, one
 //                     warp per hidden unit for the rest), writes them to the parameters' .grad tensors, applies Adam
 //                     and the Polyak average (agent_math.cuh, as adam_polyak_kernel) and sums the loss partials.  Its
-//                     gradients-only instantiation (boatagent_sac_gradients) writes the gradients and the losses times
-//                     grad_scale and leaves the parameters and the optimiser state alone, so that the gradients of
-//                     several replicas can be all-reduced before one Adam step.
+//                     gradients-only instantiation (boatagent_sac_gradients_members) writes the gradients and the
+//                     losses times grad_scale and leaves the parameters and the optimiser state alone, so that the
+//                     gradients of several replicas can be all-reduced before one Adam step ...
+//   adam_polyak_members_kernel  ... boatagent_adam_polyak_members: adam_polyak_kernel's chunk body (agent_math.cuh).
 //
-// boatagent_sac_update_members runs the same two bodies for up to 16 independent agents in one launch each:
-// member m on blockIdx.y = m, with its own arguments, workspace slice and step counter.  The data-parallel population
-// splits it as boatagent_sac_gradients splits the solo update: boatagent_sac_gradients_members (the row body and the
-// gradients-only parameter body), then, after the all-reduce, boatagent_adam_polyak_members (adam_polyak_kernel's
-// chunk body, agent_math.cuh, for every member in one launch).
+// boatagent_sac_update and boatagent_sac_gradients are the one-member case of boatagent_sac_update_members and
+// boatagent_sac_gradients_members.
 //
 // Operands in shared memory and in the workspace use the 8x8 core-matrix layout of actor_tc.cuh: element (r, c) of
 // an R-row matrix at (c / 8) * (R * 16) + r * 16 + (c % 8) * 2.  The same bytes are a K-major operand with rows = M/N
@@ -100,8 +99,8 @@ struct ParamArgs {
     float grad_scale;   // gradients-only instantiation: factor on the written gradients and losses
 };
 
-// The population launch (boatagent_sac_update_members): every member's arguments, member m on blockIdx.y = m.  Both
-// tables travel as kernel parameters, within the 32,764-byte limit of CUDA 12.1+.
+// Every member's arguments, member m on blockIdx.y = m.  Both tables travel as kernel parameters, within the
+// 32,764-byte limit of CUDA 12.1+.
 struct MemberRowArgs {
     RowArgs m[BOATAGENT_SAC_MAX_MEMBERS];
 };
@@ -327,8 +326,8 @@ __device__ __forceinline__ void put_small(unsigned char *ws, int tid, const floa
 // min(a, b)'s gradient share of a, as torch's backward of torch.min(a, b): ties split the gradient in halves
 __device__ __forceinline__ float min_share(float a, float b) { return a < b ? 1.f : (a == b ? 0.5f : 0.f); }
 
-// The row pass of one 128-row tile.  blockIdx.x is the tile and gridDim.x the tile count of ONE update: the
-// population launch puts its members on blockIdx.y, so both stay per member.
+// The row pass of one 128-row tile.  blockIdx.x is the tile and gridDim.x the tile count of ONE update: the members
+// are on blockIdx.y, so both stay per member.
 __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
@@ -439,12 +438,8 @@ __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(R.tmem) : "memory");
 }
 
-__global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_constant__ RowArgs args) {
-    sac_rows_tile(args, threadIdx.x);
-}
-
-// population launch: member blockIdx.y, its tiles on blockIdx.x
-__global__ void __launch_bounds__(kLThreads, 1) sac_rows_members_kernel(const __grid_constant__ MemberRowArgs args) {
+// member blockIdx.y, its tiles on blockIdx.x
+__global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_constant__ MemberRowArgs args) {
     sac_rows_tile(args.m[blockIdx.y], threadIdx.x);
 }
 
@@ -452,8 +447,8 @@ __global__ void __launch_bounds__(kLThreads, 1) sac_rows_members_kernel(const __
 __device__ __forceinline__ int slot_of(int n, int t) { return n == 0 ? t : 8 + 6 * (n - 1) + t; }
 
 // kAdam: write the gradients, apply Adam + Polyak and count the step; else write grad_scale times the gradients only.
-// blockIdx.x is the CTA and gridDim.x the CTA count of ONE update (the population launch: member = blockIdx.y), so
-// the step-counter ticket counts one member's CTAs.
+// blockIdx.x is the CTA and gridDim.x the CTA count of ONE update (member = blockIdx.y), so the step-counter ticket
+// counts one member's CTAs.
 template <bool kAdam>
 __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -604,21 +599,13 @@ __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const in
     }
 }
 
+// member blockIdx.y; threadIdx.x is read here, where the launch bounds bound it
 template <bool kAdam>
-__global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_constant__ ParamArgs args) {
-    sac_params_block<kAdam>(args, threadIdx.x);   // read here, where the launch bounds bound it
+__global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_constant__ MemberParamArgs args) {
+    sac_params_block<kAdam>(args.m[blockIdx.y], threadIdx.x);
 }
 
-__global__ void __launch_bounds__(kPThreads) sac_params_members_kernel(const __grid_constant__ MemberParamArgs args) {
-    sac_params_block<true>(args.m[blockIdx.y], threadIdx.x);
-}
-
-// population gradients (boatagent_sac_gradients_members): member blockIdx.y
-__global__ void __launch_bounds__(kPThreads) sac_grads_members_kernel(const __grid_constant__ MemberParamArgs args) {
-    sac_params_block<false>(args.m[blockIdx.y], threadIdx.x);
-}
-
-// population Adam + Polyak step (boatagent_adam_polyak_members): member blockIdx.y, its chunks on blockIdx.x
+// Adam + Polyak step (boatagent_adam_polyak_members): member blockIdx.y, its chunks on blockIdx.x
 __global__ void __launch_bounds__(kAdamThreads) adam_polyak_members_kernel(const __grid_constant__ MemberParamArgs args) {
     const ParamArgs &a = args.m[blockIdx.y];
     adam_polyak_chunk(a.slot, kSlots, a.beta1, a.beta2, a.eps, a.tau, a.state, blockIdx.x, gridDim.x, threadIdx.x);
@@ -652,55 +639,89 @@ extern "C" int64_t boatagent_sac_update_workspace_bytes(int64_t batch) {
 
 namespace {
 
-// The arguments of both kernels from the ABI's (checks as documented in boatenv.h); pa's optimiser fields stay unset.
-int sac_args(const float *state, const float *action, const float *reward, const float *new_state, const uint8_t *done,
-             const float *eps, const float *max_action, int64_t batch, float gamma, float reward_scale,
-             const boatagent_adam_slot *slots_host, int32_t n_slots, float *losses_out, void *workspace,
-             int64_t workspace_bytes, RowArgs &ra, ParamArgs &pa) {
-    if (!state || !action || !reward || !new_state || !done || !eps || !max_action || !slots_host || !losses_out ||
-        !workspace)
-        return BOATENV_EINVAL;
-    if (batch <= 0 || batch % kRows != 0 || n_slots != kSlots) return BOATENV_EINVAL;
-    if (workspace_bytes < (int64_t)ws_bytes(batch / kRows)) return BOATENV_EINVAL;
-    if ((reinterpret_cast<uintptr_t>(workspace) & 15u) != 0) return BOATENV_EALIGN;
+// The 26 slots of one agent in DeviceAdam's order: every pointer set, the agent's shapes, a target on the value
+// network's tensors and only on them, 16-byte aligned parameters.
+int check_slots(const boatagent_adam_slot *slots) {
     for (int k = 0; k < kSlots; ++k) {
-        const boatagent_adam_slot &s = slots_host[k];
+        const boatagent_adam_slot &s = slots[k];
         if (!s.param || !s.grad || !s.exp_avg || !s.exp_avg_sq || s.numel != expected_numel(k)) return BOATENV_EINVAL;
         if ((k >= 20) != (s.target != nullptr)) return BOATENV_EINVAL;   // the value network's tensors, and only they
         if ((reinterpret_cast<uintptr_t>(s.param) & 15u) != 0) return BOATENV_EALIGN;
-        pa.slot[k] = s;
     }
-    pa.batch = batch;
-    pa.ws = (const unsigned char *)workspace;
-    pa.losses = losses_out;
+    return 0;
+}
 
-    ra.state = state;
-    ra.action = action;
-    ra.reward = reward;
-    ra.new_state = new_state;
-    ra.eps = eps;
-    ra.max_action = max_action;
-    ra.done = done;
-    ra.batch = batch;
-    ra.gamma = gamma;
-    ra.scale = reward_scale;
-    ra.ws = (unsigned char *)workspace;
-    auto net = [&](int k0, int in, bool actor, bool target) {
-        Net n;
-        const boatagent_adam_slot *s = slots_host + k0;
-        auto p = [&](int t) { return (const float *)(target ? s[t].target : s[t].param); };
-        n.w1 = p(0); n.b1 = p(1); n.w2 = p(2); n.b2 = p(3);
-        n.w3[0] = p(4); n.b3[0] = p(5);
-        n.w3[1] = actor ? p(6) : nullptr; n.b3[1] = actor ? p(7) : nullptr;
-        n.in = in;
-        n.nh = actor ? 2 : 1;
-        return n;
-    };
-    ra.net[0] = net(0, kObs, true, false);
-    ra.net[1] = net(8, kObs + 1, false, false);
-    ra.net[2] = net(14, kObs + 1, false, false);
-    ra.net[3] = net(20, kObs, false, false);
-    ra.net[4] = net(20, kObs, false, true);
+MemberRowArgs &member_rows() {   // ~32 KB together: kept off the stack
+    static thread_local MemberRowArgs ra;
+    return ra;
+}
+MemberParamArgs &member_params() {
+    static thread_local MemberParamArgs pa;
+    return pa;
+}
+
+// The member tables of both kernels: every member checked as documented in boatenv.h (its adam_state only with
+// `adam`) before anything is launched.
+int member_tables(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch, void *workspace,
+                  int64_t workspace_bytes, bool adam, float beta1, float beta2, float adam_eps, float grad_scale,
+                  MemberRowArgs &ra, MemberParamArgs &pa) {
+    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
+    if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
+    const size_t slice = ws_bytes(batch / kRows);   // a multiple of 16: every slice stays 16-byte aligned
+    if (workspace_bytes < 0 || (uint64_t)workspace_bytes < slice * (uint64_t)n_members) return BOATENV_EINVAL;
+    if ((reinterpret_cast<uintptr_t>(workspace) & 15u) != 0) return BOATENV_EALIGN;
+    std::memset(&ra, 0, sizeof(ra));
+    std::memset(&pa, 0, sizeof(pa));
+    for (int m = 0; m < n_members; ++m) {
+        const boatagent_sac_member &b = members_host[m];
+        if ((adam && !b.adam_state) || !b.state || !b.action || !b.reward || !b.new_state || !b.done || !b.eps ||
+            !b.max_action || !b.slots || !b.losses || b.n_slots != kSlots)
+            return BOATENV_EINVAL;
+        const int rc = check_slots(b.slots);
+        if (rc != 0) return rc;
+        unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
+
+        RowArgs &r = ra.m[m];
+        r.state = b.state;
+        r.action = b.action;
+        r.reward = b.reward;
+        r.new_state = b.new_state;
+        r.eps = b.eps;
+        r.max_action = b.max_action;
+        r.done = b.done;
+        r.batch = batch;
+        r.gamma = b.gamma;
+        r.scale = b.reward_scale;
+        r.ws = ws;
+        auto net = [&](int k0, int in, bool actor, bool target) {
+            Net n;
+            const boatagent_adam_slot *s = b.slots + k0;
+            auto p = [&](int t) { return (const float *)(target ? s[t].target : s[t].param); };
+            n.w1 = p(0); n.b1 = p(1); n.w2 = p(2); n.b2 = p(3);
+            n.w3[0] = p(4); n.b3[0] = p(5);
+            n.w3[1] = actor ? p(6) : nullptr; n.b3[1] = actor ? p(7) : nullptr;
+            n.in = in;
+            n.nh = actor ? 2 : 1;
+            return n;
+        };
+        r.net[0] = net(0, kObs, true, false);
+        r.net[1] = net(8, kObs + 1, false, false);
+        r.net[2] = net(14, kObs + 1, false, false);
+        r.net[3] = net(20, kObs, false, false);
+        r.net[4] = net(20, kObs, false, true);
+
+        ParamArgs &p = pa.m[m];
+        std::memcpy(p.slot, b.slots, sizeof(p.slot));
+        p.beta1 = beta1;
+        p.beta2 = beta2;
+        p.eps = adam_eps;
+        p.tau = b.tau;
+        p.batch = batch;
+        p.ws = ws;
+        p.state = (long long *)b.adam_state;
+        p.losses = b.losses;
+        p.grad_scale = grad_scale;
+    }
     return 0;
 }
 
@@ -716,128 +737,39 @@ int set_smem_attributes() {
         CUDA_TRY(cudaFuncSetAttribute(sac_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
-        CUDA_TRY(cudaFuncSetAttribute(sac_rows_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
-        CUDA_TRY(cudaFuncSetAttribute(sac_params_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
-        CUDA_TRY(cudaFuncSetAttribute(sac_grads_members_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         set_of[dev] = true;
     }
     return 0;
 }
 
-template <bool kAdam>
-int sac_launch(const RowArgs &ra, const ParamArgs &pa, void *stream) {
+int launch(bool adam, int32_t n_members, int64_t batch, const MemberRowArgs &ra, const MemberParamArgs &pa,
+           void *stream) {
     const int rc = set_smem_attributes();
     if (rc != 0) return rc;
-    sac_rows_kernel<<<(unsigned)(ra.batch / kRows), kLThreads, kLSmem, (cudaStream_t)stream>>>(ra);
+    const cudaStream_t s = (cudaStream_t)stream;
+    sac_rows_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem, s>>>(ra);
     boatenv::count_launch();
     CUDA_TRY(cudaGetLastError());
-    sac_params_kernel<kAdam><<<kParamBlocks, kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
-    boatenv::count_launch();
-    return (int)cudaGetLastError();
-}
-
-MemberRowArgs &member_rows() {   // ~32 KB together: kept off the stack
-    static thread_local MemberRowArgs ra;
-    return ra;
-}
-MemberParamArgs &member_params() {
-    static thread_local MemberParamArgs pa;
-    return pa;
-}
-
-// The member tables of boatagent_sac_update_members and boatagent_sac_gradients_members: every member checked as
-// boatagent_sac_update checks its arguments (its adam_state only with `adam`), before anything is launched.  The
-// shared Adam hyper-parameters stay unset.
-int member_tables(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch, void *workspace,
-                  int64_t workspace_bytes, bool adam, float grad_scale, MemberRowArgs &ra, MemberParamArgs &pa) {
-    if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
-    if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
-    const size_t slice = ws_bytes(batch / kRows);   // a multiple of 16: every slice stays 16-byte aligned
-    if (workspace_bytes < 0 || (uint64_t)workspace_bytes < slice * (uint64_t)n_members) return BOATENV_EINVAL;
-    std::memset(&ra, 0, sizeof(ra));
-    std::memset(&pa, 0, sizeof(pa));
-    for (int m = 0; m < n_members; ++m) {
-        const boatagent_sac_member &b = members_host[m];
-        if (adam && !b.adam_state) return BOATENV_EINVAL;
-        unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
-        const int rc = sac_args(b.state, b.action, b.reward, b.new_state, b.done, b.eps, b.max_action, batch, b.gamma,
-                                b.reward_scale, b.slots, b.n_slots, b.losses, ws, (int64_t)slice, ra.m[m], pa.m[m]);
-        if (rc != 0) return rc;
-        pa.m[m].tau = b.tau;
-        pa.m[m].state = (long long *)b.adam_state;
-        pa.m[m].grad_scale = grad_scale;
-    }
-    return 0;
-}
-
-int members_launch(bool adam, int32_t n_members, int64_t batch, const MemberRowArgs &ra, const MemberParamArgs &pa,
-                   void *stream) {
-    const int rc = set_smem_attributes();
-    if (rc != 0) return rc;
-    sac_rows_members_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem,
-                              (cudaStream_t)stream>>>(ra);
-    boatenv::count_launch();
-    CUDA_TRY(cudaGetLastError());
+    const dim3 grid(kParamBlocks, (unsigned)n_members);
     if (adam)
-        sac_params_members_kernel<<<dim3(kParamBlocks, (unsigned)n_members), kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+        sac_params_kernel<true><<<grid, kPThreads, kPSmem, s>>>(pa);
     else
-        sac_grads_members_kernel<<<dim3(kParamBlocks, (unsigned)n_members), kPThreads, kPSmem, (cudaStream_t)stream>>>(pa);
+        sac_params_kernel<false><<<grid, kPThreads, kPSmem, s>>>(pa);
     boatenv::count_launch();
     return (int)cudaGetLastError();
 }
 
 }  // namespace
 
-extern "C" int boatagent_sac_update(const float *state, const float *action, const float *reward, const float *new_state,
-                                    const uint8_t *done, const float *eps, const float *max_action, int64_t batch,
-                                    float gamma, float reward_scale, const boatagent_adam_slot *slots_host,
-                                    int32_t n_slots, float beta1, float beta2, float adam_eps, float tau,
-                                    int64_t *adam_state, float *losses_out, void *workspace, int64_t workspace_bytes,
-                                    void *stream) {
-    if (!adam_state) return BOATENV_EINVAL;
-    RowArgs ra;
-    ParamArgs pa;
-    const int rc = sac_args(state, action, reward, new_state, done, eps, max_action, batch, gamma, reward_scale,
-                            slots_host, n_slots, losses_out, workspace, workspace_bytes, ra, pa);
-    if (rc != 0) return rc;
-    pa.beta1 = beta1;
-    pa.beta2 = beta2;
-    pa.eps = adam_eps;
-    pa.tau = tau;
-    pa.state = (long long *)adam_state;
-    pa.grad_scale = 1.0f;
-    return sac_launch<true>(ra, pa, stream);
-}
-
-extern "C" int boatagent_sac_gradients(const float *state, const float *action, const float *reward,
-                                       const float *new_state, const uint8_t *done, const float *eps,
-                                       const float *max_action, int64_t batch, float gamma, float reward_scale,
-                                       const boatagent_adam_slot *slots_host, int32_t n_slots, float grad_scale,
-                                       float *losses_out, void *workspace, int64_t workspace_bytes, void *stream) {
-    RowArgs ra;
-    ParamArgs pa;
-    const int rc = sac_args(state, action, reward, new_state, done, eps, max_action, batch, gamma, reward_scale,
-                            slots_host, n_slots, losses_out, workspace, workspace_bytes, ra, pa);
-    if (rc != 0) return rc;
-    pa.beta1 = pa.beta2 = pa.eps = pa.tau = 0.f;
-    pa.state = nullptr;
-    pa.grad_scale = grad_scale;
-    return sac_launch<false>(ra, pa, stream);
-}
-
 extern "C" int boatagent_sac_update_members(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch,
                                             float beta1, float beta2, float adam_eps, void *workspace,
                                             int64_t workspace_bytes, void *stream) {
     MemberRowArgs &ra = member_rows();
     MemberParamArgs &pa = member_params();
-    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, 1.0f, ra, pa);
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, beta1, beta2,
+                                 adam_eps, 1.0f, ra, pa);
     if (rc != 0) return rc;
-    for (int m = 0; m < n_members; ++m) {
-        pa.m[m].beta1 = beta1;
-        pa.m[m].beta2 = beta2;
-        pa.m[m].eps = adam_eps;
-    }
-    return members_launch(true, n_members, batch, ra, pa, stream);
+    return launch(true, n_members, batch, ra, pa, stream);
 }
 
 extern "C" int boatagent_sac_gradients_members(const boatagent_sac_member *members_host, int32_t n_members,
@@ -845,9 +777,31 @@ extern "C" int boatagent_sac_gradients_members(const boatagent_sac_member *membe
                                                int64_t workspace_bytes, void *stream) {
     MemberRowArgs &ra = member_rows();
     MemberParamArgs &pa = member_params();
-    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, false, grad_scale, ra, pa);
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, false, 0.f, 0.f, 0.f,
+                                 grad_scale, ra, pa);
     if (rc != 0) return rc;
-    return members_launch(false, n_members, batch, ra, pa, stream);
+    return launch(false, n_members, batch, ra, pa, stream);
+}
+
+extern "C" int boatagent_sac_update(const float *state, const float *action, const float *reward, const float *new_state,
+                                    const uint8_t *done, const float *eps, const float *max_action, int64_t batch,
+                                    float gamma, float reward_scale, const boatagent_adam_slot *slots_host,
+                                    int32_t n_slots, float beta1, float beta2, float adam_eps, float tau,
+                                    int64_t *adam_state, float *losses_out, void *workspace, int64_t workspace_bytes,
+                                    void *stream) {
+    const boatagent_sac_member m = {state, action, reward, new_state, done, eps, max_action, slots_host, n_slots,
+                                    gamma, reward_scale, tau, adam_state, losses_out};
+    return boatagent_sac_update_members(&m, 1, batch, beta1, beta2, adam_eps, workspace, workspace_bytes, stream);
+}
+
+extern "C" int boatagent_sac_gradients(const float *state, const float *action, const float *reward,
+                                       const float *new_state, const uint8_t *done, const float *eps,
+                                       const float *max_action, int64_t batch, float gamma, float reward_scale,
+                                       const boatagent_adam_slot *slots_host, int32_t n_slots, float grad_scale,
+                                       float *losses_out, void *workspace, int64_t workspace_bytes, void *stream) {
+    const boatagent_sac_member m = {state, action, reward, new_state, done, eps, max_action, slots_host, n_slots,
+                                    gamma, reward_scale, 0.f, nullptr, losses_out};
+    return boatagent_sac_gradients_members(&m, 1, batch, grad_scale, workspace, workspace_bytes, stream);
 }
 
 extern "C" int boatagent_adam_polyak_members(const boatagent_sac_member *members_host, int32_t n_members, float beta1,
@@ -858,12 +812,9 @@ extern "C" int boatagent_adam_polyak_members(const boatagent_sac_member *members
     for (int m = 0; m < n_members; ++m) {
         const boatagent_sac_member &b = members_host[m];
         if (!b.adam_state || !b.slots || b.n_slots != kSlots) return BOATENV_EINVAL;
-        for (int k = 0; k < kSlots; ++k) {
-            const boatagent_adam_slot &s = b.slots[k];
-            if (!s.param || !s.grad || !s.exp_avg || !s.exp_avg_sq || s.numel != expected_numel(k)) return BOATENV_EINVAL;
-            if ((k >= 20) != (s.target != nullptr)) return BOATENV_EINVAL;   // the value network's tensors, and only they
-            pa.m[m].slot[k] = s;
-        }
+        const int rc = check_slots(b.slots);
+        if (rc != 0) return rc;
+        std::memcpy(pa.m[m].slot, b.slots, sizeof(pa.m[m].slot));
         pa.m[m].beta1 = beta1;
         pa.m[m].beta2 = beta2;
         pa.m[m].eps = adam_eps;

@@ -14,7 +14,7 @@ the members never talk.  With one member per GPU under ``torchrun`` the members 
 
 On ONE GPU, ``AgentPopulation`` trains P members in one process: each member is an ordinary ``ContinuousAgent`` with its
 own env, ring, experiment directory and hyper-parameters, and one ``learn()`` updates all of them in four launches (one
-sample-gather for every ring, one Gaussian draw, the two kernels of ``boatagent_sac_update_members``).
+sample-gather for every ring, one Gaussian draw, the two kernels of the members' ``FusedLearner``).
 ``exploit_explore_local`` is ``exploit_explore`` over such members, with device copies instead of collectives.
 With ``data_parallel``, every member is ONE agent trained by all ranks of a process group: each rank holds its own
 env shard and ring of every member, and one update round of all members is one gradient launch pair, one all-reduce
@@ -155,7 +155,7 @@ class AgentPopulation:
         from . import _lib
         from .boat_env import BatchedBoatEnv
         from .buffer import ReplayBuffer
-        from .continuous_agent import ContinuousAgent
+        from .continuous_agent import ContinuousAgent, FusedLearner
         from .networks import TensorCorePolicy
         P = int(members)
         if not 1 <= P <= 16:
@@ -200,21 +200,23 @@ class AgentPopulation:
         B = self.batch_size
         # the members' Gaussian draws are slices of one tensor: one normal_() per learn()
         self.eps = torch.zeros((P, 2, B, 1), dtype=torch.float32, device=self.device)
+        self._sample = (_lib.SampleMember * P)()
         for m, a in enumerate(self.members):
             a._eps = self.eps[m]
-        self._ws = torch.empty(P * int(self._L.boatagent_sac_update_workspace_bytes(B)), dtype=torch.uint8,
-                               device=self.device)
-        self._sample = (_lib.SampleMember * P)()
-        self._table = None
+            s, act, r, s2, d = a._batch
+            self._sample[m] = _lib.SampleMember(a.memory._h, 0, 0, s.data_ptr(), act.data_ptr(), r.data_ptr(),
+                                                s2.data_ptr(), d.data_ptr())
         self._flat = None
         if self._dp is not None:
             self._init_data_parallel(E)
+        self._learner = FusedLearner(self.members)
 
     def _init_data_parallel(self, envs_per_member):
         """Checks that every rank holds the same population, points every member's gradients and losses into one flat
         [P, n_params + 3] buffer (one all-reduce per round) and starts every rank from rank 0's members."""
         import torch
         import torch.distributed as dist
+        from .continuous_agent import point_grads_into
         group, world = self._dp
         P = len(self.members)
         shape = torch.tensor([P, self.batch_size, envs_per_member], dtype=torch.int64, device=self.device)
@@ -224,16 +226,10 @@ class AgentPopulation:
             raise ValueError(f"AgentPopulation: every rank of the data-parallel group needs the same members, batch "
                              f"size and envs per member (this rank: {P}, {self.batch_size}, {envs_per_member}; "
                              f"largest over the ranks: {both[:3].tolist()})")
-        params = self.members[0].learner.optimizer.params
-        n = sum(p.numel() for p in params)
+        n = sum(p.numel() for p in self.members[0].learner.optimizer.params)
         self._flat = torch.zeros((P, n + 3), dtype=torch.float32, device=self.device)
         for m, a in enumerate(self.members):
-            off = 0
-            for p in a.learner.optimizer.params:
-                p.grad = self._flat[m, off:off + p.numel()].view_as(p)
-                off += p.numel()
-            a._loss_buf = self._flat[m, n:]
-            a._losses = tuple(a._loss_buf[k] for k in range(3))
+            point_grads_into(a, self._flat[m])
         src = 0 if group is None else dist.get_global_rank(group, 0)
         for a in self.members:
             for t in a.training_tensors():
@@ -259,61 +255,33 @@ class AgentPopulation:
             a._tc_policy.refresh()
             a.collect(env, steps, done_flag_mode=self.done_flag_mode)
 
-    def _build_table(self):
-        """The member table of boatagent_sac_update_members.  Every pointer in it is stable: parameters, moments,
-        gradients, the batch and the draws are updated in place."""
-        import torch
-        t = (self._lib.SacMember * len(self.members))()
-        for m, a in enumerate(self.members):
-            o, L = a.learner.optimizer, a.learner
-            for k, p in enumerate(o.params):
-                if p.grad is None:
-                    p.grad = torch.zeros_like(p)
-                o._slots[k].grad = p.grad.data_ptr()
-            s, act, r, s2, d = a._batch
-            t[m] = self._lib.SacMember(s.data_ptr(), act.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(),
-                                       a._eps.data_ptr(), L.actor.max_action.data_ptr(),
-                                       C.cast(o._slots, C.c_void_p), len(o.params), float(L.gamma), float(L.scale),
-                                       float(o.tau), o.state.data_ptr(), a._loss_buf.data_ptr())
-            self._sample[m] = self._lib.SampleMember(a.memory._h, a.memory.seed, 0, s.data_ptr(), act.data_ptr(),
-                                                     r.data_ptr(), s2.data_ptr(), d.data_ptr())
-        self._table = t   # its slot pointers are the members' own DeviceAdam arrays, which live as long as they do
-
     def learn(self):
         """One update of every member: the batched sample-gather, one Gaussian draw for all, and the two kernels of
-        boatagent_sac_update_members (no sync).  Returns each member's (value, actor, critic) losses as device
-        tensors, or None (nothing launched) while some member's ring holds less than a batch.
+        the members' fused update (``FusedLearner.update``, no sync).  Returns each member's (value, actor, critic)
+        losses as device tensors, or None (nothing launched) while some member's ring holds less than a batch.
 
-        Data-parallel: the update is boatagent_sac_gradients_members (times 1 / W), one all-reduce (SUM) of every
-        member's gradients and losses, and boatagent_adam_polyak_members; the losses are the means over the ranks.
-        The rank shards are equal, so all ranks start updating at the same call without a vote."""
+        Data-parallel: the update is ``FusedLearner.gradients`` (times 1 / W), one all-reduce (SUM) of every member's
+        gradients and losses, and ``FusedLearner.adam``; the losses are the means over the ranks.  The rank shards are
+        equal, so all ranks start updating at the same call without a vote."""
         if any(a.memory.mem_cntr < self.batch_size for a in self.members):
             return None
         import torch
-        if self._table is None:
-            self._build_table()
-        P, B = len(self.members), self.batch_size
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        for m, a in enumerate(self.members):
-            self._sample[m].counter = a.memory._samples
-        self._lib.check(self._L.boatreplay_sample_members(self._sample, P, B, stream), "boatreplay_sample_members")
+        for m, a in enumerate(self.members):   # load_state_dict may have changed the seed
+            self._sample[m].seed, self._sample[m].counter = a.memory.seed, a.memory._samples
+        self._lib.check(self._L.boatreplay_sample_members(self._sample, len(self.members), self.batch_size, stream),
+                        "boatreplay_sample_members")
         for a in self.members:
             a.memory._samples += 1
         self.eps.normal_()
-        o = self.members[0].learner.optimizer
         if self._dp is None:
-            self._lib.check(self._L.boatagent_sac_update_members(self._table, P, B, o.betas[0], o.betas[1], o.eps,
-                                                                 self._ws.data_ptr(), self._ws.numel(), stream),
-                            "boatagent_sac_update_members")
+            self._learner.update()
         else:
             import torch.distributed as dist
             group, world = self._dp
-            self._lib.check(self._L.boatagent_sac_gradients_members(self._table, P, B, 1.0 / world,
-                                                                    self._ws.data_ptr(), self._ws.numel(), stream),
-                            "boatagent_sac_gradients_members")
+            self._learner.gradients(1.0 / world)
             dist.all_reduce(self._flat, op=dist.ReduceOp.SUM, group=group)
-            self._lib.check(self._L.boatagent_adam_polyak_members(self._table, P, o.betas[0], o.betas[1], o.eps, stream),
-                            "boatagent_adam_polyak_members")
+            self._learner.adam()
         for a in self.members:
             a.updates += 1
         return [a._losses for a in self.members]
@@ -333,15 +301,12 @@ class AgentPopulation:
     def set_hyperparameters(self, m, **hp):
         """``ContinuousAgent.set_hyperparameters`` of member m, seen by the next ``learn()``."""
         self.members[m].set_hyperparameters(**hp)
-        self._table = None
 
     def exploit_explore(self, scores, rng: random.Random, bottom_fraction: float = 0.25):
         """One population round over the members (``exploit_explore_local``).  Data-parallel: every rank must call it
         with the same scores (e.g. from ``counters()``) and an identically seeded rng, so that all ranks make the same
         round and their members stay bit-identical."""
-        info = exploit_explore_local(self.members, scores, rng, bottom_fraction)
-        self._table = None
-        return info
+        return exploit_explore_local(self.members, scores, rng, bottom_fraction)
 
     def state_dict(self):
         """The members' ``ContinuousAgent.state_dict()``, in member order."""
@@ -352,7 +317,6 @@ class AgentPopulation:
             raise ValueError(f"checkpoint of {len(sd)} members for a population of {len(self.members)}")
         for a, s in zip(self.members, sd):
             a.load_state_dict(s)
-        self._table = None
 
     def close(self):
         for a, env in zip(self.members, self.envs):
