@@ -10,6 +10,8 @@ import sys
 import numpy as np
 import pytest
 
+from boat_testlib import philox4x32_10
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "boatenv.h")
 
@@ -101,24 +103,16 @@ def test_config_semantics(S, tmp_path):
     assert S.load_config(base_settings__experiment=5).base_settings.experiment == 5
 
 
-def philox4x32_10(ctr, key):
-    """Salmon et al., SC'11 -- plain-Python restatement used to pin the library's stream."""
-    c0, c1, c2, c3 = ctr
-    k0, k1 = key
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c0, 0xCD9E8D57 * c2
-        c0, c1, c2, c3 = ((p1 >> 32) ^ c1 ^ k0) & 0xffffffff, p1 & 0xffffffff, \
-                         ((p0 >> 32) ^ c3 ^ k1) & 0xffffffff, p0 & 0xffffffff
-        k0, k1 = (k0 + 0x9E3779B9) & 0xffffffff, (k1 + 0xBB67AE85) & 0xffffffff
-    return c0, c1, c2, c3
+def philox_words(*ctr_and_key):
+    return tuple(int(w) for w in philox4x32_10(*ctr_and_key))
 
 
 def test_philox_known_answers():
     """Random123 kat_vectors for philox4x32-10."""
-    assert philox4x32_10((0, 0, 0, 0), (0, 0)) == (0x6627e8d5, 0xe169c58d, 0xbc57ac4c, 0x9b00dbd8)
+    assert philox_words(0, 0, 0, 0, 0, 0) == (0x6627e8d5, 0xe169c58d, 0xbc57ac4c, 0x9b00dbd8)
     f = 0xffffffff
-    assert philox4x32_10((f, f, f, f), (f, f)) == (0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd)
-    assert philox4x32_10((0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344), (0xa4093822, 0x299f31d0)) == \
+    assert philox_words(f, f, f, f, f, f) == (0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd)
+    assert philox_words(0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344, 0xa4093822, 0x299f31d0) == \
         (0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1)
 
 
@@ -148,10 +142,10 @@ def test_host_philox_draws(S):
     for seed, env, ep in ((1, 12345, 3), (2 ** 40 + 5, 2 ** 33 + 7, 9)):
         s_y, knots = draws(seed, env, ep)
         key = (seed & 0xffffffff, seed >> 32)
-        w0 = philox4x32_10((env & 0xffffffff, env >> 32, ep, 0), key)[0]
+        w0 = philox_words(env & 0xffffffff, env >> 32, ep, 0, *key)[0]
         assert s_y == -640 + ((w0 * 1280) >> 32)
         for t in range(16):
-            w = philox4x32_10((env & 0xffffffff, env >> 32, ep, 1 + (t >> 2)), key)[t & 3]
+            w = philox_words(env & 0xffffffff, env >> 32, ep, 1 + (t >> 2), *key)[t & 3]
             assert knots[t] == ((((w >> 9) << 1) | 1) / 16777216.0)
     bad = S.params_from_config(S.load_config(base_settings__experiment=9))
     assert L.boatenv_episode_draws_host(C.byref(bad), 0, 0, 0, None, None) == -2

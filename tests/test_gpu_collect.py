@@ -14,7 +14,7 @@ import os
 import numpy as np
 import pytest
 
-from boat_testlib import ROOT
+from boat_testlib import ROOT, set_mem_cntr
 
 COUNTER_BYTES = 32 * 32 * 8   # the counter rows at the end of an export_state blob (kCounterSlots x 32 doubles)
 COUNTS = ("reached_goal", "out_of_bounds", "out_of_fuel", "timeout", "rudder_broken", "episodes")
@@ -53,11 +53,6 @@ def make_env(S, exp, n, seed=3, env_id_offset=0, auto_reset=True, precision="fp3
 
 def make_ring(S, size, obs_dim=11, n_actions=1, precision="fp32"):
     return S.ReplayBuffer(size, (obs_dim,), n_actions, precision=precision, device=0, as_torch=True)
-
-
-def set_mem_cntr(mem, value):
-    from sac_agent_b200 import _lib
-    _lib.check(mem._L.boatreplay_set_mem_cntr(mem._h, int(value)), "boatreplay_set_mem_cntr")
 
 
 def per_step(env, mem, pol, steps, done_flag_mode=1):
