@@ -95,8 +95,10 @@ def main(argv=None):
     env = S.make_sharded_env(cfg, args.envs, seed=args.seed, precision="fp32", auto_reset=False)
     mem = S.ReplayBuffer(int(cfg.agent.batch_size), (11,), 1, precision="fp32", device=local_rank, seed=args.seed,
                          as_torch=True)   # the agent needs one; evaluation stores nothing
+    # a SAC-v2 directory (train_sac.py --algorithm sac2) holds target critics instead of value networks
+    sac2 = os.path.exists(os.path.join(args.checkpoints, "checkpoints", "target_critic_network_1"))
     agent = S.ContinuousAgent(cfg, args.checkpoints, env.observation_space.shape, env, device=local_rank,
-                              seed=args.seed + rank, memory=mem)
+                              seed=args.seed + rank, memory=mem, algorithm="sac2" if sac2 else "sac1")
     agent.load_models()
     # policy draws are keyed by (seed; row, step) and rows restart at 0 on every shard: a seed per rank keeps the
     # shards' noise independent under --stochastic

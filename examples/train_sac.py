@@ -1,6 +1,8 @@
 #!/usr/bin/env python
 """End-to-end SAC (v1: actor, twin critics, value + target value) on the GPU-resident batched BoatEnv
-and the fused device replay buffer -- BASELINE.json configs[4] / SURVEY.md 8(f) rank 1.
+and the fused device replay buffer -- BASELINE.json configs[4] / SURVEY.md 8(f) rank 1.  `--algorithm sac2` trains
+SAC with twin target critics and a learned entropy temperature instead (SAC2Learner); its JSON summary adds
+`algorithm` and the final `temperature`.
 
 The loop is the reference's main.py:72-90 with every piece on the device:
 
@@ -95,7 +97,23 @@ def main(argv=None):
                          "--collect-steps.  With --data-parallel under torchrun (2+ ranks) every member is ONE agent "
                          "trained by all ranks, --envs counts each member's envs over all ranks, and --tune and "
                          "--pbt-every draw and rank the members the same way on every rank")
+    ap.add_argument("--algorithm", default="sac1", choices=["sac1", "sac2"],
+                    help="sac1: the reference's SAC-v1 (value + target value networks, entropy weight fixed by the "
+                         "reward scale); sac2: twin target critics and a learned entropy temperature (SAC2Learner)")
+    ap.add_argument("--target-entropy", type=float, default=None,
+                    help="sac2: the temperature's target entropy (default: minus the number of actions, -1)")
+    ap.add_argument("--init-temperature", type=float, default=None, help="sac2: initial alpha (default 1.0)")
+    ap.add_argument("--temperature-lr", type=float, default=None,
+                    help="sac2: Adam learning rate of log alpha (default: the critics', learning_rate_beta)")
     args = ap.parse_args(argv)
+    if args.algorithm == "sac2":   # checked before any CUDA work
+        for flag, on in (("--data-parallel", args.data_parallel), ("--overlap", args.overlap)):
+            if on:
+                ap.error(f"--algorithm sac2 and {flag} cannot be combined")
+        if args.init_temperature is not None and not args.init_temperature > 0:
+            ap.error("--init-temperature must be positive")
+    elif any(x is not None for x in (args.target_entropy, args.init_temperature, args.temperature_lr)):
+        ap.error("--target-entropy, --init-temperature and --temperature-lr need --algorithm sac2")
     if args.record_envs and not args.experiments_root:
         ap.error("--record-envs requires --experiments-root")
     if args.collect_steps < 0:
@@ -136,6 +154,9 @@ def main(argv=None):
         finally:
             if world > 1:
                 torch.distributed.destroy_process_group()
+    if args.algorithm == "sac2" and args.pbt_every and world > 1:
+        ap.error("--algorithm sac2 and --pbt-every across ranks cannot be combined (population rounds between ranks "
+                 "are SAC-v1's; use --population for SAC-v2 population rounds on one GPU)")
     if args.data_parallel:   # checked before any CUDA work
         for flag, on in (("--tune", args.tune), ("--pbt-every", args.pbt_every), ("--overlap", args.overlap)):
             if on:
@@ -168,7 +189,8 @@ def main(argv=None):
     agent = S.ContinuousAgent(cfg, exp.experiment_dir if exp else None, env.observation_space.shape, env,
                               device=local_rank, seed=args.seed + rank,
                               use_cuda_graph=not args.no_graph, memory=mem, policy_precision=args.policy_precision,
-                              learner_precision=args.learner_precision, data_parallel=args.data_parallel or None)
+                              learner_precision=args.learner_precision, data_parallel=args.data_parallel or None,
+                              **_algorithm_args(args))
     act = agent.choose_action if args.no_graph else agent.choose_action_graphed
     obs = env.reset()
     rec = None
@@ -239,7 +261,7 @@ def main(argv=None):
             c = env.counters()
             lv = [float(x) for x in losses] if losses is not None else [float("nan")] * 3
             print(f"iter {it:6d}  episodes {c['episodes']:.0f}  goals {c['reached_goal']:.0f}  "
-                  f"losses v/pi/q {lv[0]:.3g} {lv[1]:.3g} {lv[2]:.3g}", flush=True)
+                  f"losses {_loss_label(args)} {lv[0]:.3g} {lv[1]:.3g} {lv[2]:.3g}", flush=True)
     if pipe:
         pipe.finish()
     t1.record()
@@ -268,6 +290,8 @@ def main(argv=None):
                "losses_v_pi_q": [float(x) for x in losses] if losses is not None else None}
     if args.data_parallel:
         summary["data_parallel"], summary["effective_batch"] = True, world * agent.batch_size
+    if args.algorithm == "sac2":
+        summary["algorithm"], summary["temperature"] = "sac2", float(agent.temperature())
     if args.record_envs:   # over all ranks: envs recorded, and their episodes that ended (one info.csv row each)
         summary["recorded_envs"], summary["recorded_episodes"] = int(recorded[0]), int(recorded[1])
     if args.pbt_every:
@@ -292,6 +316,18 @@ def main(argv=None):
     if world > 1 or args.data_parallel:
         torch.distributed.destroy_process_group()
     return summary
+
+
+def _algorithm_args(args):
+    """ContinuousAgent / AgentPopulation keyword arguments of --algorithm and the sac2 temperature flags."""
+    if args.algorithm != "sac2":
+        return {}
+    return {"algorithm": "sac2", "target_entropy": args.target_entropy, "temperature_lr": args.temperature_lr,
+            "init_temperature": 1.0 if args.init_temperature is None else args.init_temperature}
+
+
+def _loss_label(args):
+    return "t/pi/q" if args.algorithm == "sac2" else "v/pi/q"
 
 
 def _overrides(args):
@@ -329,7 +365,7 @@ def train_population(args, rank, local_rank, world, group=None):
     pop = S.AgentPopulation(cfg, P, n_local, seed=args.seed, rank=rank, device=local_rank, configs=configs,
                             experiment_dirs=[e.experiment_dir if e else None for e in exps],
                             buffer_size=max(args.buffer, n_local * args.collect_steps),
-                            data_parallel=group if dp else None)
+                            data_parallel=group if dp else None, **_algorithm_args(args))
     pop.reset()
     losses = None
     rows, best = [[] for _ in range(P)], [float("-inf")] * P
@@ -376,8 +412,8 @@ def train_population(args, rank, local_rank, world, group=None):
                 c = counters
                 lv = [float(x) for x in losses[0]] if losses is not None else [float("nan")] * 3
                 print(f"iter {it:6d}  episodes {sum(x['episodes'] for x in c):.0f}  goals "
-                      f"{sum(x['reached_goal'] for x in c):.0f}  member 0 losses v/pi/q {lv[0]:.3g} {lv[1]:.3g} "
-                      f"{lv[2]:.3g}", flush=True)
+                      f"{sum(x['reached_goal'] for x in c):.0f}  member 0 losses {_loss_label(args)} {lv[0]:.3g} "
+                      f"{lv[1]:.3g} {lv[2]:.3g}", flush=True)
     t1.record()
     torch.cuda.synchronize()
     ms = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device="cuda")
@@ -402,6 +438,8 @@ def train_population(args, rank, local_rank, world, group=None):
     summary["env_steps_per_s_aggregate"] = summary["env_steps_per_s"]
     if dp:
         summary["data_parallel"], summary["effective_batch"] = True, world * pop.batch_size
+    if args.algorithm == "sac2":
+        summary["algorithm"], summary["temperature"] = "sac2", [float(a.temperature()) for a in pop.members]
     if args.pbt_every:
         summary["pbt_rounds"] = len(pbt_log)
         summary["pbt_adoptions"] = [e for e in pbt_log if e["adopted"]]

@@ -506,6 +506,37 @@ BOATENV_API int boatagent_sac_gradients_members(const boatagent_sac_member *memb
 BOATENV_API int boatagent_adam_polyak_members(const boatagent_sac_member *members_host, int32_t n_members, float beta1,
                                               float beta2, float adam_eps, void *stream);
 
+/* One SAC-v2 update (SAC2Learner.update: twin critics with Polyak target critics, no value network, a learned
+ * temperature alpha = exp(log_alpha)) of each of n_members BoatEnv agents, member m on blockIdx.y = m, in three
+ * launches: the forward and backward passes per 128-row tile, the fixed-order gradient reductions, then Adam and the
+ * Polyak average of the target critics over the 21 slots.  Precision and reproducibility as boatagent_sac_update.
+ * With alpha read before the update and every loss on the weights before it:
+ *   y = reward_scale r + gamma (1 - done) (min(Qt1, Qt2)(s', a') - alpha lp'),   a', lp' drawn on s' with eps[0]
+ *   critic loss 0.5 mse(Q1(s, a), y) + 0.5 mse(Q2(s, a), y)
+ *   actor loss mean(alpha lp - min(Q1, Q2)(s, a~)),   a~, lp drawn on s with eps[1] (reparameterised)
+ *   temperature loss -log_alpha mean(lp + target_entropy), lp detached
+ * Each entry: `base` as a boatagent_sac_member, with
+ *   slots / n_slots: the 21 slots in DeviceAdam's order -- actor fc1 w, b, fc2 w, b, mean w, b, std w, b; critic 1
+ *   and critic 2 fc1 w, b, fc2 w, b, q w, b with `target` the target critic's tensor; log_alpha [1] with no target.
+ *   `grad` receives the batch gradient, then Adam (the slot's lr) and the Polyak average (tau) run as in
+ *   boatagent_adam_polyak_step with adam_state int64[2] as there;
+ *   losses float32 [3] (device): temperature, actor, critic loss;
+ *   target_entropy: the temperature's target (e.g. -1, minus the action count).
+ *   workspace: n_members * boatagent_sac2_update_workspace_bytes(batch) device bytes, 16-byte aligned; member m uses
+ *   the slice at m times that size.
+ * Errors (every member checked before anything is launched): BOATENV_EINVAL for n_members outside
+ * 1..BOATAGENT_SAC_MAX_MEMBERS, a NULL table, workspace, adam_state or pointer, a batch that is not a positive
+ * multiple of 128, n_slots != 21, a slot whose numel is not the agent's shape, a missing or extra target, a workspace
+ * that is too small; BOATENV_EALIGN for a workspace or parameter that is not 16-byte aligned. */
+typedef struct boatagent_sac2_member {
+    boatagent_sac_member base;
+    float target_entropy;
+} boatagent_sac2_member;
+BOATENV_API int64_t boatagent_sac2_update_workspace_bytes(int64_t batch);   /* BOATENV_EINVAL for a bad batch */
+BOATENV_API int boatagent_sac2_update_members(const boatagent_sac2_member *members_host, int32_t n_members,
+                                              int64_t batch, float beta1, float beta2, float adam_eps, void *workspace,
+                                              int64_t workspace_bytes, void *stream);
+
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 
 typedef struct boattoy_handle *boattoy_t;

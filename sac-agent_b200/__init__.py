@@ -22,11 +22,11 @@ __all__ = ["AttrDict", "load_config", "params_from_config", "BoatEnvError", "lib
            "BatchedBoatEnv", "BoatEnv", "Box", "TERM_NAMES", "ReplayBuffer", "ToyCar", "ToyParachute",
            "BatchedRecorder", "DeviceRecorder", "all_reduce_counters", "make_sharded_env", "shard_range",
            "Experiment", "HPTuner", "get_experiment_config", "info_from_counters", "AgentPopulation",
-           "ContinuousAgent", "SACLearner", "OverlappedActorLearner"]
+           "ContinuousAgent", "SACLearner", "SAC2Learner", "OverlappedActorLearner"]
 
 
 def __getattr__(name):  # the agent pulls in torch.nn / torch.optim: imported on first use only
-    if name in ("ContinuousAgent", "SACLearner", "OverlappedActorLearner"):
+    if name in ("ContinuousAgent", "SACLearner", "SAC2Learner", "OverlappedActorLearner"):
         from . import continuous_agent
         return getattr(continuous_agent, name)
     raise AttributeError(name)

@@ -45,6 +45,11 @@ class SacMember(C.Structure):
                                                      ("tau", C.c_float), ("adam_state", vp), ("losses", vp)]
 
 
+class Sac2Member(C.Structure):
+    """boatagent_sac2_member: one agent's arguments of boatagent_sac2_update_members."""
+    _fields_ = [("base", SacMember), ("target_entropy", C.c_float)]
+
+
 class SampleMember(C.Structure):
     """boatreplay_sample_member: one ring's arguments of boatreplay_sample_members."""
     _fields_ = [("ring", vp), ("seed", u64), ("counter", u64)] + [(name, vp) for name in ("s_out", "a_out", "r_out",
@@ -94,6 +99,9 @@ SIGNATURES = {
                                                i64, vp]),
     "boatagent_sac_gradients_members": (C.c_int, [C.POINTER(SacMember), i32, i64, C.c_float, vp, i64, vp]),
     "boatagent_adam_polyak_members": (C.c_int, [C.POINTER(SacMember), i32, C.c_float, C.c_float, C.c_float, vp]),
+    "boatagent_sac2_update_workspace_bytes": (i64, [i64]),
+    "boatagent_sac2_update_members": (C.c_int, [C.POINTER(Sac2Member), i32, i64, C.c_float, C.c_float, C.c_float, vp,
+                                                i64, vp]),
     "boatreplay_sample_members": (C.c_int, [C.POINTER(SampleMember), i32, i64, vp]),
     "boatreplay_create": (C.c_int, [i64, i32, i32, C.c_int, C.c_int, C.POINTER(vp)]),
     "boatreplay_destroy": (C.c_int, [vp]),

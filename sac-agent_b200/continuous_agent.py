@@ -22,6 +22,8 @@ the data lives and how the update is driven:
 
 `SACLearner` is the update rule on plain tensors (any torch device): the parity tests drive it with
 the batch, initial weights and Gaussian draws of a recorded run of the reference's own `learn()`.
+`SAC2Learner` (`ContinuousAgent(algorithm="sac2")`) is SAC with twin target critics and a learned entropy temperature
+instead of the reference's value networks.
 """
 from __future__ import annotations
 
@@ -34,7 +36,7 @@ import torch
 import torch.nn.functional as F
 
 from .buffer import ReplayBuffer
-from .networks import ActorNetwork, CriticNetwork, ValueNetwork
+from .networks import ActorNetwork, CriticNetwork, TemperatureNetwork, ValueNetwork
 
 
 class _AdamSlot(C.Structure):
@@ -104,6 +106,8 @@ class FusedLearner:
       adam()            Adam + Polyak of every agent from its `.grad` tensors (boatagent_adam_polyak_members, one
                         launch).
 
+    Agents of algorithm "sac2" (all or none) run boatagent_sac2_update_members (three launches) and have no split
+    launches.
     The learning rates are read from the agents' DeviceAdam slots and gamma, reward scale and tau from their learners at
     every launch, so `ContinuousAgent.set_hyperparameters` reaches the next one.  The other pointers (batch, draws,
     `.grad` tensors, losses) are taken at the first launch and must stay the same tensors after it."""
@@ -117,27 +121,29 @@ class FusedLearner:
             raise ValueError("learner_precision='tcgen05': the BoatEnv agent (11 observations, one action) and a "
                              f"batch size that is a positive multiple of 128 (got {agent.input_dims}, "
                              f"{agent.get_n_actions()} actions, batch {B})")
-        if any(tuple(p.shape) != (256, 256) for p in (L.actor.fc2.weight, L.critic_1.fc2.weight,
-                                                      L.critic_2.fc2.weight, L.value.fc2.weight)):
+        if any(tuple(net.fc2.weight.shape) != (256, 256) for net in L.networks() if hasattr(net, "fc2")):
             raise ValueError("learner_precision='tcgen05': 256-wide hidden layers only")
 
     def __init__(self, agents):
         self.agents = list(agents)
         a0 = self.agents[0]
-        if not 1 <= len(self.agents) <= 16 or any(a.batch_size != a0.batch_size or a.device != a0.device
-                                                  for a in self.agents):
-            raise ValueError("FusedLearner: 1 to 16 agents (BOATAGENT_SAC_MAX_MEMBERS) of one batch size and device")
+        if not 1 <= len(self.agents) <= 16 or any(a.batch_size != a0.batch_size or a.device != a0.device or
+                                                  a.algorithm != a0.algorithm for a in self.agents):
+            raise ValueError("FusedLearner: 1 to 16 agents (BOATAGENT_SAC_MAX_MEMBERS) of one batch size, device and "
+                             "algorithm")
         for a in self.agents:
             self.check(a)
         o0 = a0.learner.optimizer
         self._lib, self._L, self.device, self.batch_size = o0._lib, o0._L, a0.device, a0.batch_size
-        self.ws = torch.empty(len(self.agents) * int(self._L.boatagent_sac_update_workspace_bytes(self.batch_size)),
-                              dtype=torch.uint8, device=self.device)
+        self.v2 = a0.algorithm == "sac2"   # boatagent_sac2_update_members (the update only)
+        ws_bytes = (self._L.boatagent_sac2_update_workspace_bytes if self.v2 else
+                    self._L.boatagent_sac_update_workspace_bytes)(self.batch_size)
+        self.ws = torch.empty(len(self.agents) * int(ws_bytes), dtype=torch.uint8, device=self.device)
         self._table = None
 
     def _launch(self, name, *args):
         if self._table is None:   # on the first launch: like the fp32 learner, no .grad before the first update
-            self._table = (self._lib.SacMember * len(self.agents))()
+            self._table = ((self._lib.Sac2Member if self.v2 else self._lib.SacMember) * len(self.agents))()
             for m, a in enumerate(self.agents):
                 o = a.learner.optimizer
                 for k, p in enumerate(o.params):   # the batch gradient goes where the fp32 learner leaves it
@@ -145,28 +151,38 @@ class FusedLearner:
                         p.grad = torch.zeros_like(p)
                     o._slots[k].grad = p.grad.data_ptr()
                 s, act, r, s2, d = a._batch
-                self._table[m] = self._lib.SacMember(
+                e = self._lib.SacMember(
                     s.data_ptr(), act.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), a._eps.data_ptr(),
                     a.learner.actor.max_action.data_ptr(), C.cast(o._slots, C.c_void_p), len(o.params), 0.0, 0.0, 0.0,
                     o.state.data_ptr(), a._loss_buf.data_ptr())
+                self._table[m] = self._lib.Sac2Member(e, 0.0) if self.v2 else e
         for e, a in zip(self._table, self.agents):
             L = a.learner
-            e.gamma, e.reward_scale, e.tau = float(L.gamma), float(L.scale), float(L.optimizer.tau)
+            b = e.base if self.v2 else e
+            b.gamma, b.reward_scale, b.tau = float(L.gamma), float(L.scale), float(L.optimizer.tau)
+            if self.v2:
+                e.target_entropy = float(L.target_entropy)
         with torch.cuda.device(self.device):   # the ABI launches on the current device
             stream = torch.cuda.current_stream().cuda_stream
             self._lib.check(getattr(self._L, name)(self._table, len(self.agents), *args, stream), name)
 
     def update(self):
         o = self.agents[0].learner.optimizer
-        self._launch("boatagent_sac_update_members", self.batch_size, o.betas[0], o.betas[1], o.eps,
-                     self.ws.data_ptr(), self.ws.numel())
+        self._launch("boatagent_sac2_update_members" if self.v2 else "boatagent_sac_update_members", self.batch_size,
+                     o.betas[0], o.betas[1], o.eps, self.ws.data_ptr(), self.ws.numel())
 
     def gradients(self, scale):
+        self._split_v1_only()
         self._launch("boatagent_sac_gradients_members", self.batch_size, scale, self.ws.data_ptr(), self.ws.numel())
 
     def adam(self):
+        self._split_v1_only()
         o = self.agents[0].learner.optimizer
         self._launch("boatagent_adam_polyak_members", o.betas[0], o.betas[1], o.eps)
+
+    def _split_v1_only(self):
+        if self.v2:
+            raise ValueError("FusedLearner: the split gradients / Adam launches (data-parallel training) are SAC-v1's")
 
 
 def point_grads_into(agent, row):
@@ -287,6 +303,118 @@ class SACLearner:
         return (value_loss.detach(), actor_loss.detach(), critic_loss.detach()), grads_v, grads_a, grads_c
 
 
+class SAC2Learner:
+    """SAC with automatic entropy tuning (Haarnoja et al. 2018, "Soft Actor-Critic Algorithms and Applications"): the
+    actor, two critics with Polyak target critics, no value network, and a temperature alpha = exp(log_alpha) learned
+    towards `target_entropy` (default -n_actions).  Same interface as SACLearner; losses are (temperature, actor,
+    critic).
+
+    Every loss of one update reads the weights and alpha as they were before it; ONE Adam step over three learning rates
+    (actor: alpha, critics: beta, log_alpha: temperature_lr, default beta) and the Polyak average of both target critics
+    follow, as SACLearner argues for v1."""
+
+    def __init__(self, input_dims, n_actions, max_action, alpha, beta, gamma, tau, reward_scale, experiment_dir=None,
+                 device="cuda", torch_reference_math=False, target_entropy=None, init_temperature=1.0,
+                 temperature_lr=None):
+        self.device = torch.device(device)
+        if self.device.type != "cuda" and not torch_reference_math:
+            raise RuntimeError("SAC2Learner needs a CUDA device; pass torch_reference_math=True for the PyTorch "
+                               "restatement of the update (parity tests only)")
+        self.gamma, self.tau, self.scale = float(gamma), float(tau), float(reward_scale)
+        self.target_entropy = float(-n_actions if target_entropy is None else target_entropy)
+        temperature_lr = beta if temperature_lr is None else temperature_lr
+        d = tuple(input_dims)
+        # a fixed creation order: identical torch seeds give identical weights
+        self.actor = ActorNetwork(experiment_dir, d, max_action, n_actions=n_actions, name="actor_network")
+        self.critic_1 = CriticNetwork(experiment_dir, d, n_actions, name="critic_network_1")
+        self.critic_2 = CriticNetwork(experiment_dir, d, n_actions, name="critic_network_2")
+        self.target_critic_1 = CriticNetwork(experiment_dir, d, n_actions, name="target_critic_network_1")
+        self.target_critic_2 = CriticNetwork(experiment_dir, d, n_actions, name="target_critic_network_2")
+        self.temperature = TemperatureNetwork(experiment_dir, init_temperature)
+        for net in self.networks():
+            net.to(self.device)
+        self._actor_params = list(self.actor.parameters())
+        self._critic_params = list(self.critic_1.parameters()) + list(self.critic_2.parameters())
+        self._temperature_params = [self.temperature.log_alpha]
+        self._target_params = list(self.target_critic_1.parameters()) + list(self.target_critic_2.parameters())
+        groups = [(self._actor_params, alpha), (self._critic_params, beta), (self._temperature_params, temperature_lr)]
+        if self.device.type == "cuda":
+            self.optimizer = DeviceAdam(groups, polyak=list(zip(self._critic_params, self._target_params)), tau=self.tau)
+        else:
+            self.optimizer = torch.optim.Adam([{"params": ps, "lr": lr} for ps, lr in groups])
+        for p in self._target_params:
+            p.requires_grad_(False)
+        self.update_network_parameters(tau=1.0)
+
+    def networks(self):
+        return (self.actor, self.critic_1, self.critic_2, self.target_critic_1, self.target_critic_2, self.temperature)
+
+    def alpha(self):
+        """alpha = exp(log_alpha), a detached [1] tensor."""
+        return self.temperature.log_alpha.detach().exp()
+
+    @torch.no_grad()
+    def update_network_parameters(self, tau=None):
+        """target_critic_k = tau * critic_k + (1 - tau) * target_critic_k."""
+        tau = self.tau if tau is None else float(tau)
+        tgt, src = self._target_params, self._critic_params
+        if tau == 1.0:
+            torch._foreach_copy_(tgt, src)
+            return
+        torch._foreach_mul_(tgt, 1.0 - tau)
+        torch._foreach_add_(tgt, src, alpha=tau)
+
+    def update(self, state, action, reward, new_state, done, eps_sample=None, eps_rsample=None):
+        """One update on a batch (shapes as SACLearner.update; eps_sample draws a' on new_state, eps_rsample the
+        reparameterised action on state).  Returns (temperature_loss, actor_loss, critic_loss) as 0-d tensors."""
+        losses, grads = self._losses_and_grads(state, action, reward, new_state, done, eps_sample, eps_rsample)
+        for p, g in zip(self.optimizer_params(), grads):
+            p.grad = g
+        if isinstance(self.optimizer, DeviceAdam):   # Adam for the three groups + both Polyak averages, one launch
+            self.optimizer.step(grads)
+        else:
+            self.optimizer.step()
+            self.update_network_parameters()
+        return losses
+
+    def optimizer_params(self):
+        """The trained tensors in DeviceAdam's order: actor 8, critic 1 6, critic 2 6, log_alpha 1."""
+        return self._actor_params + self._critic_params + self._temperature_params
+
+    def gradients(self, state, action, reward, new_state, done, eps_sample, eps_rsample, out, scale=1.0):
+        """`update` without the optimiser step, as SACLearner.gradients (out: the 21 gradients, then the 3 losses)."""
+        losses, grads = self._losses_and_grads(state, action, reward, new_state, done, eps_sample, eps_rsample)
+        torch._foreach_copy_(out, list(grads) + list(losses))
+        if scale != 1.0:
+            torch._foreach_mul_(out, scale)
+
+    def _losses_and_grads(self, state, action, reward, new_state, done, eps_sample, eps_rsample):
+        """The three losses (detached) and the gradients of the trained tensors in DeviceAdam's order."""
+        alpha = self.alpha()
+        with torch.no_grad():
+            a_next, lp_next = self.actor.sample_normal(new_state, reparameterize=False, eps=eps_sample)
+            q_next = torch.min(self.target_critic_1(new_state, a_next), self.target_critic_2(new_state, a_next)).view(-1)
+            v_next = q_next - alpha * lp_next.view(-1)
+            y = self.scale * reward + self.gamma * torch.where(done, torch.zeros_like(v_next), v_next)
+
+        actions, log_probs = self.actor.sample_normal(state, reparameterize=True, eps=eps_rsample)
+        critic_value = torch.min(self.critic_1(state, actions), self.critic_2(state, actions)).view(-1)
+        actor_loss = torch.mean(alpha * log_probs.view(-1) - critic_value)
+        # only the actor's gradients: what this loss sends into the critics is discarded, as in v1
+        grads_a = torch.autograd.grad(actor_loss, self._actor_params)
+
+        entropy_gap = torch.mean(log_probs.detach().view(-1) + self.target_entropy)
+        temperature_loss = -(self.temperature.log_alpha * entropy_gap).sum()
+        grads_t = torch.autograd.grad(temperature_loss, self._temperature_params)
+
+        q1 = self.critic_1(state, action).view(-1)
+        q2 = self.critic_2(state, action).view(-1)
+        critic_loss = 0.5 * F.mse_loss(q1, y) + 0.5 * F.mse_loss(q2, y)
+        grads_c = torch.autograd.grad(critic_loss, self._critic_params)
+        losses = (temperature_loss.detach(), actor_loss.detach(), critic_loss.detach())
+        return losses, tuple(grads_a) + tuple(grads_c) + tuple(grads_t)
+
+
 class DataParallelState(list):
     """`training_tensors()` of a data-parallel agent: ONE agent's state, held equal by every rank of its group, so
     population rounds (population.exploit_explore) must not hand it between ranks."""
@@ -302,7 +430,14 @@ class ContinuousAgent:
     same number of envs (`learn()` updates on all ranks or on none without a vote)."""
 
     def __init__(self, config, experiment_dir, input_dims, env, device=None, seed=0, use_cuda_graph=True,
-                 memory=None, policy_precision="fp32", learner_precision="fp32", data_parallel=None):
+                 memory=None, policy_precision="fp32", learner_precision="fp32", data_parallel=None, algorithm="sac1",
+                 target_entropy=None, init_temperature=1.0, temperature_lr=None):
+        if algorithm not in ("sac1", "sac2"):
+            raise ValueError(f"algorithm: sac1 or sac2, got {algorithm!r}")
+        if algorithm == "sac1" and (target_entropy is not None or init_temperature != 1.0 or temperature_lr is not None):
+            raise ValueError("target_entropy, init_temperature and temperature_lr belong to algorithm='sac2'")
+        if algorithm == "sac2" and data_parallel is not None and data_parallel is not False:
+            raise ValueError("algorithm='sac2' does not train data-parallel")
         if not torch.cuda.is_available():
             raise RuntimeError("sac_agent_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.env = env
@@ -315,12 +450,22 @@ class ContinuousAgent:
         self.memory = memory if memory is not None else ReplayBuffer(
             a.max_size, self.input_dims, self.get_n_actions(), precision="fp32", device=self.device.index, seed=seed,
             as_torch=True)
-        self.learner = SACLearner(self.input_dims, self.get_n_actions(), self.get_max_actions(), a.learning_rate_alpha,
-                                  a.learning_rate_beta, a.gamma, a.tvn_parameter_modulation_tau, a.reward_scale,
-                                  experiment_dir=experiment_dir, device=self.device)
+        # algorithm "sac2": SAC2Learner (twin target critics, learned temperature) instead of the reference's SAC-v1
+        self.algorithm = algorithm
+        learner_args = (self.input_dims, self.get_n_actions(), self.get_max_actions(), a.learning_rate_alpha,
+                        a.learning_rate_beta, a.gamma, a.tvn_parameter_modulation_tau, a.reward_scale)
+        if algorithm == "sac2":
+            self.learner = SAC2Learner(*learner_args, experiment_dir=experiment_dir, device=self.device,
+                                       target_entropy=target_entropy, init_temperature=init_temperature,
+                                       temperature_lr=temperature_lr)
+        else:
+            self.learner = SACLearner(*learner_args, experiment_dir=experiment_dir, device=self.device)
         L = self.learner
         self.actor, self.critic_1, self.critic_2 = L.actor, L.critic_1, L.critic_2
-        self.value, self.target_value = L.value, L.target_value
+        if algorithm == "sac2":
+            self.target_critic_1, self.target_critic_2 = L.target_critic_1, L.target_critic_2
+        else:
+            self.value, self.target_value = L.value, L.target_value
         self.use_cuda_graph = bool(use_cuda_graph)
         if policy_precision not in ("fp32", "tf32", "bf16", "tcgen05"):
             raise ValueError("policy_precision: fp32, tf32, bf16 or tcgen05")
@@ -617,6 +762,12 @@ class ContinuousAgent:
     def update_network_parameters(self, tau=None):
         self.learner.update_network_parameters(tau)
 
+    def temperature(self):
+        """algorithm "sac2": the entropy temperature alpha = exp(log_alpha) as a 0-d device tensor (no sync)."""
+        if self.algorithm != "sac2":
+            raise ValueError("temperature(): SAC-v1 has no learned temperature (algorithm='sac2' has)")
+        return self.learner.alpha()[0]
+
     def save_models(self):
         """base_network.py:13-14 for the five networks (weights only, the reference's checkpoint format)."""
         for net in self.learner.networks():
@@ -638,13 +789,15 @@ class ContinuousAgent:
 
     def set_hyperparameters(self, alpha=None, beta=None, gamma=None, tau=None):
         """New learning rates / discount / target smoothing for the following updates.  The captured update graph
-        holds the old values as kernel arguments, so it is dropped and re-captured by the next learn()."""
+        holds the old values as kernel arguments, so it is dropped and re-captured by the next learn().  beta is the
+        critics' (and v1's value network's) learning rate; SAC-v2's temperature keeps its own."""
         L, o = self.learner, self.learner.optimizer
         n_actor = len(L._actor_params)
+        n_beta = len(o.params) - n_actor - len(getattr(L, "_temperature_params", ()))
         for k in range(len(o.params)):
             if k < n_actor and alpha is not None:
                 o._slots[k].lr = float(alpha)
-            if k >= n_actor and beta is not None:
+            if n_actor <= k < n_actor + n_beta and beta is not None:
                 o._slots[k].lr = float(beta)
         if gamma is not None:
             L.gamma = self.gamma = float(gamma)

@@ -18,6 +18,11 @@
 // boatagent_sac_update and boatagent_sac_gradients are the one-member case of boatagent_sac_update_members and
 // boatagent_sac_gradients_members.
 //
+// SAC-v2 (boatagent_sac2_update_members: twin target critics, no value network, a learned temperature) reuses the
+// building blocks in three launches: sac2_rows_kernel (the row pass of sac2_rows_tile, six stagings as in v1),
+// sac2_params_kernel (the gradients-only parameter body over its three trained networks, plus the log alpha gradient)
+// and adam_polyak_members_kernel over its 21 slots.
+//
 // Operands in shared memory and in the workspace use the 8x8 core-matrix layout of actor_tc.cuh: element (r, c) of
 // an R-row matrix at (c / 8) * (R * 16) + r * 16 + (c % 8) * 2.  The same bytes are a K-major operand with rows = M/N
 // (LBO = R * 16, SBO = 128) and an MN-major operand with rows = K (LBO = 128, SBO = R * 16): so W2 [out][in] is the B
@@ -25,6 +30,7 @@
 // are the A and B operands of dW2 = dZ2^T . H1 without a transpose.
 #include <cstdint>
 #include <cstring>
+#include <type_traits>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
@@ -50,7 +56,12 @@ constexpr size_t kWsH2 = kWsDz2 + kRows * kHidden * 4;       // fp32 [256][128]:
 constexpr size_t kWsSmall = kWsH2 + kRows * kHidden * 4;     // fp32 [16][128]
 constexpr size_t kWsNet = kWsSmall + kSmall * kRows * 4;
 constexpr size_t kWsLoss = 4;                                // per tile: sum (V - vt)^2, sum (lp2 - minQ), sum (q_k - q_hat)^2
-constexpr size_t ws_bytes(long long tiles) { return (size_t)tiles * (kNets * kWsNet + 16 * kWsLoss); }
+constexpr size_t ws_bytes(long long tiles, int nets = kNets) { return (size_t)tiles * (nets * kWsNet + 16 * kWsLoss); }
+
+// SAC-v2 (boatagent_sac2_update_members): three trained networks in workspace order actor, critic 1, critic 2, and 21
+// slots -- actor 8, critic 1 6, critic 2 6 (their targets the target critics), log alpha 1.  slot_of and the first 20
+// slots' shapes are v1's.  Loss partials per tile: sum (lp + target_entropy), sum (alpha lp - minQ), sum (q_k - y)^2.
+constexpr int kNets2 = 3, kSlots2 = 21;
 
 // shared memory of the row kernel
 constexpr int kLW1 = 0;                                 // bf16 core [256][16]
@@ -110,6 +121,17 @@ struct MemberParamArgs {
 static_assert(sizeof(MemberRowArgs) <= 32764, "kernel parameter limit");
 static_assert(sizeof(MemberParamArgs) <= 32764, "kernel parameter limit");
 
+// SAC-v2 row arguments: net[] = actor, critic 1, critic 2, target critic 1, target critic 2
+struct Row2Args {
+    RowArgs r;
+    const float *log_alpha;
+    float target_entropy;
+};
+struct MemberRow2Args {
+    Row2Args m[BOATAGENT_SAC_MAX_MEMBERS];
+};
+static_assert(sizeof(MemberRow2Args) <= 32764, "kernel parameter limit");
+
 __device__ __forceinline__ uint32_t core_off(int r, int c, int rows) { return (uint32_t)((c >> 3) * (rows * 16) + r * 16 + (c & 7) * 2); }
 
 // Sum over the 128 threads of the CTA, fixed order (butterfly within warps, then warps 0..3).
@@ -133,6 +155,33 @@ struct Rows {
     uint64_t *bar;
     uint32_t phase;
     int tid;
+
+    // the CTA's barrier and its 512 TMEM columns (warp 0 allocates into *slot)
+    __device__ __forceinline__ void open(unsigned char *s, uint32_t *slot, int t) {
+        smem = s;
+        sbase = smem_u32(s);
+        bar = reinterpret_cast<uint64_t *>(s + kLBar);
+        phase = 0;
+        tid = t;
+        if (t == 0) {
+            mbar_init(bar, 1);
+            mbar_fence_init();
+        }
+        if ((t >> 5) == 0) {
+            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
+            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        }
+        tc_fence_before();
+        __syncthreads();
+        tc_fence_after();
+        tmem = *slot;
+        lane_base = tmem + ((uint32_t)((t >> 5) * 32) << 16);
+    }
+    __device__ __forceinline__ void close() {
+        tc_fence_before();
+        __syncthreads();
+        if ((tid >> 5) == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+    }
 
     // the hand-off from the threads' shared-memory / TMEM writes to one MMA batch, issued by thread 0
     __device__ __forceinline__ void mma_sync() {
@@ -331,26 +380,8 @@ __device__ __forceinline__ float min_share(float a, float b) { return a < b ? 1.
 __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
-    const int warp = tid >> 5;
     Rows R;
-    R.smem = smem;
-    R.sbase = smem_u32(smem);
-    R.bar = reinterpret_cast<uint64_t *>(smem + kLBar);
-    R.phase = 0;
-    R.tid = tid;
-    if (tid == 0) {
-        mbar_init(R.bar, 1);
-        mbar_fence_init();
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    R.tmem = tmem_slot;
-    R.lane_base = R.tmem + ((uint32_t)(warp * 32) << 16);
+    R.open(smem, &tmem_slot, tid);
 
     const long long B = args.batch, row = (long long)blockIdx.x * kRows + tid;
     const float invB = 1.0f / (float)B;
@@ -432,10 +463,7 @@ __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid
                      (q_sa[1] - q_hat) * (q_sa[1] - q_hat)};
     cta_sum4(part, reinterpret_cast<float *>(smem + kLRed));
     if (tid < 4) loss_part[tid] = part[tid];
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(R.tmem) : "memory");
+    R.close();
 }
 
 // member blockIdx.y, its tiles on blockIdx.x
@@ -443,13 +471,111 @@ __global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_con
     sac_rows_tile(args.m[blockIdx.y], threadIdx.x);
 }
 
+// The SAC-v2 row pass of one 128-row tile, with alpha = exp(log_alpha) read before the update:
+//   y = scale r + gamma (1 - done) (min(Qt1, Qt2)(s', a') - alpha lp'),   a', lp' = actor(s', eps[0])
+//   critics: 0.5 mse(Q_k(s, a), y);  actor: mean(alpha lp - min(Q1, Q2)(s, a~)),   a~, lp = actor(s, eps[1])
+// Six stagings, as in v1: actor, the two target critics, the two critics, the actor again for its backward pass.
+__device__ __forceinline__ void sac2_rows_tile(const Row2Args &a2, const int tid) {
+    extern __shared__ __align__(1024) unsigned char smem[];
+    __shared__ uint32_t tmem_slot;
+    const RowArgs &args = a2.r;
+    Rows R;
+    R.open(smem, &tmem_slot, tid);
+
+    const long long B = args.batch, row = (long long)blockIdx.x * kRows + tid;
+    const float invB = 1.0f / (float)B;
+    unsigned char *ws_tile = args.ws + (size_t)blockIdx.x * kNets2 * kWsNet;
+    unsigned char *ws_net[kNets2];
+#pragma unroll
+    for (int k = 0; k < kNets2; ++k) ws_net[k] = ws_tile + (size_t)k * kWsNet;
+    float *loss_part = reinterpret_cast<float *>(args.ws + (size_t)gridDim.x * kNets2 * kWsNet) + blockIdx.x * kWsLoss;
+
+    float s[kK1], s2[kK1];
+#pragma unroll
+    for (int q = 0; q < kK1; ++q) {
+        s[q] = q < kObs ? __ldg(args.state + row * kObs + q) : 0.f;
+        s2[q] = q < kObs ? __ldg(args.new_state + row * kObs + q) : 0.f;
+    }
+    const float a_batch = __ldg(args.action + row), rew = __ldg(args.reward + row);
+    const bool done = __ldg(args.done + row) != 0;
+    const float e0 = __ldg(args.eps + row), e1 = __ldg(args.eps + B + row), ma = __ldg(args.max_action);
+    const float alpha = expf(__ldg(a2.log_alpha));
+    float y[2];
+    uint32_t m1[8], m2[8];
+
+    // actor: the target's draw on new_state, then the trained pass on state (its activations to the workspace)
+    uint32_t am1[8], am2[8];
+    R.stage(args.net[0]);
+    R.forward(s2, y, m1, m2, nullptr);
+    float a_next, a_pi;
+    const float lp_next = gaussian_head_fwd(y[0], y[1], e0, ma, a_next);
+    R.forward(s, y, am1, am2, ws_net[0]);
+    const float mean = y[0], raw_std = y[1];
+    const float lp = gaussian_head_fwd(mean, raw_std, e1, ma, a_pi);
+
+    // target critics at (s', a')
+    float qt[2];
+#pragma unroll 1
+    for (int k = 0; k < 2; ++k) {
+        R.stage(args.net[3 + k]);
+        float x[kK1];
+#pragma unroll
+        for (int q = 0; q < kK1; ++q) x[q] = s2[q];
+        x[kObs] = a_next;
+        R.forward(x, y, m1, m2, nullptr);
+        qt[k] = y[0];
+    }
+    const float q_hat = args.scale * rew + args.gamma * (done ? 0.f : fminf(qt[0], qt[1]) - alpha * lp_next);
+
+    // the critics: Q and dQ/da at (s, a~) for the actor, the trained pass at (s, a)
+    float q_pi[2], dq_pi[2], q_sa[2];
+#pragma unroll 1
+    for (int k = 0; k < 2; ++k) {
+        R.stage(args.net[1 + k]);
+        float x[kK1];
+#pragma unroll
+        for (int q = 0; q < kK1; ++q) x[q] = s[q];
+        x[kObs] = a_pi;
+        R.forward(x, y, m1, m2, nullptr);
+        q_pi[k] = y[0];
+        const float one[2] = {1.f, 0.f};
+        dq_pi[k] = R.backward(one, m1, m2, nullptr);
+        x[kObs] = a_batch;
+        R.forward(x, y, m1, m2, ws_net[1 + k]);
+        q_sa[k] = y[0];
+        const float dq[2] = {(q_sa[k] - q_hat) * invB, 0.f};
+        R.backward(dq, m1, m2, ws_net[1 + k]);
+        put_small(ws_net[1 + k], tid, x, dq[0], 0.f);
+    }
+
+    // actor: d loss / d lp = alpha / B; the critics' gradients of this loss are discarded
+    const float w1 = min_share(q_pi[0], q_pi[1]), w2 = min_share(q_pi[1], q_pi[0]);
+    const float grad_action = -(w1 * dq_pi[0] + w2 * dq_pi[1]) * invB;
+    float dyh[2];
+    gaussian_head_bwd(mean, raw_std, e1, ma, grad_action, alpha * invB, dyh[0], dyh[1]);
+    R.stage(args.net[0]);
+    R.backward(dyh, am1, am2, ws_net[0]);
+    put_small(ws_net[0], tid, s, dyh[0], dyh[1]);
+
+    float part[4] = {lp + a2.target_entropy, alpha * lp - fminf(q_pi[0], q_pi[1]),
+                     (q_sa[0] - q_hat) * (q_sa[0] - q_hat), (q_sa[1] - q_hat) * (q_sa[1] - q_hat)};
+    cta_sum4(part, reinterpret_cast<float *>(smem + kLRed));
+    if (tid < 4) loss_part[tid] = part[tid];
+    R.close();
+}
+
+__global__ void __launch_bounds__(kLThreads, 1) sac2_rows_kernel(const __grid_constant__ MemberRow2Args args) {
+    sac2_rows_tile(args.m[blockIdx.y], threadIdx.x);
+}
+
 // slot of tensor `t` (0 w1, 1 b1, 2 w2, 3 b2, 4 / 6 head weights, 5 / 7 head biases) of trained network `n`
 __device__ __forceinline__ int slot_of(int n, int t) { return n == 0 ? t : 8 + 6 * (n - 1) + t; }
 
 // kAdam: write the gradients, apply Adam + Polyak and count the step; else write grad_scale times the gradients only.
 // blockIdx.x is the CTA and gridDim.x the CTA count of ONE update (member = blockIdx.y), so the step-counter ticket
-// counts one member's CTAs.
-template <bool kAdam>
+// counts one member's CTAs.  kN: the trained networks of the workspace, kNets (SAC-v1) or kNets2 (SAC-v2, whose last
+// CTA also writes the log alpha gradient).
+template <bool kAdam, int kN = kNets>
 __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
@@ -472,7 +598,7 @@ __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const in
         }
     };
     const int blk = blockIdx.x;
-    if (blk < 2 * kNets) {
+    if (blk < 2 * kN) {
         // ---- fc2 weight gradient of network blk / 2, output rows 128 (blk % 2) .. + 127: dW2 = dZ2^T . H1 on tcgen05
         const int n = blk >> 1, half = blk & 1;
         uint64_t *bar = reinterpret_cast<uint64_t *>(smem + kPBar);
@@ -489,7 +615,7 @@ __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const in
         tc_fence_after();
         const uint32_t tmem = tmem_slot, sbase = smem_u32(smem);
         for (long long t = 0; t < tiles; ++t) {   // K = the batch, one 128-row tile at a time
-            const unsigned char *w = args.ws + ((size_t)t * kNets + n) * kWsNet;
+            const unsigned char *w = args.ws + ((size_t)t * kN + n) * kWsNet;
             const uint4 *srcA = reinterpret_cast<const uint4 *>(w + kWsDz2b + (size_t)half * (kRows * 128 * 2));
             const uint4 *srcB = reinterpret_cast<const uint4 *>(w + kWsH1);
 #pragma unroll
@@ -526,16 +652,16 @@ __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const in
         tc_fence_before();
         __syncthreads();
         if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
-    } else if (blk < 2 * kNets + kNets * (kHidden / 8)) {
+    } else if (blk < 2 * kN + kN * (kHidden / 8)) {
         // ---- one warp per hidden unit j of network n: fc1 weights and bias, fc2 bias, head weights (+ head biases at
         // j = 0), reduced over the batch in a fixed order (rows strided over the lanes, then a butterfly)
-        const int u = (blk - 2 * kNets) * 8 + warp, n = u / kHidden, j = u % kHidden;
+        const int u = (blk - 2 * kN) * 8 + warp, n = u / kHidden, j = u % kHidden;
         const int in = n == 1 || n == 2 ? kObs + 1 : kObs, nh = n == 0 ? 2 : 1;
         float acc[18];
 #pragma unroll
         for (int q = 0; q < 18; ++q) acc[q] = 0.f;
         for (long long t = 0; t < tiles; ++t) {
-            const unsigned char *w = args.ws + ((size_t)t * kNets + n) * kWsNet;
+            const unsigned char *w = args.ws + ((size_t)t * kN + n) * kWsNet;
             const float *dz1 = reinterpret_cast<const float *>(w + kWsDz1) + j * kRows;
             const float *dz2 = reinterpret_cast<const float *>(w + kWsDz2) + j * kRows;
             const float *h2 = reinterpret_cast<const float *>(w + kWsH2) + j * kRows;
@@ -571,12 +697,19 @@ __device__ __forceinline__ void sac_params_block(const ParamArgs &args, const in
         else if (lane == 17 && j == 0 && nh > 1) adam(slot_of(n, 7), 0, g);
     } else if (tid == 0) {
         // ---- the three losses from the tiles' partial sums, in tile order
-        const float *p = reinterpret_cast<const float *>(args.ws + (size_t)tiles * kNets * kWsNet);
+        const float *p = reinterpret_cast<const float *>(args.ws + (size_t)tiles * kN * kWsNet);
         float s[4] = {0.f, 0.f, 0.f, 0.f};
         for (long long t = 0; t < tiles; ++t)
             for (int q = 0; q < 4; ++q) s[q] += p[t * kWsLoss + q];
         const float invB = 1.0f / (float)B;
-        if constexpr (kAdam) {
+        if constexpr (kN == kNets2) {
+            // temperature loss -log_alpha mean(lp + target_entropy), lp detached: its log alpha gradient is -mean(...)
+            const float ent = s[0] * invB;
+            adam(kSlots2 - 1, 0, -ent);
+            args.losses[0] = (-args.slot[kSlots2 - 1].param[0] * ent) * args.grad_scale;
+            args.losses[1] = (s[1] * invB) * args.grad_scale;
+            args.losses[2] = (0.5f * (s[2] * invB) + 0.5f * (s[3] * invB)) * args.grad_scale;
+        } else if constexpr (kAdam) {
             args.losses[0] = 0.5f * (s[0] * invB);
             args.losses[1] = s[1] * invB;
             args.losses[2] = 0.5f * (s[2] * invB) + 0.5f * (s[3] * invB);
@@ -605,6 +738,11 @@ __global__ void __launch_bounds__(kPThreads) sac_params_kernel(const __grid_cons
     sac_params_block<kAdam>(args.m[blockIdx.y], threadIdx.x);
 }
 
+// SAC-v2 gradients of every member (Adam follows as adam_polyak_members_kernel over the 21 slots)
+__global__ void __launch_bounds__(kPThreads) sac2_params_kernel(const __grid_constant__ MemberParamArgs args) {
+    sac_params_block<false, kNets2>(args.m[blockIdx.y], threadIdx.x);
+}
+
 // Adam + Polyak step (boatagent_adam_polyak_members): member blockIdx.y, its chunks on blockIdx.x
 __global__ void __launch_bounds__(kAdamThreads) adam_polyak_members_kernel(const __grid_constant__ MemberParamArgs args) {
     const ParamArgs &a = args.m[blockIdx.y];
@@ -612,6 +750,7 @@ __global__ void __launch_bounds__(kAdamThreads) adam_polyak_members_kernel(const
 }
 
 constexpr int kParamBlocks = 2 * kNets + kNets * (kHidden / 8) + 1;
+constexpr int kParamBlocks2 = 2 * kNets2 + kNets2 * (kHidden / 8) + 1;
 
 // numel of slot k, in DeviceAdam's order (actor: fc1 w, b, fc2 w, b, mean w, b, std w, b; critics and value: fc1 w, b,
 // fc2 w, b, head w, b)
@@ -620,10 +759,14 @@ constexpr long long expected_numel(int k) {
     return t == 0 ? (long long)kHidden * in : t == 2 ? (long long)kHidden * kHidden : (t == 5 || t == 7) ? 1 : kHidden;
 }
 
-// the CTAs of one agent's Adam step: the chunks of its 26 slots, as boatagent_adam_polyak_step counts them
-constexpr int adam_chunks() {
+// numel of SAC-v2 slot k: v1's actor and critics, then log alpha
+constexpr long long expected_numel2(int k) { return k < kSlots2 - 1 ? expected_numel(k) : 1; }
+
+// the CTAs of one agent's Adam step: the chunks of its 26 (v2: 21) slots, as boatagent_adam_polyak_step counts them
+constexpr int adam_chunks(bool v2 = false) {
     long long n = 0;
-    for (int k = 0; k < kSlots; ++k) n += (expected_numel(k) + kAdamChunk - 1) / kAdamChunk;
+    for (int k = 0; k < (v2 ? kSlots2 : kSlots); ++k)
+        n += ((v2 ? expected_numel2(k) : expected_numel(k)) + kAdamChunk - 1) / kAdamChunk;
     return (int)n;
 }
 
@@ -637,15 +780,22 @@ extern "C" int64_t boatagent_sac_update_workspace_bytes(int64_t batch) {
     return (int64_t)ws_bytes(batch / kRows);
 }
 
+extern "C" int64_t boatagent_sac2_update_workspace_bytes(int64_t batch) {
+    if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
+    return (int64_t)ws_bytes(batch / kRows, kNets2);
+}
+
 namespace {
 
 // The 26 slots of one agent in DeviceAdam's order: every pointer set, the agent's shapes, a target on the value
-// network's tensors and only on them, 16-byte aligned parameters.
-int check_slots(const boatagent_adam_slot *slots) {
-    for (int k = 0; k < kSlots; ++k) {
+// network's tensors and only on them, 16-byte aligned parameters.  v2: the 21 slots, targets on the critics' tensors
+// and only on them.
+int check_slots(const boatagent_adam_slot *slots, bool v2 = false) {
+    for (int k = 0; k < (v2 ? kSlots2 : kSlots); ++k) {
         const boatagent_adam_slot &s = slots[k];
-        if (!s.param || !s.grad || !s.exp_avg || !s.exp_avg_sq || s.numel != expected_numel(k)) return BOATENV_EINVAL;
-        if ((k >= 20) != (s.target != nullptr)) return BOATENV_EINVAL;   // the value network's tensors, and only they
+        if (!s.param || !s.grad || !s.exp_avg || !s.exp_avg_sq || s.numel != (v2 ? expected_numel2(k) : expected_numel(k)))
+            return BOATENV_EINVAL;
+        if ((v2 ? k >= 8 && k < 20 : k >= 20) != (s.target != nullptr)) return BOATENV_EINVAL;
         if ((reinterpret_cast<uintptr_t>(s.param) & 15u) != 0) return BOATENV_EALIGN;
     }
     return 0;
@@ -659,29 +809,42 @@ MemberParamArgs &member_params() {
     static thread_local MemberParamArgs pa;
     return pa;
 }
+MemberRow2Args &member_rows2() {
+    static thread_local MemberRow2Args ra;
+    return ra;
+}
 
-// The member tables of both kernels: every member checked as documented in boatenv.h (its adam_state only with
+const boatagent_sac_member &base_of(const boatagent_sac_member &e) { return e; }
+const boatagent_sac_member &base_of(const boatagent_sac2_member &e) { return e.base; }
+RowArgs &rows_of(RowArgs &r) { return r; }
+RowArgs &rows_of(Row2Args &r) { return r.r; }
+
+// The member tables of the kernels of SAC-v1 (Entry boatagent_sac_member, rows MemberRowArgs) or SAC-v2
+// (boatagent_sac2_member, MemberRow2Args): every member checked as documented in boatenv.h (its adam_state only with
 // `adam`) before anything is launched.
-int member_tables(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch, void *workspace,
+template <class Entry, class RowTable>
+int member_tables(const Entry *members_host, int32_t n_members, int64_t batch, void *workspace,
                   int64_t workspace_bytes, bool adam, float beta1, float beta2, float adam_eps, float grad_scale,
-                  MemberRowArgs &ra, MemberParamArgs &pa) {
+                  RowTable &ra, MemberParamArgs &pa) {
+    constexpr bool v2 = std::is_same<Entry, boatagent_sac2_member>::value;
     if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
     if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
-    const size_t slice = ws_bytes(batch / kRows);   // a multiple of 16: every slice stays 16-byte aligned
+    // a multiple of 16: every slice stays 16-byte aligned
+    const size_t slice = ws_bytes(batch / kRows, v2 ? kNets2 : kNets);
     if (workspace_bytes < 0 || (uint64_t)workspace_bytes < slice * (uint64_t)n_members) return BOATENV_EINVAL;
     if ((reinterpret_cast<uintptr_t>(workspace) & 15u) != 0) return BOATENV_EALIGN;
     std::memset(&ra, 0, sizeof(ra));
     std::memset(&pa, 0, sizeof(pa));
     for (int m = 0; m < n_members; ++m) {
-        const boatagent_sac_member &b = members_host[m];
+        const boatagent_sac_member &b = base_of(members_host[m]);
         if ((adam && !b.adam_state) || !b.state || !b.action || !b.reward || !b.new_state || !b.done || !b.eps ||
-            !b.max_action || !b.slots || !b.losses || b.n_slots != kSlots)
+            !b.max_action || !b.slots || !b.losses || b.n_slots != (v2 ? kSlots2 : kSlots))
             return BOATENV_EINVAL;
-        const int rc = check_slots(b.slots);
+        const int rc = check_slots(b.slots, v2);
         if (rc != 0) return rc;
         unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
 
-        RowArgs &r = ra.m[m];
+        RowArgs &r = rows_of(ra.m[m]);
         r.state = b.state;
         r.action = b.action;
         r.reward = b.reward;
@@ -707,11 +870,18 @@ int member_tables(const boatagent_sac_member *members_host, int32_t n_members, i
         r.net[0] = net(0, kObs, true, false);
         r.net[1] = net(8, kObs + 1, false, false);
         r.net[2] = net(14, kObs + 1, false, false);
-        r.net[3] = net(20, kObs, false, false);
-        r.net[4] = net(20, kObs, false, true);
+        if constexpr (v2) {
+            r.net[3] = net(8, kObs + 1, false, true);
+            r.net[4] = net(14, kObs + 1, false, true);
+            ra.m[m].log_alpha = b.slots[kSlots2 - 1].param;
+            ra.m[m].target_entropy = members_host[m].target_entropy;
+        } else {
+            r.net[3] = net(20, kObs, false, false);
+            r.net[4] = net(20, kObs, false, true);
+        }
 
-        ParamArgs &p = pa.m[m];
-        std::memcpy(p.slot, b.slots, sizeof(p.slot));
+        ParamArgs &p = pa.m[m];   // v2: slots 21.. stay zero
+        std::memcpy(p.slot, b.slots, sizeof(boatagent_adam_slot) * (v2 ? kSlots2 : kSlots));
         p.beta1 = beta1;
         p.beta2 = beta2;
         p.eps = adam_eps;
@@ -737,6 +907,8 @@ int set_smem_attributes() {
         CUDA_TRY(cudaFuncSetAttribute(sac_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac2_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac2_params_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         set_of[dev] = true;
     }
     return 0;
@@ -759,7 +931,35 @@ int launch(bool adam, int32_t n_members, int64_t batch, const MemberRowArgs &ra,
     return (int)cudaGetLastError();
 }
 
+// SAC-v2: the row pass, the gradients, then one coalesced Adam + Polyak launch over the 21 slots (the
+// adam_polyak_members_kernel of v1's split update, on the v2 chunk count; slots 21.. of the table are empty).
+int launch2(int32_t n_members, int64_t batch, const MemberRow2Args &ra, const MemberParamArgs &pa, void *stream) {
+    const int rc = set_smem_attributes();
+    if (rc != 0) return rc;
+    const cudaStream_t s = (cudaStream_t)stream;
+    sac2_rows_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem, s>>>(ra);
+    boatenv::count_launch();
+    CUDA_TRY(cudaGetLastError());
+    sac2_params_kernel<<<dim3(kParamBlocks2, (unsigned)n_members), kPThreads, kPSmem, s>>>(pa);
+    boatenv::count_launch();
+    CUDA_TRY(cudaGetLastError());
+    adam_polyak_members_kernel<<<dim3(adam_chunks(true), (unsigned)n_members), kAdamThreads, 0, s>>>(pa);
+    boatenv::count_launch();
+    return (int)cudaGetLastError();
+}
+
 }  // namespace
+
+extern "C" int boatagent_sac2_update_members(const boatagent_sac2_member *members_host, int32_t n_members,
+                                             int64_t batch, float beta1, float beta2, float adam_eps, void *workspace,
+                                             int64_t workspace_bytes, void *stream) {
+    MemberRow2Args &ra = member_rows2();
+    MemberParamArgs &pa = member_params();
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, beta1, beta2,
+                                 adam_eps, 1.0f, ra, pa);
+    if (rc != 0) return rc;
+    return launch2(n_members, batch, ra, pa, stream);
+}
 
 extern "C" int boatagent_sac_update_members(const boatagent_sac_member *members_host, int32_t n_members, int64_t batch,
                                             float beta1, float beta2, float adam_eps, void *workspace,

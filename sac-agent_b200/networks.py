@@ -176,6 +176,20 @@ class ValueNetwork(BaseNetwork):
         return self.v(x)
 
 
+class TemperatureNetwork(BaseNetwork):
+    """SAC-v2's entropy temperature alpha = exp(log_alpha), log_alpha a one-element parameter, so that checkpoints,
+    state dicts and population hand-overs carry it like a network's weights."""
+
+    def __init__(self, experiment_dir, init_temperature=1.0, name="log_alpha"):
+        super().__init__(name, experiment_dir)
+        if not init_temperature > 0:
+            raise ValueError(f"init_temperature must be positive, got {init_temperature}")
+        self.log_alpha = nn.Parameter(torch.tensor([math.log(init_temperature)], dtype=torch.float32))
+
+    def forward(self):
+        return self.log_alpha.exp()
+
+
 class TensorCorePolicy:
     """choose_action over N envs as ONE tcgen05 kernel (csrc/policy_mlp.cu): the actor's three dense layers
     with bf16 inputs / fp32 accumulation and the tanh-squashed draw, a 128-env tile staying on chip from

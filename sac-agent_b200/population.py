@@ -147,10 +147,15 @@ class AgentPopulation:
 
     ``configs``: one config per member (e.g. its tuned_configs.yaml draw), else ``config`` for all; the batch size must
     be the same.  Change a member's hyper-parameters through ``set_hyperparameters`` or ``exploit_explore`` so that
-    the next ``learn()`` sees them."""
+    the next ``learn()`` sees them.
+
+    ``algorithm``: "sac1" or "sac2" (``ContinuousAgent(algorithm=...)``; every member's SAC-v2 update runs in the same
+    launches).  ``target_entropy``, ``init_temperature`` and ``temperature_lr`` (sac2 only): one value for every member
+    or a sequence of one per member.  SAC-v2 does not train data-parallel."""
 
     def __init__(self, config, members, envs_per_member, seed=0, rank=0, device=None, configs=None,
-                 experiment_dirs=None, buffer_size=None, done_flag_mode=1, data_parallel=None):
+                 experiment_dirs=None, buffer_size=None, done_flag_mode=1, data_parallel=None, algorithm="sac1",
+                 target_entropy=None, init_temperature=1.0, temperature_lr=None):
         import torch
         from . import _lib
         from .boat_env import BatchedBoatEnv
@@ -160,6 +165,25 @@ class AgentPopulation:
         P = int(members)
         if not 1 <= P <= 16:
             raise ValueError(f"AgentPopulation: 1 to 16 members per process (BOATAGENT_SAC_MAX_MEMBERS), got {P}")
+        if algorithm not in ("sac1", "sac2"):
+            raise ValueError(f"AgentPopulation: algorithm sac1 or sac2, got {algorithm!r}")
+        if algorithm == "sac2" and data_parallel is not None and data_parallel is not False:
+            raise ValueError("AgentPopulation: algorithm='sac2' does not train data-parallel")
+        if algorithm == "sac1" and (target_entropy is not None or init_temperature != 1.0 or temperature_lr is not None):
+            raise ValueError("AgentPopulation: target_entropy, init_temperature and temperature_lr belong to "
+                             "algorithm='sac2'")
+
+        def per_member(x, name):
+            xs = list(x) if isinstance(x, (list, tuple)) else [x] * P
+            if len(xs) != P:
+                raise ValueError(f"AgentPopulation: {name} needs one value or one per member ({P})")
+            return xs
+        v2 = [{} for _ in range(P)]
+        if algorithm == "sac2":
+            for name, x in (("target_entropy", target_entropy), ("init_temperature", init_temperature),
+                            ("temperature_lr", temperature_lr)):
+                for m, v in enumerate(per_member(x, name)):
+                    v2[m][name] = v
         configs = list(configs) if configs is not None else [config] * P
         dirs = list(experiment_dirs) if experiment_dirs is not None else [None] * P
         if len(configs) != P or len(dirs) != P:
@@ -193,7 +217,7 @@ class AgentPopulation:
                 torch.manual_seed(weight_seed)
                 agent = ContinuousAgent(cfg, dirs[m], env.observation_space.shape, env, device=self.device.index,
                                         seed=seed + g, memory=mem, policy_precision="tcgen05",
-                                        learner_precision="tcgen05")
+                                        learner_precision="tcgen05", algorithm=algorithm, **v2[m])
             agent._tc_policy = TensorCorePolicy(agent.actor, seed=0x5ac + g)
             self.envs.append(env)
             self.members.append(agent)
@@ -257,8 +281,8 @@ class AgentPopulation:
 
     def learn(self):
         """One update of every member: the batched sample-gather, one Gaussian draw for all, and the two kernels of
-        the members' fused update (``FusedLearner.update``, no sync).  Returns each member's (value, actor, critic)
-        losses as device tensors, or None (nothing launched) while some member's ring holds less than a batch.
+        the members' fused update (``FusedLearner.update``, no sync; SAC-v2: three kernels).  Returns each member's
+        (value, actor, critic) losses -- SAC-v2: (temperature, actor, critic) -- as device tensors, or None (nothing launched) while some member's ring holds less than a batch.
 
         Data-parallel: the update is ``FusedLearner.gradients`` (times 1 / W), one all-reduce (SUM) of every member's
         gradients and losses, and ``FusedLearner.adam``; the losses are the means over the ranks.  The rank shards are
