@@ -2,7 +2,8 @@
 """End-to-end SAC (v1: actor, twin critics, value + target value) on the GPU-resident batched BoatEnv
 and the fused device replay buffer -- BASELINE.json configs[4] / SURVEY.md 8(f) rank 1.  `--algorithm sac2` trains
 SAC with twin target critics and a learned entropy temperature instead (SAC2Learner); its JSON summary adds
-`algorithm` and the final `temperature`.
+`algorithm` and the final `temperature`.  `--prioritized` draws the updates' batches by prioritized experience replay
+(ContinuousAgent(prioritized=True)); its JSON summary adds `prioritized` and the four priority parameters.
 
 The loop is the reference's main.py:72-90 with every piece on the device:
 
@@ -105,7 +106,30 @@ def main(argv=None):
     ap.add_argument("--init-temperature", type=float, default=None, help="sac2: initial alpha (default 1.0)")
     ap.add_argument("--temperature-lr", type=float, default=None,
                     help="sac2: Adam learning rate of log alpha (default: the critics', learning_rate_beta)")
+    ap.add_argument("--prioritized", action="store_true",
+                    help="prioritized experience replay (Schaul et al. 2016): batches drawn by priority, critic loss "
+                         "rows weighted by importance, priorities set from the TD errors")
+    ap.add_argument("--priority-alpha", type=float, default=None, help="--prioritized: priority exponent (default 0.6)")
+    ap.add_argument("--priority-beta", type=float, default=None,
+                    help="--prioritized: initial importance-weight exponent (default 0.4)")
+    ap.add_argument("--priority-beta-updates", type=int, default=None,
+                    help="--prioritized: updates over which beta rises linearly to 1 (default 0: constant)")
+    ap.add_argument("--priority-eps", type=float, default=None,
+                    help="--prioritized: added to |TD| before the exponent (default 1e-6)")
     args = ap.parse_args(argv)
+    priority_flags = (args.priority_alpha, args.priority_beta, args.priority_beta_updates, args.priority_eps)
+    if not args.prioritized and any(x is not None for x in priority_flags):   # checked before any CUDA work
+        ap.error("--priority-alpha, --priority-beta, --priority-beta-updates and --priority-eps need --prioritized")
+    if args.prioritized:
+        for flag, on in (("--data-parallel", args.data_parallel), ("--population", args.population),
+                         ("--overlap", args.overlap)):
+            if on:
+                ap.error(f"--prioritized and {flag} cannot be combined")
+        p = _priority_args(args)
+        if not (p["priority_alpha"] >= 0 and 0 <= p["priority_beta"] <= 1 and p["priority_beta_updates"] >= 0
+                and p["priority_eps"] > 0):
+            ap.error("--priority-alpha >= 0, 0 <= --priority-beta <= 1, --priority-beta-updates >= 0 and "
+                     "--priority-eps > 0")
     if args.algorithm == "sac2":   # checked before any CUDA work
         for flag, on in (("--data-parallel", args.data_parallel), ("--overlap", args.overlap)):
             if on:
@@ -154,6 +178,9 @@ def main(argv=None):
         finally:
             if world > 1:
                 torch.distributed.destroy_process_group()
+    if args.prioritized and args.pbt_every and world > 1:
+        ap.error("--prioritized and --pbt-every across ranks cannot be combined (population rounds between ranks hand "
+                 "over weights, not the priorities of each rank's ring)")
     if args.algorithm == "sac2" and args.pbt_every and world > 1:
         ap.error("--algorithm sac2 and --pbt-every across ranks cannot be combined (population rounds between ranks "
                  "are SAC-v1's; use --population for SAC-v2 population rounds on one GPU)")
@@ -184,13 +211,18 @@ def main(argv=None):
         if args.tune:
             cfg = tuned
     env = S.make_sharded_env(cfg, args.envs, seed=args.seed, precision="fp32", auto_reset=True)
-    mem = S.ReplayBuffer(max(args.buffer, env.n_envs * max(args.collect_steps, 1)), (11,), 1, precision="fp32", device=local_rank,
-                         seed=args.seed + rank, as_torch=True)
+    size = max(args.buffer, env.n_envs * max(args.collect_steps, 1))
+    if args.prioritized:
+        p = _priority_args(args)
+        mem = S.PrioritizedReplayBuffer(size, (11,), 1, precision="fp32", device=local_rank, seed=args.seed + rank,
+                                        as_torch=True, alpha=p["priority_alpha"], eps=p["priority_eps"])
+    else:
+        mem = S.ReplayBuffer(size, (11,), 1, precision="fp32", device=local_rank, seed=args.seed + rank, as_torch=True)
     agent = S.ContinuousAgent(cfg, exp.experiment_dir if exp else None, env.observation_space.shape, env,
                               device=local_rank, seed=args.seed + rank,
                               use_cuda_graph=not args.no_graph, memory=mem, policy_precision=args.policy_precision,
                               learner_precision=args.learner_precision, data_parallel=args.data_parallel or None,
-                              **_algorithm_args(args))
+                              **_algorithm_args(args), **(_priority_args(args) if args.prioritized else {}))
     act = agent.choose_action if args.no_graph else agent.choose_action_graphed
     obs = env.reset()
     rec = None
@@ -292,6 +324,9 @@ def main(argv=None):
         summary["data_parallel"], summary["effective_batch"] = True, world * agent.batch_size
     if args.algorithm == "sac2":
         summary["algorithm"], summary["temperature"] = "sac2", float(agent.temperature())
+    if args.prioritized:
+        summary["prioritized"] = True
+        summary.update(_priority_args(args))
     if args.record_envs:   # over all ranks: envs recorded, and their episodes that ended (one info.csv row each)
         summary["recorded_envs"], summary["recorded_episodes"] = int(recorded[0]), int(recorded[1])
     if args.pbt_every:
@@ -324,6 +359,15 @@ def _algorithm_args(args):
         return {}
     return {"algorithm": "sac2", "target_entropy": args.target_entropy, "temperature_lr": args.temperature_lr,
             "init_temperature": 1.0 if args.init_temperature is None else args.init_temperature}
+
+
+def _priority_args(args):
+    """ContinuousAgent keyword arguments of --prioritized and the priority flags, their defaults filled in."""
+    d = {"priority_alpha": 0.6, "priority_beta": 0.4, "priority_beta_updates": 0, "priority_eps": 1e-6}
+    for k in d:
+        if getattr(args, k) is not None:
+            d[k] = type(d[k])(getattr(args, k))
+    return {"prioritized": True, **d}
 
 
 def _loss_label(args):

@@ -286,6 +286,51 @@ BOATENV_API int boatreplay_set_mem_cntr(boatreplay_t r, int64_t mem_cntr);
 BOATENV_API int64_t boatreplay_mem_cntr(boatreplay_t r); /* buffer.py:6  */
 BOATENV_API int64_t boatreplay_mem_size(boatreplay_t r); /* buffer.py:5  */
 
+/* ---- prioritized experience replay (Schaul et al. 2016) over one ring -------------------
+ * A sum tree of the ring's mem_size slots: fp32 leaf priorities (0 for a slot never filled), above them fp64 sums of
+ * 1024 consecutive entries per level up to the total, each block summed in one fixed order, and a device scalar
+ * max_priority that starts at 1.  No float atomics: fills, draws and updates are bit-reproducible.  The ring's store
+ * kernels do not know the tree; the caller fills the rows stored since its last call before it draws.
+ *
+ * boatper_fill_new: the leaves of rows first_row .. first_row + n_rows - 1 (slots modulo mem_size) become
+ *   max_priority, then the sums above them are recomputed.  Rows older than the last mem_size are skipped.
+ * boatper_sample: batch stratified draws.  Row j draws u in [0, 1) from Philox (counter (j, counter), key seed, the
+ *   stream 0xE of DESIGN.md "Random streams"), descends the tree to t = ((j + u) / batch) total and writes the leaf to
+ *   idx_out int64[batch] (device) and the importance weight (n P(j))^-beta / max over the batch = (p_min / p_j)^beta
+ *   to weight_out float[batch] (device).  A leaf of priority 0 is never drawn.  Gather the rows with
+ *   boatreplay_gather.  Errors: BOATENV_EINVAL for batch <= 0, NULL outputs, beta < 0 or an empty tree.
+ * boatper_find: the descent of boatper_sample for given targets (inverse CDF): idx_out[j] (int64, device) is the
+ *   slot whose priority prefix range holds targets[j] (double[n], device, in [0, total) where total is the last
+ *   level's entry), with the same clamp: a target on or past an edge by rounding takes the last non-zero entry, so a
+ *   zero-priority slot is never returned.  Errors: BOATENV_EINVAL for n <= 0, NULL pointers or an empty tree.
+ * boatper_update: leaf idx[j] becomes (td[j] + eps)^alpha (float32 td[batch], int64 idx[batch], device); a slot drawn
+ *   twice takes the larger value; max_priority rises to the batch maximum; the sums above are recomputed.  Errors:
+ *   BOATENV_EINVAL for batch <= 0, NULL pointers, alpha < 0, eps <= 0 or an empty tree.  The kernels do not trust the
+ *   inputs: a row with an index outside the ring, a negative or NaN td (td holds absolute TD errors) or a priority that
+ *   is not finite is skipped and flagged, and the next boatper_check returns BOATENV_EINVAL.
+ * boatper_check: waits for `stream`; BOATENV_EINVAL (and clears the flag) if an update skipped a row since the last
+ *   check.
+ * boatper_level_size: the entries of tree level `level` (0: leaves, mem_size of them; the last level holds 1, the
+ *   total); BOATENV_EINVAL past the last level.  boatper_filled: slots given a priority so far.
+ * boatper_read: copies level `level` (0: float leaves, >= 1: double sums, -1: the float max_priority) to device `out`.
+ * boatper_load: checkpoint restore: leaves 0 .. n-1 from device `leaves`, the rest 0, max_priority from a device
+ *   float, the filled count; every sum is recomputed. */
+typedef struct boatper_handle *boatper_t;
+BOATENV_API int boatper_create(int64_t mem_size, int device, boatper_t *out);
+BOATENV_API int boatper_destroy(boatper_t p);
+BOATENV_API int boatper_fill_new(boatper_t p, int64_t first_row, int64_t n_rows, void *stream);
+BOATENV_API int boatper_sample(boatper_t p, int64_t batch, uint64_t seed, uint64_t counter, double beta,
+                               int64_t *idx_out, float *weight_out, void *stream);
+BOATENV_API int boatper_find(boatper_t p, int64_t n, const double *targets, int64_t *idx_out, void *stream);
+BOATENV_API int boatper_update(boatper_t p, int64_t batch, const int64_t *idx, const float *td, double alpha,
+                               double eps, void *stream);
+BOATENV_API int boatper_check(boatper_t p, void *stream);
+BOATENV_API int64_t boatper_level_size(boatper_t p, int32_t level);
+BOATENV_API int64_t boatper_filled(boatper_t p);
+BOATENV_API int boatper_read(boatper_t p, int32_t level, void *out, void *stream);
+BOATENV_API int boatper_load(boatper_t p, const float *leaves, int64_t n, const float *max_priority, int64_t filled,
+                             void *stream);
+
 /* env.step + agent.remember (main.py:81-88) in ONE kernel: steps every env and writes
  * the transition (obs_inout as s, action, reward, new obs as s', done) straight into
  * the ring.  obs_inout T[n_envs][11] holds the current observations on entry and the
@@ -536,6 +581,31 @@ BOATENV_API int64_t boatagent_sac2_update_workspace_bytes(int64_t batch);   /* B
 BOATENV_API int boatagent_sac2_update_members(const boatagent_sac2_member *members_host, int32_t n_members,
                                               int64_t batch, float beta1, float beta2, float adam_eps, void *workspace,
                                               int64_t workspace_bytes, void *stream);
+
+/* The updates of boatagent_sac_update_members / boatagent_sac2_update_members with importance weights (prioritized
+ * replay): row i's critic loss terms are scaled by weights[i], i.e. the critic loss is
+ * 0.5 mean(w (Q1 - target)^2) + 0.5 mean(w (Q2 - target)^2) (target: q_hat for v1, y for v2); the value (v1), actor
+ * and temperature (v2) losses stay unweighted means.  td_out[i] receives 0.5 (|Q1_i - target_i| + |Q2_i - target_i|).
+ * weights, td_out: float32 [batch], device.  With every weight 1 the update equals the unweighted call bit for bit.
+ * Workspace, tables and errors as the unweighted calls, and BOATENV_EINVAL for a NULL weights or td_out. */
+typedef struct boatagent_sac_prioritized_member {
+    boatagent_sac_member base;
+    const float *weights;
+    float *td_out;
+} boatagent_sac_prioritized_member;
+typedef struct boatagent_sac2_prioritized_member {
+    boatagent_sac2_member base;
+    const float *weights;
+    float *td_out;
+} boatagent_sac2_prioritized_member;
+BOATENV_API int boatagent_sac_update_prioritized_members(const boatagent_sac_prioritized_member *members_host,
+                                                         int32_t n_members, int64_t batch, float beta1, float beta2,
+                                                         float adam_eps, void *workspace, int64_t workspace_bytes,
+                                                         void *stream);
+BOATENV_API int boatagent_sac2_update_prioritized_members(const boatagent_sac2_prioritized_member *members_host,
+                                                          int32_t n_members, int64_t batch, float beta1, float beta2,
+                                                          float adam_eps, void *workspace, int64_t workspace_bytes,
+                                                          void *stream);
 
 /* ---- toy integrator envs (environment/toy_car.py, toy_parachute.py) ---------------- */
 

@@ -10,7 +10,7 @@ raises.
 from .config import AttrDict, load_config, params_from_config  # noqa: F401
 from ._lib import BoatEnvError, lib, library_path  # noqa: F401
 from .boat_env import BatchedBoatEnv, BoatEnv, Box, TERM_NAMES  # noqa: F401
-from .buffer import ReplayBuffer  # noqa: F401
+from .buffer import PrioritizedReplayBuffer, ReplayBuffer  # noqa: F401
 from .toy_envs import ToyCar, ToyParachute  # noqa: F401
 from .csv_export import BatchedRecorder, DeviceRecorder  # noqa: F401
 from .sharding import all_reduce_counters, make_sharded_env, shard_range  # noqa: F401
@@ -19,7 +19,7 @@ from . import population  # noqa: F401
 from .population import AgentPopulation  # noqa: F401
 
 __all__ = ["AttrDict", "load_config", "params_from_config", "BoatEnvError", "lib", "library_path",
-           "BatchedBoatEnv", "BoatEnv", "Box", "TERM_NAMES", "ReplayBuffer", "ToyCar", "ToyParachute",
+           "BatchedBoatEnv", "BoatEnv", "Box", "TERM_NAMES", "PrioritizedReplayBuffer", "ReplayBuffer", "ToyCar", "ToyParachute",
            "BatchedRecorder", "DeviceRecorder", "all_reduce_counters", "make_sharded_env", "shard_range",
            "Experiment", "HPTuner", "get_experiment_config", "info_from_counters", "AgentPopulation",
            "ContinuousAgent", "SACLearner", "SAC2Learner", "OverlappedActorLearner"]

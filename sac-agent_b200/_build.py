@@ -34,6 +34,7 @@ UNITS = {
     "record.cu": [],
     "rollout.cu": [],
     "learner.cu": [],
+    "priority.cu": [],
 }
 
 

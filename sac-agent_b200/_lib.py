@@ -50,6 +50,16 @@ class Sac2Member(C.Structure):
     _fields_ = [("base", SacMember), ("target_entropy", C.c_float)]
 
 
+class SacPrioritizedMember(C.Structure):
+    """boatagent_sac_prioritized_member: a SacMember with its rows' importance weights and TD-error output."""
+    _fields_ = [("base", SacMember), ("weights", vp), ("td_out", vp)]
+
+
+class Sac2PrioritizedMember(C.Structure):
+    """boatagent_sac2_prioritized_member: a Sac2Member with its rows' importance weights and TD-error output."""
+    _fields_ = [("base", Sac2Member), ("weights", vp), ("td_out", vp)]
+
+
 class SampleMember(C.Structure):
     """boatreplay_sample_member: one ring's arguments of boatreplay_sample_members."""
     _fields_ = [("ring", vp), ("seed", u64), ("counter", u64)] + [(name, vp) for name in ("s_out", "a_out", "r_out",
@@ -102,6 +112,10 @@ SIGNATURES = {
     "boatagent_sac2_update_workspace_bytes": (i64, [i64]),
     "boatagent_sac2_update_members": (C.c_int, [C.POINTER(Sac2Member), i32, i64, C.c_float, C.c_float, C.c_float, vp,
                                                 i64, vp]),
+    "boatagent_sac_update_prioritized_members": (C.c_int, [C.POINTER(SacPrioritizedMember), i32, i64, C.c_float,
+                                                           C.c_float, C.c_float, vp, i64, vp]),
+    "boatagent_sac2_update_prioritized_members": (C.c_int, [C.POINTER(Sac2PrioritizedMember), i32, i64, C.c_float,
+                                                            C.c_float, C.c_float, vp, i64, vp]),
     "boatreplay_sample_members": (C.c_int, [C.POINTER(SampleMember), i32, i64, vp]),
     "boatreplay_create": (C.c_int, [i64, i32, i32, C.c_int, C.c_int, C.POINTER(vp)]),
     "boatreplay_destroy": (C.c_int, [vp]),
@@ -111,6 +125,17 @@ SIGNATURES = {
     "boatreplay_mem_cntr": (i64, [vp]),
     "boatreplay_set_mem_cntr": (C.c_int, [vp, i64]),
     "boatreplay_mem_size": (i64, [vp]),
+    "boatper_create": (C.c_int, [i64, C.c_int, C.POINTER(vp)]),
+    "boatper_destroy": (C.c_int, [vp]),
+    "boatper_fill_new": (C.c_int, [vp, i64, i64, vp]),
+    "boatper_sample": (C.c_int, [vp, i64, u64, u64, dbl, vp, vp, vp]),
+    "boatper_find": (C.c_int, [vp, i64, vp, vp, vp]),
+    "boatper_update": (C.c_int, [vp, i64, vp, vp, dbl, dbl, vp]),
+    "boatper_check": (C.c_int, [vp, vp]),
+    "boatper_level_size": (i64, [vp, i32]),
+    "boatper_filled": (i64, [vp]),
+    "boatper_read": (C.c_int, [vp, i32, vp, vp]),
+    "boatper_load": (C.c_int, [vp, vp, i64, vp, i64, vp]),
     "boatenv_step_store": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, C.c_int, u32, vp]),
     "boattoy_create": (C.c_int, [C.c_int, i64, C.POINTER(dbl), i32, dbl, u64, C.c_int, C.c_int, C.POINTER(vp)]),
     "boattoy_destroy": (C.c_int, [vp]),

@@ -35,7 +35,7 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-from .buffer import ReplayBuffer
+from .buffer import PrioritizedReplayBuffer, ReplayBuffer
 from .networks import ActorNetwork, CriticNetwork, TemperatureNetwork, ValueNetwork
 
 
@@ -107,7 +107,8 @@ class FusedLearner:
                         launch).
 
     Agents of algorithm "sac2" (all or none) run boatagent_sac2_update_members (three launches) and have no split
-    launches.
+    launches.  A prioritized agent (one member only) runs boatagent_sac[2]_update_prioritized_members: its `_weights`
+    scale the critic loss rows and its `_td` receives the rows' TD errors.
     The learning rates are read from the agents' DeviceAdam slots and gamma, reward scale and tau from their learners at
     every launch, so `ContinuousAgent.set_hyperparameters` reaches the next one.  The other pointers (batch, draws,
     `.grad` tensors, losses) are taken at the first launch and must stay the same tensors after it."""
@@ -136,6 +137,9 @@ class FusedLearner:
         o0 = a0.learner.optimizer
         self._lib, self._L, self.device, self.batch_size = o0._lib, o0._L, a0.device, a0.batch_size
         self.v2 = a0.algorithm == "sac2"   # boatagent_sac2_update_members (the update only)
+        self.per = a0.prioritized          # boatagent_sac[2]_update_prioritized_members (the update only)
+        if any(a.prioritized for a in self.agents) and len(self.agents) > 1:
+            raise ValueError("FusedLearner: a prioritized agent is updated on its own, not as a population member")
         ws_bytes = (self._L.boatagent_sac2_update_workspace_bytes if self.v2 else
                     self._L.boatagent_sac_update_workspace_bytes)(self.batch_size)
         self.ws = torch.empty(len(self.agents) * int(ws_bytes), dtype=torch.uint8, device=self.device)
@@ -143,7 +147,9 @@ class FusedLearner:
 
     def _launch(self, name, *args):
         if self._table is None:   # on the first launch: like the fp32 learner, no .grad before the first update
-            self._table = ((self._lib.Sac2Member if self.v2 else self._lib.SacMember) * len(self.agents))()
+            entry = {(False, False): self._lib.SacMember, (True, False): self._lib.Sac2Member,
+                     (False, True): self._lib.SacPrioritizedMember, (True, True): self._lib.Sac2PrioritizedMember}
+            self._table = (entry[self.v2, self.per] * len(self.agents))()
             for m, a in enumerate(self.agents):
                 o = a.learner.optimizer
                 for k, p in enumerate(o.params):   # the batch gradient goes where the fp32 learner leaves it
@@ -155,20 +161,26 @@ class FusedLearner:
                     s.data_ptr(), act.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), a._eps.data_ptr(),
                     a.learner.actor.max_action.data_ptr(), C.cast(o._slots, C.c_void_p), len(o.params), 0.0, 0.0, 0.0,
                     o.state.data_ptr(), a._loss_buf.data_ptr())
-                self._table[m] = self._lib.Sac2Member(e, 0.0) if self.v2 else e
+                e = self._lib.Sac2Member(e, 0.0) if self.v2 else e
+                if self.per:
+                    e = (self._lib.Sac2PrioritizedMember if self.v2 else self._lib.SacPrioritizedMember)(
+                        e, a._weights.data_ptr(), a._td.data_ptr())
+                self._table[m] = e
         for e, a in zip(self._table, self.agents):
             L = a.learner
-            b = e.base if self.v2 else e
+            e2 = e.base if self.per else e   # the (v1 or v2) member entry
+            b = e2.base if self.v2 else e2
             b.gamma, b.reward_scale, b.tau = float(L.gamma), float(L.scale), float(L.optimizer.tau)
             if self.v2:
-                e.target_entropy = float(L.target_entropy)
+                e2.target_entropy = float(L.target_entropy)
         with torch.cuda.device(self.device):   # the ABI launches on the current device
             stream = torch.cuda.current_stream().cuda_stream
             self._lib.check(getattr(self._L, name)(self._table, len(self.agents), *args, stream), name)
 
     def update(self):
         o = self.agents[0].learner.optimizer
-        self._launch("boatagent_sac2_update_members" if self.v2 else "boatagent_sac_update_members", self.batch_size,
+        name = "boatagent_sac2_update" if self.v2 else "boatagent_sac_update"
+        self._launch(name + ("_prioritized_members" if self.per else "_members"), self.batch_size,
                      o.betas[0], o.betas[1], o.eps, self.ws.data_ptr(), self.ws.numel())
 
     def gradients(self, scale):
@@ -181,8 +193,9 @@ class FusedLearner:
         self._launch("boatagent_adam_polyak_members", o.betas[0], o.betas[1], o.eps)
 
     def _split_v1_only(self):
-        if self.v2:
-            raise ValueError("FusedLearner: the split gradients / Adam launches (data-parallel training) are SAC-v1's")
+        if self.v2 or self.per:
+            raise ValueError("FusedLearner: the split gradients / Adam launches (data-parallel training) are for "
+                             "SAC-v1 with uniform replay")
 
 
 def point_grads_into(agent, row):
@@ -194,6 +207,18 @@ def point_grads_into(agent, row):
         off += p.numel()
     agent._loss_buf = row[off:off + 3]
     agent._losses = tuple(agent._loss_buf[k] for k in range(3))
+
+
+def _critic_loss(q1, q2, target, weights, td_out):
+    """0.5 mse(q1, target) + 0.5 mse(q2, target); with importance weights (prioritized replay) the means are weighted,
+    0.5 mean(w (q1 - target)^2) + 0.5 mean(w (q2 - target)^2), which equals the unweighted loss and its gradients bit
+    for bit when every weight is 1 and the batch size is a power of two.  td_out receives the rows' TD errors."""
+    if td_out is not None:
+        with torch.no_grad():
+            td_out.copy_(0.5 * ((q1 - target).abs() + (q2 - target).abs()))
+    if weights is None:
+        return 0.5 * F.mse_loss(q1, target) + 0.5 * F.mse_loss(q2, target)
+    return 0.5 * torch.mean(weights * (q1 - target) ** 2) + 0.5 * torch.mean(weights * (q2 - target) ** 2)
 
 
 class SACLearner:
@@ -249,12 +274,15 @@ class SACLearner:
         torch._foreach_mul_(tgt, 1.0 - tau)
         torch._foreach_add_(tgt, src, alpha=tau)
 
-    def update(self, state, action, reward, new_state, done, eps_sample=None, eps_rsample=None):
+    def update(self, state, action, reward, new_state, done, eps_sample=None, eps_rsample=None, weights=None,
+               td_out=None):
         """One update on a batch (state [B, obs], action [B, n_actions], reward [B], new_state [B, obs],
         done [B] bool).  eps_*: optional standard-normal draws for the two `sample_normal` calls.
+        weights [B] (prioritized replay): importance weights of the critic loss rows; td_out [B] receives the rows' TD
+        errors 0.5 (|Q1 - q_hat| + |Q2 - q_hat|).
         Returns (value_loss, actor_loss, critic_loss) as 0-d tensors."""
         losses, grads_v, grads_a, grads_c = self._losses_and_grads(state, action, reward, new_state, done, eps_sample,
-                                                                   eps_rsample)
+                                                                   eps_rsample, weights, td_out)
         for p, g in zip(self._value_params + self._actor_params + self._critic_params, grads_v + grads_a + grads_c):
             p.grad = g
         if isinstance(self.optimizer, DeviceAdam):   # Adam for all four networks + update_network_parameters (:154)
@@ -274,7 +302,8 @@ class SACLearner:
         if scale != 1.0:
             torch._foreach_mul_(out, scale)
 
-    def _losses_and_grads(self, state, action, reward, new_state, done, eps_sample, eps_rsample):
+    def _losses_and_grads(self, state, action, reward, new_state, done, eps_sample, eps_rsample, weights=None,
+                          td_out=None):
         """The three losses (detached) and the gradients of the value, actor and critic parameters."""
         with torch.no_grad():
             value_ = self.target_value(new_state).view(-1)
@@ -298,7 +327,7 @@ class SACLearner:
 
         q1_old = self.critic_1(state, action).view(-1)                          # :138-152
         q2_old = self.critic_2(state, action).view(-1)
-        critic_loss = 0.5 * F.mse_loss(q1_old, q_hat) + 0.5 * F.mse_loss(q2_old, q_hat)
+        critic_loss = _critic_loss(q1_old, q2_old, q_hat, weights, td_out)
         grads_c = torch.autograd.grad(critic_loss, self._critic_params)
         return (value_loss.detach(), actor_loss.detach(), critic_loss.detach()), grads_v, grads_a, grads_c
 
@@ -364,10 +393,13 @@ class SAC2Learner:
         torch._foreach_mul_(tgt, 1.0 - tau)
         torch._foreach_add_(tgt, src, alpha=tau)
 
-    def update(self, state, action, reward, new_state, done, eps_sample=None, eps_rsample=None):
+    def update(self, state, action, reward, new_state, done, eps_sample=None, eps_rsample=None, weights=None,
+               td_out=None):
         """One update on a batch (shapes as SACLearner.update; eps_sample draws a' on new_state, eps_rsample the
-        reparameterised action on state).  Returns (temperature_loss, actor_loss, critic_loss) as 0-d tensors."""
-        losses, grads = self._losses_and_grads(state, action, reward, new_state, done, eps_sample, eps_rsample)
+        reparameterised action on state; weights and td_out as SACLearner.update, with y in place of q_hat).
+        Returns (temperature_loss, actor_loss, critic_loss) as 0-d tensors."""
+        losses, grads = self._losses_and_grads(state, action, reward, new_state, done, eps_sample, eps_rsample,
+                                               weights, td_out)
         for p, g in zip(self.optimizer_params(), grads):
             p.grad = g
         if isinstance(self.optimizer, DeviceAdam):   # Adam for the three groups + both Polyak averages, one launch
@@ -388,7 +420,8 @@ class SAC2Learner:
         if scale != 1.0:
             torch._foreach_mul_(out, scale)
 
-    def _losses_and_grads(self, state, action, reward, new_state, done, eps_sample, eps_rsample):
+    def _losses_and_grads(self, state, action, reward, new_state, done, eps_sample, eps_rsample, weights=None,
+                          td_out=None):
         """The three losses (detached) and the gradients of the trained tensors in DeviceAdam's order."""
         alpha = self.alpha()
         with torch.no_grad():
@@ -409,7 +442,7 @@ class SAC2Learner:
 
         q1 = self.critic_1(state, action).view(-1)
         q2 = self.critic_2(state, action).view(-1)
-        critic_loss = 0.5 * F.mse_loss(q1, y) + 0.5 * F.mse_loss(q2, y)
+        critic_loss = _critic_loss(q1, q2, y, weights, td_out)
         grads_c = torch.autograd.grad(critic_loss, self._critic_params)
         losses = (temperature_loss.detach(), actor_loss.detach(), critic_loss.detach())
         return losses, tuple(grads_a) + tuple(grads_c) + tuple(grads_t)
@@ -427,17 +460,42 @@ class ContinuousAgent:
     rank keeps its own env shard, ring, sampler seed and Gaussian draws; every update averages the ranks' gradients and
     losses with one all-reduce and applies the same Adam step everywhere, so the weights stay bit-identical without
     being re-broadcast.  Rank 0's weights and optimiser state are broadcast at construction.  Every rank must hold the
-    same number of envs (`learn()` updates on all ranks or on none without a vote)."""
+    same number of envs (`learn()` updates on all ranks or on none without a vote).
+
+    prioritized: prioritized experience replay (Schaul et al. 2016).  The memory is a PrioritizedReplayBuffer (created
+    here with priority_alpha and priority_eps unless one is passed in, whose own alpha and eps then apply); `learn()`
+    draws its batch by priority, weights the critic loss rows by their importance weights and sets the drawn rows'
+    priorities from their TD errors.  The weights' exponent beta rises linearly from priority_beta to 1 over
+    priority_beta_updates updates (0: it stays priority_beta).  Works with both algorithms and both learner
+    precisions; not with data_parallel, as an AgentPopulation member or under OverlappedActorLearner."""
 
     def __init__(self, config, experiment_dir, input_dims, env, device=None, seed=0, use_cuda_graph=True,
                  memory=None, policy_precision="fp32", learner_precision="fp32", data_parallel=None, algorithm="sac1",
-                 target_entropy=None, init_temperature=1.0, temperature_lr=None):
+                 target_entropy=None, init_temperature=1.0, temperature_lr=None, prioritized=False,
+                 priority_alpha=0.6, priority_beta=0.4, priority_beta_updates=0, priority_eps=1e-6):
         if algorithm not in ("sac1", "sac2"):
             raise ValueError(f"algorithm: sac1 or sac2, got {algorithm!r}")
         if algorithm == "sac1" and (target_entropy is not None or init_temperature != 1.0 or temperature_lr is not None):
             raise ValueError("target_entropy, init_temperature and temperature_lr belong to algorithm='sac2'")
         if algorithm == "sac2" and data_parallel is not None and data_parallel is not False:
             raise ValueError("algorithm='sac2' does not train data-parallel")
+        self.prioritized = bool(prioritized)
+        if not self.prioritized:
+            if (priority_alpha, priority_beta, priority_beta_updates, priority_eps) != (0.6, 0.4, 0, 1e-6):
+                raise ValueError("priority_alpha, priority_beta, priority_beta_updates and priority_eps belong to "
+                                 "prioritized=True")
+            if isinstance(memory, PrioritizedReplayBuffer):
+                raise ValueError("a PrioritizedReplayBuffer memory needs prioritized=True")
+        else:
+            if data_parallel is not None and data_parallel is not False:
+                raise ValueError("prioritized=True does not train data-parallel")
+            if not (priority_alpha >= 0 and priority_eps > 0 and 0 <= priority_beta <= 1 and priority_beta_updates >= 0):
+                raise ValueError("prioritized: priority_alpha >= 0, 0 <= priority_beta <= 1, priority_beta_updates >= 0 "
+                                 f"and priority_eps > 0 (got {priority_alpha}, {priority_beta}, {priority_beta_updates}, "
+                                 f"{priority_eps})")
+            if memory is not None and not isinstance(memory, PrioritizedReplayBuffer):
+                raise ValueError("prioritized=True needs a PrioritizedReplayBuffer memory (or none: it is created)")
+        self._beta = (float(priority_beta), int(priority_beta_updates))
         if not torch.cuda.is_available():
             raise RuntimeError("sac_agent_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.env = env
@@ -447,9 +505,15 @@ class ContinuousAgent:
         self.batch_size = int(a.batch_size)
         self.input_dims = tuple(input_dims)
         self.device = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
-        self.memory = memory if memory is not None else ReplayBuffer(
-            a.max_size, self.input_dims, self.get_n_actions(), precision="fp32", device=self.device.index, seed=seed,
-            as_torch=True)
+        if memory is not None:
+            self.memory = memory
+        elif self.prioritized:
+            self.memory = PrioritizedReplayBuffer(a.max_size, self.input_dims, self.get_n_actions(), precision="fp32",
+                                                  device=self.device.index, seed=seed, as_torch=True,
+                                                  alpha=priority_alpha, eps=priority_eps)
+        else:
+            self.memory = ReplayBuffer(a.max_size, self.input_dims, self.get_n_actions(), precision="fp32",
+                                       device=self.device.index, seed=seed, as_torch=True)
         # algorithm "sac2": SAC2Learner (twin target critics, learned temperature) instead of the reference's SAC-v1
         self.algorithm = algorithm
         learner_args = (self.input_dims, self.get_n_actions(), self.get_max_actions(), a.learning_rate_alpha,
@@ -487,6 +551,10 @@ class ContinuousAgent:
         self._batch = (torch.zeros((B, O), **kw), torch.zeros((B, A), **kw), torch.zeros(B, **kw),
                        torch.zeros((B, O), **kw), torch.zeros(B, dtype=torch.uint8, device=self.device))
         self._eps = torch.zeros((2, B, A), **kw)  # the Gaussian draws of the two sample_normal calls of one update
+        if self.prioritized:   # the drawn slots, their importance weights and the TD errors of one update
+            self._idx = torch.zeros(B, dtype=torch.int64, device=self.device)
+            self._weights = torch.ones(B, **kw)
+            self._td = torch.zeros(B, **kw)
         self._graph = None
         self.capture_stream = None   # stream the update graph is captured on (None: torch's own capture stream)
         self._losses = None
@@ -610,7 +678,8 @@ class ContinuousAgent:
     # -- learning -------------------------------------------------------------------------
     def _update_static(self):
         s, a, r, s2, d = self._batch
-        return self.learner.update(s, a, r, s2, d.bool(), eps_sample=self._eps[0], eps_rsample=self._eps[1])
+        per = dict(weights=self._weights, td_out=self._td) if self.prioritized else {}
+        return self.learner.update(s, a, r, s2, d.bool(), eps_sample=self._eps[0], eps_rsample=self._eps[1], **per)
 
     def _fused_learner(self):
         """This agent's one-member FusedLearner.  Created on first use, so that the members of an AgentPopulation,
@@ -720,9 +789,22 @@ class ContinuousAgent:
         "tcgen05": the two kernels of the fused update)."""
         if self.memory.mem_cntr < self.batch_size:
             return None
+        if self.prioritized:   # draw by priority, update with the importance weights, re-prioritise from the TD errors
+            self.memory.sample_buffer(self.batch_size, self.priority_beta(), out=self._batch, idx_out=self._idx,
+                                      weight_out=self._weights)
+            self._eps.normal_()
+            losses = self._run_update()
+            self.memory.update_priorities(self._idx, self._td)
+            return losses
         self.memory.sample_buffer(self.batch_size, as_torch=True, out=self._batch)
         self._eps.normal_()
         return self._run_update()
+
+    def priority_beta(self):
+        """prioritized: the importance-weight exponent of the next learn(), priority_beta rising linearly to 1 over
+        priority_beta_updates updates."""
+        b0, n = self._beta
+        return b0 if n <= 0 else b0 + (1.0 - b0) * min(1.0, self.updates / n)
 
     def learn_from(self, state, action, reward, new_state, done, eps=None):
         """One update on a caller-supplied batch (device or host arrays of the batch size); `eps`
@@ -733,6 +815,8 @@ class ContinuousAgent:
             self._eps.normal_()
         else:
             self._eps.copy_(torch.as_tensor(eps).reshape(self._eps.shape))
+        if self.prioritized:   # a caller's batch carries no priorities: unit weights, no re-prioritisation
+            self._weights.fill_(1.0)
         return self._run_update()
 
     def _capture(self):
@@ -884,6 +968,8 @@ class OverlappedActorLearner:
     def __init__(self, agent: ContinuousAgent, env, done_flag_mode=1, recorder=None):
         if agent.data_parallel:
             raise ValueError("OverlappedActorLearner: a data-parallel agent is not supported")
+        if agent.prioritized:
+            raise ValueError("OverlappedActorLearner: a prioritized agent is not supported")
         self.agent, self.env, self.done_flag_mode = agent, env, int(done_flag_mode)
         self.recorder = recorder   # a DeviceRecorder: captures every step on the env stream
         dev = agent.device

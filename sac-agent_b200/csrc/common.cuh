@@ -165,6 +165,7 @@ constexpr uint32_t kStreamEpisode = 0x00000000u;  // block 0: s_y_start; block 1
 constexpr uint32_t kStreamAction = 0xA0000000u;   // uniform(-1,1) test / bench policy
 constexpr uint32_t kStreamReplay = 0xB0000000u;   // replay-buffer sample indices
 constexpr uint32_t kStreamToy = 0xC0000000u;      // toy-env parameter jitter
+constexpr uint32_t kStreamPer = 0xE0000000u;      // prioritized replay: stratified draws (priority.cu)
 
 // np.random.sample() stand-in: 23 random bits -> (2k+1) * 2^-24, strictly inside (0,1)
 // and exactly representable in fp32 AND fp64 (both precisions see identical knots).

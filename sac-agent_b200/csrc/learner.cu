@@ -23,6 +23,10 @@
 // sac2_params_kernel (the gradients-only parameter body over its three trained networks, plus the log alpha gradient)
 // and adam_polyak_members_kernel over its 21 slots.
 //
+// Prioritized replay (boatagent_sac[2]_update_prioritized_members) runs the kPer instantiation of either row pass
+// (sac_rows_prioritized_kernel, sac2_rows_prioritized_kernel: importance-weighted critic rows and per-row TD errors)
+// and the same parameter and Adam kernels.
+//
 // Operands in shared memory and in the workspace use the 8x8 core-matrix layout of actor_tc.cuh: element (r, c) of
 // an R-row matrix at (c / 8) * (R * 16) + r * 16 + (c % 8) * 2.  The same bytes are a K-major operand with rows = M/N
 // (LBO = R * 16, SBO = 128) and an MN-major operand with rows = K (LBO = 128, SBO = R * 16): so W2 [out][in] is the B
@@ -131,6 +135,26 @@ struct MemberRow2Args {
     Row2Args m[BOATAGENT_SAC_MAX_MEMBERS];
 };
 static_assert(sizeof(MemberRow2Args) <= 32764, "kernel parameter limit");
+
+// prioritized replay: the row arguments with each row's importance weight and TD-error output
+struct PerRowArgs {
+    RowArgs r;
+    const float *weights;
+    float *td;
+};
+struct MemberPerRowArgs {
+    PerRowArgs m[BOATAGENT_SAC_MAX_MEMBERS];
+};
+struct PerRow2Args {
+    Row2Args r;
+    const float *weights;
+    float *td;
+};
+struct MemberPerRow2Args {
+    PerRow2Args m[BOATAGENT_SAC_MAX_MEMBERS];
+};
+static_assert(sizeof(MemberPerRowArgs) <= 32764, "kernel parameter limit");
+static_assert(sizeof(MemberPerRow2Args) <= 32764, "kernel parameter limit");
 
 __device__ __forceinline__ uint32_t core_off(int r, int c, int rows) { return (uint32_t)((c >> 3) * (rows * 16) + r * 16 + (c & 7) * 2); }
 
@@ -376,8 +400,10 @@ __device__ __forceinline__ void put_small(unsigned char *ws, int tid, const floa
 __device__ __forceinline__ float min_share(float a, float b) { return a < b ? 1.f : (a == b ? 0.5f : 0.f); }
 
 // The row pass of one 128-row tile.  blockIdx.x is the tile and gridDim.x the tile count of ONE update: the members
-// are on blockIdx.y, so both stay per member.
-__device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid) {
+// are on blockIdx.y, so both stay per member.  kPer (prioritized replay): row i's critic output gradient and critic
+// loss partial are scaled by weights[i], and td_out[i] receives its TD error 0.5 (|q1 - q_hat| + |q2 - q_hat|).
+template <bool kPer>
+__device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const float *weights, float *td_out, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
     Rows R;
@@ -400,6 +426,7 @@ __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid
     const float a_batch = __ldg(args.action + row), rew = __ldg(args.reward + row);
     const bool done = __ldg(args.done + row) != 0;
     const float e0 = __ldg(args.eps + row), e1 = __ldg(args.eps + B + row), ma = __ldg(args.max_action);
+    const float w_row = kPer ? __ldg(weights + row) : 1.f;
     float y[2];
     uint32_t m1[8], m2[8];
 
@@ -436,7 +463,7 @@ __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid
         x[kObs] = a_batch;
         R.forward(x, y, m1, m2, ws_net[1 + k]);
         q_sa[k] = y[0];
-        const float dq[2] = {(q_sa[k] - q_hat) * invB, 0.f};
+        const float dq[2] = {kPer ? (q_sa[k] - q_hat) * w_row * invB : (q_sa[k] - q_hat) * invB, 0.f};
         R.backward(dq, m1, m2, ws_net[1 + k]);
         put_small(ws_net[1 + k], tid, x, dq[0], 0.f);
     }
@@ -461,6 +488,11 @@ __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid
 
     float part[4] = {v_err * v_err, lp2 - fminf(q_a2[0], q_a2[1]), (q_sa[0] - q_hat) * (q_sa[0] - q_hat),
                      (q_sa[1] - q_hat) * (q_sa[1] - q_hat)};
+    if constexpr (kPer) {
+        part[2] = w_row * part[2];
+        part[3] = w_row * part[3];
+        td_out[row] = 0.5f * (fabsf(q_sa[0] - q_hat) + fabsf(q_sa[1] - q_hat));
+    }
     cta_sum4(part, reinterpret_cast<float *>(smem + kLRed));
     if (tid < 4) loss_part[tid] = part[tid];
     R.close();
@@ -468,14 +500,22 @@ __device__ __forceinline__ void sac_rows_tile(const RowArgs &args, const int tid
 
 // member blockIdx.y, its tiles on blockIdx.x
 __global__ void __launch_bounds__(kLThreads, 1) sac_rows_kernel(const __grid_constant__ MemberRowArgs args) {
-    sac_rows_tile(args.m[blockIdx.y], threadIdx.x);
+    sac_rows_tile<false>(args.m[blockIdx.y], nullptr, nullptr, threadIdx.x);
+}
+
+__global__ void __launch_bounds__(kLThreads, 1) sac_rows_prioritized_kernel(
+    const __grid_constant__ MemberPerRowArgs args) {
+    const PerRowArgs &a = args.m[blockIdx.y];
+    sac_rows_tile<true>(a.r, a.weights, a.td, threadIdx.x);
 }
 
 // The SAC-v2 row pass of one 128-row tile, with alpha = exp(log_alpha) read before the update:
 //   y = scale r + gamma (1 - done) (min(Qt1, Qt2)(s', a') - alpha lp'),   a', lp' = actor(s', eps[0])
 //   critics: 0.5 mse(Q_k(s, a), y);  actor: mean(alpha lp - min(Q1, Q2)(s, a~)),   a~, lp = actor(s, eps[1])
 // Six stagings, as in v1: actor, the two target critics, the two critics, the actor again for its backward pass.
-__device__ __forceinline__ void sac2_rows_tile(const Row2Args &a2, const int tid) {
+// kPer: importance weights and TD errors as in sac_rows_tile, with y in place of q_hat.
+template <bool kPer>
+__device__ __forceinline__ void sac2_rows_tile(const Row2Args &a2, const float *weights, float *td_out, const int tid) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t tmem_slot;
     const RowArgs &args = a2.r;
@@ -500,6 +540,7 @@ __device__ __forceinline__ void sac2_rows_tile(const Row2Args &a2, const int tid
     const bool done = __ldg(args.done + row) != 0;
     const float e0 = __ldg(args.eps + row), e1 = __ldg(args.eps + B + row), ma = __ldg(args.max_action);
     const float alpha = expf(__ldg(a2.log_alpha));
+    const float w_row = kPer ? __ldg(weights + row) : 1.f;
     float y[2];
     uint32_t m1[8], m2[8];
 
@@ -543,7 +584,7 @@ __device__ __forceinline__ void sac2_rows_tile(const Row2Args &a2, const int tid
         x[kObs] = a_batch;
         R.forward(x, y, m1, m2, ws_net[1 + k]);
         q_sa[k] = y[0];
-        const float dq[2] = {(q_sa[k] - q_hat) * invB, 0.f};
+        const float dq[2] = {kPer ? (q_sa[k] - q_hat) * w_row * invB : (q_sa[k] - q_hat) * invB, 0.f};
         R.backward(dq, m1, m2, ws_net[1 + k]);
         put_small(ws_net[1 + k], tid, x, dq[0], 0.f);
     }
@@ -559,13 +600,24 @@ __device__ __forceinline__ void sac2_rows_tile(const Row2Args &a2, const int tid
 
     float part[4] = {lp + a2.target_entropy, alpha * lp - fminf(q_pi[0], q_pi[1]),
                      (q_sa[0] - q_hat) * (q_sa[0] - q_hat), (q_sa[1] - q_hat) * (q_sa[1] - q_hat)};
+    if constexpr (kPer) {
+        part[2] = w_row * part[2];
+        part[3] = w_row * part[3];
+        td_out[row] = 0.5f * (fabsf(q_sa[0] - q_hat) + fabsf(q_sa[1] - q_hat));
+    }
     cta_sum4(part, reinterpret_cast<float *>(smem + kLRed));
     if (tid < 4) loss_part[tid] = part[tid];
     R.close();
 }
 
 __global__ void __launch_bounds__(kLThreads, 1) sac2_rows_kernel(const __grid_constant__ MemberRow2Args args) {
-    sac2_rows_tile(args.m[blockIdx.y], threadIdx.x);
+    sac2_rows_tile<false>(args.m[blockIdx.y], nullptr, nullptr, threadIdx.x);
+}
+
+__global__ void __launch_bounds__(kLThreads, 1) sac2_rows_prioritized_kernel(
+    const __grid_constant__ MemberPerRow2Args args) {
+    const PerRow2Args &a = args.m[blockIdx.y];
+    sac2_rows_tile<true>(a.r, a.weights, a.td, threadIdx.x);
 }
 
 // slot of tensor `t` (0 w1, 1 b1, 2 w2, 3 b2, 4 / 6 head weights, 5 / 7 head biases) of trained network `n`
@@ -813,20 +865,37 @@ MemberRow2Args &member_rows2() {
     static thread_local MemberRow2Args ra;
     return ra;
 }
+template <class RowTable>
+RowTable &member_rows_of() {   // the prioritized tables
+    static thread_local RowTable ra;
+    return ra;
+}
 
 const boatagent_sac_member &base_of(const boatagent_sac_member &e) { return e; }
 const boatagent_sac_member &base_of(const boatagent_sac2_member &e) { return e.base; }
+const boatagent_sac_member &base_of(const boatagent_sac_prioritized_member &e) { return e.base; }
+const boatagent_sac_member &base_of(const boatagent_sac2_prioritized_member &e) { return e.base.base; }
+float entropy_of(const boatagent_sac2_member &e) { return e.target_entropy; }
+float entropy_of(const boatagent_sac2_prioritized_member &e) { return e.base.target_entropy; }
 RowArgs &rows_of(RowArgs &r) { return r; }
 RowArgs &rows_of(Row2Args &r) { return r.r; }
+RowArgs &rows_of(PerRowArgs &r) { return r.r; }
+RowArgs &rows_of(PerRow2Args &r) { return r.r.r; }
+Row2Args &row2_of(Row2Args &r) { return r; }
+Row2Args &row2_of(PerRow2Args &r) { return r.r; }
 
 // The member tables of the kernels of SAC-v1 (Entry boatagent_sac_member, rows MemberRowArgs) or SAC-v2
-// (boatagent_sac2_member, MemberRow2Args): every member checked as documented in boatenv.h (its adam_state only with
-// `adam`) before anything is launched.
+// (boatagent_sac2_member, MemberRow2Args), or of their prioritized updates (boatagent_sac[2]_prioritized_member,
+// MemberPerRow[2]Args): every member checked as documented in boatenv.h (its adam_state only with `adam`) before
+// anything is launched.
 template <class Entry, class RowTable>
 int member_tables(const Entry *members_host, int32_t n_members, int64_t batch, void *workspace,
                   int64_t workspace_bytes, bool adam, float beta1, float beta2, float adam_eps, float grad_scale,
                   RowTable &ra, MemberParamArgs &pa) {
-    constexpr bool v2 = std::is_same<Entry, boatagent_sac2_member>::value;
+    constexpr bool v2 = std::is_same<Entry, boatagent_sac2_member>::value ||
+                        std::is_same<Entry, boatagent_sac2_prioritized_member>::value;
+    constexpr bool per = std::is_same<Entry, boatagent_sac_prioritized_member>::value ||
+                         std::is_same<Entry, boatagent_sac2_prioritized_member>::value;
     if (!members_host || n_members < 1 || n_members > BOATAGENT_SAC_MAX_MEMBERS || !workspace) return BOATENV_EINVAL;
     if (batch <= 0 || batch % kRows != 0) return BOATENV_EINVAL;
     // a multiple of 16: every slice stays 16-byte aligned
@@ -842,6 +911,11 @@ int member_tables(const Entry *members_host, int32_t n_members, int64_t batch, v
             return BOATENV_EINVAL;
         const int rc = check_slots(b.slots, v2);
         if (rc != 0) return rc;
+        if constexpr (per) {
+            if (!members_host[m].weights || !members_host[m].td_out) return BOATENV_EINVAL;
+            ra.m[m].weights = members_host[m].weights;
+            ra.m[m].td = members_host[m].td_out;
+        }
         unsigned char *ws = static_cast<unsigned char *>(workspace) + slice * (size_t)m;
 
         RowArgs &r = rows_of(ra.m[m]);
@@ -873,8 +947,8 @@ int member_tables(const Entry *members_host, int32_t n_members, int64_t batch, v
         if constexpr (v2) {
             r.net[3] = net(8, kObs + 1, false, true);
             r.net[4] = net(14, kObs + 1, false, true);
-            ra.m[m].log_alpha = b.slots[kSlots2 - 1].param;
-            ra.m[m].target_entropy = members_host[m].target_entropy;
+            row2_of(ra.m[m]).log_alpha = b.slots[kSlots2 - 1].param;
+            row2_of(ra.m[m]).target_entropy = entropy_of(members_host[m]);
         } else {
             r.net[3] = net(20, kObs, false, false);
             r.net[4] = net(20, kObs, false, true);
@@ -909,17 +983,29 @@ int set_smem_attributes() {
         CUDA_TRY(cudaFuncSetAttribute(sac_params_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac2_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
         CUDA_TRY(cudaFuncSetAttribute(sac2_params_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac_rows_prioritized_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
+        CUDA_TRY(cudaFuncSetAttribute(sac2_rows_prioritized_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLSmem));
         set_of[dev] = true;
     }
     return 0;
 }
 
-int launch(bool adam, int32_t n_members, int64_t batch, const MemberRowArgs &ra, const MemberParamArgs &pa,
-           void *stream) {
+// the row pass of a member table
+void launch_rows(const MemberRowArgs &ra, dim3 grid, cudaStream_t s) { sac_rows_kernel<<<grid, kLThreads, kLSmem, s>>>(ra); }
+void launch_rows(const MemberPerRowArgs &ra, dim3 grid, cudaStream_t s) {
+    sac_rows_prioritized_kernel<<<grid, kLThreads, kLSmem, s>>>(ra);
+}
+void launch_rows(const MemberRow2Args &ra, dim3 grid, cudaStream_t s) { sac2_rows_kernel<<<grid, kLThreads, kLSmem, s>>>(ra); }
+void launch_rows(const MemberPerRow2Args &ra, dim3 grid, cudaStream_t s) {
+    sac2_rows_prioritized_kernel<<<grid, kLThreads, kLSmem, s>>>(ra);
+}
+
+template <class RowTable>
+int launch(bool adam, int32_t n_members, int64_t batch, const RowTable &ra, const MemberParamArgs &pa, void *stream) {
     const int rc = set_smem_attributes();
     if (rc != 0) return rc;
     const cudaStream_t s = (cudaStream_t)stream;
-    sac_rows_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem, s>>>(ra);
+    launch_rows(ra, dim3((unsigned)(batch / kRows), (unsigned)n_members), s);
     boatenv::count_launch();
     CUDA_TRY(cudaGetLastError());
     const dim3 grid(kParamBlocks, (unsigned)n_members);
@@ -933,11 +1019,12 @@ int launch(bool adam, int32_t n_members, int64_t batch, const MemberRowArgs &ra,
 
 // SAC-v2: the row pass, the gradients, then one coalesced Adam + Polyak launch over the 21 slots (the
 // adam_polyak_members_kernel of v1's split update, on the v2 chunk count; slots 21.. of the table are empty).
-int launch2(int32_t n_members, int64_t batch, const MemberRow2Args &ra, const MemberParamArgs &pa, void *stream) {
+template <class RowTable>
+int launch2(int32_t n_members, int64_t batch, const RowTable &ra, const MemberParamArgs &pa, void *stream) {
     const int rc = set_smem_attributes();
     if (rc != 0) return rc;
     const cudaStream_t s = (cudaStream_t)stream;
-    sac2_rows_kernel<<<dim3((unsigned)(batch / kRows), (unsigned)n_members), kLThreads, kLSmem, s>>>(ra);
+    launch_rows(ra, dim3((unsigned)(batch / kRows), (unsigned)n_members), s);
     boatenv::count_launch();
     CUDA_TRY(cudaGetLastError());
     sac2_params_kernel<<<dim3(kParamBlocks2, (unsigned)n_members), kPThreads, kPSmem, s>>>(pa);
@@ -954,6 +1041,30 @@ extern "C" int boatagent_sac2_update_members(const boatagent_sac2_member *member
                                              int64_t batch, float beta1, float beta2, float adam_eps, void *workspace,
                                              int64_t workspace_bytes, void *stream) {
     MemberRow2Args &ra = member_rows2();
+    MemberParamArgs &pa = member_params();
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, beta1, beta2,
+                                 adam_eps, 1.0f, ra, pa);
+    if (rc != 0) return rc;
+    return launch2(n_members, batch, ra, pa, stream);
+}
+
+extern "C" int boatagent_sac_update_prioritized_members(const boatagent_sac_prioritized_member *members_host,
+                                                        int32_t n_members, int64_t batch, float beta1, float beta2,
+                                                        float adam_eps, void *workspace, int64_t workspace_bytes,
+                                                        void *stream) {
+    MemberPerRowArgs &ra = member_rows_of<MemberPerRowArgs>();
+    MemberParamArgs &pa = member_params();
+    const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, beta1, beta2,
+                                 adam_eps, 1.0f, ra, pa);
+    if (rc != 0) return rc;
+    return launch(true, n_members, batch, ra, pa, stream);
+}
+
+extern "C" int boatagent_sac2_update_prioritized_members(const boatagent_sac2_prioritized_member *members_host,
+                                                         int32_t n_members, int64_t batch, float beta1, float beta2,
+                                                         float adam_eps, void *workspace, int64_t workspace_bytes,
+                                                         void *stream) {
+    MemberPerRow2Args &ra = member_rows_of<MemberPerRow2Args>();
     MemberParamArgs &pa = member_params();
     const int rc = member_tables(members_host, n_members, batch, workspace, workspace_bytes, true, beta1, beta2,
                                  adam_eps, 1.0f, ra, pa);
